@@ -276,7 +276,7 @@ class Dist:
         return int(t.item())
 
 
-def measure(args, D, engine, name, steps, warmup, e2e_steps, with_cpu, peaks, fp64_peak):
+def measure(args, D, engine, name, steps, warmup, e2e_steps, with_cpu, peaks, fp64_peak, dump=False):
     """One workload at D.world GPUs: device-timed value, end-to-end value through optb_trace_host, rooflines, CPU
     baseline. Returns the dict that becomes the JSON line (headline) or an entry of "workloads"."""
     import torch
@@ -337,6 +337,7 @@ def measure(args, D, engine, name, steps, warmup, e2e_steps, with_cpu, peaks, fp
     total_ms = D.max_f(ev[0].elapsed_time(ev[-1]))
     trace_ms = float(np.mean([a.elapsed_time(b) for a, b in kern]))
     clocks = sampler.stop()
+    dumped = dump_outputs(args.dump_outputs, dt, n, D.world) if args.dump_outputs and dump and D.rank == 0 else None
     inter_all = D.sum_i(inter)
     ms_per_step = total_ms / steps
     value = inter_all / (ms_per_step * 1e-3)
@@ -366,6 +367,8 @@ def measure(args, D, engine, name, steps, warmup, e2e_steps, with_cpu, peaks, fp
                             "inputs+outputs per step (%.3f GB) fit the L2: a 256 MB buffer is written between timed steps (inside ms_per_step)" % (step_bytes / 1e9),
                       "parallelism": f"rays sharded over {D.world} GPU(s), scene tables replicated, histograms all-reduced"},
            "clocks": clocks, "gpu_launches": launches * steps, "e2e": e2e}
+    if dumped:
+        out["outputs_dump"] = dumped
     if e2e_hist:
         out["e2e_histograms_only"] = e2e_hist
     if D.rank == 0:
@@ -398,6 +401,56 @@ def measure(args, D, engine, name, steps, warmup, e2e_steps, with_cpu, peaks, fp
     del dt
     torch.cuda.empty_cache()
     return out
+
+
+DUMP_SEED = 0
+DUMP_MAX_BYTES = 48 << 20  # monitor rows of the output sample; histograms and counts come on top (< 1 MB)
+
+
+def dump_outputs(out_dir, dt, n_rays, world_size):
+    """Write what the last timed step left in the device result buffers as DIR/<name>.npy (float64):
+    the monitor histograms, the result counts (pops, interactions, monitor rows) and the monitor rows of a fixed,
+    seeded sample of the initial rays, in (root, monitor, pop) order. Rows are appended in device order, so they are
+    selected by their root ray and sorted by their packed key: two builds that compute the same rows write the same
+    files. The sample has as many rays as keep the rows under DUMP_MAX_BYTES; if the chosen rays still yield more
+    rows, the first rows in key order are kept. Only rank 0 writes: with --gpus > 1 the histograms are the
+    all-reduced ones of every GPU, but the rows and counts are rank 0's shard (its own rays), and "world_size" in the
+    line's "outputs_dump" says how many GPUs shared the batch."""
+    import torch
+
+    from optable_b200 import _abi as A
+
+    os.makedirs(out_dir, exist_ok=True)
+    cnt = dt.counters()
+    rows = int(cnt[A.C_HITS])
+    cols = ("hit_px", "hit_py", "hit_pz", "hit_intensity", "hit_t")
+    row_bytes = 8 * (len(cols) + 3)  # + root, monitor and pop
+    max_rows = DUMP_MAX_BYTES // row_bytes
+    per_ray = rows / max(n_rays, 1)
+    k = n_rays if per_ray * n_rays <= max_rows else max(1, int(max_rows / per_ray))
+    roots = np.sort(np.random.default_rng(DUMP_SEED).choice(n_rays, size=k, replace=False)) if k < n_rays else None
+    if "hit_key" in dt.t:
+        key = dt.t["hit_key"][:rows]
+    else:  # --e2e-columns all: the key is three columns
+        u32 = lambda c: dt.t[c][:rows].to(torch.int64) & 0xffffffff  # noqa: E731
+        key = (u32("hit_root") << 32) | (u32("hit_monitor") << 24) | u32("hit_pop")
+    if roots is not None:
+        chosen = torch.zeros(n_rays, dtype=torch.bool, device=key.device)
+        chosen[torch.from_numpy(roots).to(key.device)] = True
+        sel = torch.nonzero(chosen[key >> 32]).flatten()
+    else:
+        sel = torch.arange(rows, device=key.device)
+    order = sel[torch.argsort(key[sel])][:max_rows]
+    key = key[order]
+    arrays = {"hit_root": key >> 32, "hit_monitor": (key >> 24) & 0xff, "hit_pop": key & 0xffffff}
+    arrays.update({c: dt.t[c][:rows][order] for c in cols})
+    arrays["hist_y"], arrays["hist_yz"] = dt.t["hist_y"], dt.t["hist_yz"]
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), cnt[[A.C_SEGMENTS, A.C_INTERACTIONS, A.C_HITS]].astype(np.float64))
+    return {"dir": out_dir, "rows": int(order.numel()), "rows_per_step": rows,
+            "sampled_rays": n_rays if roots is None else k, "seed": DUMP_SEED, "world_size": world_size,
+            "rows_from": "rank 0 (its own rays)" if world_size > 1 else "the whole batch"}
 
 
 def bundle_bytes(bundle):
@@ -533,7 +586,8 @@ def run_cuda(args):
     fp64 = engine.fp64_peak_tflops()
     c = s.stop()
     fp64_peak = {"tflops": fp64, "sm_mhz": c.get("sm_mhz"), "reasons": c.get("reasons")}
-    head = measure(args, D, engine, args.workload, args.steps, args.warmup, args.e2e_steps, True, peaks, fp64_peak)
+    head = measure(args, D, engine, args.workload, args.steps, args.warmup, min(args.e2e_steps, args.steps), True, peaks, fp64_peak,
+                   dump=True)
     extra = {}
     if not args.only:
         for name in workloads():
@@ -583,7 +637,7 @@ def flagged_fraction(engine, workload, n):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20, help="timed steps of the headline workload (also caps --e2e-steps)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--rays", type=int, default=0, help="rays per GPU per step (0 = the workload's default)")
@@ -600,7 +654,11 @@ def main():
                     help="largest per-GPU row set the end-to-end leg copies to pinned host memory; above it e2e returns histograms")
     ap.add_argument("--flag-rays", type=int, default=1_000_000, help="rays of the ambiguity-flag pass (0 = skip)")
     ap.add_argument("--chain-len", type=int, default=0, help="max in-register pops per launch (0 = unlimited); scheduling only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline workload's results of the last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "cuda":
         args.warmup = 3
     if args.impl == "reference":

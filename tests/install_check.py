@@ -63,3 +63,60 @@ def check_install(name, engine, q_rtol=1e-9):
     for cw, cg in zip(leaves_w, leaves_g):
         assert sorted(cw._interact_count.values()) == sorted(cg._interact_count.values()) or cw.max_interact_count is None
     return len(tb.rays), sum(len(m._data_raw) for m in tb.monitors)
+
+
+def golden_fields(want, k):
+    """`fields` of segment k of a stored reference result (tests/golden/<name>.npz, (root, pop) order)."""
+    import math
+
+    return (want["seg_o"][k], want["seg_d"][k], None if math.isinf(want["seg_length"][k]) else float(want["seg_length"][k]),
+            bool(want["seg_alive"][k]), float(want["seg_intensity"][k]), float(want["seg_wavelength"][k]),
+            complex(want["seg_q"][k]) if want["seg_hasq"][k] else None, float(want["seg_pathlength"][k]),
+            float(want["seg_n"][k]))
+
+
+def check_monitor_rows_against_golden(monitors, want, segments):
+    """Every monitor's `_data_raw` rows against the stored reference rows, in order; each row must point at one of
+    `segments` (the objects of the traced table)."""
+    on_table = {id(s) for s in segments}
+    for mi, mon in enumerate(monitors):
+        sel = want["hit_monitor"] == mi
+        assert mon.ndata == len(mon._data_raw) == int(sel.sum())
+        for Pw, Iw, tw, (Pg, Ig, tg, rg) in zip(want["hit_P"][sel], want["hit_intensity"][sel], want["hit_t"][sel], mon._data_raw):
+            assert np.linalg.norm(Pw - np.asarray(Pg)) <= 1e-9 * max(np.linalg.norm(Pw), 1.0)
+            assert Iw == pytest.approx(Ig, rel=1e-9) and tw == pytest.approx(tg, rel=1e-9)
+            assert id(rg) in on_table
+
+
+def check_against_golden(name, q_rtol=1e-9):
+    """`check_install` where the reference package is not installed: this package's own classes traced by its
+    `OpticalTable.ray_tracing` (the CUDA engine) against the reference's results for the same scene as
+    oracle/make_golden.py stored them (tests/golden/<name>.npz): `table.rays` segment by segment, the `_id` family
+    partition, every monitor's `_data_raw` rows (pointing at the objects of `table.rays`) and `_interact_count`."""
+    import optable_b200 as ob
+    from optable_b200.flatten import pack_rays
+    from tests import golden_io
+
+    want = golden_io.load(name)[3]
+    sc = scenes.REGISTRY[name](ob)
+    table = ob.OpticalTable()
+    table.add_components(sc.components)
+    table.add_monitors(sc.monitors)
+    got = table.ray_tracing(sc.rays, perfomance_limit=sc.limit)
+    assert len(got) == len(table.rays) == len(want["seg_root"])
+    for k, rg in enumerate(table.rays):
+        assert_same_segment(golden_fields(want, k), fields(rg), q_rtol)
+    # families: every segment descends from the initial ray of its root and keeps that ray's `_id`
+    fam_w, fam_g = {}, {}
+    for k, rg in enumerate(table.rays):
+        fam_w.setdefault(sc.rays[int(want["seg_root"][k])]._id, []).append(k)
+        fam_g.setdefault(rg._id, []).append(k)
+    assert sorted(fam_w.values()) == sorted(fam_g.values())
+    check_monitor_rows_against_golden(table.monitors, want, table.rays)
+    flat = sc.flat()   # (the same component objects the table traced: cap slots point at their `_interact_count`)
+    if flat.n_capslots:
+        _, fam_ids, _ = pack_rays(sc.rays)
+        for s, comp in enumerate(flat.capslots):
+            for f, rid in enumerate(fam_ids):
+                assert comp._interact_count.get(rid, 0) == int(want["cap_counts"][s, f])
+    return len(table.rays), sum(len(m._data_raw) for m in table.monitors)

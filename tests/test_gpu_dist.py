@@ -26,7 +26,7 @@ def test_sharded_trace_over_nccl_equals_single_gpu():
 
     n = torch.cuda.device_count()
     if n < 2:
-        pytest.skip("needs >= 2 GPUs (run with gpurun --gpus 2)")
+        pytest.skip("needs >= 2 GPUs (one rank per GPU under torch.distributed.run)")
     world = 2 if n < 4 else (4 if n < 8 else 8)
     run = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
                           "--master-addr", "127.0.0.1", "--master-port", str(_free_port()),

@@ -123,7 +123,7 @@ def test_random_constructions_match_reference_classes(block):
     from oracle import ref_harness as RH
 
     if not RH.reference_available():
-        pytest.skip("/root/reference not present")
+        pytest.skip("the unmodified optable reference package is not installed (baseline/_ref, or OPTABLE_REFERENCE_ROOT)")
     ref = RH.load_reference()
     for seed in range(7000 + 50 * block, 7050 + 50 * block):
         caps, extended = bool(seed % 2), bool(seed % 4 < 2)   # extended: the whole zoo incl. MMA, roof mirrors, prisms

@@ -4,7 +4,7 @@ import pytest
 
 from oracle import ref_harness as RH
 
-pytestmark = pytest.mark.skipif(not RH.reference_available(), reason="/root/reference not present")
+pytestmark = pytest.mark.skipif(not RH.reference_available(), reason="the unmodified optable reference package is not installed (baseline/_ref, or OPTABLE_REFERENCE_ROOT)")
 
 
 def test_solver_helpers_equal_reference():
