@@ -346,6 +346,26 @@ const char* optb_last_error(const optb_ctx* ctx);
 int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* desc, optb_scene** out);
 int optb_scene_destroy(optb_ctx* ctx, optb_scene* scene);
 
+/* Sweep scene: K = n_configs configurations of one scene with the same topology (descs[0..K-1], host pointers), e.g.
+ * one table built over a parameter grid (the GUI's scan, optimize: optable/interact.py:465-630) or the draws of a
+ * tolerance study. The handle is an ordinary optb_scene; every optb_trace / optb_trace_host on it traces the bundle
+ * of rays.n = N rays through all K configurations in one call:
+ *   - K * N roots: root k * N + r is ray r in configuration k (seg_root, hit_root and hit_key carry that number, so
+ *     optb_sort_rows gives configuration-major order); K * N must stay below 2^32 (-7 otherwise);
+ *   - hist_y / hist_yz are [K][n_monitors][...]; root_flags would be [K * N]; counters are totals over all configurations;
+ *   - rays.family must be NULL (every root is its own family); a scene with interact caps needs params.caps_slack
+ *     (sweeps have no family-serial path; -7 otherwise); flag_ambiguity and reference_roots are rejected (-7);
+ *   - optb_workspace_bytes(scene, N, max_live) sizes for K * N roots (max_live counts over all configurations);
+ *   - optb_scene_update_nodes is rejected (-7): upload the configurations again.
+ * Every desc must have the same n_nodes, n_leaves, n_materials, n_monitors, n_capslots and n_aux, identical node_i rows
+ * except column OPTB_NI_ORTHO (a leaf index, skip pointer, material and cap slot mean the same in every configuration)
+ * and identical mat_kind; node_f, mat_f, mon_f and aux may differ (poses, boxes, apertures, lattice descriptors,
+ * reflectivity, glass coefficients, monitor placement). Violations fail with -5 and name the configuration.
+ * Added without a change of OPTB_ABI_VERSION: that number stamps the layout and meaning of the structs above, which every
+ * consumer of a scene description (this library, the C restatement in oracle/) checks, and none of them changed; a host
+ * written for this entry point against an older library fails to link instead.                                     */
+int optb_scene_upload_sweep(optb_ctx* ctx, const optb_scene_desc* descs, int32_t n_configs, optb_scene** out);
+
 /* Rewrite the rows of the listed nodes of an uploaded scene from `desc` (the tables the scene was uploaded from, with
  * those rows changed in place: same node count, kinds, skip pointers, materials and aux pool). What a GUI loop needs
  * when one component moved (optable/interact.py:455-457 re-runs the user's script per slider event): a few hundred
@@ -355,7 +375,8 @@ int optb_scene_update_nodes(optb_ctx* ctx, optb_scene* scene, const optb_scene_d
                             const int32_t* nodes, int32_t n_nodes, void* stream);
 
 /* Bytes of device workspace optb_trace needs for `n_rays` roots when at most
- * `max_live` rays are alive at once (max_live >= n_rays).                             */
+ * `max_live` rays are alive at once (max_live >= n_rays). Sweep scene: n_rays rays per configuration, sized for
+ * n_configs * n_rays roots.                                                            */
 int64_t optb_workspace_bytes(const optb_scene* scene, int64_t n_rays, int64_t max_live);
 
 /* The bounce loop: replaces OpticalTable.ray_tracing/_single_ray_tracing for a whole batch of
@@ -422,7 +443,8 @@ int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_t first, in
  *   optb_comm_init        all ranks: joins the communicator (collective call)
  *   optb_monitor_merge    all ranks: in-place sum over ranks of hist_y [n_monitors][30], hist_yz [n_monitors][30][30]
  *                         and counters [OPTB_C_COUNT] (device pointers; any may be NULL; the status word is OR-ed,
- *                         OPTB_C_GENERATIONS takes the maximum), enqueued on `stream`
+ *                         OPTB_C_GENERATIONS takes the maximum), enqueued on `stream`. The histograms of a sweep
+ *                         scene are contiguous [K][n_monitors][...]: pass n_monitors = K * n_monitors
  *   optb_comm_destroy     leaves the communicator                                                                  */
 int optb_comm_unique_id(optb_ctx* ctx, void* id128);
 int optb_comm_init(optb_ctx* ctx, const void* id128, int rank, int nranks);

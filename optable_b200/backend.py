@@ -35,6 +35,7 @@ def lib():
         L.optb_last_error.restype = C.c_char_p
         L.optb_last_error.argtypes = [C.c_void_p]
         L.optb_scene_upload.argtypes = [C.c_void_p, C.POINTER(A.SceneDesc), C.POINTER(C.c_void_p)]
+        L.optb_scene_upload_sweep.argtypes = [C.c_void_p, C.POINTER(A.SceneDesc), C.c_int32, C.POINTER(C.c_void_p)]
         L.optb_scene_destroy.argtypes = [C.c_void_p, C.c_void_p]
         L.optb_workspace_bytes.restype = C.c_int64
         L.optb_workspace_bytes.argtypes = [C.c_void_p, C.c_int64, C.c_int64]
@@ -77,13 +78,23 @@ def _result_fields(torch):
 
 
 class Scene:
-    """Device-resident scene tables (optb_scene handle)."""
+    """Device-resident scene tables (optb_scene handle). With `configs` (a list of FlatScene of one topology) it is a
+    sweep scene (optb_scene_upload_sweep): `flat` is then configs[0], and every trace runs its bundle through all
+    `n_configs` configurations."""
 
-    def __init__(self, engine, flat: FlatScene):
+    def __init__(self, engine, flat: FlatScene, configs=None):
         self.engine, self.flat = engine, flat
+        self.configs = list(configs) if configs is not None else [flat]
+        self.n_configs = len(self.configs)
+        self.sweep = configs is not None
+        self.max_children = max(f.max_children for f in self.configs)
         h = C.c_void_p()
-        desc = flat.desc()
-        engine._check(lib().optb_scene_upload(engine._ctx, C.byref(desc), C.byref(h)))
+        if self.sweep:
+            descs = (A.SceneDesc * self.n_configs)(*[f.desc() for f in self.configs])   # (the arrays stay alive in configs)
+            engine._check(lib().optb_scene_upload_sweep(engine._ctx, descs, self.n_configs, C.byref(h)))
+        else:
+            desc = flat.desc()
+            engine._check(lib().optb_scene_upload(engine._ctx, C.byref(desc), C.byref(h)))
         self._h = h
 
     def update_nodes(self, nodes, stream=None):
@@ -136,6 +147,10 @@ class Engine:
 
     def upload(self, flat: FlatScene) -> Scene:
         return Scene(self, flat)
+
+    def upload_sweep(self, flats) -> Scene:
+        """One sweep scene from the FlatScenes of K configurations with the same topology (optb_scene_upload_sweep)."""
+        return Scene(self, flats[0], configs=flats)
 
     def fp64_peak_tflops(self) -> float:
         v = C.c_double(0)
@@ -192,7 +207,7 @@ class Engine:
         torch = self.torch
         dev = f"cuda:{self.device}"
         dt = _result_fields(torch)
-        nm = max(scene.flat.n_monitors, 1)
+        nm = max(scene.flat.n_monitors, 1) * scene.n_configs   # a sweep: [n_configs][n_monitors] histograms
         spec = [(k, dt[k], (int(seg_capacity),)) for k in A.SEG_F64 + A.SEG_U32 + A.SEG_I32]
         # `hit_columns`: the monitor-row columns the caller wants (default: all but the packed key); the others stay
         # NULL in the result struct: neither allocated nor written
@@ -248,14 +263,14 @@ class Engine:
         split rays; returns after the last generation otherwise."""
         torch = self.torch
         rs = self._rays_struct(rays_t)
-        n = int(rs.n)
+        n = int(rs.n) * scene.n_configs   # roots
         has_pass = bool((scene.flat.node_i[:, A.NI_INTER] == A.I_PASS).any())   # runs the general (wavefront) variants
-        splitting = (scene.flat.max_children > 1 or params.chain_len > 0 or scene.flat.n_capslots > 0 or params.flag_ambiguity
+        splitting = (scene.max_children > 1 or params.chain_len > 0 or scene.flat.n_capslots > 0 or params.flag_ambiguity
                      or params.reference_roots or has_pass)
         live = 0 if not splitting else int(max_live if max_live is not None else max(4 * n, 1024))
         if scene.flat.n_capslots and not params.caps_slack:  # family-serial mode: total FIFO entries over all families
             live = max(live, min(64 * max(n, 16), n * (int(params.max_trace_num) + 2)))
-        nbytes = lib().optb_workspace_bytes(scene._h, n, live)
+        nbytes = lib().optb_workspace_bytes(scene._h, int(rs.n), live)
         ws = self._ws(nbytes)
         st = torch.cuda.current_stream(self.device).cuda_stream if stream is None else stream
         self._check(lib().optb_trace(self._ctx, scene._h, C.byref(rs), C.byref(params), C.byref(result),

@@ -109,15 +109,17 @@ HIT_COLUMNS_ALL = A.HIT_I32 + A.HIT_U32 + A.HIT_F64
 
 class DeviceTrace:
     """Reusable device-side state for repeated traces of same-shaped bundles through one scene: scene tables,
-    result buffers and workspace are allocated once; `run` only enqueues kernels."""
+    result buffers and workspace are allocated once; `run` only enqueues kernels. With `configs` (the FlatScenes of a
+    sweep, `flat` = configs[0]) the scene is a sweep scene and one run traces the bundle through every configuration."""
 
     def __init__(self, engine, flat, n_rays, hit_capacity, seg_capacity=0, hit_columns=HIT_COLUMNS_ALL,
-                 max_trace_num=2000, unit=1e-2, record_hist=False, chain_len=0, flag_ambiguity=False):
+                 max_trace_num=2000, unit=1e-2, record_hist=False, chain_len=0, flag_ambiguity=False, configs=None):
         import torch
 
         self.engine, self.flat, self.torch = engine, flat, torch
-        self.scene = engine.upload(flat)
-        self.res, self.t = engine.alloc_result(self.scene, seg_capacity, hit_capacity, n_rays,
+        self.scene = engine.upload(flat) if configs is None else engine.upload_sweep(configs)
+        n_roots = n_rays * self.scene.n_configs
+        self.res, self.t = engine.alloc_result(self.scene, seg_capacity, hit_capacity, n_roots,
                                                hit_columns=tuple(hit_columns) + (() if "hit_key" in hit_columns else ("hit_monitor",)))
         if flag_ambiguity:
             self.t["root_flags"] = torch.zeros(max(int(n_rays), 1), dtype=torch.int32, device=f"cuda:{engine.device}")
@@ -126,12 +128,12 @@ class DeviceTrace:
         if flat.n_capslots:
             # a bundle ray is its own `_id` family starting from zero counts: a cap can only bind if it is
             # smaller than the pop budget. Binding caps need Ray objects (OpticalTable.ray_tracing).
-            capmax = flat.node_f[flat.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX].min()
+            capmax = min(f.node_f[f.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX].min() for f in self.scene.configs)
             if capmax < max_trace_num:
                 raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped component")
             slack = 1
         self.prm = engine.make_params(max_trace_num, unit, seg_capacity > 0, hit_capacity > 0, record_hist, chain_len,
-                                      n_rays, slack, flag_ambiguity)
+                                      n_roots, slack, flag_ambiguity)
         self.hit_columns = tuple(k for k in HIT_COLUMNS_ALL + ("hit_key",) if k in self.t)
 
     def run(self, rays_t, max_live=None):
@@ -146,7 +148,7 @@ class DeviceTrace:
         and move components with `scene.update_nodes(flat.refresh(component))` between replays (SURVEY 8f item 3)."""
         torch = self.torch
         has_pass = bool((self.flat.node_i[:, A.NI_INTER] == A.I_PASS).any())   # pass-through leaves run the wavefront variants
-        if self.flat.max_children > 1 or self.prm.chain_len > 0 or self.flat.n_capslots or has_pass:
+        if self.scene.max_children > 1 or self.prm.chain_len > 0 or self.flat.n_capslots or has_pass:
             raise NotImplementedError("CUDA-graph replay needs a scene whose interactions emit one ray at most (no host round trips)")
         self.run(rays_t, max_live)          # warm-up: workspace and kernel attributes exist before the capture
         torch.cuda.synchronize()
@@ -186,26 +188,35 @@ def trace_bundle(table, bundle: RayBundle, perfomance_limit=None, record_hits=Tr
     cap = int(hit_capacity if hit_capacity is not None else bundle.n * max(flat.n_monitors, 1) * 2) if record_hits else 0
     limit = trace_cap(perfomance_limit)
     rays_t = bundle.to_torch(device=f"cuda:{engine.device}")
-    # live-ray budget of a splitting scene: grow on overflow towards the bound 2 n max_trace_num (a root pops at most
-    # max_trace_num rays and each pop queues at most two); row capacity: the counters keep counting past it, so an
-    # overflowing attempt is repeated once with the exact size
-    live, bound = max_live, max(2 * bundle.n * max(limit, 1), 1024)
-    resized = False
-    while True:
-        dt = DeviceTrace(engine, flat, bundle.n, cap, max_trace_num=limit, record_hist=record_hist, hit_columns=hit_columns)
-        dt.run(rays_t, live)
-        cnt = dt.counters()
-        st = int(cnt[A.C_STATUS])
-        cur = live if live is not None else max(4 * bundle.n, 1024)
-        if st & A.ST_WORK_OVERFLOW and cur < bound:
-            live = min(4 * cur, bound)
-        elif st & A.ST_HIT_OVERFLOW and not resized and hit_capacity is None:
-            cap, resized = int(cnt[A.C_HITS]), True
-        else:
-            break
-        dt.scene.close()
-    engine._raise_status(cnt)
+    dt, cnt = run_to_fit(lambda c: DeviceTrace(engine, flat, bundle.n, c, max_trace_num=limit, record_hist=record_hist,
+                                               hit_columns=hit_columns),
+                         rays_t, bundle.n, limit, cap, hit_capacity is not None, max_live)
     nh = int(cnt[A.C_HITS]) if record_hits else 0
     out = {k: dt.t[k][:nh] for k in dt.hit_columns}
     out["hist_y"], out["hist_yz"], out["counters"] = dt.t["hist_y"], dt.t["hist_yz"], cnt
     return out
+
+
+def run_to_fit(make, rays_t, n_roots, limit, cap, fixed_cap=False, max_live=None):
+    """Trace with `make(hit_capacity)` (a DeviceTrace) until the run fits; returns (DeviceTrace, counters).
+
+    Live-ray budget of a splitting scene: grow on overflow towards the bound 2 n max_trace_num (a root pops at most
+    max_trace_num rays and each pop queues at most two); row capacity (unless `fixed_cap`): the counters keep counting
+    past it, so an overflowing attempt is repeated once with the exact size."""
+    live, bound = max_live, max(2 * n_roots * max(limit, 1), 1024)
+    resized = False
+    while True:
+        dt = make(cap)
+        dt.run(rays_t, live)
+        cnt = dt.counters()
+        st = int(cnt[A.C_STATUS])
+        cur = live if live is not None else max(4 * n_roots, 1024)
+        if st & A.ST_WORK_OVERFLOW and cur < bound:
+            live = min(4 * cur, bound)
+        elif st & A.ST_HIT_OVERFLOW and not resized and not fixed_cap:
+            cap, resized = int(cnt[A.C_HITS]), True
+        else:
+            break
+        dt.scene.close()
+    dt.engine._raise_status(cnt)
+    return dt, cnt

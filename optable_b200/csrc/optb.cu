@@ -101,6 +101,7 @@ struct TraceArgs {
   const unsigned char* blob; uint32_t blob_bytes; SceneOff off; int n_nodes, n_mons;
   // input wavefront: either the caller's rays (gen0) or the workspace wavefront
   optb_rays in0; RayBuf w; int gen0;
+  int hist_mons;       // SWEEP kernels: histograms this launch accumulates (n_configs * n_mons)
   long long n_in; const unsigned int* n_in_dev;  // n_in_dev overrides when non-null
   const uint32_t* gen_first; const uint32_t* gen_last;
   const uint32_t* perm;  // processing order of the wavefront (sorted by coherence key), or null
@@ -118,6 +119,8 @@ struct TraceArgs {
   const uint32_t* fam_off; uint32_t* fam_roots; uint32_t qcap;
   uint32_t root_base;  // global index of ray 0 of this launch (chunked host traces)
   int has_boxes;       // some node carries a lab-box test
+  uint32_t sweep_n;    // SWEEP kernels: rays per configuration (root k * sweep_n + r = ray r in configuration k);
+                       // blob_bytes is then the stride between the configurations' blobs
 };
 
 OPTB_DEV uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -151,11 +154,14 @@ OPTB_DEV unsigned long long warp_alloc(unsigned long long* ctr) {
   return base + __popc(m & ((1u << lane) - 1u));
 }
 
+template <bool SWEEP = false>
 OPTB_DEV void load_ray(const TraceArgs& a, long long i, Ray& r, bool& solo, uint32_t& gcount, uint32_t& pop_base) {
   if (a.gen0) {
     const optb_rays& s = a.in0;
     const uint32_t bc = s.broadcast;
-#define OPTB_COL(ptr, bit) ((ptr)[((bc >> (bit)) & 1u) ? 0 : i])
+    // a sweep traces the one bundle through every configuration: root i reads input ray i % N
+    const long long in = SWEEP ? i % a.sweep_n : i;
+#define OPTB_COL(ptr, bit) ((ptr)[((bc >> (bit)) & 1u) ? 0 : in])
     r.ox = OPTB_COL(s.ox, 0); r.oy = OPTB_COL(s.oy, 1); r.oz = OPTB_COL(s.oz, 2);
     r.dx = OPTB_COL(s.dx, 3); r.dy = OPTB_COL(s.dy, 4); r.dz = OPTB_COL(s.dz, 5);
     r.I = OPTB_COL(s.intensity, 6); r.wl = OPTB_COL(s.wavelength, 7);
@@ -163,7 +169,7 @@ OPTB_DEV void load_ray(const TraceArgs& a, long long i, Ray& r, bool& solo, uint
     r.pl = OPTB_COL(s.pathlength, 10); r.n = OPTB_COL(s.n_medium, 11);
     r.len = s.length ? OPTB_COL(s.length, 12) : INFINITY;
 #undef OPTB_COL
-    r.flags = s.flags ? s.flags[i] : (OPTB_RF_ALIVE | OPTB_RF_HASQ);
+    r.flags = s.flags ? s.flags[in] : (OPTB_RF_ALIVE | OPTB_RF_HASQ);
     r.root = (uint32_t)i + a.root_base; r.pop = 0;
     r.family = s.family ? s.family[i] : (int32_t)r.root;
     solo = true; gcount = 1; pop_base = 0;
@@ -209,7 +215,20 @@ OPTB_DEV void ring_get(const RayBuf& w, long long j, Ray& r) {
   r.flags = q.flags;
 }
 
+// The tables of one configuration of a sweep scene (configuration blobs back to back at stride a.blob_bytes).
+OPTB_DEV void sweep_view(const TraceArgs& a, uint32_t root, SceneView& sv) {
+  const unsigned char* base = a.blob + (size_t)(root / a.sweep_n) * a.blob_bytes;
+  sv.trav = (const double*)(base + a.off.trav);
+  sv.nf = (const double*)(base + a.off.nf);
+  sv.ni = (const int32_t*)(base + a.off.ni);
+  sv.matk = (const int32_t*)(base + a.off.matk);
+  sv.matf = (const double*)(base + a.off.matf);
+  sv.mon = (const double*)(base + a.off.mon);
+  sv.aux = (const double*)(base + a.off.aux);
+}
+
 // One pop's dead segment: append to the segment log and test it against every monitor (monitor.py:183-193).
+template <bool SWEEP = false>
 OPTB_COLD void emit_segment(const TraceArgs& a, const SceneView& sv, const Ray& r, double seg_len, uint32_t seg_flags,
                            int leaf, unsigned int* s_hist, unsigned int& n_hits_local) {
   if (a.rec_seg) {
@@ -254,6 +273,7 @@ OPTB_COLD void emit_segment(const TraceArgs& a, const SceneView& sv, const Ray& 
     const double Px = fma(t, dx, ox), Py = fma(t, dy, oy), Pz = fma(t, dz, oz);
     if (!(fabs(Py) <= mf[OPTB_MON_HW] && fabs(Pz) <= mf[OPTB_MON_HH])) continue;
     if (a.rec_hist) {
+      const int hm = SWEEP ? (int)(r.root / a.sweep_n) * sv.n_mons + m : m;  // sweeps: histograms [config][monitor]
       double y = dot3(Px, Py, Pz, mf[OPTB_MON_TY], mf[OPTB_MON_TY + 1], mf[OPTB_MON_TY + 2]);
       double z = dot3(Px, Py, Pz, mf[OPTB_MON_TZ], mf[OPTB_MON_TZ + 1], mf[OPTB_MON_TZ + 2]);
       int by = hist_bin(y, -mf[OPTB_MON_HW], mf[OPTB_MON_HW], mf[OPTB_MON_STRIDE], mf[OPTB_MON_STRIDE + 1]);
@@ -261,12 +281,12 @@ OPTB_COLD void emit_segment(const TraceArgs& a, const SceneView& sv, const Ray& 
       const int per = OPTB_HIST_BINS * (OPTB_HIST_BINS + 1);
       if (by >= 0) {
         if (a.hist_smem) {
-          atomicAdd(&s_hist[m * per + by], 1u);
-          if (bz >= 0) atomicAdd(&s_hist[m * per + OPTB_HIST_BINS + by * OPTB_HIST_BINS + bz], 1u);
+          atomicAdd(&s_hist[hm * per + by], 1u);
+          if (bz >= 0) atomicAdd(&s_hist[hm * per + OPTB_HIST_BINS + by * OPTB_HIST_BINS + bz], 1u);
         } else {
-          atomicAdd((unsigned long long*)&a.out.hist_y[m * OPTB_HIST_BINS + by], 1ull);
+          atomicAdd((unsigned long long*)&a.out.hist_y[hm * OPTB_HIST_BINS + by], 1ull);
           if (bz >= 0)
-            atomicAdd((unsigned long long*)&a.out.hist_yz[(m * OPTB_HIST_BINS + by) * OPTB_HIST_BINS + bz], 1ull);
+            atomicAdd((unsigned long long*)&a.out.hist_yz[(hm * OPTB_HIST_BINS + by) * OPTB_HIST_BINS + bz], 1ull);
         }
       }
     }
@@ -537,13 +557,17 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
 // BRENT = params.reference_roots: curved-surface roots from the reference's own brentq iteration (brentq_dev) instead
 // of the closed-form / Newton root.
 // PASSK = the scene has an OPTB_I_PASS leaf (a Monitor listed as a component): only the general variants carry that body.
-template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = false, bool BRENT = false, bool PASSK = false>
+// SWEEP = a sweep scene (optb_scene_upload_sweep): every lane reads the tables of its root's configuration from global
+// memory (a warp may straddle configurations); the kernels of ordinary scenes do not carry it.
+template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = false, bool BRENT = false, bool PASSK = false,
+          bool SWEEP = false>
 // Resident CTAs per SM: scenes staged in shared memory are bound by dependent fp64 chains and lose more to the
 // spills of a tighter register budget than they gain from a fifth CTA (measured 6.32 -> 7.62 ms on c2); scenes
 // whose tables stay in L1/L2 (thousands of leaves) are memory-latency bound and gain from it (ripa 30.6 -> 29.8 ms).
 __global__ void __launch_bounds__(kBlock, kResident((SMEM || ASPH || SERIAL) ? OPTB_MIN_BLOCKS : OPTB_MIN_BLOCKS + OPTB_BIG_EXTRA))
 trace_kernel(const __grid_constant__ TraceArgs a) {
   constexpr int MAXCH = (SPLIT || SERIAL) ? 2 : 1;
+  static_assert(!SWEEP || (!SMEM && !SERIAL && !FLAG && !BRENT), "sweeps run the parallel path from global memory");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) unsigned long long mbar;
   // The closest-hit search only needs a ray's geometry. Its radiometric state (intensity, wavelength, q, path
@@ -585,7 +609,7 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
   const int per = OPTB_HIST_BINS * (OPTB_HIST_BINS + 1);
   unsigned int* s_hist = (unsigned int*)(smem_raw + (SMEM ? ((a.blob_bytes + 15u) & ~15u) : 0u));
   if (a.hist_smem) {
-    for (int k = threadIdx.x; k < a.n_mons * per; k += blockDim.x) s_hist[k] = 0u;
+    for (int k = threadIdx.x; k < (SWEEP ? a.hist_mons : a.n_mons) * per; k += blockDim.x) s_hist[k] = 0u;
     __syncthreads();
   }
 
@@ -673,7 +697,8 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
     }
 
     Ray ray; bool solo = true; uint32_t gcount = 1, pop_base0 = 0;
-    if (has) load_ray(a, i, ray, solo, gcount, pop_base0);
+    if (has) load_ray<SWEEP>(a, i, ray, solo, gcount, pop_base0);
+    if constexpr (SWEEP) { if (has) sweep_view(a, ray.root, sv); }
     if (!SPLIT) solo = true;
     uint32_t pop_base_next = (!SPLIT || a.gen0) ? 0u : (pop_base0 + gcount);
     int nch = 0;
@@ -705,8 +730,8 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
       const bool hit = node >= 0;
       const int32_t* ni = sv.ni + (hit ? node : 0) * OPTB_NI_STRIDE;
       const double* nf = sv.nf + (hit ? node : 0) * OPTB_NF_STRIDE;
-      emit_segment(a, sv, ray, hit ? t : ray.len, hit ? (ray.flags & ~OPTB_RF_ALIVE) : ray.flags,
-                   hit ? ni[OPTB_NI_LEAF] : -1, s_hist, c_hits);
+      emit_segment<SWEEP>(a, sv, ray, hit ? t : ray.len, hit ? (ray.flags & ~OPTB_RF_ALIVE) : ray.flags,
+                          hit ? ni[OPTB_NI_LEAF] : -1, s_hist, c_hits);
       if (!hit) { nch = 0; return false; }
       c_inter++;
       hit_leaf = ni[OPTB_NI_LEAF];
@@ -753,7 +778,8 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
             i = (long long)base + __popc(need & ((1u << lane) - 1u));
             if (i < n_in) {
               if (a.perm) i = a.perm[i];
-              load_ray(a, i, ray, solo, gcount, pop_base0);
+              load_ray<SWEEP>(a, i, ray, solo, gcount, pop_base0);
+              if constexpr (SWEEP) sweep_view(a, ray.root, sv);
               pop_base_next = a.gen0 ? 0u : (pop_base0 + gcount);
               nch = 0; chained = 0; hit_leaf = 0; ch.n = 0;
               active = true;
@@ -801,7 +827,7 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
   }
   if (a.hist_smem) {
     __syncthreads();
-    for (int k = threadIdx.x; k < a.n_mons * per; k += blockDim.x) {
+    for (int k = threadIdx.x; k < (SWEEP ? a.hist_mons : a.n_mons) * per; k += blockDim.x) {
       unsigned int cnt = s_hist[k];
       if (!cnt) continue;
       int m = k / per, r = k % per;
@@ -1010,7 +1036,11 @@ struct optb_scene {
   // not for the whole device (other streams, NCCL and unrelated kernels keep running)
   cudaEvent_t last_use; bool used;
   std::vector<unsigned char>* cull;  // cullable bit per node as uploaded (optb_scene_update_nodes keeps it current)
+  int n_cfg; uint32_t cfg_stride;    // sweep scenes: configurations, bytes per configuration blob (0, 0 otherwise)
 };
+
+// histograms a trace of the scene fills: [n_cfg][n_mons] for a sweep
+static int hist_mons(const optb_scene* s) { return s->n_mons * std::max(s->n_cfg, 1); }
 
 static int fail(optb_ctx* ctx, int code, const char* what, cudaError_t e = cudaSuccess) {
   if (ctx) {
@@ -1137,11 +1167,10 @@ static void asphere_constants(double* nf, const int32_t* ni) {
   else nf[OPTB_NF_FOCAL] = (c[1] + 1.0) / ((c[1] - 1.0) * c[0] * c[0]);
 }
 
-extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_scene** out) {
-  if (!ctx || !d || !out) return -1;
+// The kernels index the tables without bounds checks: reject anything that could walk out of them.
+static int validate_desc(optb_ctx* ctx, const optb_scene_desc* d) {
   if (d->abi_version != OPTB_ABI_VERSION) return fail(ctx, -4, "scene ABI version mismatch");
   if (d->n_nodes < 0 || d->n_materials < 1) return fail(ctx, -5, "bad scene counts");
-  // The kernels index the tables without bounds checks: reject anything that could walk out of them.
   for (int i = 0; i < d->n_nodes; i++) {
     const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
     const int g = ni[OPTB_NI_GEOM];
@@ -1206,30 +1235,32 @@ extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_s
       }
     }
   }
-  cudaSetDevice(ctx->device);
-  optb_scene* s = new (std::nothrow) optb_scene();
-  if (!s) return -3;
-  memset(s, 0, sizeof *s);
-  s->n_nodes = d->n_nodes; s->n_leaves = d->n_leaves; s->n_mats = d->n_materials; s->n_mons = d->n_monitors;
-  s->n_caps = d->n_capslots; s->n_aux = d->n_aux;
+  return 0;
+}
+
+// Byte layout of one scene blob; returns its size.
+static size_t blob_layout(const optb_scene_desc* d, SceneOff& off) {
   size_t b_nf = (size_t)d->n_nodes * OPTB_NF_STRIDE * 8, b_ni = (size_t)d->n_nodes * OPTB_NI_STRIDE * 4;
   size_t b_mk = (size_t)d->n_materials * 4, b_mf = (size_t)d->n_materials * OPTB_MF_STRIDE * 8;
   size_t b_mon = (size_t)std::max(d->n_monitors, 1) * kMonBlobStride * 8, b_aux = (size_t)std::max<long long>(d->n_aux, 1) * 8;
   size_t o = 0;
   const size_t b_trav = (size_t)std::max(d->n_nodes, 1) * 64;
-  s->off.trav = (uint32_t)o; o = align_up(o + b_trav, 16);
-  s->off.nf = (uint32_t)o; o = align_up(o + b_nf, 16);
-  s->off.ni = (uint32_t)o; o = align_up(o + b_ni, 16);
-  s->off.matk = (uint32_t)o; o = align_up(o + b_mk, 16);
-  s->off.matf = (uint32_t)o; o = align_up(o + b_mf, 16);
-  s->off.mon = (uint32_t)o; o = align_up(o + b_mon, 16);
-  s->off.aux = (uint32_t)o; o = align_up(o + b_aux, 16);
-  if (o > 0xfff00000ull) { delete s; return fail(ctx, -6, "scene too large"); }
-  s->blob_bytes = (uint32_t)o;
-  std::vector<unsigned char> host(o, 0);
+  off.trav = (uint32_t)o; o = align_up(o + b_trav, 16);
+  off.nf = (uint32_t)o; o = align_up(o + b_nf, 16);
+  off.ni = (uint32_t)o; o = align_up(o + b_ni, 16);
+  off.matk = (uint32_t)o; o = align_up(o + b_mk, 16);
+  off.matf = (uint32_t)o; o = align_up(o + b_mf, 16);
+  off.mon = (uint32_t)o; o = align_up(o + b_mon, 16);
+  off.aux = (uint32_t)o; o = align_up(o + b_aux, 16);
+  return o;
+}
+
+// Host image of one scene blob (zeroed `host`, blob_layout bytes); `cull` receives the cullable bit of every node.
+static void fill_blob(const optb_scene_desc* d, const SceneOff& off, unsigned char* host, std::vector<unsigned char>& cull) {
+  const size_t b_nf = (size_t)d->n_nodes * OPTB_NF_STRIDE * 8, b_ni = (size_t)d->n_nodes * OPTB_NI_STRIDE * 4;
   if (d->n_nodes) {
-    memcpy(host.data() + s->off.nf, d->node_f, b_nf);
-    memcpy(host.data() + s->off.ni, d->node_i, b_ni);
+    memcpy(host + off.nf, d->node_f, b_nf);
+    memcpy(host + off.ni, d->node_i, b_ni);
     // parent of every node, from the skip pointers (pre-order: the innermost open group that still covers i)
     std::vector<int32_t> parent(d->n_nodes, -1), open;
     for (int i = 0; i < d->n_nodes; i++) {
@@ -1238,11 +1269,9 @@ extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_s
       parent[i] = open.empty() ? -1 : open.back();
       if (ni[OPTB_NI_GEOM] == OPTB_G_GROUP || ni[OPTB_NI_GEOM] == OPTB_G_GRID) open.push_back(i);
     }
-    s->cull = new std::vector<unsigned char>();
-    std::vector<unsigned char>& cull = *s->cull;
     cull_bits(d, cull);
     for (int i = 0; i < d->n_nodes; i++) {  // compact traversal records
-      unsigned char* tv = host.data() + s->off.trav + (size_t)i * 64;
+      unsigned char* tv = host + off.trav + (size_t)i * 64;
       const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
       memcpy(tv, d->node_f + (size_t)i * OPTB_NF_STRIDE + OPTB_NF_AABB, 48);
       // box word: bit 0 = test the box (component_group.py:98-107), bit 1 = the box may dismiss by distance (cull_bits)
@@ -1250,27 +1279,32 @@ extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_s
       memcpy(tv + 48, pack, 16);
     }
   }
-  memcpy(host.data() + s->off.matk, d->mat_kind, b_mk);
-  memcpy(host.data() + s->off.matf, d->mat_f, b_mf);
+  memcpy(host + off.matk, d->mat_kind, (size_t)d->n_materials * 4);
+  memcpy(host + off.matf, d->mat_f, (size_t)d->n_materials * OPTB_MF_STRIDE * 8);
   for (int m = 0; m < d->n_monitors; m++) {  // ABI record + the histogram constants derived from it (kMonBlobStride)
-    double* mf = (double*)(host.data() + s->off.mon) + (size_t)m * kMonBlobStride;
+    double* mf = (double*)(host + off.mon) + (size_t)m * kMonBlobStride;
     memcpy(mf, d->mon_f + (size_t)m * OPTB_MON_STRIDE, OPTB_MON_STRIDE * 8);
     const double w = mf[OPTB_MON_HW] - (-mf[OPTB_MON_HW]), h = mf[OPTB_MON_HH] - (-mf[OPTB_MON_HH]);  // hi - lo as hist_bin forms it
     mf[OPTB_MON_STRIDE] = OPTB_HIST_BINS / w; mf[OPTB_MON_STRIDE + 1] = w / OPTB_HIST_BINS;
     mf[OPTB_MON_STRIDE + 2] = OPTB_HIST_BINS / h; mf[OPTB_MON_STRIDE + 3] = h / OPTB_HIST_BINS;
   }
-  for (int i = 0; i < d->n_nodes; i++) asphere_constants((double*)(host.data() + s->off.nf) + (size_t)i * OPTB_NF_STRIDE,
+  for (int i = 0; i < d->n_nodes; i++) asphere_constants((double*)(host + off.nf) + (size_t)i * OPTB_NF_STRIDE,
                                                          d->node_i + (size_t)i * OPTB_NI_STRIDE);
-  if (d->n_aux) memcpy(host.data() + s->off.aux, d->aux, (size_t)d->n_aux * 8);
-  // most children one interaction can emit (decides whether the wavefront machinery is needed)
-  int mc = 0;
+  if (d->n_aux) memcpy(host + off.aux, d->aux, (size_t)d->n_aux * 8);
+}
+
+// Scene-wide properties that pick the kernel variant. max_children: most children one interaction can emit (decides
+// whether the wavefront machinery is needed).
+struct SceneProps { int max_children, has_boxes, has_asph, has_grid, has_pass; };
+static SceneProps scene_props(const optb_scene_desc* d) {
+  SceneProps p{0, 0, 0, 0, 0};
   for (int i = 0; i < d->n_nodes; i++) {
     const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
     const double* nf = d->node_f + (size_t)i * OPTB_NF_STRIDE;
-    if (ni[OPTB_NI_AABB]) s->has_boxes = 1;
-    if (ni[OPTB_NI_GEOM] == OPTB_G_ASPHERE) s->has_asph = 1;
-    if (ni[OPTB_NI_GEOM] == OPTB_G_GRID) s->has_grid = 1;
-    if (ni[OPTB_NI_INTER] == OPTB_I_PASS) s->has_pass = 1;
+    if (ni[OPTB_NI_AABB]) p.has_boxes = 1;
+    if (ni[OPTB_NI_GEOM] == OPTB_G_ASPHERE) p.has_asph = 1;
+    if (ni[OPTB_NI_GEOM] == OPTB_G_GRID) p.has_grid = 1;
+    if (ni[OPTB_NI_INTER] == OPTB_I_PASS) p.has_pass = 1;
     int k = 0;
     switch (ni[OPTB_NI_INTER]) {
       case OPTB_I_MIRROR: k = (nf[OPTB_NF_REFL] > 0) + (nf[OPTB_NF_TRANS] > 0); break;
@@ -1278,12 +1312,41 @@ extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_s
       case OPTB_I_THINLENS: case OPTB_I_PASS: k = 1; break;
       default: k = 0;
     }
-    mc = std::max(mc, k);
+    p.max_children = std::max(p.max_children, k);
   }
-  s->max_children = mc;
-  size_t hist_bytes = (size_t)d->n_monitors * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 4;
+  return p;
+}
+
+// One scene (n_cfg = 0) or a sweep of n_cfg configurations of one topology (descs checked by the caller): the
+// configuration blobs lie back to back at a stride of one blob.
+static int scene_upload(optb_ctx* ctx, const optb_scene_desc* ds, int n_cfg, optb_scene** out) {
+  const int K = std::max(n_cfg, 1);
+  for (int k = 0; k < K; k++)
+    if (int rc = validate_desc(ctx, &ds[k])) return rc;
+  const optb_scene_desc* d = &ds[0];
+  cudaSetDevice(ctx->device);
+  optb_scene* s = new (std::nothrow) optb_scene();
+  if (!s) return -3;
+  memset(s, 0, sizeof *s);
+  s->n_nodes = d->n_nodes; s->n_leaves = d->n_leaves; s->n_mats = d->n_materials; s->n_mons = d->n_monitors;
+  s->n_caps = d->n_capslots; s->n_aux = d->n_aux;
+  s->n_cfg = n_cfg;
+  const size_t stride = blob_layout(d, s->off);
+  const size_t o = stride * K;
+  if (o > 0xfff00000ull) { delete s; return fail(ctx, -6, "scene too large"); }
+  s->blob_bytes = (uint32_t)o; s->cfg_stride = (uint32_t)stride;
+  std::vector<unsigned char> host(o, 0);
+  if (d->n_nodes) s->cull = new std::vector<unsigned char>();
+  for (int k = 0; k < K; k++) {
+    std::vector<unsigned char> cull_k;  // (cull bits are per configuration; the scene keeps the first one's)
+    fill_blob(&ds[k], s->off, host.data() + stride * k, k == 0 && s->cull ? *s->cull : cull_k);
+    const SceneProps p = scene_props(&ds[k]);
+    s->max_children = std::max(s->max_children, p.max_children);
+    s->has_boxes |= p.has_boxes; s->has_asph |= p.has_asph; s->has_grid |= p.has_grid; s->has_pass |= p.has_pass;
+  }
+  size_t hist_bytes = (size_t)K * d->n_monitors * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 4;
   size_t budget = ctx->smem_optin > 2048 ? ctx->smem_optin - 2048 : 0;
-  s->in_smem = (o <= budget);
+  s->in_smem = !n_cfg && (o <= budget);  // sweep kernels read the tables from global memory (L1/L2)
   size_t used = s->in_smem ? o : 0;
   s->hist_smem = (hist_bytes > 0 && used + hist_bytes <= std::min<size_t>(budget, used + 65536));
   s->smem_bytes = (uint32_t)(used + (s->hist_smem ? hist_bytes : 0));
@@ -1297,18 +1360,51 @@ extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_s
   } else {
     s->blob_cap = (o + 65535) & ~(size_t)65535;
     e = cudaMalloc((void**)&s->d_blob, s->blob_cap);
-    if (e != cudaSuccess) { delete s; return fail(ctx, -10, "cudaMalloc(scene)", e); }
+    if (e != cudaSuccess) { delete s->cull; delete s; return fail(ctx, -10, "cudaMalloc(scene)", e); }
   }
   e = cudaMemcpy(s->d_blob, host.data(), o, cudaMemcpyHostToDevice);
   if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->last_use, cudaEventDisableTiming);
-  if (e != cudaSuccess) { cudaFree(s->d_blob); delete s; return fail(ctx, -10, "cudaMemcpy(scene)", e); }
+  if (e != cudaSuccess) { cudaFree(s->d_blob); delete s->cull; delete s; return fail(ctx, -10, "cudaMemcpy(scene)", e); }
   *out = s;
   return 0;
+}
+
+extern "C" int optb_scene_upload(optb_ctx* ctx, const optb_scene_desc* d, optb_scene** out) {
+  if (!ctx || !d || !out) return -1;
+  return scene_upload(ctx, d, 0, out);
+}
+
+extern "C" int optb_scene_upload_sweep(optb_ctx* ctx, const optb_scene_desc* descs, int32_t n_configs, optb_scene** out) {
+  if (!ctx || !descs || !out) return -1;
+  if (n_configs < 1) return fail(ctx, -5, "optb_scene_upload_sweep: n_configs must be >= 1");
+  const optb_scene_desc* d0 = &descs[0];
+  char msg[160];
+  for (int k = 1; k < n_configs; k++) {
+    const optb_scene_desc* d = &descs[k];
+    if (d->n_nodes != d0->n_nodes || d->n_leaves != d0->n_leaves || d->n_materials != d0->n_materials ||
+        d->n_monitors != d0->n_monitors || d->n_capslots != d0->n_capslots || d->n_aux != d0->n_aux) {
+      snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in its table sizes", k);
+      return fail(ctx, -5, msg);
+    }
+    // a leaf index, skip pointer, material slot and cap slot must mean the same in every configuration
+    for (int i = 0; i < d0->n_nodes; i++)
+      for (int c = 0; c < OPTB_NI_STRIDE; c++)
+        if (c != OPTB_NI_ORTHO && d->node_i[(size_t)i * OPTB_NI_STRIDE + c] != d0->node_i[(size_t)i * OPTB_NI_STRIDE + c]) {
+          snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in node_i row %d column %d", k, i, c);
+          return fail(ctx, -5, msg);
+        }
+    if (memcmp(d->mat_kind, d0->mat_kind, (size_t)d0->n_materials * 4)) {
+      snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in its material kinds", k);
+      return fail(ctx, -5, msg);
+    }
+  }
+  return scene_upload(ctx, descs, n_configs, out);
 }
 
 extern "C" int optb_scene_update_nodes(optb_ctx* ctx, optb_scene* s, const optb_scene_desc* d, const int32_t* nodes,
                                        int32_t n, void* stream_v) {
   if (!ctx || !s || !d || (n > 0 && !nodes)) return -1;
+  if (s->n_cfg) return fail(ctx, -7, "optb_scene_update_nodes: not available on a sweep scene (upload the configurations again)");
   if (d->n_nodes != s->n_nodes || d->n_leaves != s->n_leaves || d->n_materials != s->n_mats || d->n_aux != s->n_aux ||
       d->n_capslots != s->n_caps)
     return fail(ctx, -5, "optb_scene_update_nodes: the tables no longer have the shape of the uploaded scene");
@@ -1339,23 +1435,8 @@ extern "C" int optb_scene_update_nodes(optb_ctx* ctx, optb_scene* s, const optb_
     s->cull->swap(now);
   }
   // scene-wide properties that pick the kernel variant follow the new rows
-  int mc = 0, boxes = 0, asph = 0, pass = 0;
-  for (int i = 0; i < d->n_nodes; i++) {
-    const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
-    const double* nf = d->node_f + (size_t)i * OPTB_NF_STRIDE;
-    if (ni[OPTB_NI_AABB]) boxes = 1;
-    if (ni[OPTB_NI_GEOM] == OPTB_G_ASPHERE) asph = 1;
-    if (ni[OPTB_NI_INTER] == OPTB_I_PASS) pass = 1;
-    int k = 0;
-    switch (ni[OPTB_NI_INTER]) {
-      case OPTB_I_MIRROR: k = (nf[OPTB_NF_REFL] > 0) + (nf[OPTB_NF_TRANS] > 0); break;
-      case OPTB_I_REFRACT: k = nf[OPTB_NF_REFL] > 0 ? 2 : 1; break;
-      case OPTB_I_THINLENS: case OPTB_I_PASS: k = 1; break;
-      default: k = 0;
-    }
-    mc = std::max(mc, k);
-  }
-  s->max_children = mc; s->has_boxes = boxes; s->has_asph = asph; s->has_pass = pass;
+  const SceneProps p = scene_props(d);
+  s->max_children = p.max_children; s->has_boxes = p.has_boxes; s->has_asph = p.has_asph; s->has_pass = p.has_pass;
   return 0;
 }
 
@@ -1442,6 +1523,7 @@ SerialLayout serial_layout(long long n_rays, long long n_fam, long long ring_ent
 
 extern "C" int64_t optb_workspace_bytes(const optb_scene* scene, int64_t n_rays, int64_t max_live) {
   if (!scene || n_rays < 0) return -1;
+  if (scene->n_cfg) n_rays *= scene->n_cfg;  // sweep: n_rays per configuration, one root per (configuration, ray)
   // the caller may later pass chain_len > 0, so always size for the wavefront when asked for max_live > 0
   bool split = scene->max_children > 1 || max_live > 0 || scene->has_pass;
   int64_t need = (int64_t)ws_layout(n_rays, std::max<int64_t>(max_live, n_rays), split).total;
@@ -1466,6 +1548,16 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   cudaSetDevice(ctx->device);
   if (!out->counters) return fail(ctx, -7, "result.counters is required");
   if (rays->n >= 0xffffffffll) return fail(ctx, -7, "at most 2^32-1 rays per call");
+  // a sweep scene traces every ray through every configuration: root k * rays.n + r = ray r in configuration k
+  const long long n_roots = scene->n_cfg ? rays->n * scene->n_cfg : rays->n;
+  if (scene->n_cfg) {
+    if (n_roots >= 0xffffffffll) return fail(ctx, -7, "sweep: n_configs * rays.n must stay below 2^32");
+    if (needs_serial(scene, rays, prm))
+      return fail(ctx, -7, "sweep: the scene has interact caps; set params.caps_slack (sweeps have no family-serial path)");
+    if (prm->flag_ambiguity || prm->reference_roots)
+      return fail(ctx, -7, "sweep: flag_ambiguity and reference_roots are not available on sweep scenes");
+    if (rays->family) return fail(ctx, -7, "sweep: rays.family must be NULL (every root is its own family)");
+  }
   if (prm->record_hits && out->hit_capacity > 0 && !out->hit_monitor && !out->hit_key) return fail(ctx, -7, "record_hits needs hit_monitor or hit_key");
   if (prm->record_hits && out->hit_key && (prm->max_trace_num > (1ll << 24) || scene->n_mons > 256))
     return fail(ctx, -7, "hit_key packs pop into 24 bits and the monitor into 8: max_trace_num <= 2^24 and <= 256 monitors");
@@ -1473,12 +1565,12 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   if (scene->n_caps > 0 && (!out->cap_counts || prm->n_families < 1)) return fail(ctx, -7, "scene has interact caps: cap_counts/n_families required");
   // cap_counts is [n_capslots][n_families]; without a family column every initial ray is its own family (column
   // index = ray index), so the table must have a column per ray
-  if (scene->n_caps > 0 && !rays->family && (long long)prm->n_families < rays->n)
-    return fail(ctx, -7, "scene has interact caps and rays.family is NULL: n_families must be >= rays.n");
+  if (scene->n_caps > 0 && !rays->family && (long long)prm->n_families < n_roots)
+    return fail(ctx, -7, "scene has interact caps and rays.family is NULL: n_families must be >= rays.n (times n_configs for a sweep)");
   const bool serial = needs_serial(scene, rays, prm);
   if (serial && prm->flag_ambiguity) return fail(ctx, -7, "flag_ambiguity is not available on the family-serial path (binding interact caps)");
   const bool split = !serial && needs_wavefront(scene, prm);
-  WsLayout L = ws_layout(rays->n, 0, false);
+  WsLayout L = ws_layout(n_roots, 0, false);
   long long cap = 0;
   SerialLayout SL{};
   long long n_fam = 0, qcap = 0;
@@ -1499,18 +1591,18 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
     L.hdr = SL.hdr;
   } else if (split) {
     // find the largest wavefront capacity the given workspace supports
-    if (workspace_bytes < (int64_t)ws_layout(rays->n, rays->n, true).total) return fail(ctx, -8, "workspace too small (see optb_workspace_bytes)");
+    if (workspace_bytes < (int64_t)ws_layout(n_roots, n_roots, true).total) return fail(ctx, -8, "workspace too small (see optb_workspace_bytes)");
     // upper end of the search: what the workspace could hold at ~100 B per live ray (far above the real cost of
     // ~540 B), so the capacity is set by the caller's workspace and never by the size of the batch: one initial ray
     // through cascaded beam splitters may need thousands of live rays (the reference allows 2000 pops)
-    long long lo = rays->n, hi = std::max<long long>(rays->n, (long long)(workspace_bytes / 100));
+    long long lo = n_roots, hi = std::max<long long>(n_roots, (long long)(workspace_bytes / 100));
     hi = std::min<long long>(hi, 0x7ffffff0ll);
     while (lo < hi) {
       long long mid = lo + (hi - lo + 1) / 2;
-      if ((int64_t)ws_layout(rays->n, mid, true).total <= workspace_bytes) lo = mid; else hi = mid - 1;
+      if ((int64_t)ws_layout(n_roots, mid, true).total <= workspace_bytes) lo = mid; else hi = mid - 1;
     }
     cap = lo;
-    L = ws_layout(rays->n, cap, true);
+    L = ws_layout(n_roots, cap, true);
   } else if (workspace_bytes < (int64_t)L.total) {
     return fail(ctx, -8, "workspace too small (see optb_workspace_bytes)");
   }
@@ -1522,8 +1614,8 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   if (prm->record_hist && scene->n_mons && !out->hist_y) return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
   if (prm->record_hist && scene->n_mons && zero_hist) {
     if (!out->hist_y || !out->hist_yz) return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
-    CK(cudaMemsetAsync(out->hist_y, 0, sizeof(int64_t) * OPTB_HIST_BINS * scene->n_mons, st), "memset hist");
-    CK(cudaMemsetAsync(out->hist_yz, 0, sizeof(int64_t) * OPTB_HIST_BINS * OPTB_HIST_BINS * scene->n_mons, st), "memset hist");
+    CK(cudaMemsetAsync(out->hist_y, 0, sizeof(int64_t) * OPTB_HIST_BINS * hist_mons(scene), st), "memset hist");
+    CK(cudaMemsetAsync(out->hist_yz, 0, sizeof(int64_t) * OPTB_HIST_BINS * OPTB_HIST_BINS * hist_mons(scene), st), "memset hist");
   }
 
   if (prm->flag_ambiguity) CK(cudaMemsetAsync(out->root_flags, 0, sizeof(uint32_t) * (size_t)rays->n, st), "memset root flags");
@@ -1531,7 +1623,8 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   memset(&a, 0, sizeof a);
   a.blob = scene->d_blob; a.blob_bytes = scene->blob_bytes; a.off = scene->off;
   a.n_nodes = scene->n_nodes; a.n_mons = scene->n_mons;
-  a.in0 = *rays; a.gen0 = 1; a.n_in = rays->n; a.n_in_dev = nullptr;
+  a.in0 = *rays; a.gen0 = 1; a.n_in = n_roots; a.n_in_dev = nullptr;
+  if (scene->n_cfg) { a.blob_bytes = scene->cfg_stride; a.sweep_n = (uint32_t)rays->n; a.hist_mons = hist_mons(scene); }
   a.max_trace = prm->max_trace_num; a.unit = prm->unit;
   a.rec_seg = prm->record_segments; a.rec_hit = prm->record_hits; a.rec_hist = prm->record_hist && scene->n_mons > 0;
   a.chain_len = prm->chain_len; a.n_families = prm->n_families;
@@ -1571,6 +1664,15 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
                                      trace_kernel<true, false, 1, true, true, false, false, true>};
   if (scene->has_pass && !serial) kern = pass_table[scene->in_smem ? 1 : 0];
   if (prm->flag_ambiguity) kern = flag_table[scene->in_smem ? 1 : 0];
+  // sweep scenes: the same production kinds, each lane on its root's configuration (tables in global memory)
+#define OPTB_K(B, A, P) trace_kernel<false, false, B, A, P, false, false, false, true>
+#define OPTB_KROW(B) {{OPTB_K(B, false, false), OPTB_K(B, false, true)}, {OPTB_K(B, true, false), OPTB_K(B, true, true)}}
+  static const Kern sweep_table[3][2][2] = {OPTB_KROW(0), OPTB_KROW(1), OPTB_KROW(2)};
+#undef OPTB_KROW
+#undef OPTB_K
+  if (scene->n_cfg)
+    kern = scene->has_pass ? trace_kernel<false, false, 1, true, true, false, false, true, true>
+                           : sweep_table[boxmode][scene->has_asph ? 1 : 0][split ? 1 : 0];
   // params.reference_roots: the general variants with brentq_dev (parallel and family-serial)
   static const Kern brent_table[2][2] = {{trace_kernel<false, false, 1, true, true, false, true>, trace_kernel<true, false, 1, true, true, false, true>},
                                          {trace_kernel<false, true, 1, true, true, false, true>, trace_kernel<true, true, 1, true, true, false, true>}};
@@ -1585,7 +1687,7 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   const int full_grid = ctx->sm_count * occ;
 
   unsigned long long gens = 0, launches = 0;
-  long long n_in = rays->n;
+  long long n_in = n_roots;
   if (serial && n_in > 0) {
     unsigned int* off = (unsigned int*)(ws + SL.off);
     unsigned int* cursor = (unsigned int*)(ws + SL.cursor);
@@ -1873,21 +1975,22 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
 extern "C" int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
                                optb_result* out) {
   if (!ctx || !scene || !rays || !prm || !out) return -1;
-  if (!needs_wavefront(scene, prm) && scene->n_caps == 0 && rays->n >= (3ll << 20)) {
+  if (!needs_wavefront(scene, prm) && scene->n_caps == 0 && !scene->n_cfg && rays->n >= (3ll << 20)) {
     int rc = trace_host_pipelined(ctx, scene, rays, prm, out);
     if (rc <= 0) return rc;  // 1 = a chunk outgrew its estimated share of the result capacity: one-shot path
   }
   // The live ray set of a splitting scene is not known in advance: grow the workspace until it fits. A root pops at
   // most max_trace_num rays and every pop queues at most two, so 2 n max_trace_num live rays always suffice.
-  const double bound_d = 2.0 * (double)std::max<int64_t>(rays->n, 1) * (double)std::max<int64_t>(prm->max_trace_num, 1);
+  const int64_t n_roots = rays->n * std::max(scene->n_cfg, 1);
+  const double bound_d = 2.0 * (double)std::max<int64_t>(n_roots, 1) * (double)std::max<int64_t>(prm->max_trace_num, 1);
   const int64_t bound = bound_d > 4e9 ? (int64_t)4e9 : (int64_t)bound_d;
   const int64_t per_ray = std::max<int64_t>(4, ctx->live_per_ray_hint);
-  for (int64_t live = std::min<int64_t>(std::max<int64_t>(per_ray * rays->n, 1024), std::max<int64_t>(bound, 1024));;
+  for (int64_t live = std::min<int64_t>(std::max<int64_t>(per_ray * n_roots, 1024), std::max<int64_t>(bound, 1024));;
        live = std::min<int64_t>(live * 2, bound)) {
     int rc = trace_host_once(ctx, scene, rays, prm, out, live);
     if (rc) return rc;
     if (!(ctx->h_counters[OPTB_C_STATUS] & OPTB_ST_WORK_OVERFLOW)) {
-      if (rays->n > 0 && needs_wavefront(scene, prm)) ctx->live_per_ray_hint = (live + rays->n - 1) / rays->n;
+      if (n_roots > 0 && needs_wavefront(scene, prm)) ctx->live_per_ray_hint = (live + n_roots - 1) / n_roots;
       return 0;
     }
     if (live >= bound) break;
@@ -1898,16 +2001,16 @@ extern "C" int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const opt
 static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
                            optb_result* out, int64_t live) {
   cudaSetDevice(ctx->device);
-  const int64_t n = rays->n;
+  const int64_t n = rays->n, n_roots = n * std::max(scene->n_cfg, 1);
   const bool split = needs_wavefront(scene, prm) || needs_serial(scene, rays, prm);
   const int64_t segcap = prm->record_segments ? out->seg_capacity : 0, hitcap = prm->record_hits ? out->hit_capacity : 0;
-  const int64_t max_live = split ? std::max<int64_t>(live, n) : 0;
+  const int64_t max_live = split ? std::max<int64_t>(live, n_roots) : 0;
   const int64_t wsb = needs_serial(scene, rays, prm) ? optb_workspace_bytes(scene, n, 16 * std::max<int64_t>(live, 64))
-                                               : (int64_t)ws_layout(n, max_live, split).total;
+                                               : (int64_t)ws_layout(n_roots, max_live, split).total;
   const int nfam = std::max(prm->n_families, 1);
   const int64_t sortb = prm->sorted_rows ? optb_sort_workspace_bytes(std::max(segcap, hitcap)) : 0;
   size_t need = 256 * 64 + (size_t)sortb + (size_t)n * (8 * 13 + 8) + (size_t)segcap * (13 * 8 + 16) + (size_t)hitcap * (10 * 8 + 12 + 8) +
-                (size_t)std::max(scene->n_mons, 1) * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 8 +
+                (size_t)std::max(hist_mons(scene), 1) * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 8 +
                 (size_t)std::max(scene->n_caps, 1) * nfam * 4 + 64 * 8 + (size_t)wsb;
   if (ctx->arena_bytes < need) {
     if (ctx->arena) cudaFree(ctx->arena);
@@ -1951,7 +2054,7 @@ static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_ra
   for (auto& c : cols) if (!*c.dev) return fail(ctx, -9, "arena sizing");
   void* sort_ws = sortb ? ac.take((size_t)sortb) : nullptr;
   if (sortb && !sort_ws) return fail(ctx, -9, "arena sizing");
-  const size_t hy = (size_t)std::max(scene->n_mons, 1) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
+  const size_t hy = (size_t)std::max(hist_mons(scene), 1) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
   dv.hist_y = (int64_t*)ac.take(hy); dv.hist_yz = (int64_t*)ac.take(hyz);
   const size_t capb = (size_t)std::max(scene->n_caps, 1) * nfam * 4;
   dv.cap_counts = (int32_t*)ac.take(capb);
@@ -1974,8 +2077,8 @@ static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_ra
     if (rows > 0) CK(cudaMemcpyAsync(c.host, *c.dev, (size_t)rows * c.elt, cudaMemcpyDeviceToHost, st), "D2H results");
   }
   if (prm->record_hist && scene->n_mons) {
-    if (out->hist_y) CK(cudaMemcpyAsync(out->hist_y, dv.hist_y, (size_t)scene->n_mons * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
-    if (out->hist_yz) CK(cudaMemcpyAsync(out->hist_yz, dv.hist_yz, (size_t)scene->n_mons * OPTB_HIST_BINS * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
+    if (out->hist_y) CK(cudaMemcpyAsync(out->hist_y, dv.hist_y, (size_t)hist_mons(scene) * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
+    if (out->hist_yz) CK(cudaMemcpyAsync(out->hist_yz, dv.hist_yz, (size_t)hist_mons(scene) * OPTB_HIST_BINS * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
   }
   if (scene->n_caps > 0 && out->cap_counts) CK(cudaMemcpyAsync(out->cap_counts, dv.cap_counts, capb, cudaMemcpyDeviceToHost, st), "D2H caps");
   CK(cudaStreamSynchronize(st), "sync results");

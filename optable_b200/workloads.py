@@ -77,6 +77,17 @@ def telescope_4f(ns, n_rays=7, disc=True):
     return Scene([l0, l1], rays, [mon0, mon1])
 
 
+def telescope_4f_grid(ns, F1, F2):
+    """The C2 relay as `calibrate_symmetric_4f` scans it (optical_table.py:328-336): lens 1 stays at its focal length
+    F0 = 43.17, lens 2 sits at F0 + F1 + F2 and monitor 1 at F0 + F1 + 2 F2 (F1 = F2 = F0: the C2 scene). No rays."""
+    F0 = 43.17
+    l0 = asphere_lens9(ns, [F0, 0, 0])
+    l1 = asphere_lens9(ns, [F0 + F1 + F2, 0, 0]).RotZ(np.pi)
+    mon0 = ns.Monitor([0, 0, 0], width=5, height=5)
+    mon1 = ns.Monitor([F0 + F1 + 2 * F2, 0, 0], width=5, height=5)
+    return Scene([l0, l1], [], [mon0, mon1])
+
+
 def ripa(ns, n_rays=1, limit=300, jitter=True):
     """C5: examples/ripa_gen2_lensless.py:54-299 (7,689 leaves: two MMA arrays of 80x15 and 80x80 spherical
     micro-mirrors, a 80x1 back MMA, fold mirrors, a TriangularPrism, a Block; nesting depth 2; 3 monitors).
