@@ -77,6 +77,15 @@ def _result_fields(torch):
     return _RESULT_DTYPES
 
 
+def runs_wavefront(flats, params: A.Params) -> bool:
+    """Whether a trace of the scene made of `flats` (its configurations) with `params` can run the wavefront path (or
+    the family-serial one): it then needs workspace for the live rays of every generation and synchronises with the
+    host once per generation, so it cannot be captured into a CUDA graph. Splitting scenes, capped scenes, pass-through
+    leaves, chain_len > 0 and the two diagnostics modes do."""
+    return bool(params.chain_len > 0 or params.flag_ambiguity or params.reference_roots
+                or any(f.max_children > 1 or f.n_capslots > 0 or f.has_pass for f in flats))
+
+
 class Scene:
     """Device-resident scene tables (optb_scene handle). With `configs` (a list of FlatScene of one topology) it is a
     sweep scene (optb_scene_upload_sweep): `flat` is then configs[0], and every trace runs its bundle through all
@@ -264,10 +273,7 @@ class Engine:
         torch = self.torch
         rs = self._rays_struct(rays_t)
         n = int(rs.n) * scene.n_configs   # roots
-        has_pass = bool((scene.flat.node_i[:, A.NI_INTER] == A.I_PASS).any())   # runs the general (wavefront) variants
-        splitting = (scene.max_children > 1 or params.chain_len > 0 or scene.flat.n_capslots > 0 or params.flag_ambiguity
-                     or params.reference_roots or has_pass)
-        live = 0 if not splitting else int(max_live if max_live is not None else max(4 * n, 1024))
+        live = 0 if not runs_wavefront(scene.configs, params) else int(max_live if max_live is not None else max(4 * n, 1024))
         if scene.flat.n_capslots and not params.caps_slack:  # family-serial mode: total FIFO entries over all families
             live = max(live, min(64 * max(n, 16), n * (int(params.max_trace_num) + 2)))
         nbytes = lib().optb_workspace_bytes(scene._h, int(rs.n), live)

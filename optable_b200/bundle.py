@@ -146,10 +146,11 @@ class DeviceTrace:
         is a fixed sequence of launches). `replay()` then re-issues it with one driver call; the ray columns, the
         result buffers and the scene blob are read at replay time, so the caller may overwrite the rays in place
         and move components with `scene.update_nodes(flat.refresh(component))` between replays (SURVEY 8f item 3)."""
+        from .backend import runs_wavefront
+
         torch = self.torch
-        has_pass = bool((self.flat.node_i[:, A.NI_INTER] == A.I_PASS).any())   # pass-through leaves run the wavefront variants
-        if self.scene.max_children > 1 or self.prm.chain_len > 0 or self.flat.n_capslots or has_pass:
-            raise NotImplementedError("CUDA-graph replay needs a scene whose interactions emit one ray at most (no host round trips)")
+        if runs_wavefront(self.scene.configs, self.prm):
+            raise NotImplementedError("CUDA-graph replay needs a trace without host round trips (backend.runs_wavefront)")
         self.run(rays_t, max_live)          # warm-up: workspace and kernel attributes exist before the capture
         torch.cuda.synchronize()
         self._graph_rays = rays_t

@@ -28,40 +28,7 @@ using namespace optb;
 
 namespace {
 
-#ifndef OPTB_MIN_BLOCKS
-#define OPTB_MIN_BLOCKS 4
-#endif
-#ifndef OPTB_GRID_WALK
-#define OPTB_GRID_WALK 1   // 0: ignore the lattice descriptors (A/B switch; OPTB_G_GRID nodes are then plain groups)
-#endif
-#ifndef OPTB_BLOCK
-#define OPTB_BLOCK 128
-#endif
-#ifndef OPTB_LANE_REFILL
-#define OPTB_LANE_REFILL 1   // 0: a warp works through one 32-ray chunk at a time in every variant (A/B switch)
-#endif
-#ifndef OPTB_BIG_EXTRA
-#define OPTB_BIG_EXTRA 1   // extra resident CTAs per SM for the variants whose scene tables stay in L1/L2
-#endif
-#ifndef OPTB_CULL_FAR
-#define OPTB_CULL_FAR 1   // 0: boxes are only tested the reference's way, never used to dismiss by distance (A/B switch)
-#endif
-#ifndef OPTB_VOTE_SMEM
-#define OPTB_VOTE_SMEM 0   // 1: the walk of shared-memory scenes also re-converges its lanes with a vote before each leaf test
-#endif
-#ifndef OPTB_PARK_ALWAYS
-#define OPTB_PARK_ALWAYS 0   // 1: every variant parks the radiometric ray state in shared memory during the hit search
-                             // (0: only asphere / lattice variants; measured r2u: c4 115.0 -> 110.8 ms, c3 8.00 -> 7.81)
-#endif
-#ifndef OPTB_WIN_BATCH
-#define OPTB_WIN_BATCH 1   // lattice windows of up to 8 x 8 cells: the cells' box tests as one batch, two at a time
-                           // (ripa 21.45 -> 21.19 ms per 1e6 rays; 0 = one candidate at a time, A/B switch)
-#endif
-#ifndef OPTB_PHASE_SYNC
-#define OPTB_PHASE_SYNC 1   // 0: no per-pop CTA barrier in any variant (A/B switch)
-#endif
-constexpr int kBlock = OPTB_BLOCK;
-constexpr int kResident(int ctas_of_128) { return ctas_of_128 * 128 / kBlock > 0 ? ctas_of_128 * 128 / kBlock : 1; }
+constexpr int kBlock = 128;  // trace_kernel threads per CTA
 constexpr int kTile = 2048;  // children-scan tile (entries per block)
 constexpr int kScanBlock = 256;
 constexpr int kRayF64 = 13;
@@ -229,7 +196,7 @@ OPTB_DEV void sweep_view(const TraceArgs& a, uint32_t root, SceneView& sv) {
 
 // One pop's dead segment: append to the segment log and test it against every monitor (monitor.py:183-193).
 template <bool SWEEP = false>
-OPTB_COLD void emit_segment(const TraceArgs& a, const SceneView& sv, const Ray& r, double seg_len, uint32_t seg_flags,
+OPTB_DEV void emit_segment(const TraceArgs& a, const SceneView& sv, const Ray& r, double seg_len, uint32_t seg_flags,
                            int leaf, unsigned int* s_hist, unsigned int& n_hits_local) {
   if (a.rec_seg) {
     unsigned long long j = warp_alloc(&a.counters[OPTB_C_SEGMENTS]);
@@ -333,10 +300,10 @@ struct HitSearch {
     // a capped surface counts every geometric hit, closest or not (optical_component.py:359-362): no early exit
     const double t_beat = slot >= 0 ? INFINITY : best_t;
     double t;
-    if (OPTB_STAGED_PLANAR && is_planar_kind(ni[OPTB_NI_GEOM])) {
+    if (is_planar_kind(ni[OPTB_NI_GEOM])) {
       t = intersect_planar(sv, ni, nf, ray, t_beat);
     } else {
-      if (!is_planar_kind(ni[OPTB_NI_GEOM])) atomicAdd(cnt + kBlock, 1u);
+      atomicAdd(cnt + kBlock, 1u);
       double ox, oy, oz, dx, dy, dz;
       to_local(nf + OPTB_NF_ORIGIN, nf + OPTB_NF_TINV, ray, ni[OPTB_NI_ORTHO] != 0, ox, oy, oz, dx, dy, dz);
       t = intersect_leaf<ASPH, BRENT>(sv, ni, nf, ox, oy, oz, dx, dy, dz, ray.len, t_beat);
@@ -410,10 +377,8 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
     best_t = hs.best_t; best_node = hs.best_node;
     return;
   }
-  // front-to-back dismissal (slab_hit_far): 1 = in the walk and before a parked test; 2 = asphere variants only before a
-  // parked test (their walks stay as they were)
-  constexpr bool kCullWalk = OPTB_CULL_FAR == 1 || (OPTB_CULL_FAR == 2 && !ASPH);
-  constexpr bool kCullPark = OPTB_CULL_FAR != 0;
+  // Boxes the upload marked cullable are tested with front-to-back dismissal (slab_hit_far), in the walk and before a
+  // parked test.
   unsigned int n_box = 0;
   constexpr int kPark = 4;
   int parked[kPark];
@@ -424,7 +389,7 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
   const BoxRay br(ray.ox, ray.oy, ray.oz, BOXES ? ray.dx : 1.0, BOXES ? ray.dy : 1.0, BOXES ? ray.dz : 1.0);
   // lattice cursor (BOXES = 2): group being listed (-1: none), cell cursor, window, cursor over the extra children
   int g_node = -1, g_i = 0, g_j = 0, g_i1 = -1, g_j0 = 0, g_j1 = -1, g_x = 0;
-  unsigned long long g_mask = 0ull;  // (OPTB_WIN_BATCH) window cells whose box test passed and that are still to be visited
+  unsigned long long g_mask = 0ull;  // window cells whose box test passed and that are still to be visited
   const double* gd = nullptr;
   // Warp-synchronous "walk, then test": in every round each lane walks boxes until it holds a leaf (or runs out of
   // nodes and takes a parked asphere), then the lanes that called in together meet again at the vote and run the
@@ -442,12 +407,12 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
         if (BOXES == 2 && g_node >= 0) {
           // next candidate child of the lattice group: window cells in list order, then the off-lattice children
           int cand;
-          if (OPTB_WIN_BATCH && g_mask) {
+          if (g_mask) {
             // (batched window: the boxes of all window cells were tested when the window was set up)
             const int b = __ffsll((long long)g_mask) - 1;
             g_mask &= g_mask - 1ull;
             cand = (int)gd[OPTB_GRID_CELLS + (g_i + (b >> 3)) * (int)gd[OPTB_GRID_NINNER] + g_j0 + (b & 7)];
-            if (kCullWalk && (*reinterpret_cast<const int*>(sv.trav + cand * 8 + 7) & 2) && hs.best_t < INFINITY &&
+            if ((*reinterpret_cast<const int*>(sv.trav + cand * 8 + 7) & 2) && hs.best_t < INFINITY &&
                 slab_far_only(br, sv.trav + cand * 8, hs.best_t)) continue;
             leaf = cand;
             break;
@@ -464,7 +429,7 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
             continue;
           }
           n_box++;
-          if (kCullWalk && (*reinterpret_cast<const int*>(sv.trav + cand * 8 + 7) & 2)) {
+          if (*reinterpret_cast<const int*>(sv.trav + cand * 8 + 7) & 2) {
             if (slab_hit_far(br, sv.trav + cand * 8, hs.best_t) != 1) continue;
           } else if (!slab_hit(br, sv.trav + cand * 8)) continue;  // the child's own lab box (component_group.py:104-107)
           leaf = cand;  // (lattice children are leaves without interact caps, never aspheres to park: flatten._grid)
@@ -477,7 +442,7 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
           const int word = *reinterpret_cast<const int*>(tv + 7);  // bit 0: test the box; bit 1: may dismiss by distance
           if (word) {
             n_box++;
-            if (kCullWalk && (word & 2)) {
+            if (word & 2) {
               // front to back: a cullable box entered beyond the closest hit so far cannot hold the winner
               if (slab_hit_far(br, tv, hs.best_t) != 1) { i = gs.y; continue; }
             } else if (!slab_hit(br, tv)) { i = gs.y; continue; }
@@ -490,11 +455,12 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
           int i0;
           if (grid_window(gd, ray, i0, g_i1, g_j0, g_j1)) {
             g_node = cur; g_i = i0; g_j = g_j0; g_x = 0;
-            if (OPTB_WIN_BATCH && g_i1 - i0 < 8 && g_j1 - g_j0 < 8 && g_i1 >= i0 && g_j1 >= g_j0) {
+            if (g_i1 - i0 < 8 && g_j1 - g_j0 < 8 && g_i1 >= i0 && g_j1 >= g_j0) {
               // The window's box tests as one batch, two at a time: they are independent (each child's own stored box,
               // component_group.py:104-107), and taken one by one each is a dependent chain of L2 round trips (cell
-              // index -> box -> test -> branch). Bit (row * 8 + column) of g_mask = that cell's box is hit; the walk
-              // then visits the set bits in list order and applies the front-to-back dismissal when it gets to each.
+              // index -> box -> test -> branch; ripa 21.45 -> 21.19 ms per 1e6 rays). Bit (row * 8 + column) of g_mask
+              // = that cell's box is hit; the walk then visits the set bits in list order and applies the front-to-back
+              // dismissal when it gets to each.
               const int nin = (int)gd[OPTB_GRID_NINNER];
               const int total = (g_i1 - i0 + 1) * (g_j1 - g_j0 + 1);
               int ii = i0, jj = g_j0;
@@ -537,7 +503,7 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
           for (int k = 0; k < kPark; k++) if (k == n_done) leaf = parked[k];
           n_done++;
           // parked while the closest cheap hit was not known yet: its box may be out of reach by now
-          if (kCullPark && BOXES && (*reinterpret_cast<const int*>(sv.trav + leaf * 8 + 7) & 2) &&
+          if (BOXES && (*reinterpret_cast<const int*>(sv.trav + leaf * 8 + 7) & 2) &&
               slab_hit_far(br, sv.trav + leaf * 8, hs.best_t) == 2) leaf = -1;
         } else {
           searching = false;
@@ -564,7 +530,7 @@ template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = 
 // Resident CTAs per SM: scenes staged in shared memory are bound by dependent fp64 chains and lose more to the
 // spills of a tighter register budget than they gain from a fifth CTA (measured 6.32 -> 7.62 ms on c2); scenes
 // whose tables stay in L1/L2 (thousands of leaves) are memory-latency bound and gain from it (ripa 30.6 -> 29.8 ms).
-__global__ void __launch_bounds__(kBlock, kResident((SMEM || ASPH || SERIAL) ? OPTB_MIN_BLOCKS : OPTB_MIN_BLOCKS + OPTB_BIG_EXTRA))
+__global__ void __launch_bounds__(kBlock, (SMEM || ASPH || SERIAL) ? 4 : 5)
 trace_kernel(const __grid_constant__ TraceArgs a) {
   constexpr int MAXCH = (SPLIT || SERIAL) ? 2 : 1;
   static_assert(!SWEEP || (!SMEM && !SERIAL && !FLAG && !BRENT), "sweeps run the parallel path from global memory");
@@ -618,12 +584,12 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
   unsigned int c_pops = 0, c_inter = 0, c_drop = 0, c_hits = 0;  // per thread; widened when reduced
 
   while (true) {
-    constexpr bool PHASE = OPTB_PHASE_SYNC && !SERIAL && !FLAG && BOXES != 0 && !ASPH;
+    constexpr bool PHASE = !SERIAL && !FLAG && BOXES != 0 && !ASPH;
     // REFILL: a lane whose ray is finished (its chain ended, or it was a one-pop ray) takes the next ray from the work
     // counter at once instead of idling until the slowest of its warp's 32 rays is done. Chains of a splitting scene end
     // after very different numbers of pops (ripa generation 0: 23.8 of 32 lanes busy on average). The work counter of
     // these variants counts rays, not 32-ray chunks.
-    constexpr bool REFILL = OPTB_LANE_REFILL && PHASE && SPLIT;
+    constexpr bool REFILL = PHASE && SPLIT;
     unsigned int chunk = 0;
     if (lane == 0) chunk = atomicAdd(&a.hdr->work_ctr, REFILL ? 32u : 1u);
     chunk = __shfl_sync(0xffffffffu, chunk, 0);
@@ -710,15 +676,17 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
     auto pop_step = [&]() -> bool {
       if ((long long)ray.pop >= a.max_trace) { c_drop++; nch = 0; return false; }  // queued but never popped
       double t; int node;
-      if constexpr (OPTB_PARK_ALWAYS || ASPH || BOXES == 2) {
+      // Only the asphere and lattice variants park: for the others it measured slower on B200 (c4 110.8 -> 115.0 ms,
+      // c3 7.81 -> 8.00 ms).
+      if constexpr (ASPH || BOXES == 2) {
         volatile double* pk = &s_park[0][threadIdx.x];
         pk[0 * kBlock] = ray.I; pk[1 * kBlock] = ray.wl; pk[2 * kBlock] = ray.qre;
         pk[3 * kBlock] = ray.qim; pk[4 * kBlock] = ray.pl; pk[5 * kBlock] = ray.n;
-        closest_hit<BOXES, ASPH, BRENT, OPTB_VOTE_SMEM || SMEM != 1>(a, sv, ray, solo, t, node, my_cnt);
+        closest_hit<BOXES, ASPH, BRENT, !SMEM>(a, sv, ray, solo, t, node, my_cnt);
         ray.I = pk[0 * kBlock]; ray.wl = pk[1 * kBlock]; ray.qre = pk[2 * kBlock];
         ray.qim = pk[3 * kBlock]; ray.pl = pk[4 * kBlock]; ray.n = pk[5 * kBlock];
       } else {
-        closest_hit<BOXES, ASPH, BRENT, OPTB_VOTE_SMEM || SMEM != 1>(a, sv, ray, solo, t, node, my_cnt);
+        closest_hit<BOXES, ASPH, BRENT, !SMEM>(a, sv, ray, solo, t, node, my_cnt);
       }
       c_pops++;
       if constexpr (FLAG) {
@@ -797,15 +765,7 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
       while (pop_step()) {}
     }
     if constexpr (SPLIT) {
-      if (a.nchild && has) {
-        a.nchild[i] = (uint8_t)nch;
-        uint32_t pb = solo ? ray.pop + 1u : pop_base_next;
-        if (nch > 0) store_child(a.c, 2 * i, ray, ch.ox, ch.oy, ch.oz, ch.pl, ch.dx[0], ch.dy[0], ch.dz[0], ch.I[0],
-                                 ch.qre[0], ch.qim[0], ch.nmed[0], 0, pb, hit_leaf);
-        if (nch > 1) store_child(a.c, 2 * i + 1, ray, ch.ox, ch.oy, ch.oz, ch.pl, ch.dx[MAXCH - 1], ch.dy[MAXCH - 1],
-                                 ch.dz[MAXCH - 1], ch.I[MAXCH - 1], ch.qre[MAXCH - 1], ch.qim[MAXCH - 1],
-                                 ch.nmed[MAXCH - 1], 1, pb, hit_leaf);
-      }
+      if (a.nchild && has) store_children();
     }
   }
 
@@ -1519,6 +1479,41 @@ SerialLayout serial_layout(long long n_rays, long long n_fam, long long ring_ent
   L.total = o;
   return L;
 }
+
+using Kern = void (*)(const TraceArgs);
+// The parallel-path kinds, indexed by [box mode][aspheres][split]; SWEEP: each lane on its root's configuration
+template <bool SMEM, bool SWEEP = false>
+Kern parallel_kernel(int boxmode, bool asph, bool split) {
+#define OPTB_K(B, A, P) trace_kernel<SMEM, false, B, A, P, false, false, false, SWEEP>
+#define OPTB_KROW(B) {{OPTB_K(B, false, false), OPTB_K(B, false, true)}, {OPTB_K(B, true, false), OPTB_K(B, true, true)}}
+  static const Kern k[3][2][2] = {OPTB_KROW(0), OPTB_KROW(1), OPTB_KROW(2)};
+#undef OPTB_KROW
+#undef OPTB_K
+  return k[boxmode][asph ? 1 : 0][split ? 1 : 0];
+}
+// The general kind (box walk, aspheres, split) with one of the options only it carries
+template <bool SERIAL, bool FLAG, bool BRENT, bool PASSK>
+Kern general_kernel(bool smem) {
+  return smem ? trace_kernel<true, SERIAL, 1, true, true, FLAG, BRENT, PASSK>
+              : trace_kernel<false, SERIAL, 1, true, true, FLAG, BRENT, PASSK>;
+}
+// The trace_kernel instantiation that runs a trace. Sweep scenes read their tables from global memory. The
+// family-serial path, the two diagnostics modes (params.reference_roots: brentq_dev roots; params.flag_ambiguity: the
+// A.9 pass at every pop) and pass-through leaves (OPTB_I_PASS) only exist in the general kind.
+Kern select_kernel(const optb_scene* scene, const optb_params* prm, bool serial, bool split) {
+  // box mode: 0 none, 1 pre-order walk with culling, 2 walk + lattice windows (scenes with OPTB_G_GRID groups)
+  const int boxmode = !scene->has_boxes ? 0 : (scene->has_grid ? 2 : 1);
+  const bool smem = scene->in_smem, asph = scene->has_asph;
+  if (scene->n_cfg)
+    return scene->has_pass ? trace_kernel<false, false, 1, true, true, false, false, true, true>
+                           : parallel_kernel<false, true>(boxmode, asph, split);
+  if (prm->reference_roots)
+    return serial ? general_kernel<true, false, true, false>(smem) : general_kernel<false, false, true, false>(smem);
+  if (prm->flag_ambiguity) return general_kernel<false, true, false, false>(smem);
+  if (serial) return general_kernel<true, false, false, false>(smem);
+  if (scene->has_pass) return general_kernel<false, false, false, true>(smem);
+  return smem ? parallel_kernel<true>(boxmode, asph, split) : parallel_kernel<false>(boxmode, asph, split);
+}
 }  // namespace
 
 extern "C" int64_t optb_workspace_bytes(const optb_scene* scene, int64_t n_rays, int64_t max_live) {
@@ -1569,6 +1564,9 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
     return fail(ctx, -7, "scene has interact caps and rays.family is NULL: n_families must be >= rays.n (times n_configs for a sweep)");
   const bool serial = needs_serial(scene, rays, prm);
   if (serial && prm->flag_ambiguity) return fail(ctx, -7, "flag_ambiguity is not available on the family-serial path (binding interact caps)");
+  if (prm->reference_roots && prm->flag_ambiguity) return fail(ctx, -7, "reference_roots and flag_ambiguity are separate diagnostics modes");
+  if (prm->record_hist && scene->n_mons && (!out->hist_y || (zero_hist && !out->hist_yz)))
+    return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
   const bool split = !serial && needs_wavefront(scene, prm);
   WsLayout L = ws_layout(n_roots, 0, false);
   long long cap = 0;
@@ -1611,9 +1609,7 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
 
   CK(cudaMemsetAsync(out->counters, 0, sizeof(int64_t) * OPTB_C_COUNT, st), "memset counters");
   CK(cudaMemsetAsync(hdr, 0, sizeof(Header), st), "memset header");
-  if (prm->record_hist && scene->n_mons && !out->hist_y) return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
   if (prm->record_hist && scene->n_mons && zero_hist) {
-    if (!out->hist_y || !out->hist_yz) return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
     CK(cudaMemsetAsync(out->hist_y, 0, sizeof(int64_t) * OPTB_HIST_BINS * hist_mons(scene), st), "memset hist");
     CK(cudaMemsetAsync(out->hist_yz, 0, sizeof(int64_t) * OPTB_HIST_BINS * OPTB_HIST_BINS * hist_mons(scene), st), "memset hist");
   }
@@ -1643,43 +1639,7 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
     a.gen_last = (uint32_t*)(ws + L.gen_last);
   }
   uint32_t smem = scene->in_smem ? scene->smem_bytes : (a.hist_smem ? scene->smem_bytes : 0);
-  using Kern = void (*)(const TraceArgs);
-  // box mode: 0 none, 1 pre-order walk with culling, 2 walk + lattice windows (scenes with OPTB_G_GRID groups)
-  const int boxmode = !scene->has_boxes ? 0 : ((scene->has_grid && OPTB_GRID_WALK) ? 2 : 1);
-  // [smem][box mode][aspheres][split] for the parallel path; the family-serial path keeps one general variant per
-  // staging mode
-#define OPTB_K(S, B, A, P) trace_kernel<S, false, B, A, P>
-#define OPTB_KROW(S, B) {{OPTB_K(S, B, false, false), OPTB_K(S, B, false, true)}, {OPTB_K(S, B, true, false), OPTB_K(S, B, true, true)}}
-  static const Kern table[2][3][2][2] = {{OPTB_KROW(false, 0), OPTB_KROW(false, 1), OPTB_KROW(false, 2)},
-                                         {OPTB_KROW(true, 0), OPTB_KROW(true, 1), OPTB_KROW(true, 2)}};
-#undef OPTB_KROW
-#undef OPTB_K
-  static const Kern serial_table[2] = {trace_kernel<false, true, 1, true, true>, trace_kernel<true, true, 1, true, true>};
-  // diagnostics (params.flag_ambiguity): the general variant of the parallel path + the A.9 pass at every pop
-  static const Kern flag_table[2] = {trace_kernel<false, false, 1, true, true, true>, trace_kernel<true, false, 1, true, true, true>};
-  Kern kern = serial ? serial_table[scene->in_smem ? 1 : 0]
-                     : table[scene->in_smem ? 1 : 0][boxmode][scene->has_asph ? 1 : 0][split ? 1 : 0];
-  // a pass-through leaf (OPTB_I_PASS) only exists in the general variants: this one, or the three kinds below
-  static const Kern pass_table[2] = {trace_kernel<false, false, 1, true, true, false, false, true>,
-                                     trace_kernel<true, false, 1, true, true, false, false, true>};
-  if (scene->has_pass && !serial) kern = pass_table[scene->in_smem ? 1 : 0];
-  if (prm->flag_ambiguity) kern = flag_table[scene->in_smem ? 1 : 0];
-  // sweep scenes: the same production kinds, each lane on its root's configuration (tables in global memory)
-#define OPTB_K(B, A, P) trace_kernel<false, false, B, A, P, false, false, false, true>
-#define OPTB_KROW(B) {{OPTB_K(B, false, false), OPTB_K(B, false, true)}, {OPTB_K(B, true, false), OPTB_K(B, true, true)}}
-  static const Kern sweep_table[3][2][2] = {OPTB_KROW(0), OPTB_KROW(1), OPTB_KROW(2)};
-#undef OPTB_KROW
-#undef OPTB_K
-  if (scene->n_cfg)
-    kern = scene->has_pass ? trace_kernel<false, false, 1, true, true, false, false, true, true>
-                           : sweep_table[boxmode][scene->has_asph ? 1 : 0][split ? 1 : 0];
-  // params.reference_roots: the general variants with brentq_dev (parallel and family-serial)
-  static const Kern brent_table[2][2] = {{trace_kernel<false, false, 1, true, true, false, true>, trace_kernel<true, false, 1, true, true, false, true>},
-                                         {trace_kernel<false, true, 1, true, true, false, true>, trace_kernel<true, true, 1, true, true, false, true>}};
-  if (prm->reference_roots) {
-    if (prm->flag_ambiguity) return fail(ctx, -7, "reference_roots and flag_ambiguity are separate diagnostics modes");
-    kern = brent_table[serial ? 1 : 0][scene->in_smem ? 1 : 0];
-  }
+  const Kern kern = select_kernel(scene, prm, serial, split);
   CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<uint32_t>(smem, 1024)), "smem attr");
   int occ = 1;
   CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kBlock, smem), "occupancy");
@@ -1800,10 +1760,7 @@ static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_ra
 static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
                                 optb_result* out) {
   cudaSetDevice(ctx->device);
-#ifndef OPTB_HOST_CHUNK
-#define OPTB_HOST_CHUNK (1 << 20)
-#endif
-  constexpr int64_t kChunk = OPTB_HOST_CHUNK;
+  constexpr int64_t kChunk = 1 << 20;  // rays per chunk
   const int64_t n = rays->n;
   const int nch = (int)((n + kChunk - 1) / kChunk);
   const int64_t segcap = prm->record_segments ? out->seg_capacity : 0, hitcap = prm->record_hits ? out->hit_capacity : 0;

@@ -10,27 +10,10 @@
 #include <stdint.h>
 #include "../../include/optb.h"
 
+// Everything is inlined, the once-per-pop physics and segment code included (measured on B200: 10 % faster than
+// __noinline__ calls for those). Deciding the special operands of divisions (1/0, 0/x, x/inf) up front measured
+// slower or equal on B200 (DESIGN.md §4), so the divisions below are plain.
 #define OPTB_DEV __device__ __forceinline__
-#ifndef OPTB_CH_REGS
-#define OPTB_CH_REGS 0   // 1: Children slots written through selects (registers) instead of indexed stores (local
-                         // memory). Measured on B200 (r2a): no difference on c2/c3/c4; 0 has fewer spills
-#endif
-// bit 0/3: BoxRay skips 1/0 on parallel axes; bit 1: cdiv decides 0/x itself; bit 2: x/inf of planar ROC terms decided
-// up front. Each removes a ~70-instruction special-operand division path from most pops of the benchmark scenes, and
-// each measured slower or equal on B200 (c2 -1..+3 %, c3 +0.4..+4 %, c4 +1.4 %, ripa -2 %): off.
-#ifndef OPTB_DIVSP
-#define OPTB_DIVSP 0
-#endif
-#ifndef OPTB_STAGED_PLANAR
-#define OPTB_STAGED_PLANAR 1  // planar leaves: x row of Tinv first (intersect_planar) instead of a full to_local
-#endif
-// cold, register-hungry code (once per pop) is kept out of line so that the closest-hit loop gets the registers
-// (measured on B200: keeping them inline is 10 % faster than __noinline__ calls; -DOPTB_NOINLINE_COLD flips it)
-#ifdef OPTB_NOINLINE_COLD
-#define OPTB_COLD __device__ __noinline__
-#else
-#define OPTB_COLD __device__ __forceinline__
-#endif
 
 namespace optb {
 
@@ -118,9 +101,7 @@ struct BoxRay {
     for (int ax = 0; ax < 3; ax++) {
       par[ax] = fabs(d[ax]) <= 1e-8;
       any_par |= par[ax];
-      // (a parallel axis never reads inv; 1/0 would take the division's ~70-instruction special-operand path on
-      // every pop of an axis-aligned beam)
-      inv[ax] = (OPTB_DIVSP & 8) ? 1.0 / (par[ax] ? 1.0 : d[ax]) : ((OPTB_DIVSP & 1) && par[ax]) ? 0.0 : 1.0 / d[ax];
+      inv[ax] = 1.0 / d[ax];
       near[ax] = inv[ax] < 0.0 ? 1 : 0;
     }
   }
@@ -551,25 +532,7 @@ OPTB_DEV double intersect_leaf(const SceneView& sv, const int32_t* __restrict__ 
   // only ever reports roots inside its bracket [a, b], so a bracket that starts beyond t_beat is skipped whole.
   const int g = ni[OPTB_NI_GEOM];
   const double* p = nf + OPTB_NF_P;
-#if !OPTB_STAGED_PLANAR
-  if (is_planar_kind(g)) {
-    // planar branch :165-196: plane x = 0
-    if (!((ox < 0.0 && dx > 0.0) || (ox > 0.0 && dx < 0.0))) return -1.0;
-    double t = -ox / dx;
-    if (!(t >= 1e-9) || t > len) return -1.0;  // |t|<EPS, t<0, t>length, NaN
-    double Px = fma(t, dx, ox), Py = fma(t, dy, oy), Pz = fma(t, dz, oz);
-    bool in;
-    if (g == OPTB_G_CSG) {
-      in = csg_within(sv, ni, p, Px, Py, Pz);
-    } else if (g == OPTB_G_POLY2D) {
-      in = poly_within(sv.aux + ni[OPTB_NI_AUX], Px, Py, Pz);
-    } else {
-      in = planar_within(sv, g, p[0], p[1], Px, Py, Pz);
-    }
-    return in ? t : -1.0;
-  }
-#endif
-  // (with OPTB_STAGED_PLANAR planar kinds never get here: intersect_planar)
+  // (planar kinds never get here: intersect_planar)
   // curved branch :197-233. Local AABB (Surface.get_bbox_local) -> bracket -> 10-point sign scan -> roots.
   double bb[6];
   if (g == OPTB_G_SPHERE) {
@@ -776,20 +739,10 @@ OPTB_DEV double material_n_cached(const SceneView& sv, const IndexCache& c, int 
   return n;
 }
 
-// num / den, bit for bit, with the two special-operand cases the path meets all the time decided up front: 0 / x (the
-// imaginary part of a planar interface's ABCD denominator) and x / inf (curvature terms of a planar surface, ROC = inf).
-// The hardware division handles them in a ~70-instruction out-of-line path; the result is a zero with the XOR of the signs.
-OPTB_DEV double div_special(double num, double den) {
-  const bool zero_num = (num == 0.0) && (den != 0.0) && (fabs(den) < INFINITY);
-  const bool inf_den = (fabs(den) == INFINITY) && (fabs(num) < INFINITY);
-  if (zero_num || inf_den) return copysign(0.0, num) * copysign(1.0, den);
-  return num / den;
-}
-
 // numpy complex128 division (Smith)
 OPTB_DEV void cdiv(double a, double b, double c, double d, double& re, double& im) {
   if (fabs(c) >= fabs(d)) {
-    double r = (OPTB_DIVSP & 2) ? div_special(d, c) : d / c, den = fma(d, r, c);
+    double r = d / c, den = fma(d, r, c);
     double id = 1.0 / den;
     re = fma(b, r, a) * id; im = fma(-a, r, b) * id;
   } else {
@@ -807,16 +760,11 @@ struct Children {
   double ox, oy, oz;    // lab origin
   double pl;            // _pathlength of the children
   double dx[N], dy[N], dz[N], I[N], qre[N], qim[N], nmed[N];
-  // slot k with k a run-time value: written as selects so that the arrays stay in registers
+  // slot k with k a run-time value: an indexed store (writing it through selects to keep the arrays in registers
+  // measured no faster on B200 and spilled more)
   OPTB_DEV void set(int k, double ax, double ay, double az, double i, double qr, double qi, double nm) {
-#if OPTB_CH_REGS
-#pragma unroll
-    for (int j = 0; j < N; j++)
-      if (j == k) { dx[j] = ax; dy[j] = ay; dz[j] = az; I[j] = i; qre[j] = qr; qim[j] = qi; nmed[j] = nm; }
-#else
     if (N == 1) k = 0;
     dx[k] = ax; dy[k] = ay; dz[k] = az; I[k] = i; qre[k] = qr; qim[k] = qi; nmed[k] = nm;
-#endif
   }
 };
 
@@ -836,7 +784,7 @@ OPTB_DEV void dir_to_lab(const double* __restrict__ T, bool ortho, double lx, do
 
 // interact_local bodies for the winning leaf. (ox..dz) is the ray in the leaf's local frame, t the hit parameter.
 template <bool ASPH, int N, bool PASSK>
-OPTB_COLD void interact(const SceneView& sv, const int32_t* __restrict__ ni, const double* __restrict__ nf,
+OPTB_DEV void interact(const SceneView& sv, const int32_t* __restrict__ ni, const double* __restrict__ nf,
                        const Ray& ray, double unit, double ox, double oy, double oz, double dx, double dy, double dz,
                        double t, Children<N>& ch, const IndexCache& ic) {
   const double* T = nf + OPTB_NF_T;
@@ -913,11 +861,11 @@ OPTB_COLD void interact(const SceneView& sv, const int32_t* __restrict__ ni, con
   if (hasq) {  // ABCD of the refraction / of the reflection (:648-666); each only when a child will carry it
     double qr = ray.qre + t, qi = ray.qim;
     if (sin_t < 1 && trans > 0) {
-      double Cc = (OPTB_DIVSP & 4) ? div_special(nin - nout, ROC * nout) : (nin - nout) / (ROC * nout);
+      double Cc = (nin - nout) / (ROC * nout);
       cdiv(qr, qi, fma(Cc, qr, ratio), Cc * qi, qtr, qti);
     }
     if (!(sin_t < 1) || want_refl) {
-      double C2 = (OPTB_DIVSP & 4) ? div_special(2.0, ROC) : 2.0 / ROC;
+      double C2 = 2.0 / ROC;
       cdiv(qr, qi, fma(C2, qr, 1.0), C2 * qi, qrr, qri);
     }
   }

@@ -16,6 +16,7 @@ Flatten map = SURVEY.md Appendix D. What is read, and where the reference define
 from __future__ import annotations
 
 import ctypes as C
+import functools
 import math
 import os
 
@@ -178,6 +179,11 @@ class FlatScene:
         self.n_materials = int(self.mat_kind.shape[0])  # >= 1 (a dummy row when nothing refracts)
         self.n_monitors = len(self.monitors)
         self.n_capslots = len(self.capslots)
+
+    @functools.cached_property
+    def has_pass(self) -> bool:
+        """Some leaf hands every ray that reaches it back unchanged (A.I_PASS: a Monitor listed as a component)."""
+        return bool((self.node_i[:, A.NI_INTER] == A.I_PASS).any())
 
     def _finish_inverses(self):
         if self._pending_inv:

@@ -404,3 +404,52 @@ def test_gui_loop_refresh_update_nodes_and_graph_replay():
             assert torch.equal(torch.sort(live.t[col][:nh]).values, torch.sort(fresh.t[col][:nh]).values), col
         fresh.close()
     live.close()
+
+
+def test_rejected_option_combinations_enqueue_nothing():
+    """Option combinations the library refuses fail with -7 and their message before anything is enqueued: the
+    caller's counters are left as they were."""
+    import re
+
+    import torch
+
+    from optable_b200.backend import BackendError, Engine
+    from optable_b200.bundle import DeviceTrace, RayBundle
+    from optable_b200.flatten import FlatScene
+
+    engine = Engine.get(0)
+    n = 64
+    rays = RayBundle.collimated_disc(n, radius=2.5).to_torch(device="cuda:0")
+    root_flags = torch.zeros(n, dtype=torch.int32, device="cuda:0")
+    sc = scenes.telescope_4f(ob, n_rays=0)
+    flat = FlatScene(sc.components, sc.monitors)
+    caps = scenes.caps_binding(ob)
+
+    def refused(scene, msg, rays_t=rays, **kw):
+        res, t = engine.alloc_result(scene, 0, 0, n * scene.n_configs)
+        res.root_flags = root_flags.data_ptr()
+        t["counters"].fill_(-1)
+        prm = engine.make_params(80, record_segments=False, record_hits=False, n_families=n * scene.n_configs, **kw)
+        with pytest.raises(BackendError, match=re.escape(f"liboptb error -7: {msg}")):
+            engine.trace_device(scene, rays_t, prm, res)
+        torch.cuda.synchronize()
+        assert (t["counters"] == -1).all()
+
+    single, sweep, capped = engine.upload(flat), engine.upload_sweep([flat, flat]), engine.upload(FlatScene(caps.components, caps.monitors))
+    refused(single, "reference_roots and flag_ambiguity are separate diagnostics modes", reference_roots=True, flag_ambiguity=True)
+    sweep_msg = "sweep: flag_ambiguity and reference_roots are not available on sweep scenes"
+    refused(sweep, sweep_msg, flag_ambiguity=True)
+    refused(sweep, sweep_msg, reference_roots=True)
+    refused(sweep, "sweep: rays.family must be NULL (every root is its own family)",
+            rays_t=dict(rays, family=torch.arange(n, dtype=torch.int32, device="cuda:0")))
+    refused(capped, "flag_ambiguity is not available on the family-serial path (binding interact caps)", flag_ambiguity=True)
+    for s in (single, sweep, capped):
+        s.close()
+    # the graph capture of a flag_ambiguity trace (one host round trip per generation) is refused before it begins
+    dt = DeviceTrace(engine, flat, n, 2 * n + 64, flag_ambiguity=True)
+    dt.t["counters"].fill_(-1)
+    with pytest.raises(NotImplementedError):
+        dt.capture(rays)
+    assert not torch.cuda.is_current_stream_capturing()
+    assert (dt.t["counters"] == -1).all()   # not even the warm-up run
+    dt.close()
