@@ -421,6 +421,11 @@ enum {
   OPTB_MS_COUNT = 0, OPTB_MS_SUM_I = 1, OPTB_MS_SUM_Y = 2, OPTB_MS_SUM_YY = 3, OPTB_MS_SUM_Z = 4, OPTB_MS_SUM_ZZ = 5,
   OPTB_MS_SUM_WD = 6, OPTB_MS_MIN_Y = 7, OPTB_MS_MAX_Y = 8, OPTB_MS_MIN_Z = 9, OPTB_MS_MAX_Z = 10,
   OPTB_MS_SUM_TY = 11, OPTB_MS_SUM_TYTY = 12,
+  /* sums of (y - mean_y)^2, (z - mean_z)^2, (tY - mean_tY)^2 over the selected rows, taken in a second pass about the
+   * means of the first (std_y = sqrt(M2_Y / count) keeps full precision where SUM_YY / count - mean_y^2 cancels, e.g.
+   * a small spot far off the monitor's axis). M2_TY is 0 without hit_dx..dz. Added in slots that were unused before,
+   * without a change of OPTB_ABI_VERSION: no struct changed.                                                      */
+  OPTB_MS_M2_Y = 13, OPTB_MS_M2_Z = 14, OPTB_MS_M2_TY = 15,
   OPTB_MS_HIST = 16, /* 30 counts */
   OPTB_MS_STRIDE = 48
 };

@@ -96,5 +96,5 @@ class MonitorFrame(C.Structure):
 
 
 (MS_COUNT, MS_SUM_I, MS_SUM_Y, MS_SUM_YY, MS_SUM_Z, MS_SUM_ZZ, MS_SUM_WD, MS_MIN_Y, MS_MAX_Y, MS_MIN_Z, MS_MAX_Z,
- MS_SUM_TY, MS_SUM_TYTY) = range(13)
+ MS_SUM_TY, MS_SUM_TYTY, MS_M2_Y, MS_M2_Z, MS_M2_TY) = range(16)
 MS_HIST, MS_STRIDE = 16, 48

@@ -81,7 +81,7 @@ class DeviceMonitor:
             self._stats = {
                 "count": int(s[A.MS_COUNT]), "sum_intensity": float(s[A.MS_SUM_I]), "avg_intensity": float(s[A.MS_SUM_I] / n),
                 "mean_y": float(my), "mean_z": float(mz),
-                "std_y": float(np.sqrt(max(s[A.MS_SUM_YY] / n - my * my, 0.0))), "std_z": float(np.sqrt(max(s[A.MS_SUM_ZZ] / n - mz * mz, 0.0))),
+                "std_y": float(np.sqrt(s[A.MS_M2_Y] / n)), "std_z": float(np.sqrt(s[A.MS_M2_Z] / n)),
                 "min_y": float(s[A.MS_MIN_Y]), "max_y": float(s[A.MS_MAX_Y]), "min_z": float(s[A.MS_MIN_Z]), "max_z": float(s[A.MS_MAX_Z]),
                 "mean_waist_distance": float(s[A.MS_SUM_WD] / n), "mean_tY": float(s[A.MS_SUM_TY] / n),
                 "hist_y": s[A.MS_HIST:A.MS_HIST + A.HIST_BINS].astype(np.int64),

@@ -2322,6 +2322,40 @@ __global__ void __launch_bounds__(256) monitor_stats_kernel(const StatsArgs a) {
   __syncthreads();
   if (threadIdx.x < OPTB_HIST_BINS && s_hist[threadIdx.x]) atomicAdd(&a.stats[OPTB_MS_HIST + threadIdx.x], (double)s_hist[threadIdx.x]);
 }
+// Second pass: sums of squares about the means the first pass left in `stats`. sum_yy / n - mean^2 cancels for a spot
+// far off axis (|mean| / std = 1e4 already loses 8 digits); centred sums keep the spread to rounding.
+__global__ void __launch_bounds__(256) monitor_m2_kernel(const StatsArgs a) {
+  __shared__ double s_red[3][8];
+  const double n = a.stats[OPTB_MS_COUNT];
+  if (n == 0.0) return;
+  const double my = a.stats[OPTB_MS_SUM_Y] / n, mz = a.stats[OPTB_MS_SUM_Z] / n, mty = a.stats[OPTB_MS_SUM_TY] / n;
+  double v[3] = {0.0, 0.0, 0.0};
+  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < a.n; k += (long long)gridDim.x * blockDim.x) {
+    const long long j = a.first + k;
+    if (a.monitor >= 0 && (a.mon ? a.mon[j] != a.monitor : (int)((a.key[j] >> 24) & 0xffu) != a.monitor)) continue;
+    const double Px = a.px[j], Py = a.py[j], Pz = a.pz[j];
+    const double y = dot3(Px, Py, Pz, a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]) - my;
+    const double z = dot3(Px, Py, Pz, a.f.tangent_z[0], a.f.tangent_z[1], a.f.tangent_z[2]) - mz;
+    v[0] = fma(y, y, v[0]); v[1] = fma(z, z, v[1]);
+    if (a.dx) {
+      const double ty = dot3(a.dx[j], a.dy[j], a.dz[j], a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]) - mty;
+      v[2] = fma(ty, ty, v[2]);
+    }
+  }
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int q = 0; q < 3; q++) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
+    if (lane == 0) s_red[q][wid] = v[q];
+  }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    double tot = 0;
+    for (int w = 0; w < 8; w++) tot += s_red[threadIdx.x][w];
+    if (tot != 0.0) atomicAdd(&a.stats[OPTB_MS_M2_Y + threadIdx.x], tot);
+  }
+}
 }  // namespace
 
 extern "C" int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_t first, int64_t n, int monitor,
@@ -2345,6 +2379,7 @@ extern "C" int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_
   if (n > 0) {
     const int grid = (int)std::min<long long>((n + 255) / 256, (long long)ctx->sm_count * 8);
     monitor_stats_kernel<<<grid, 256, 0, st>>>(a);
+    monitor_m2_kernel<<<grid, 256, 0, st>>>(a);
   }
   CK(cudaGetLastError(), "monitor_stats_kernel");
   return 0;

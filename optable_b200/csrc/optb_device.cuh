@@ -897,13 +897,15 @@ OPTB_DEV void interact(const SceneView& sv, const int32_t* __restrict__ ni, cons
 
 // np.histogram(x, bins=30, range=(lo, hi)) bin index, -1 outside
 // (norm = nb / (hi - lo) and step = (hi - lo) / nb depend on the monitor only: the upload precomputes them)
+// The edges are np.linspace's: i * step and + lo each rounded, the last edge = hi. A fused i * step + lo differs from
+// them by one ulp at many interior edges and would put a value on such an edge into the neighbouring bin.
 OPTB_DEV int hist_bin(double x, double lo, double hi, double norm, double step) {
   const int nb = OPTB_HIST_BINS;
   if (!(x >= lo && x <= hi)) return -1;
   int idx = (int)((x - lo) * norm);
   if (idx == nb) idx = nb - 1;
-  double e0 = fma((double)idx, step, lo);
-  double e1 = (idx + 1 == nb) ? hi : fma((double)(idx + 1), step, lo);
+  double e0 = __dadd_rn(__dmul_rn((double)idx, step), lo);
+  double e1 = (idx + 1 == nb) ? hi : __dadd_rn(__dmul_rn((double)(idx + 1), step), lo);
   if (x < e0) idx--;
   else if (x >= e1 && idx != nb - 1) idx++;
   return idx;

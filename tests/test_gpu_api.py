@@ -252,6 +252,10 @@ def test_device_monitor_analytics_match_host_monitor(tmp_path):
         counts, _ = host._get_hist_y()
         np.testing.assert_array_equal(dm._get_hist_y()[0], counts)           # the fused kernel's own binning
         np.testing.assert_array_equal(out["hist_y"][m].cpu().numpy(), counts)  # = the histogram the trace accumulated
+        y, z = dm.get_yList(sort=None).cpu().numpy(), dm.get_zList(sort=None).cpu().numpy()
+        hw, hh = float(mon.width) / 2, float(mon.height) / 2
+        want2 = np.histogram2d(y, z, 30, [[-hw, hw], [-hh, hh]])[0].astype(np.int64)
+        np.testing.assert_array_equal(out["hist_yz"][m].cpu().numpy(), want2)
         dy, dz = dm.get_delta_pos()
         hy, hz = host.get_delta_pos()
         np.testing.assert_allclose(dy.cpu().numpy(), hy, rtol=0, atol=1e-15)

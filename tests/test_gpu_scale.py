@@ -111,9 +111,11 @@ def test_full_size_properties_c2(engine):
     assert int(dt.t["hist_y"].sum()) == nh
     for m in (0, 1):
         sel = mon == m
-        h = torch.histc(py[sel], bins=30, min=-2.5, max=2.5)
-        # bin edges are not exactly representable: allow the few rows that sit within rounding of an edge
-        assert int((h.to(torch.int64) - dt.t["hist_y"][m]).abs().sum()) <= 4
+        mf = flat.mon_f[m]
+        assert list(mf[A.MON_TY:A.MON_TY + 3]) == [0.0, 1.0, 0.0]   # unrotated: the histogram's y is hit_py itself
+        hw = float(mf[A.MON_HW])
+        want = np.histogram(py[sel].cpu().numpy(), bins=30, range=(-hw, hw))[0]
+        np.testing.assert_array_equal(dt.t["hist_y"][m].cpu().numpy(), want, err_msg=f"monitor {m}")
     # a 4f relay images the input plane inverted: monitor-1 position = -input position within aberrations
     r1 = dt.t["hit_root"][:nh][mon == 1].long()
     assert float((py[mon == 1] + oy[r1]).abs().max()) < 0.05 and float((pz[mon == 1] + oz[r1]).abs().max()) < 0.05
