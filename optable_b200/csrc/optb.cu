@@ -976,7 +976,7 @@ struct optb_ctx {
   void* arena; size_t arena_bytes;
   unsigned long long* h_counters;  // pinned
   unsigned int* h_hdr;             // pinned
-  cudaStream_t s_h2d, s_run, s_d2h;  // pipelined optb_trace_host
+  cudaStream_t s_h2d, s_run, s_d2h;  // optb_trace_host
   unsigned long long* h_chunk; size_t h_chunk_n;  // pinned per-chunk counters
   // Retired scene blobs, kept for the next upload: cudaMalloc/cudaFree cost milliseconds each (and cudaFree
   // synchronises the device), which is most of the latency of a small trace that re-uploads its scene per call.
@@ -1017,8 +1017,6 @@ extern "C" int64_t optb_sort_workspace_bytes(int64_t n_rows);
 static int sort_rows_dev(optb_ctx* ctx, const optb_result* res, const optb_result* dst, int64_t n_seg, int64_t n_hit,
                          const unsigned long long* d_counters, void* workspace, int64_t workspace_bytes, cudaStream_t st,
                          int end_bit);
-extern "C" int optb_sort_rows(optb_ctx* ctx, const optb_result* res, int64_t n_seg, int64_t n_hit, void* workspace,
-                              int64_t workspace_bytes, void* stream_v);
 
 extern "C" int optb_ctx_create(int device, optb_ctx** out) {
   if (!out) return -1;
@@ -1743,30 +1741,40 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
 }
 
 namespace {
+// Bump allocator over the optb_trace_host arena. With no base it only measures: the same carve run once without a
+// base and once over an arena of the measured size takes the same offsets.
 struct ArenaCursor {
-  unsigned char* base; size_t off, cap;
-  void* take(size_t bytes) { size_t o = align_up(off, 256); off = o + bytes; return off <= cap ? base + o : nullptr; }
+  unsigned char* base; size_t off;
+  void* take(size_t bytes) { size_t o = align_up(off, 256); off = o + bytes; return base ? base + o : nullptr; }
 };
 }  // namespace
 
-static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
-                           optb_result* out, int64_t live);
-
-// Chunked, three-stream version of optb_trace_host for scenes that cannot split: the host->device copy of chunk
-// c+1, the trace of chunk c and the device->host copy of chunk c-1 overlap (PCIe is full duplex). Rows of chunk c
-// land behind the rows of chunks < c, so the host result is the same set of rows as the one-shot path; row keys
-// stay global through root_base. Returns 1 when a chunk overflowed its (estimated) device capacity: the caller
-// then repeats the whole batch on the one-shot path.
-static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
-                                optb_result* out) {
+// optb_trace_host in chunks of `chunk` rays over three streams: the host->device copy of chunk c+1, the trace of
+// chunk c and the device->host copy of chunk c-1 overlap (PCIe is full duplex). Rows of chunk c land behind the rows
+// of chunks < c; row keys stay global through root_base. chunk >= rays.n is the one-shot trace: one result set of the
+// caller's capacity, nothing overlapped. `live`: the live-ray budget of a splitting scene. Returns 1 when one of
+// several chunks overflowed its (estimated) share of the result capacity: the caller then repeats the whole batch as
+// one chunk.
+static int trace_host(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
+                      optb_result* out, int64_t chunk, int64_t live) {
   cudaSetDevice(ctx->device);
-  constexpr int64_t kChunk = 1 << 20;  // rays per chunk
-  const int64_t n = rays->n;
-  const int nch = (int)((n + kChunk - 1) / kChunk);
+  const int64_t n = rays->n, n_roots = n * std::max(scene->n_cfg, 1);
+  const int nch = chunk >= n ? 1 : (int)((n + chunk - 1) / chunk);
+  const bool chunked = nch > 1;
   const int64_t segcap = prm->record_segments ? out->seg_capacity : 0, hitcap = prm->record_hits ? out->hit_capacity : 0;
-  auto chunk_cap = [&](int64_t total) { return total ? std::min<int64_t>(total, (int64_t)((double)total * kChunk / n * 1.25) + 4096) : 0; };
+  auto chunk_cap = [&](int64_t total) { return chunked && total ? std::min<int64_t>(total, (int64_t)((double)total * chunk / n * 1.25) + 4096) : total; };
   const int64_t cseg = chunk_cap(segcap), chit = chunk_cap(hitcap);
-  const int64_t wsb = (int64_t)ws_layout(kChunk, 0, false).total;
+  const bool serial = needs_serial(scene, rays, prm), split = needs_wavefront(scene, prm) || serial;
+  const int64_t croots = std::min(chunk, n) * std::max(scene->n_cfg, 1);  // roots of the largest chunk
+  const int64_t wsb = serial ? optb_workspace_bytes(scene, n, 16 * std::max<int64_t>(live, 64))
+                             : (int64_t)ws_layout(croots, split ? std::max(live, croots) : 0, split).total;
+  // sorted_rows: one chunk is sorted in place once its row counts are known; several chunks are each gathered into a
+  // sorted copy right behind their trace, so that the copy back never waits for a later chunk's trace
+  const bool sorted = prm->sorted_rows != 0, gather = sorted && chunked;
+  const int64_t sortb = sorted ? optb_sort_workspace_bytes(std::max(cseg, chit)) : 0;
+  const bool hist = prm->record_hist && scene->n_mons;
+  const size_t hy = (size_t)hist_mons(scene) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
+  const size_t capb = (size_t)scene->n_caps * std::max(prm->n_families, 1) * 4;
   if (!ctx->s_h2d) {
     CK(cudaStreamCreateWithFlags(&ctx->s_h2d, cudaStreamNonBlocking), "stream");
     CK(cudaStreamCreateWithFlags(&ctx->s_run, cudaStreamNonBlocking), "stream");
@@ -1778,49 +1786,39 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
     CK(cudaMallocHost((void**)&ctx->h_chunk, sizeof(unsigned long long) * OPTB_C_COUNT * nch), "pinned counters");
     ctx->h_chunk_n = nch;
   }
-  const int64_t sortb = prm->sorted_rows ? optb_sort_workspace_bytes(std::max(cseg, chit)) : 0;
-  size_t need = 256 * 128 + (size_t)n * (8 * 13 + 8) + (prm->sorted_rows ? 4 : 2) * ((size_t)cseg * (13 * 8 + 16) + (size_t)chit * (10 * 8 + 12 + 8) + 40 * 256) +
-                (size_t)std::max(scene->n_mons, 1) * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 8 + 2 * (64 * 8 + (size_t)wsb) +
-                (size_t)sortb + 4096;
-  if (ctx->arena_bytes < need) {
-    if (ctx->arena) cudaFree(ctx->arena);
-    ctx->arena = nullptr; ctx->arena_bytes = 0;
-    CK(cudaMalloc(&ctx->arena, need), "cudaMalloc(arena)");
-    ctx->arena_bytes = need;
-  }
-  ArenaCursor ac{(unsigned char*)ctx->arena, 0, ctx->arena_bytes};
-  // full-length device input columns; chunks are slices of them
+  // full-length device input columns (chunks are slices of them); dev: the result sets the traces of even / odd
+  // chunks append to; srt: their sorted copies
   optb_rays dr = *rays;
   const double* const* src_f = &rays->ox;
   const double** dst_f = &dr.ox;
-  for (int f = 0; f < kRayF64; f++) {
-    if (!src_f[f]) { dst_f[f] = nullptr; continue; }
-    const size_t rows = ((rays->broadcast >> f) & 1u) ? 1 : (size_t)n;
-    dst_f[f] = (const double*)ac.take(rows * 8);
-    if (!dst_f[f]) return fail(ctx, -9, "arena sizing");
-    if (rows == 1) CK(cudaMemcpyAsync((void*)dst_f[f], src_f[f], 8, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D rays");
-  }
-  if (rays->flags) dr.flags = (const uint32_t*)ac.take((size_t)n * 4);
-  if (rays->family) dr.family = (const int32_t*)ac.take((size_t)n * 4);
-  // dev: the two result sets the traces of even / odd chunks append to; srt (sorted_rows): the same rows in reference
-  // order, gathered there right behind the trace, so that the copy back never waits for a later chunk's trace
-  struct Col { void* dev[2]; void* srt[2]; unsigned char* host; size_t elt; int kind; };
+  struct Col { void* dev[2]; void* srt[2]; unsigned char* host; size_t elt; int kind; };  // kind 0 seg, 1 hit
   std::vector<Col> cols;
   optb_result dv[2] = {*out, *out}, sv[2] = {*out, *out};
-  const bool sorted = prm->sorted_rows != 0;
-  auto add = [&](size_t field_off, void* host_ptr, size_t elt, int64_t capn, int kind) {
-    for (int s = 0; s < 2; s++) *(void**)((unsigned char*)&dv[s] + field_off) = *(void**)((unsigned char*)&sv[s] + field_off) = nullptr;
-    if (!host_ptr || capn == 0) return;
-    Col c{{ac.take((size_t)capn * elt), ac.take((size_t)capn * elt)}, {nullptr, nullptr}, (unsigned char*)host_ptr, elt, kind};
-    if (sorted) { c.srt[0] = ac.take((size_t)capn * elt); c.srt[1] = ac.take((size_t)capn * elt); }
-    for (int s = 0; s < 2; s++) {
-      *(void**)((unsigned char*)&dv[s] + field_off) = c.dev[s];
-      *(void**)((unsigned char*)&sv[s] + field_off) = c.srt[s];
-    }
-    cols.push_back(c);
-  };
+  int64_t *d_hy = nullptr, *d_hyz = nullptr;
+  int32_t* d_caps = nullptr;
+  void* ws[2] = {nullptr, nullptr};
+  void* sort_ws = nullptr;
+  for (int pass = 0; pass < 2; pass++) {  // pass 0 measures the carve, pass 1 takes it from an arena of that size
+    ArenaCursor ac{pass ? (unsigned char*)ctx->arena : nullptr, 0};
+    for (int f = 0; f < kRayF64; f++)
+      dst_f[f] = src_f[f] ? (const double*)ac.take((((rays->broadcast >> f) & 1u) ? 1 : (size_t)n) * 8) : nullptr;
+    if (rays->flags) dr.flags = (const uint32_t*)ac.take((size_t)n * 4);
+    if (rays->family) dr.family = (const int32_t*)ac.take((size_t)n * 4);
+    cols.clear();
+    auto add = [&](size_t field_off, void* host_ptr, size_t elt, int64_t capn, int kind) {
+      Col c{{nullptr, nullptr}, {nullptr, nullptr}, (unsigned char*)host_ptr, elt, kind};
+      const bool want = host_ptr && capn;
+      for (int s = 0; s < (chunked ? 2 : 1) && want; s++) {
+        c.dev[s] = ac.take((size_t)capn * elt);
+        if (gather) c.srt[s] = ac.take((size_t)capn * elt);
+      }
+      for (int s = 0; s < 2; s++) {
+        *(void**)((unsigned char*)&dv[s] + field_off) = c.dev[s];
+        *(void**)((unsigned char*)&sv[s] + field_off) = c.srt[s];
+      }
+      if (want) cols.push_back(c);
+    };
 #define OPTB_FIELD(name) offsetof(optb_result, name), (void*)out->name
-  {
     const size_t seg0 = offsetof(optb_result, seg_ox), hit0 = offsetof(optb_result, hit_px);
     double* const* seg_h = &out->seg_ox; double* const* hit_h = &out->hit_px;
     for (int f = 0; f < 13; f++) add(seg0 + 8 * f, seg_h[f], 8, cseg, 0);
@@ -1829,34 +1827,41 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
     add(OPTB_FIELD(hit_monitor), 4, chit, 1); add(OPTB_FIELD(hit_root), 4, chit, 1); add(OPTB_FIELD(hit_pop), 4, chit, 1);
     for (int f = 0; f < 10; f++) add(hit0 + 8 * f, hit_h[f], 8, chit, 1);
     add(OPTB_FIELD(hit_key), 8, chit, 1);
-  }
 #undef OPTB_FIELD
-  for (auto& c : cols) if (!c.dev[0] || !c.dev[1] || (sorted && (!c.srt[0] || !c.srt[1]))) return fail(ctx, -9, "arena sizing");
+    if (hist) { d_hy = (int64_t*)ac.take(hy); d_hyz = (int64_t*)ac.take(hyz); }
+    if (capb) d_caps = (int32_t*)ac.take(capb);
+    for (int s = 0; s < (chunked ? 2 : 1); s++) {
+      dv[s].seg_capacity = cseg; dv[s].hit_capacity = chit;
+      dv[s].hist_y = d_hy; dv[s].hist_yz = d_hyz; dv[s].cap_counts = d_caps; dv[s].root_flags = nullptr;
+      dv[s].counters = (int64_t*)ac.take(OPTB_C_COUNT * 8);
+      ws[s] = ac.take((size_t)wsb);
+    }
+    if (sortb) sort_ws = ac.take((size_t)sortb);
+    if (pass == 0 && ctx->arena_bytes < ac.off) {
+      if (ctx->arena) cudaFree(ctx->arena);
+      ctx->arena = nullptr; ctx->arena_bytes = 0;
+      CK(cudaMalloc(&ctx->arena, ac.off), "cudaMalloc(arena)");
+      ctx->arena_bytes = ac.off;
+    }
+  }
   int end_bit = 33;  // keys are root << 32 | ...: sort only the bits a root index of this batch can occupy
-  while (end_bit < 64 && (1ull << (end_bit - 32)) <= (unsigned long long)n) end_bit++;
-  const size_t hy = (size_t)std::max(scene->n_mons, 1) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
-  int64_t* d_hy = (int64_t*)ac.take(hy); int64_t* d_hyz = (int64_t*)ac.take(hyz);
-  void* ws[2];
-  for (int s = 0; s < 2; s++) {
-    dv[s].seg_capacity = cseg; dv[s].hit_capacity = chit;
-    dv[s].hist_y = d_hy; dv[s].hist_yz = d_hyz; dv[s].cap_counts = nullptr;
-    dv[s].counters = (int64_t*)ac.take(OPTB_C_COUNT * 8);
-    ws[s] = ac.take((size_t)wsb);
-    if (!ws[s] || !dv[s].counters) return fail(ctx, -9, "arena sizing");
-    dv[s].root_flags = nullptr;
-  }
-  void* sort_ws = sortb ? ac.take((size_t)sortb) : nullptr;
-  if (sortb && !sort_ws) return fail(ctx, -9, "arena sizing");
-  if (prm->record_hist && scene->n_mons) {
-    CK(cudaMemsetAsync(d_hy, 0, hy, ctx->s_run), "memset hist");
-    CK(cudaMemsetAsync(d_hyz, 0, hyz, ctx->s_run), "memset hist");
-  }
+  while (end_bit < 64 && (1ull << (end_bit - 32)) <= (unsigned long long)n_roots) end_bit++;
   struct Events {  // destroyed on every exit path
     std::vector<cudaEvent_t> v;
     explicit Events(int n) : v(n) { for (auto& e : v) cudaEventCreateWithFlags(&e, cudaEventDisableTiming); }
     ~Events() { for (auto& e : v) cudaEventDestroy(e); }
     cudaEvent_t& operator[](int i) { return v[i]; }
-  } ev_h2d(nch), ev_run(nch), ev_d2h(nch);
+  } ev_in(1), ev_h2d(nch), ev_run(nch), ev_d2h(nch);
+  // the call comes after the caller's earlier work on the legacy default stream and on every blocking stream
+  CK(cudaEventRecord(ev_in[0], 0), "event");
+  CK(cudaStreamWaitEvent(ctx->s_h2d, ev_in[0], 0), "wait");
+  CK(cudaStreamWaitEvent(ctx->s_run, ev_in[0], 0), "wait");
+  if (hist) {
+    CK(cudaMemsetAsync(d_hy, 0, hy, ctx->s_run), "memset hist");
+    CK(cudaMemsetAsync(d_hyz, 0, hyz, ctx->s_run), "memset hist");
+  }
+  if (capb && out->cap_counts) CK(cudaMemcpyAsync(d_caps, out->cap_counts, capb, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D caps");
+  else if (capb) CK(cudaMemsetAsync(d_caps, 0, capb, ctx->s_h2d), "memset caps");  // no table given: every family starts at zero
   unsigned long long tot[OPTB_C_COUNT] = {0};
   int64_t seg_off = 0, hit_off = 0;
   bool chunk_overflow = false;
@@ -1864,49 +1869,49 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
   auto drain = [&](int k) -> int {
     CK(cudaEventSynchronize(ev_run[k]), "sync chunk");
     const unsigned long long* hc = ctx->h_chunk + (size_t)k * OPTB_C_COUNT;
-    if (hc[OPTB_C_STATUS] & (OPTB_ST_SEG_OVERFLOW | OPTB_ST_HIT_OVERFLOW)) chunk_overflow = true;
+    if (chunked && (hc[OPTB_C_STATUS] & (OPTB_ST_SEG_OVERFLOW | OPTB_ST_HIT_OVERFLOW))) chunk_overflow = true;
     int64_t rows[2] = {std::min<int64_t>((int64_t)hc[OPTB_C_SEGMENTS], cseg), std::min<int64_t>((int64_t)hc[OPTB_C_HITS], chit)};
     int64_t room[2] = {segcap - seg_off, hitcap - hit_off};
     for (int kind = 0; kind < 2; kind++)
       if (rows[kind] > room[kind]) { rows[kind] = std::max<int64_t>(room[kind], 0); tot[OPTB_C_STATUS] |= kind ? OPTB_ST_HIT_OVERFLOW : OPTB_ST_SEG_OVERFLOW; }
+    if (sorted && !gather)
+      if (int src = sort_rows_dev(ctx, &dv[0], nullptr, rows[0], rows[1], nullptr, sort_ws, sortb, ctx->s_d2h, end_bit)) return src;
     for (auto& c : cols) {
       const int64_t r = rows[c.kind], off = c.kind ? hit_off : seg_off;
-      if (r > 0) CK(cudaMemcpyAsync(c.host + (size_t)off * c.elt, sorted ? c.srt[k & 1] : c.dev[k & 1], (size_t)r * c.elt, cudaMemcpyDeviceToHost, ctx->s_d2h), "D2H rows");
+      if (r > 0) CK(cudaMemcpyAsync(c.host + (size_t)off * c.elt, gather ? c.srt[k & 1] : c.dev[k & 1], (size_t)r * c.elt, cudaMemcpyDeviceToHost, ctx->s_d2h), "D2H rows");
     }
     CK(cudaEventRecord(ev_d2h[k], ctx->s_d2h), "event");
-    if (prm->record_segments) seg_off += rows[0];
-    if (prm->record_hits) hit_off += rows[1];
-    for (int q : {OPTB_C_SEGMENTS, OPTB_C_INTERACTIONS, OPTB_C_HITS, OPTB_C_TESTS, OPTB_C_DROPPED, OPTB_C_LAUNCHES}) tot[q] += hc[q];
-    tot[OPTB_C_STATUS] |= hc[OPTB_C_STATUS];
-    tot[OPTB_C_GENERATIONS] = std::max(tot[OPTB_C_GENERATIONS], hc[OPTB_C_GENERATIONS]);
+    seg_off += rows[0];
+    hit_off += rows[1];
+    for (int q = 0; q < OPTB_C_COUNT; q++)
+      tot[q] = q == OPTB_C_STATUS ? tot[q] | hc[q] : q == OPTB_C_GENERATIONS ? std::max(tot[q], hc[q]) : tot[q] + hc[q];
     return 0;
   };
   for (int c = 0; c < nch && !rc; c++) {
-    const int64_t lo = (int64_t)c * kChunk, m = std::min<int64_t>(kChunk, n - lo);
-    for (int f = 0; f < kRayF64; f++) {
-      if (!src_f[f] || ((rays->broadcast >> f) & 1u)) continue;
-      CK(cudaMemcpyAsync((void*)(dst_f[f] + lo), src_f[f] + lo, (size_t)m * 8, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D rays");
-    }
-    if (rays->flags) CK(cudaMemcpyAsync((void*)(dr.flags + lo), rays->flags + lo, (size_t)m * 4, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D flags");
-    if (rays->family) CK(cudaMemcpyAsync((void*)(dr.family + lo), rays->family + lo, (size_t)m * 4, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D family");
-    CK(cudaEventRecord(ev_h2d[c], ctx->s_h2d), "event");
-    CK(cudaStreamWaitEvent(ctx->s_run, ev_h2d[c], 0), "wait");
-    if (c >= 2 && !sorted) CK(cudaStreamWaitEvent(ctx->s_run, ev_d2h[c - 2], 0), "wait");  // the result set is free again
+    const int64_t lo = (int64_t)c * chunk, m = std::min<int64_t>(chunk, n - lo);
     optb_rays cr = dr;
     cr.n = m;
     const double** cf = &cr.ox;
-    for (int f = 0; f < kRayF64; f++) if (cf[f] && !((rays->broadcast >> f) & 1u)) cf[f] += lo;
-    if (cr.flags) cr.flags += lo;
-    if (cr.family) cr.family += lo;
+    for (int f = 0; f < kRayF64; f++) {
+      if (!src_f[f]) continue;
+      const bool bc = (rays->broadcast >> f) & 1u;  // one value for all rays: staged with the first chunk
+      if (!bc) cf[f] += lo;
+      if (!bc || c == 0) CK(cudaMemcpyAsync((void*)cf[f], src_f[f] + (bc ? 0 : lo), (bc ? 1 : (size_t)m) * 8, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D rays");
+    }
+    if (cr.flags) { cr.flags += lo; CK(cudaMemcpyAsync((void*)cr.flags, rays->flags + lo, (size_t)m * 4, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D flags"); }
+    if (cr.family) { cr.family += lo; CK(cudaMemcpyAsync((void*)cr.family, rays->family + lo, (size_t)m * 4, cudaMemcpyHostToDevice, ctx->s_h2d), "H2D family"); }
+    CK(cudaEventRecord(ev_h2d[c], ctx->s_h2d), "event");
+    CK(cudaStreamWaitEvent(ctx->s_run, ev_h2d[c], 0), "wait");
+    if (c >= 2 && !gather) CK(cudaStreamWaitEvent(ctx->s_run, ev_d2h[c - 2], 0), "wait");  // the result set is free again
     rc = trace_impl(ctx, scene, &cr, prm, &dv[c & 1], ws[c & 1], wsb, ctx->s_run, (uint32_t)lo, false);
     if (rc) break;
-    if (sorted) {
+    if (gather) {
       // reference order inside the chunk (chunks follow each other in ray order): keys + radix sort + one gather of
       // all columns into the sorted set, on the trace stream right behind the trace. The row counts stay on the
       // device (rows beyond them sort to the end), so nothing here waits for the host.
       if (c >= 2) CK(cudaStreamWaitEvent(ctx->s_run, ev_d2h[c - 2], 0), "wait");  // the sorted set is free again
-      rc = sort_rows_dev(ctx, &dv[c & 1], &sv[c & 1], prm->record_segments ? cseg : 0, prm->record_hits ? chit : 0,
-                         (const unsigned long long*)dv[c & 1].counters, sort_ws, sortb, ctx->s_run, end_bit);
+      rc = sort_rows_dev(ctx, &dv[c & 1], &sv[c & 1], cseg, chit, (const unsigned long long*)dv[c & 1].counters, sort_ws,
+                         sortb, ctx->s_run, end_bit);
       if (rc) break;
     }
     CK(cudaMemcpyAsync(ctx->h_chunk + (size_t)c * OPTB_C_COUNT, dv[c & 1].counters, OPTB_C_COUNT * 8, cudaMemcpyDeviceToHost, ctx->s_run), "D2H counters");
@@ -1914,15 +1919,15 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
     if (c >= 1) rc = drain(c - 1);
   }
   if (!rc) rc = drain(nch - 1);
-  if (!rc && prm->record_hist && scene->n_mons) {
-    cudaStreamWaitEvent(ctx->s_d2h, ev_run[nch - 1], 0);
-    if (out->hist_y) cudaMemcpyAsync(out->hist_y, d_hy, (size_t)scene->n_mons * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, ctx->s_d2h);
-    if (out->hist_yz) cudaMemcpyAsync(out->hist_yz, d_hyz, (size_t)scene->n_mons * OPTB_HIST_BINS * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, ctx->s_d2h);
+  if (!rc && hist) {
+    if (out->hist_y) CK(cudaMemcpyAsync(out->hist_y, d_hy, hy, cudaMemcpyDeviceToHost, ctx->s_d2h), "D2H hist");
+    if (out->hist_yz) CK(cudaMemcpyAsync(out->hist_yz, d_hyz, hyz, cudaMemcpyDeviceToHost, ctx->s_d2h), "D2H hist");
   }
+  if (!rc && capb && out->cap_counts) CK(cudaMemcpyAsync(out->cap_counts, d_caps, capb, cudaMemcpyDeviceToHost, ctx->s_d2h), "D2H caps");
   cudaStreamSynchronize(ctx->s_h2d); cudaStreamSynchronize(ctx->s_run);
   cudaError_t e = cudaStreamSynchronize(ctx->s_d2h);
   if (rc) return rc;
-  if (e != cudaSuccess) return fail(ctx, -10, "pipelined trace", e);
+  if (e != cudaSuccess) return fail(ctx, -10, "host trace", e);
   if (chunk_overflow) return 1;
   memcpy(ctx->h_counters, tot, sizeof tot);
   if (out->counters) memcpy(out->counters, tot, sizeof tot);
@@ -1932,9 +1937,10 @@ static int trace_host_pipelined(optb_ctx* ctx, const optb_scene* scene, const op
 extern "C" int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
                                optb_result* out) {
   if (!ctx || !scene || !rays || !prm || !out) return -1;
+  constexpr int64_t kChunk = 1 << 20;  // rays per chunk
   if (!needs_wavefront(scene, prm) && scene->n_caps == 0 && !scene->n_cfg && rays->n >= (3ll << 20)) {
-    int rc = trace_host_pipelined(ctx, scene, rays, prm, out);
-    if (rc <= 0) return rc;  // 1 = a chunk outgrew its estimated share of the result capacity: one-shot path
+    int rc = trace_host(ctx, scene, rays, prm, out, kChunk, 0);
+    if (rc <= 0) return rc;  // 1 = a chunk outgrew its estimated share of the result capacity: rerun as one chunk
   }
   // The live ray set of a splitting scene is not known in advance: grow the workspace until it fits. A root pops at
   // most max_trace_num rays and every pop queues at most two, so 2 n max_trace_num live rays always suffice.
@@ -1944,7 +1950,7 @@ extern "C" int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const opt
   const int64_t per_ray = std::max<int64_t>(4, ctx->live_per_ray_hint);
   for (int64_t live = std::min<int64_t>(std::max<int64_t>(per_ray * n_roots, 1024), std::max<int64_t>(bound, 1024));;
        live = std::min<int64_t>(live * 2, bound)) {
-    int rc = trace_host_once(ctx, scene, rays, prm, out, live);
+    int rc = trace_host(ctx, scene, rays, prm, out, rays->n, live);
     if (rc) return rc;
     if (!(ctx->h_counters[OPTB_C_STATUS] & OPTB_ST_WORK_OVERFLOW)) {
       if (n_roots > 0 && needs_wavefront(scene, prm)) ctx->live_per_ray_hint = (live + n_roots - 1) / n_roots;
@@ -1953,93 +1959,6 @@ extern "C" int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const opt
     if (live >= bound) break;
   }
   return fail(ctx, -8, "live ray set exceeds 2 * n * max_trace_num: workspace overflow");
-}
-
-static int trace_host_once(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
-                           optb_result* out, int64_t live) {
-  cudaSetDevice(ctx->device);
-  const int64_t n = rays->n, n_roots = n * std::max(scene->n_cfg, 1);
-  const bool split = needs_wavefront(scene, prm) || needs_serial(scene, rays, prm);
-  const int64_t segcap = prm->record_segments ? out->seg_capacity : 0, hitcap = prm->record_hits ? out->hit_capacity : 0;
-  const int64_t max_live = split ? std::max<int64_t>(live, n_roots) : 0;
-  const int64_t wsb = needs_serial(scene, rays, prm) ? optb_workspace_bytes(scene, n, 16 * std::max<int64_t>(live, 64))
-                                               : (int64_t)ws_layout(n_roots, max_live, split).total;
-  const int nfam = std::max(prm->n_families, 1);
-  const int64_t sortb = prm->sorted_rows ? optb_sort_workspace_bytes(std::max(segcap, hitcap)) : 0;
-  size_t need = 256 * 64 + (size_t)sortb + (size_t)n * (8 * 13 + 8) + (size_t)segcap * (13 * 8 + 16) + (size_t)hitcap * (10 * 8 + 12 + 8) +
-                (size_t)std::max(hist_mons(scene), 1) * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 8 +
-                (size_t)std::max(scene->n_caps, 1) * nfam * 4 + 64 * 8 + (size_t)wsb;
-  if (ctx->arena_bytes < need) {
-    if (ctx->arena) cudaFree(ctx->arena);
-    ctx->arena = nullptr; ctx->arena_bytes = 0;
-    CK(cudaMalloc(&ctx->arena, need), "cudaMalloc(arena)");
-    ctx->arena_bytes = need;
-  }
-  ArenaCursor ac{(unsigned char*)ctx->arena, 0, ctx->arena_bytes};
-  cudaStream_t st = 0;
-  optb_rays dr = *rays;
-  const double* const* src_f = &rays->ox;
-  const double** dst_f = &dr.ox;
-  for (int f = 0; f < kRayF64; f++) {
-    if (!src_f[f]) { dst_f[f] = nullptr; continue; }
-    const size_t rows = ((rays->broadcast >> f) & 1u) ? 1 : (size_t)n;
-    void* d = ac.take(rows * 8);
-    if (!d) return fail(ctx, -9, "arena sizing");
-    CK(cudaMemcpyAsync(d, src_f[f], rows * 8, cudaMemcpyHostToDevice, st), "H2D rays");
-    dst_f[f] = (const double*)d;
-  }
-  if (rays->flags) { void* d = ac.take((size_t)n * 4); CK(cudaMemcpyAsync(d, rays->flags, (size_t)n * 4, cudaMemcpyHostToDevice, st), "H2D flags"); dr.flags = (const uint32_t*)d; }
-  if (rays->family) { void* d = ac.take((size_t)n * 4); CK(cudaMemcpyAsync(d, rays->family, (size_t)n * 4, cudaMemcpyHostToDevice, st), "H2D family"); dr.family = (const int32_t*)d; }
-  optb_result dv = *out;
-  struct Col { void** dev; void* host; size_t elt; int64_t cap; int kind; };  // kind 0 seg, 1 hit
-  std::vector<Col> cols;
-  auto add = [&](void** dev_field, void* host_ptr, size_t elt, int64_t capn, int kind) {
-    if (!host_ptr || capn == 0) { *dev_field = nullptr; return; }
-    *dev_field = ac.take((size_t)capn * elt);
-    cols.push_back({dev_field, host_ptr, elt, capn, kind});
-  };
-  double** seg_d = &dv.seg_ox; double* const* seg_h = &out->seg_ox;
-  for (int f = 0; f < 13; f++) add((void**)&seg_d[f], seg_h[f], 8, segcap, 0);
-  add((void**)&dv.seg_flags, out->seg_flags, 4, segcap, 0); add((void**)&dv.seg_root, out->seg_root, 4, segcap, 0);
-  add((void**)&dv.seg_pop, out->seg_pop, 4, segcap, 0); add((void**)&dv.seg_leaf, out->seg_leaf, 4, segcap, 0);
-  add((void**)&dv.hit_monitor, out->hit_monitor, 4, hitcap, 1); add((void**)&dv.hit_root, out->hit_root, 4, hitcap, 1);
-  add((void**)&dv.hit_pop, out->hit_pop, 4, hitcap, 1);
-  double** hit_d = &dv.hit_px; double* const* hit_h = &out->hit_px;
-  for (int f = 0; f < 10; f++) add((void**)&hit_d[f], hit_h[f], 8, hitcap, 1);
-  add((void**)&dv.hit_key, out->hit_key, 8, hitcap, 1);
-  dv.root_flags = nullptr;
-  for (auto& c : cols) if (!*c.dev) return fail(ctx, -9, "arena sizing");
-  void* sort_ws = sortb ? ac.take((size_t)sortb) : nullptr;
-  if (sortb && !sort_ws) return fail(ctx, -9, "arena sizing");
-  const size_t hy = (size_t)std::max(hist_mons(scene), 1) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
-  dv.hist_y = (int64_t*)ac.take(hy); dv.hist_yz = (int64_t*)ac.take(hyz);
-  const size_t capb = (size_t)std::max(scene->n_caps, 1) * nfam * 4;
-  dv.cap_counts = (int32_t*)ac.take(capb);
-  dv.counters = (int64_t*)ac.take(OPTB_C_COUNT * 8);
-  void* ws = ac.take((size_t)wsb);
-  if (!ws || !dv.counters) return fail(ctx, -9, "arena sizing");
-  if (scene->n_caps > 0 && out->cap_counts) CK(cudaMemcpyAsync(dv.cap_counts, out->cap_counts, capb, cudaMemcpyHostToDevice, st), "H2D caps");
-  else CK(cudaMemsetAsync(dv.cap_counts, 0, capb, st), "memset caps");  // no table given: every family starts at zero
-  int rc = optb_trace(ctx, scene, &dr, prm, &dv, ws, wsb, st);
-  if (rc) return rc;
-  CK(cudaMemcpyAsync(ctx->h_counters, dv.counters, OPTB_C_COUNT * 8, cudaMemcpyDeviceToHost, st), "D2H counters");
-  CK(cudaStreamSynchronize(st), "sync trace");
-  if (out->counters) memcpy(out->counters, ctx->h_counters, OPTB_C_COUNT * 8);
-  int64_t nseg = std::min<int64_t>((int64_t)ctx->h_counters[OPTB_C_SEGMENTS], segcap);
-  int64_t nhit = std::min<int64_t>((int64_t)ctx->h_counters[OPTB_C_HITS], hitcap);
-  if (prm->sorted_rows)
-    if (int src = optb_sort_rows(ctx, &dv, prm->record_segments ? nseg : 0, prm->record_hits ? nhit : 0, sort_ws, sortb, st)) return src;
-  for (auto& c : cols) {
-    int64_t rows = c.kind == 0 ? nseg : nhit;
-    if (rows > 0) CK(cudaMemcpyAsync(c.host, *c.dev, (size_t)rows * c.elt, cudaMemcpyDeviceToHost, st), "D2H results");
-  }
-  if (prm->record_hist && scene->n_mons) {
-    if (out->hist_y) CK(cudaMemcpyAsync(out->hist_y, dv.hist_y, (size_t)hist_mons(scene) * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
-    if (out->hist_yz) CK(cudaMemcpyAsync(out->hist_yz, dv.hist_yz, (size_t)hist_mons(scene) * OPTB_HIST_BINS * OPTB_HIST_BINS * 8, cudaMemcpyDeviceToHost, st), "D2H hist");
-  }
-  if (scene->n_caps > 0 && out->cap_counts) CK(cudaMemcpyAsync(out->cap_counts, dv.cap_counts, capb, cudaMemcpyDeviceToHost, st), "D2H caps");
-  CK(cudaStreamSynchronize(st), "sync results");
-  return 0;
 }
 
 extern "C" int optb_measure_fp64_peak(optb_ctx* ctx, double* tflops_out) {
@@ -2107,11 +2026,6 @@ __global__ void __launch_bounds__(256) gather_rows_kernel(const GatherCols g, co
     }
   }
 }
-template <class T>
-__global__ void gather_kernel(const T* __restrict__ src, const uint32_t* __restrict__ idx, long long n, T* __restrict__ dst) {
-  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
-    dst[i] = src[idx[i]];
-}
 struct SortLayout { size_t key_a, key_b, idx_a, idx_b, tmp, cub, cub_bytes, total; };
 SortLayout sort_layout(long long n) {
   SortLayout L{};
@@ -2128,13 +2042,6 @@ SortLayout sort_layout(long long n) {
   L.cub = o; L.cub_bytes = align_up(tb + 256, 256); o += L.cub_bytes;
   L.total = o;
   return L;
-}
-template <class T>
-int reorder_column(optb_ctx* ctx, T* col, const uint32_t* order, long long n, void* tmp, int grid, cudaStream_t st) {
-  if (!col) return 0;
-  gather_kernel<T><<<grid, 256, 0, st>>>(col, order, n, (T*)tmp);
-  CK(cudaMemcpyAsync(col, tmp, (size_t)n * sizeof(T), cudaMemcpyDeviceToDevice, st), "reorder column");
-  return 0;
 }
 }  // namespace
 
@@ -2174,41 +2081,31 @@ static int sort_rows_dev(optb_ctx* ctx, const optb_result* res, const optb_resul
     size_t tb = L.cub_bytes;
     CK(cub::DeviceRadixSort::SortPairs(ws + L.cub, tb, (const unsigned long long*)key_a, key_b, (const uint32_t*)idx_a, idx_b,
                                        (int)n, 0, end_bit, st), "radix sort of the row keys");
+    const optb_result* to = dst ? dst : res;
+    GatherCols g;
+    g.ncol = 0;
+    auto col = [&](const void* sp, void* dp, int elt) { if (sp && dp) { g.src[g.ncol] = sp; g.dst[g.ncol] = dp; g.elt[g.ncol] = elt; g.ncol++; } };
+    if (pass == 0) {
+      double* const* f = &res->seg_ox; double* const* fd = &to->seg_ox;
+      for (int c = 0; c < 13; c++) col(f[c], fd[c], 8);
+      col(res->seg_flags, to->seg_flags, 4); col(res->seg_root, to->seg_root, 4);
+      col(res->seg_pop, to->seg_pop, 4); col(res->seg_leaf, to->seg_leaf, 4);
+    } else {
+      double* const* f = &res->hit_px; double* const* fd = &to->hit_px;
+      for (int c = 0; c < 10; c++) col(f[c], fd[c], 8);
+      col(res->hit_monitor, to->hit_monitor, 4); col(res->hit_root, to->hit_root, 4);
+      col(res->hit_pop, to->hit_pop, 4); col(res->hit_key, to->hit_key, 8);
+    }
     if (dst) {
-      GatherCols g;
-      g.ncol = 0;
-      auto col = [&](const void* sp, void* dp, int elt) { if (sp && dp) { g.src[g.ncol] = sp; g.dst[g.ncol] = dp; g.elt[g.ncol] = elt; g.ncol++; } };
-      if (pass == 0) {
-        double* const* f = &res->seg_ox; double* const* fd = &dst->seg_ox;
-        for (int c = 0; c < 13; c++) col(f[c], fd[c], 8);
-        col(res->seg_flags, dst->seg_flags, 4); col(res->seg_root, dst->seg_root, 4);
-        col(res->seg_pop, dst->seg_pop, 4); col(res->seg_leaf, dst->seg_leaf, 4);
-      } else {
-        double* const* f = &res->hit_px; double* const* fd = &dst->hit_px;
-        for (int c = 0; c < 10; c++) col(f[c], fd[c], 8);
-        col(res->hit_monitor, dst->hit_monitor, 4); col(res->hit_root, dst->hit_root, 4);
-        col(res->hit_pop, dst->hit_pop, 4); col(res->hit_key, dst->hit_key, 8);
-      }
       if (g.ncol) gather_rows_kernel<<<grid, 256, 0, st>>>(g, idx_b, n);
       continue;
     }
-    int rc = 0;
-    if (pass == 0) {
-      double* const* f = &res->seg_ox;
-      for (int c = 0; c < 13 && !rc; c++) rc = reorder_column<double>(ctx, f[c], idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<uint32_t>(ctx, res->seg_flags, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<uint32_t>(ctx, res->seg_root, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<uint32_t>(ctx, res->seg_pop, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<int32_t>(ctx, res->seg_leaf, idx_b, n, tmp, grid, st);
-    } else {
-      double* const* f = &res->hit_px;
-      for (int c = 0; c < 10 && !rc; c++) rc = reorder_column<double>(ctx, f[c], idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<int32_t>(ctx, res->hit_monitor, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<uint32_t>(ctx, res->hit_root, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<uint32_t>(ctx, res->hit_pop, idx_b, n, tmp, grid, st);
-      if (!rc) rc = reorder_column<unsigned long long>(ctx, (unsigned long long*)res->hit_key, idx_b, n, tmp, grid, st);
+    for (int c = 0; c < g.ncol; c++) {  // in place: each column through the scratch column
+      GatherCols one;
+      one.src[0] = g.src[c]; one.dst[0] = tmp; one.elt[0] = g.elt[c]; one.ncol = 1;
+      gather_rows_kernel<<<grid, 256, 0, st>>>(one, idx_b, n);
+      CK(cudaMemcpyAsync(g.dst[c], tmp, (size_t)n * g.elt[c], cudaMemcpyDeviceToDevice, st), "reorder column");
     }
-    if (rc) return rc;
   }
   CK(cudaGetLastError(), "optb_sort_rows");
   return 0;
