@@ -436,6 +436,35 @@ int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_t first, in
                        const optb_monitor_frame* frame, double* stats, double* y, double* z, double* ty, double* tz,
                        double* waist, void* stream);
 
+/* The same summaries for every (configuration, monitor) group of the rows [first, first + n) in one call: what a scan,
+ * an optimizer or a tolerance study ranks after one sweep (optb_scene_upload_sweep), or all monitors of one trace.
+ *   - group of a row: g = k * n_monitors + m, k = root / rays_per_config (the K x N root numbering of a sweep scene;
+ *     rays_per_config = 0: one configuration, k = 0), root from hit_root or else hit_key >> 32, m from hit_monitor or
+ *     else (hit_key >> 24) & 0xff. A row with k >= n_configs or m outside [0, n_monitors) belongs to no group: its
+ *     per-row outputs are NaN and it is counted nowhere (the counts then add up to less than n).
+ *   - frames: DEVICE optb_monitor_frame[n_configs * n_monitors], group g evaluated in frames[g].
+ *   - stats: DEVICE double[n_configs * n_monitors][OPTB_MS_STRIDE], overwritten; every group's slots mean what the
+ *     OPTB_MS_* slots of optb_monitor_stats mean (M2_* about that group's own means; the histogram bins like
+ *     np.histogram); a group without rows reads like optb_monitor_stats over no rows (zeros, min +inf, max -inf).
+ *   - y, z, ty, tz, waist: DEVICE double[n] or NULL, row first + i at [i], evaluated in its group's frame; bit-identical
+ *     to what optb_monitor_stats writes for that row and frame.
+ *   - rows may come in any order (sorted by optb_sort_rows, or in device append order).
+ *   - deterministic: the same rows in the same order give bit-identical stats on every call, on any stream, whatever
+ *     the device's SM count (rows are sorted by group, each group is reduced in tiles of a fixed size in a fixed order,
+ *     and its tile partials are combined in tile order).
+ *   - workspace: optb_monitor_stats_grouped_workspace_bytes(n, n_configs * n_monitors) bytes of device memory
+ *     (-1: n >= 2^31 - 1 or a group count outside [1, 2^20]).
+ * Fails with -7 when a required column is missing (the monitor column; the root column when rays_per_config > 0),
+ * slopes or waist distances are requested without hit_dx..dz / hit_q_re, n_monitors > 256, n_configs * n_monitors
+ * > 2^20, n >= 2^31 - 1, or the workspace is too small. Enqueued on `stream`, without a host synchronisation.
+ * Added without a change of OPTB_ABI_VERSION: no struct changed, and a host written for this entry point against an
+ * older library fails to link instead.                                                                           */
+int64_t optb_monitor_stats_grouped_workspace_bytes(int64_t n_rows, int32_t n_groups);
+int optb_monitor_stats_grouped(optb_ctx* ctx, const optb_result* rows, int64_t first, int64_t n,
+                               int64_t rays_per_config, int32_t n_configs, int32_t n_monitors,
+                               const optb_monitor_frame* frames, double* stats, double* y, double* z, double* ty,
+                               double* tz, double* waist, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- multi-GPU monitor merge (SURVEY 8e) -----------------------------------------------------------------------
  * The path shards without a data-path collective: every rank (one process per GPU, one ctx each) traces its own block
  * of the initial rays against its own copy of the scene. The only exchange is the merge of the monitors at the end,

@@ -86,6 +86,7 @@ EXPORTED_SYMBOLS = (
     "optb_scene_upload", "optb_scene_upload_sweep", "optb_scene_destroy", "optb_scene_update_nodes", "optb_workspace_bytes", "optb_trace",
     "optb_trace_host", "optb_measure_fp64_peak",
     "optb_sort_workspace_bytes", "optb_sort_rows", "optb_monitor_stats",
+    "optb_monitor_stats_grouped_workspace_bytes", "optb_monitor_stats_grouped",
     "optb_comm_unique_id", "optb_comm_init", "optb_monitor_merge", "optb_comm_destroy",
 )
 

@@ -18,6 +18,67 @@ import numpy as np
 from . import _abi as A
 
 
+def _frame(monitor) -> A.MonitorFrame:
+    fr = A.MonitorFrame()
+    fr.tangent_y[:] = [float(v) for v in monitor.tangent_Y]
+    fr.tangent_z[:] = [float(v) for v in monitor.tangent_Z]
+    fr.normal[:] = [float(v) for v in monitor.normal]
+    fr.half_width, fr.half_height = float(monitor.width) / 2, float(monitor.height) / 2
+    return fr
+
+
+def stats_arrays(s, widths) -> dict:
+    """`DeviceMonitor.stats()` of many monitors at once: stats slots s [..., OPTB_MS_STRIDE] (numpy) -> the same keys as
+    arrays shaped s.shape[:-1] (hist_y: [..., 30]), plus `std_tY` (from OPTB_MS_M2_TY) and `std_histy` (the formula of
+    `DeviceMonitor.std_histy`; NaN for a monitor without rows in its histogram) for monitors of widths `widths`."""
+    s = np.asarray(s, np.float64)
+    n = np.maximum(s[..., A.MS_COUNT], 1.0)
+    hist = s[..., A.MS_HIST:A.MS_HIST + A.HIST_BINS].astype(np.int64)
+    w = np.asarray(widths, np.float64)
+    c = hist.astype(np.float64)
+    left = np.linspace(-w / 2, w / 2, A.HIST_BINS + 1, axis=-1)[..., :-1]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        mean = (c * left).sum(-1) / c.sum(-1)
+        std_histy = np.sqrt((c * left ** 2).sum(-1) / c.sum(-1) - mean ** 2)
+    return {
+        "count": s[..., A.MS_COUNT].astype(np.int64), "sum_intensity": s[..., A.MS_SUM_I],
+        "avg_intensity": s[..., A.MS_SUM_I] / n, "mean_y": s[..., A.MS_SUM_Y] / n, "mean_z": s[..., A.MS_SUM_Z] / n,
+        "std_y": np.sqrt(s[..., A.MS_M2_Y] / n), "std_z": np.sqrt(s[..., A.MS_M2_Z] / n),
+        "min_y": s[..., A.MS_MIN_Y], "max_y": s[..., A.MS_MAX_Y], "min_z": s[..., A.MS_MIN_Z], "max_z": s[..., A.MS_MAX_Z],
+        "mean_waist_distance": s[..., A.MS_SUM_WD] / n, "mean_tY": s[..., A.MS_SUM_TY] / n,
+        "hist_y": hist, "std_tY": np.sqrt(s[..., A.MS_M2_TY] / n), "std_histy": std_histy,
+    }
+
+
+def grouped_stats(out: dict, monitors, rays_per_config=0, engine=None):
+    """Summaries of every (configuration k, monitor m) of the hit rows in `out` (CUDA tensors of one result) in one
+    device call (`optb_monitor_stats_grouped`), each group in the frame of monitors[k][m]. A row's configuration is
+    root // rays_per_config (0: one configuration). Returns (stats_arrays dict of [K, M] arrays, per-row values
+    [5, n]: y, z, tY, tZ, waist distance as a CUDA tensor aligned with the rows). Raises ValueError when a row belongs
+    to no group (its monitor or configuration is out of range): the counts would not add up to the rows."""
+    from .backend import Engine
+
+    K, M = len(monitors), len(monitors[0])
+    any_col = out["hit_px"]
+    engine = engine or Engine.get(any_col.device.index or 0)
+    frames = (A.MonitorFrame * (K * M))(*[_frame(monitors[k][m]) for k in range(K) for m in range(M)])
+    stats, per_row = engine.monitor_stats_grouped(out, frames, K, M, rays_per_config)
+    s = stats.cpu().numpy().reshape(K, M, A.MS_STRIDE)
+    n, counted = int(any_col.numel()), int(s[..., A.MS_COUNT].sum())
+    if counted != n:
+        raise ValueError(f"{n - counted} of {n} monitor rows belong to no (configuration, monitor) group of this "
+                         f"{K} x {M} result: their monitor or configuration index is out of range")
+    widths = [[float(monitors[k][m].width) for m in range(M)] for k in range(K)]
+    return stats_arrays(s, widths), per_row
+
+
+def monitor_stats(monitors, out: dict, engine=None) -> dict:
+    """`DeviceMonitor(monitors[m], out, m).stats()` of every monitor of a `trace_bundle` result in one device call:
+    the same keys as arrays shaped [M] (hist_y [M, 30]), plus `std_tY` and `std_histy` (see `stats_arrays`)."""
+    s, _ = grouped_stats(out, [list(monitors)], 0, engine)
+    return {k: v[0] for k, v in s.items()}
+
+
 class DeviceMonitor:
     def __init__(self, monitor, out: dict, index: int, engine=None):
         import torch
@@ -34,11 +95,7 @@ class DeviceMonitor:
         for k in A.HIT_I32 + A.HIT_U32 + A.HIT_F64 + ("hit_key",):
             if out.get(k) is not None:
                 setattr(res, k, out[k].data_ptr())
-        fr = A.MonitorFrame()
-        fr.tangent_y[:] = [float(v) for v in monitor.tangent_Y]
-        fr.tangent_z[:] = [float(v) for v in monitor.tangent_Z]
-        fr.normal[:] = [float(v) for v in monitor.normal]
-        fr.half_width, fr.half_height = float(monitor.width) / 2, float(monitor.height) / 2
+        fr = _frame(monitor)
         f64 = torch.float64
         has_d, has_q = out.get("hit_dx") is not None, out.get("hit_q_re") is not None
         cols = torch.empty((5, max(n, 1)), dtype=f64, device=dev)

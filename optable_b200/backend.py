@@ -46,6 +46,10 @@ def lib():
         L.optb_sort_workspace_bytes.restype = C.c_int64
         L.optb_sort_workspace_bytes.argtypes = [C.c_int64]
         L.optb_sort_rows.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]
+        L.optb_monitor_stats_grouped_workspace_bytes.restype = C.c_int64
+        L.optb_monitor_stats_grouped_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
+        L.optb_monitor_stats_grouped.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_int64, C.c_int32,
+                                                 C.c_int32, C.c_void_p, C.c_void_p] + [C.c_void_p] * 6 + [C.c_int64, C.c_void_p]
         if L.optb_abi_version() != A.ABI_VERSION:
             raise BackendError("liboptb.so ABI version does not match optable_b200._abi")
         _lib = L
@@ -387,6 +391,33 @@ class Engine:
         st = self.torch.cuda.current_stream(self.device).cuda_stream
         self._check(lib().optb_sort_rows(self._ctx, C.byref(res), int(nseg), int(nhit), ws.data_ptr(), int(ws.numel()), C.c_void_p(st)))
         return True
+
+    def monitor_stats_grouped(self, cols, frames, n_configs, n_monitors, rays_per_config=0):
+        """optb_monitor_stats_grouped over every row of `cols` (the CUDA hit columns of one result) on the current
+        stream. `frames`: a ctypes array of n_configs * n_monitors MonitorFrame, group k * n_monitors + m at its place.
+        Returns the device tensors stats [n_configs * n_monitors, OPTB_MS_STRIDE] and per-row values [5, n] (y, z, tY,
+        tZ, waist distance in each row's own frame; the last three rows are unwritten without hit_dx..dz / hit_q_re)."""
+        torch = self.torch
+        dev = f"cuda:{self.device}"
+        n, G = int(cols["hit_px"].numel()), int(n_configs) * int(n_monitors)
+        res = A.Result()
+        for k in A.HIT_I32 + A.HIT_U32 + A.HIT_F64 + ("hit_key",):
+            if cols.get(k) is not None:
+                setattr(res, k, cols[k].data_ptr())
+        frames_dev = torch.frombuffer(bytearray(frames), dtype=torch.uint8).to(dev)
+        stats = torch.empty((G, A.MS_STRIDE), dtype=torch.float64, device=dev)
+        per_row = torch.empty((5, max(n, 1)), dtype=torch.float64, device=dev)
+        has_d, has_q = cols.get("hit_dx") is not None, cols.get("hit_q_re") is not None
+        ptr = lambda r, ok=True: C.c_void_p(per_row[r].data_ptr()) if ok else None
+        L = lib()
+        # a group count the library refuses gets no workspace size (-1): the call then reports why
+        ws = self._ws(max(int(L.optb_monitor_stats_grouped_workspace_bytes(n, G)), 1))
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(L.optb_monitor_stats_grouped(self._ctx, C.byref(res), 0, n, int(rays_per_config), int(n_configs),
+                                                 int(n_monitors), C.c_void_p(frames_dev.data_ptr()), C.c_void_p(stats.data_ptr()),
+                                                 ptr(0), ptr(1), ptr(2, has_d), ptr(3, has_d), ptr(4, has_d and has_q),
+                                                 C.c_void_p(ws.data_ptr()), int(ws.numel()), C.c_void_p(st)))
+        return stats, per_row[:, :n]
 
     @staticmethod
     def _raise_status(counters):

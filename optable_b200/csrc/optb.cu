@@ -14,6 +14,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 #include <stddef.h>
 #include <stdio.h>
 #include <string.h>
@@ -2149,6 +2150,27 @@ __global__ void stats_init_kernel(double* s) {
   const int k = threadIdx.x;
   if (k < OPTB_MS_STRIDE) s[k] = (k == OPTB_MS_MIN_Y || k == OPTB_MS_MIN_Z) ? INFINITY : (k == OPTB_MS_MAX_Y || k == OPTB_MS_MAX_Z) ? -INFINITY : 0.0;
 }
+// What the Monitor accessors derive for row j in frame f: y, z (local point . lab tangent), tY, tZ and the signed waist
+// distance (NaN without hit_dx..dz, resp. hit_q_re); returns the row's bin of the 30-bin histogram of y (-1 outside).
+// One definition for the single-monitor and the grouped kernels, so that their per-row columns agree bit for bit.
+template <class Cols>
+OPTB_DEV int eval_row(const Cols& a, long long j, const optb_monitor_frame& f, double& y, double& z, double& ty,
+                      double& tz, double& wd) {
+  const double Px = a.px[j], Py = a.py[j], Pz = a.pz[j];
+  y = dot3(Px, Py, Pz, f.tangent_y[0], f.tangent_y[1], f.tangent_y[2]);
+  z = dot3(Px, Py, Pz, f.tangent_z[0], f.tangent_z[1], f.tangent_z[2]);
+  ty = NAN; tz = NAN; wd = NAN;
+  if (a.dx) {
+    const double dx = a.dx[j], dy = a.dy[j], dz = a.dz[j];
+    ty = dot3(dx, dy, dz, f.tangent_y[0], f.tangent_y[1], f.tangent_y[2]);
+    tz = dot3(dx, dy, dz, f.tangent_z[0], f.tangent_z[1], f.tangent_z[2]);
+    if (a.qre) {
+      const double dist = a.qre[j] + a.t[j];  // Re(q_at_z(t)) = distance to the waist plane (ray.py:17-25)
+      wd = dot3(dx, dy, dz, f.normal[0], f.normal[1], f.normal[2]) > 0.0 ? -dist : dist;
+    }
+  }
+  return hist_bin(y, -f.half_width, f.half_width);
+}
 __global__ void __launch_bounds__(256) monitor_stats_kernel(const StatsArgs a) {
   __shared__ unsigned int s_hist[OPTB_HIST_BINS];
   __shared__ double s_red[8][8];
@@ -2162,23 +2184,13 @@ __global__ void __launch_bounds__(256) monitor_stats_kernel(const StatsArgs a) {
     if (a.monitor >= 0) mine = a.mon ? (a.mon[j] == a.monitor) : (int)((a.key[j] >> 24) & 0xffu) == a.monitor;
     double y = NAN, z = NAN, ty = NAN, tz = NAN, wd = NAN;
     if (mine) {
-      const double Px = a.px[j], Py = a.py[j], Pz = a.pz[j];
-      y = dot3(Px, Py, Pz, a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]);
-      z = dot3(Px, Py, Pz, a.f.tangent_z[0], a.f.tangent_z[1], a.f.tangent_z[2]);
+      const int b = eval_row(a, j, a.f, y, z, ty, tz, wd);
       cnt += 1.0; sI += a.I[j]; sy += y; syy = fma(y, y, syy); sz += z; szz = fma(z, z, szz);
       ymin = fmin(ymin, y); ymax = fmax(ymax, y); zmin = fmin(zmin, z); zmax = fmax(zmax, z);
-      const int b = hist_bin(y, -a.f.half_width, a.f.half_width);
       if (b >= 0) atomicAdd(&s_hist[b], 1u);
       if (a.dx) {
-        const double dx = a.dx[j], dy = a.dy[j], dz = a.dz[j];
-        ty = dot3(dx, dy, dz, a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]);
-        tz = dot3(dx, dy, dz, a.f.tangent_z[0], a.f.tangent_z[1], a.f.tangent_z[2]);
         sty += ty; styty = fma(ty, ty, styty);
-        if (a.qre) {
-          const double dist = a.qre[j] + a.t[j];  // Re(q_at_z(t)) = distance to the waist plane (ray.py:17-25)
-          wd = dot3(dx, dy, dz, a.f.normal[0], a.f.normal[1], a.f.normal[2]) > 0.0 ? -dist : dist;
-          swd += wd;
-        }
+        if (a.qre) swd += wd;
       }
     }
     if (a.y) a.y[k] = y;
@@ -2230,12 +2242,12 @@ __global__ void __launch_bounds__(256) monitor_m2_kernel(const StatsArgs a) {
   for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < a.n; k += (long long)gridDim.x * blockDim.x) {
     const long long j = a.first + k;
     if (a.monitor >= 0 && (a.mon ? a.mon[j] != a.monitor : (int)((a.key[j] >> 24) & 0xffu) != a.monitor)) continue;
-    const double Px = a.px[j], Py = a.py[j], Pz = a.pz[j];
-    const double y = dot3(Px, Py, Pz, a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]) - my;
-    const double z = dot3(Px, Py, Pz, a.f.tangent_z[0], a.f.tangent_z[1], a.f.tangent_z[2]) - mz;
+    double y, z, ty, tz, wd;
+    eval_row(a, j, a.f, y, z, ty, tz, wd);
+    y -= my; z -= mz;
     v[0] = fma(y, y, v[0]); v[1] = fma(z, z, v[1]);
     if (a.dx) {
-      const double ty = dot3(a.dx[j], a.dy[j], a.dz[j], a.f.tangent_y[0], a.f.tangent_y[1], a.f.tangent_y[2]) - mty;
+      ty -= mty;
       v[2] = fma(ty, ty, v[2]);
     }
   }
@@ -2279,6 +2291,275 @@ extern "C" int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_
     monitor_m2_kernel<<<grid, 256, 0, st>>>(a);
   }
   CK(cudaGetLastError(), "monitor_stats_kernel");
+  return 0;
+}
+
+// ---- grouped monitor analytics: every (configuration, monitor) of a result in one call, deterministically ---------
+// Rows are sorted by group (stable radix sort of (group, row index)), each group's run is cut into tiles of kGroupTile
+// rows, a block reduces one tile in a fixed order and a warp combines a group's tile partials in tile order. Nothing
+// depends on the grid or the SM count, so the same rows in the same order give the same bits on every call.
+namespace {
+constexpr int kGroupThreads = 256;
+constexpr int kGroupTile = kGroupThreads * 16;
+constexpr long long kMaxGroups = 1ll << 20;
+struct GroupArgs {
+  const double *px, *py, *pz, *I, *t, *dx, *dy, *dz, *qre;
+  const uint32_t* root; const int32_t* mon; const unsigned long long* key;
+  long long first, n, per_config; int n_configs, n_monitors, n_groups;
+  const optb_monitor_frame* frames;
+  double *stats, *y, *z, *ty, *tz, *wd;
+  uint32_t *key_a, *key_b, *idx_a, *idx_b, *start, *ntiles, *tile_first;
+  double* part; long long part_stride;  // tile partials, slot-major: part[slot * part_stride + tile]
+};
+struct GroupLayout { size_t key_a, key_b, idx_a, idx_b, start, ntiles, tile_first, part, cub, cub_bytes, total;
+                     long long tiles_cap; int end_bit; };
+GroupLayout group_layout(long long n, int G) {
+  GroupLayout L{};
+  const long long nn = std::max<long long>(n, 1);
+  // sum over groups of ceil(count / tile) <= floor(n / tile) + (number of non-empty groups)
+  L.tiles_cap = n / kGroupTile + std::min<long long>(G, n) + 1;
+  L.end_bit = 32 - __builtin_clz((unsigned)G);  // keys 0..G (G: the row belongs to no group)
+  size_t o = 0;
+  L.key_a = o; o += align_up((size_t)nn * 4, 256);
+  L.key_b = o; o += align_up((size_t)nn * 4, 256);
+  L.idx_a = o; o += align_up((size_t)nn * 4, 256);
+  L.idx_b = o; o += align_up((size_t)nn * 4, 256);
+  L.start = o; o += align_up((size_t)(G + 1) * 4, 256);
+  L.ntiles = o; o += align_up((size_t)(G + 1) * 4, 256);
+  L.tile_first = o; o += align_up((size_t)(G + 1) * 4, 256);
+  L.part = o; o += align_up((size_t)L.tiles_cap * OPTB_MS_STRIDE * 8, 256);
+  size_t tb_sort = 0, tb_scan = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, tb_sort, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const uint32_t*)nullptr,
+                                  (uint32_t*)nullptr, (int)std::min<long long>(nn, 0x7fffffffll), 0, L.end_bit);
+  cub::DeviceScan::ExclusiveSum(nullptr, tb_scan, (const uint32_t*)nullptr, (uint32_t*)nullptr, G + 1);
+  L.cub = o; L.cub_bytes = align_up(std::max(tb_sort, tb_scan) + 256, 256); o += L.cub_bytes;
+  L.total = o;
+  return L;
+}
+OPTB_DEV bool slot_is_min(int q) { return q == OPTB_MS_MIN_Y || q == OPTB_MS_MIN_Z; }
+OPTB_DEV bool slot_is_max(int q) { return q == OPTB_MS_MAX_Y || q == OPTB_MS_MAX_Z; }
+// group of every row (n_groups: none; its per-row outputs are NaN here, the passes never see it) and the identity
+// permutation for the sort
+__global__ void group_keys_kernel(const GroupArgs a) {
+  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < a.n; k += (long long)gridDim.x * blockDim.x) {
+    const long long j = a.first + k;
+    const int m = a.mon ? a.mon[j] : (int)((a.key[j] >> 24) & 0xffu);
+    long long cfg = 0;
+    if (a.per_config > 0) cfg = (long long)(a.root ? a.root[j] : (uint32_t)(a.key[j] >> 32)) / a.per_config;
+    const bool ok = m >= 0 && m < a.n_monitors && cfg < a.n_configs;
+    a.key_a[k] = ok ? (uint32_t)(cfg * a.n_monitors + m) : (uint32_t)a.n_groups;
+    a.idx_a[k] = (uint32_t)k;
+    if (!ok) {
+      if (a.y) a.y[k] = NAN;
+      if (a.z) a.z[k] = NAN;
+      if (a.ty) a.ty[k] = NAN;
+      if (a.tz) a.tz[k] = NAN;
+      if (a.wd) a.wd[k] = NAN;
+    }
+  }
+}
+OPTB_DEV uint32_t lower_bound_u32(const uint32_t* v, uint32_t n, uint32_t x) {
+  uint32_t lo = 0, hi = n;
+  while (lo < hi) { const uint32_t mid = (lo + hi) >> 1; if (v[mid] < x) lo = mid + 1; else hi = mid; }
+  return lo;
+}
+// start[g] = first sorted row of group g (start[G] = rows in some group); ntiles[g] = tiles of its run (ntiles[G] = 0)
+__global__ void group_bounds_kernel(const GroupArgs a) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g > a.n_groups) return;
+  const uint32_t s0 = lower_bound_u32(a.key_b, (uint32_t)a.n, (uint32_t)g);
+  a.start[g] = s0;
+  if (g == a.n_groups) { a.ntiles[g] = 0; return; }
+  const uint32_t s1 = lower_bound_u32(a.key_b, (uint32_t)a.n, (uint32_t)g + 1);
+  a.ntiles[g] = (s1 - s0 + kGroupTile - 1) / kGroupTile;
+}
+// the tile this block reduces: its group (the last g with tile_first[g] <= tile) and its sorted rows [row0, row1)
+OPTB_DEV bool find_tile(const GroupArgs& a, long long tile, int& g, uint32_t& row0, uint32_t& row1) {
+  if (tile >= a.tile_first[a.n_groups]) return false;
+  int lo = 0, hi = a.n_groups;  // invariant: tile_first[lo] <= tile < tile_first[hi]
+  while (hi - lo > 1) { const int mid = (lo + hi) >> 1; if (a.tile_first[mid] <= tile) lo = mid; else hi = mid; }
+  g = lo;
+  row0 = a.start[g] + (uint32_t)(tile - a.tile_first[g]) * kGroupTile;
+  row1 = min(row0 + (uint32_t)kGroupTile, a.start[g + 1]);
+  return true;
+}
+// first pass over one tile: the sums, extrema and histogram of optb_monitor_stats, and the per-row outputs
+__global__ void __launch_bounds__(kGroupThreads) group_stats_kernel(const GroupArgs a) {
+  __shared__ unsigned int s_hist[OPTB_HIST_BINS];
+  __shared__ double s_red[OPTB_MS_M2_Y][kGroupThreads / 32];
+  int g; uint32_t row0, row1;
+  const long long tile = blockIdx.x;
+  if (!find_tile(a, tile, g, row0, row1)) return;
+  if (threadIdx.x < OPTB_HIST_BINS) s_hist[threadIdx.x] = 0u;
+  __syncthreads();
+  const optb_monitor_frame f = a.frames[g];
+  double v[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};  // count, I, y, yy, z, zz, waist, tY, tYtY
+  double ymin = INFINITY, ymax = -INFINITY, zmin = INFINITY, zmax = -INFINITY;
+  for (uint32_t i = row0 + threadIdx.x; i < row1; i += kGroupThreads) {
+    const uint32_t k = a.idx_b[i];
+    const long long j = a.first + k;
+    double y, z, ty, tz, wd;
+    const int b = eval_row(a, j, f, y, z, ty, tz, wd);
+    v[0] += 1.0; v[1] += a.I[j]; v[2] += y; v[3] = fma(y, y, v[3]); v[4] += z; v[5] = fma(z, z, v[5]);
+    ymin = fmin(ymin, y); ymax = fmax(ymax, y); zmin = fmin(zmin, z); zmax = fmax(zmax, z);
+    if (b >= 0) atomicAdd(&s_hist[b], 1u);  // integer counts: the order of the atomics does not matter
+    if (a.dx) {
+      v[7] += ty; v[8] = fma(ty, ty, v[8]);
+      if (a.qre) v[6] += wd;
+    }
+    if (a.y) a.y[k] = y;
+    if (a.z) a.z[k] = z;
+    if (a.ty) a.ty[k] = ty;
+    if (a.tz) a.tz[k] = tz;
+    if (a.wd) a.wd[k] = wd;
+  }
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+    for (int q = 0; q < 9; q++) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
+    ymin = fmin(ymin, __shfl_xor_sync(0xffffffffu, ymin, o)); ymax = fmax(ymax, __shfl_xor_sync(0xffffffffu, ymax, o));
+    zmin = fmin(zmin, __shfl_xor_sync(0xffffffffu, zmin, o)); zmax = fmax(zmax, __shfl_xor_sync(0xffffffffu, zmax, o));
+  }
+  if (lane == 0) {  // s_red is indexed by stats slot: these are slots 0..12
+    s_red[OPTB_MS_COUNT][wid] = v[0]; s_red[OPTB_MS_SUM_I][wid] = v[1]; s_red[OPTB_MS_SUM_Y][wid] = v[2];
+    s_red[OPTB_MS_SUM_YY][wid] = v[3]; s_red[OPTB_MS_SUM_Z][wid] = v[4]; s_red[OPTB_MS_SUM_ZZ][wid] = v[5];
+    s_red[OPTB_MS_SUM_WD][wid] = v[6]; s_red[OPTB_MS_SUM_TY][wid] = v[7]; s_red[OPTB_MS_SUM_TYTY][wid] = v[8];
+    s_red[OPTB_MS_MIN_Y][wid] = ymin; s_red[OPTB_MS_MAX_Y][wid] = ymax; s_red[OPTB_MS_MIN_Z][wid] = zmin; s_red[OPTB_MS_MAX_Z][wid] = zmax;
+  }
+  __syncthreads();
+  if (threadIdx.x < 13) {
+    const int q = threadIdx.x;
+    const bool mn = slot_is_min(q), mx = slot_is_max(q);
+    double tot = s_red[q][0];
+    for (int w = 1; w < kGroupThreads / 32; w++) tot = mn ? fmin(tot, s_red[q][w]) : mx ? fmax(tot, s_red[q][w]) : tot + s_red[q][w];
+    a.part[q * a.part_stride + tile] = tot;
+  }
+  if (threadIdx.x < OPTB_HIST_BINS) a.part[(OPTB_MS_HIST + threadIdx.x) * a.part_stride + tile] = (double)s_hist[threadIdx.x];
+  // the slots this pass does not fill (M2_*: the second pass; the two after the histogram: unused) combine to zero
+  if (threadIdx.x >= 32 && threadIdx.x < 37) {
+    const int r = threadIdx.x - 32;
+    a.part[(r < 3 ? OPTB_MS_M2_Y + r : OPTB_MS_HIST + OPTB_HIST_BINS + r - 3) * a.part_stride + tile] = 0.0;
+  }
+}
+// second pass over one tile: sums of squares about the group's means (what monitor_m2_kernel does for one monitor)
+__global__ void __launch_bounds__(kGroupThreads) group_m2_kernel(const GroupArgs a) {
+  __shared__ double s_red[3][kGroupThreads / 32];
+  int g; uint32_t row0, row1;
+  const long long tile = blockIdx.x;
+  if (!find_tile(a, tile, g, row0, row1)) return;
+  const optb_monitor_frame f = a.frames[g];
+  const double* s = a.stats + (long long)g * OPTB_MS_STRIDE;
+  const double n = s[OPTB_MS_COUNT];
+  const double my = s[OPTB_MS_SUM_Y] / n, mz = s[OPTB_MS_SUM_Z] / n, mty = s[OPTB_MS_SUM_TY] / n;
+  double v[3] = {0.0, 0.0, 0.0};
+  for (uint32_t i = row0 + threadIdx.x; i < row1; i += kGroupThreads) {
+    const long long j = a.first + a.idx_b[i];
+    double y, z, ty, tz, wd;
+    eval_row(a, j, f, y, z, ty, tz, wd);
+    y -= my; z -= mz;
+    v[0] = fma(y, y, v[0]); v[1] = fma(z, z, v[1]);
+    if (a.dx) {
+      ty -= mty;
+      v[2] = fma(ty, ty, v[2]);
+    }
+  }
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+#pragma unroll
+  for (int q = 0; q < 3; q++) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
+    if (lane == 0) s_red[q][wid] = v[q];
+  }
+  __syncthreads();
+  if (threadIdx.x < 3) {
+    double tot = s_red[threadIdx.x][0];
+    for (int w = 1; w < kGroupThreads / 32; w++) tot += s_red[threadIdx.x][w];
+    a.part[(OPTB_MS_M2_Y + threadIdx.x) * a.part_stride + tile] = tot;
+  }
+}
+// one warp per group: slots [q0, q1) of stats[g] from the group's tile partials, in tile order (lane l takes tiles
+// l, l + 32, ...; then a fixed shuffle tree). A group without rows gets the values of optb_monitor_stats over no rows.
+__global__ void group_combine_kernel(const GroupArgs a, int q0, int q1) {
+  const long long g = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  if (g >= a.n_groups) return;
+  const int lane = threadIdx.x & 31;
+  const uint32_t t0 = a.tile_first[g], t1 = a.tile_first[g + 1];
+  for (int q = q0; q < q1; q++) {
+    const bool mn = slot_is_min(q), mx = slot_is_max(q);
+    double v = mn ? INFINITY : mx ? -INFINITY : 0.0;
+    for (uint32_t t = t0 + lane; t < t1; t += 32) {
+      const double p = a.part[q * a.part_stride + t];
+      v = mn ? fmin(v, p) : mx ? fmax(v, p) : v + p;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const double w = __shfl_xor_sync(0xffffffffu, v, o);
+      v = mn ? fmin(v, w) : mx ? fmax(v, w) : v + w;
+    }
+    if (lane == 0) a.stats[g * OPTB_MS_STRIDE + q] = v;
+  }
+}
+}  // namespace
+
+extern "C" int64_t optb_monitor_stats_grouped_workspace_bytes(int64_t n_rows, int32_t n_groups) {
+  if (n_rows < 0 || n_rows >= 0x7fffffffll || n_groups < 1 || n_groups > kMaxGroups) return -1;
+  return (int64_t)group_layout(n_rows, n_groups).total;
+}
+
+extern "C" int optb_monitor_stats_grouped(optb_ctx* ctx, const optb_result* rows, int64_t first, int64_t n,
+                                          int64_t rays_per_config, int32_t n_configs, int32_t n_monitors,
+                                          const optb_monitor_frame* frames, double* stats, double* y, double* z,
+                                          double* ty, double* tz, double* waist, void* workspace,
+                                          int64_t workspace_bytes, void* stream_v) {
+  if (!ctx || !rows || !frames || !stats || first < 0 || n < 0 || rays_per_config < 0 || n_configs < 1 || n_monitors < 1)
+    return -1;
+  if (!rows->hit_px || !rows->hit_py || !rows->hit_pz || !rows->hit_intensity || !rows->hit_t)
+    return fail(ctx, -7, "optb_monitor_stats_grouped: hit_px/py/pz, hit_intensity and hit_t are required");
+  if (!rows->hit_monitor && !rows->hit_key)
+    return fail(ctx, -7, "optb_monitor_stats_grouped: the monitor of a row needs hit_monitor or hit_key");
+  if (rays_per_config > 0 && !rows->hit_root && !rows->hit_key)
+    return fail(ctx, -7, "optb_monitor_stats_grouped: the configuration of a row needs hit_root or hit_key");
+  if ((ty || tz || waist) && !(rows->hit_dx && rows->hit_dy && rows->hit_dz)) return fail(ctx, -7, "optb_monitor_stats_grouped: slopes / waist distances need hit_dx, hit_dy, hit_dz");
+  if (waist && !rows->hit_q_re) return fail(ctx, -7, "optb_monitor_stats_grouped: waist distances need hit_q_re");
+  if (n_monitors > 256) return fail(ctx, -7, "optb_monitor_stats_grouped: at most 256 monitors");
+  if ((long long)n_configs * n_monitors > kMaxGroups) return fail(ctx, -7, "optb_monitor_stats_grouped: n_configs * n_monitors must be at most 2^20");
+  if (n >= 0x7fffffffll) return fail(ctx, -7, "optb_monitor_stats_grouped: at most 2^31-1 rows");
+  const int G = n_configs * n_monitors;
+  const GroupLayout L = group_layout(n, G);
+  if (!workspace || workspace_bytes < (int64_t)L.total)
+    return fail(ctx, -7, "optb_monitor_stats_grouped: workspace too small (optb_monitor_stats_grouped_workspace_bytes)");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream_v;
+  unsigned char* ws = (unsigned char*)workspace;
+  GroupArgs a;
+  a.px = rows->hit_px; a.py = rows->hit_py; a.pz = rows->hit_pz; a.I = rows->hit_intensity; a.t = rows->hit_t;
+  a.dx = rows->hit_dx && rows->hit_dy && rows->hit_dz ? rows->hit_dx : nullptr; a.dy = rows->hit_dy; a.dz = rows->hit_dz;
+  a.qre = rows->hit_q_re;
+  a.root = rows->hit_root; a.mon = rows->hit_monitor; a.key = (const unsigned long long*)rows->hit_key;
+  a.first = first; a.n = n; a.per_config = rays_per_config; a.n_configs = n_configs; a.n_monitors = n_monitors; a.n_groups = G;
+  a.frames = frames;
+  a.stats = stats; a.y = y; a.z = z; a.ty = ty; a.tz = tz; a.wd = waist;
+  a.key_a = (uint32_t*)(ws + L.key_a); a.key_b = (uint32_t*)(ws + L.key_b);
+  a.idx_a = (uint32_t*)(ws + L.idx_a); a.idx_b = (uint32_t*)(ws + L.idx_b);
+  a.start = (uint32_t*)(ws + L.start); a.ntiles = (uint32_t*)(ws + L.ntiles); a.tile_first = (uint32_t*)(ws + L.tile_first);
+  a.part = (double*)(ws + L.part); a.part_stride = L.tiles_cap;
+  if (n > 0) {
+    const int grid = (int)std::min<long long>((n + 255) / 256, (long long)ctx->sm_count * 16);
+    group_keys_kernel<<<grid, 256, 0, st>>>(a);
+    size_t tb = L.cub_bytes;
+    CK(cub::DeviceRadixSort::SortPairs(ws + L.cub, tb, (const uint32_t*)a.key_a, a.key_b, (const uint32_t*)a.idx_a, a.idx_b,
+                                       (int)n, 0, L.end_bit, st), "radix sort of the row groups");
+  }
+  group_bounds_kernel<<<(G + 1 + 255) / 256, 256, 0, st>>>(a);
+  size_t tb = L.cub_bytes;
+  CK(cub::DeviceScan::ExclusiveSum(ws + L.cub, tb, (const uint32_t*)a.ntiles, a.tile_first, G + 1, st), "scan of the tile counts");
+  const long long gw = ((long long)G * 32 + 255) / 256;
+  group_stats_kernel<<<(unsigned)L.tiles_cap, kGroupThreads, 0, st>>>(a);
+  group_combine_kernel<<<(unsigned)gw, 256, 0, st>>>(a, 0, OPTB_MS_STRIDE);
+  group_m2_kernel<<<(unsigned)L.tiles_cap, kGroupThreads, 0, st>>>(a);
+  group_combine_kernel<<<(unsigned)gw, 256, 0, st>>>(a, OPTB_MS_M2_Y, OPTB_MS_HIST);
+  CK(cudaGetLastError(), "optb_monitor_stats_grouped");
   return 0;
 }
 

@@ -104,6 +104,32 @@ class SweepResult:
             self._bounds = torch.searchsorted(root.long() & 0xFFFFFFFF, starts).tolist()
         else:
             self._bounds = [0] * (K + 1)
+        self._grouped = None
+
+    def _grouped_stats(self):
+        from .analytics import grouped_stats
+
+        if "hit_px" not in self.hits:
+            raise ValueError("SweepResult.stats / row_values: this sweep was traced with record_hits=False, so it kept no "
+                             "monitor rows to summarise")
+        if self._grouped is None:
+            M = len(self.tables[0].monitors)
+            monitors = [[t.monitors[m] for m in range(M)] for t in self.tables]
+            self._grouped = grouped_stats(self.hits, monitors, self.n, self.engine)
+        return self._grouped
+
+    def stats(self) -> dict:
+        """Summaries of every configuration k and monitor m from one device call over all monitor rows
+        (`optb_monitor_stats_grouped`; each in the frame of tables[k].monitors[m]) and one copy back: the keys of
+        `DeviceMonitor.stats()` as numpy arrays [K, M] (hist_y [K, M, 30]), plus `std_tY` and `std_histy`. The same
+        sweep gives the same bits on every call, so a ranking of configurations does not change between calls."""
+        return self._grouped_stats()[0]
+
+    def row_values(self) -> dict:
+        """Per-row y, z, tY, tZ and waist_distance, each row evaluated in its own configuration's monitor frame: CUDA
+        tensors aligned with `hits`, from the same device call as `stats()`."""
+        v = self._grouped_stats()[1]
+        return dict(zip(("y", "z", "tY", "tZ", "waist_distance"), v))
 
     def rows(self, k: int) -> dict:
         """Configuration k's monitor rows (views of the sorted columns) with `hit_root` (and `hit_key`) rebased to the
