@@ -366,6 +366,25 @@ int optb_scene_destroy(optb_ctx* ctx, optb_scene* scene);
  * written for this entry point against an older library fails to link instead.                                     */
 int optb_scene_upload_sweep(optb_ctx* ctx, const optb_scene_desc* descs, int32_t n_configs, optb_scene** out);
 
+/* Sweep scene from one base scene plus the rows that differ: for a sweep that varies a few components and monitors of
+ * a large scene (a tolerance or Monte Carlo study), only those rows travel, and the K configuration blobs are written on
+ * the device. Configuration k is `base` with
+ *   - node_i / node_f row nodes[v] replaced by node_i[k][v] / node_f[k][v] (host arrays [K][n_var_nodes][OPTB_NI_STRIDE]
+ *     and [K][n_var_nodes][OPTB_NF_STRIDE]), and
+ *   - mon_f record monitors[w] replaced by mon_f[k][w] ([K][n_var_monitors][OPTB_MON_STRIDE]);
+ * mat_kind, mat_f and aux are the base's in every configuration. The handle has exactly the contract of
+ * optb_scene_upload_sweep (the K * N root numbering, [K][n_monitors] histograms, the same -7 rejections, update_nodes
+ * refused), and every configuration blob is byte for byte the one optb_scene_upload_sweep builds from the K materialised
+ * descriptions, cull bits and kernel choice included (a reflectivity that is > 0 in one configuration picks the
+ * splitting kernels). Synchronous: the scene is ready when the call returns.
+ * Fails with -5 when a node or monitor index is out of range or repeated, when a varied node_i row differs from the
+ * base's in a column other than OPTB_NI_ORTHO (naming the configuration, row and column) or a varied row fails the checks
+ * optb_scene_upload applies to a node (naming the configuration and row); with -6 when the K blobs exceed the scene
+ * size limit. Added without a change of OPTB_ABI_VERSION: no struct changed.                                        */
+int optb_scene_upload_sweep_rows(optb_ctx* ctx, const optb_scene_desc* base, int32_t n_configs,
+                                 const int32_t* nodes, int32_t n_var_nodes, const double* node_f, const int32_t* node_i,
+                                 const int32_t* monitors, int32_t n_var_monitors, const double* mon_f, optb_scene** out);
+
 /* Rewrite the rows of the listed nodes of an uploaded scene from `desc` (the tables the scene was uploaded from, with
  * those rows changed in place: same node count, kinds, skip pointers, materials and aux pool). What a GUI loop needs
  * when one component moved (optable/interact.py:455-457 re-runs the user's script per slider event): a few hundred

@@ -83,7 +83,8 @@ class Result(C.Structure):
 
 EXPORTED_SYMBOLS = (
     "optb_abi_version", "optb_ctx_create", "optb_ctx_destroy", "optb_last_error",
-    "optb_scene_upload", "optb_scene_upload_sweep", "optb_scene_destroy", "optb_scene_update_nodes", "optb_workspace_bytes", "optb_trace",
+    "optb_scene_upload", "optb_scene_upload_sweep", "optb_scene_upload_sweep_rows", "optb_scene_destroy",
+    "optb_scene_update_nodes", "optb_workspace_bytes", "optb_trace",
     "optb_trace_host", "optb_measure_fp64_peak",
     "optb_sort_workspace_bytes", "optb_sort_rows", "optb_monitor_stats",
     "optb_monitor_stats_grouped_workspace_bytes", "optb_monitor_stats_grouped",

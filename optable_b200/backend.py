@@ -36,6 +36,9 @@ def lib():
         L.optb_last_error.argtypes = [C.c_void_p]
         L.optb_scene_upload.argtypes = [C.c_void_p, C.POINTER(A.SceneDesc), C.POINTER(C.c_void_p)]
         L.optb_scene_upload_sweep.argtypes = [C.c_void_p, C.POINTER(A.SceneDesc), C.c_int32, C.POINTER(C.c_void_p)]
+        L.optb_scene_upload_sweep_rows.argtypes = [C.c_void_p, C.POINTER(A.SceneDesc), C.c_int32, C.c_void_p, C.c_int32,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                                   C.POINTER(C.c_void_p)]
         L.optb_scene_destroy.argtypes = [C.c_void_p, C.c_void_p]
         L.optb_workspace_bytes.restype = C.c_int64
         L.optb_workspace_bytes.argtypes = [C.c_void_p, C.c_int64, C.c_int64]
@@ -91,18 +94,28 @@ def runs_wavefront(flats, params: A.Params) -> bool:
 
 
 class Scene:
-    """Device-resident scene tables (optb_scene handle). With `configs` (a list of FlatScene of one topology) it is a
-    sweep scene (optb_scene_upload_sweep): `flat` is then configs[0], and every trace runs its bundle through all
-    `n_configs` configurations."""
+    """Device-resident scene tables (optb_scene handle). With `configs` it is a sweep scene, and every trace runs its
+    bundle through all `n_configs` configurations: `configs` is a list of FlatScene of one topology
+    (optb_scene_upload_sweep; `flat` is then configs[0]) or a sweep.SweepRows, a base scene plus the rows that differ
+    (optb_scene_upload_sweep_rows; `flat` is then its base). `self.configs` holds what runs_wavefront and the cap check
+    read: the FlatScenes, or the one SweepRows, whose properties cover all its configurations."""
 
     def __init__(self, engine, flat: FlatScene, configs=None):
+        from .sweep import SweepRows
+
         self.engine, self.flat = engine, flat
-        self.configs = list(configs) if configs is not None else [flat]
-        self.n_configs = len(self.configs)
+        rows = configs if isinstance(configs, SweepRows) else None
+        self.configs = [rows] if rows is not None else list(configs) if configs is not None else [flat]
+        self.n_configs = rows.n_configs if rows is not None else len(self.configs)
         self.sweep = configs is not None
         self.max_children = max(f.max_children for f in self.configs)
         h = C.c_void_p()
-        if self.sweep:
+        if rows is not None:
+            desc = flat.desc()
+            engine._check(lib().optb_scene_upload_sweep_rows(
+                engine._ctx, C.byref(desc), rows.n_configs, rows.nodes.ctypes.data, rows.nodes.size, rows.node_f.ctypes.data,
+                rows.node_i.ctypes.data, rows.monitors.ctypes.data, rows.monitors.size, rows.mon_f.ctypes.data, C.byref(h)))
+        elif self.sweep:
             descs = (A.SceneDesc * self.n_configs)(*[f.desc() for f in self.configs])   # (the arrays stay alive in configs)
             engine._check(lib().optb_scene_upload_sweep(engine._ctx, descs, self.n_configs, C.byref(h)))
         else:
@@ -161,9 +174,12 @@ class Engine:
     def upload(self, flat: FlatScene) -> Scene:
         return Scene(self, flat)
 
-    def upload_sweep(self, flats) -> Scene:
-        """One sweep scene from the FlatScenes of K configurations with the same topology (optb_scene_upload_sweep)."""
-        return Scene(self, flats[0], configs=flats)
+    def upload_sweep(self, configs) -> Scene:
+        """One sweep scene from the FlatScenes of K configurations with the same topology (optb_scene_upload_sweep), or
+        from a sweep.SweepRows (optb_scene_upload_sweep_rows)."""
+        from .sweep import SweepRows
+
+        return Scene(self, configs.flat if isinstance(configs, SweepRows) else configs[0], configs=configs)
 
     def fp64_peak_tflops(self) -> float:
         v = C.c_double(0)

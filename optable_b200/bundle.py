@@ -110,7 +110,8 @@ HIT_COLUMNS_ALL = A.HIT_I32 + A.HIT_U32 + A.HIT_F64
 class DeviceTrace:
     """Reusable device-side state for repeated traces of same-shaped bundles through one scene: scene tables,
     result buffers and workspace are allocated once; `run` only enqueues kernels. With `configs` (the FlatScenes of a
-    sweep, `flat` = configs[0]) the scene is a sweep scene and one run traces the bundle through every configuration."""
+    sweep, `flat` = configs[0], or a SweepRows, `flat` = its base) the scene is a sweep scene and one run traces the
+    bundle through every configuration."""
 
     def __init__(self, engine, flat, n_rays, hit_capacity, seg_capacity=0, hit_columns=HIT_COLUMNS_ALL,
                  max_trace_num=2000, unit=1e-2, record_hist=False, chain_len=0, flag_ambiguity=False, configs=None):
@@ -128,8 +129,7 @@ class DeviceTrace:
         if flat.n_capslots:
             # a bundle ray is its own `_id` family starting from zero counts: a cap can only bind if it is
             # smaller than the pop budget. Binding caps need Ray objects (OpticalTable.ray_tracing).
-            capmax = min(f.node_f[f.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX].min() for f in self.scene.configs)
-            if capmax < max_trace_num:
+            if min(f.cap_min for f in self.scene.configs) < max_trace_num:
                 raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped component")
             slack = 1
         self.prm = engine.make_params(max_trace_num, unit, seg_capacity > 0, hit_capacity > 0, record_hist, chain_len,

@@ -963,6 +963,44 @@ __global__ void __launch_bounds__(256) dfma_kernel(double* out, int iters) {
   out[blockIdx.x * blockDim.x + threadIdx.x] = a0 + a1 + a2 + a3 + a4 + a5 + a6 + a7;
 }
 
+// Bytes of one varied node's rows in blob form (traversal record, node_f, node_i) and of one monitor record; every
+// blob section starts 16-byte aligned and these row sizes are multiples of 16, so no 16-byte word straddles two rows.
+constexpr uint32_t kTravBytes = 64, kNfBytes = OPTB_NF_STRIDE * 8, kNiBytes = OPTB_NI_STRIDE * 4;
+constexpr uint32_t kVarNodeBytes = kTravBytes + kNfBytes + kNiBytes, kMonBytes = kMonBlobStride * 8;
+static_assert(kNfBytes % 16 == 0 && kNiBytes % 16 == 0 && kMonBytes % 16 == 0, "blob rows must be whole 16-byte words");
+
+// optb_scene_upload_sweep_rows: writes the K configuration blobs of a sweep scene, each 16-byte word once. A word of
+// configuration k is the base blob's word unless it lies in the row of a node or monitor with a slot (slot >= 0), in
+// which case it comes from configuration k's rows: `rows` holds per configuration [n_var_nodes][kVarNodeBytes] then
+// [n_var_mons][kMonBytes], `cfg_bytes` apart. The base blob is read by every configuration and stays in L2.
+__global__ void __launch_bounds__(256) sweep_build_kernel(uint4* __restrict__ out, const uint4* __restrict__ base,
+                                                         const unsigned char* __restrict__ rows,
+                                                         const int32_t* __restrict__ node_slot,
+                                                         const int32_t* __restrict__ mon_slot, SceneOff off, int n_nodes,
+                                                         int n_mons, uint32_t stride_words, uint32_t total_words,
+                                                         uint32_t cfg_bytes, uint32_t mon_rows_at) {
+  for (uint32_t w = blockIdx.x * blockDim.x + threadIdx.x; w < total_words; w += gridDim.x * blockDim.x) {
+    const uint32_t k = w / stride_words, o = (w - k * stride_words) * 16;
+    const unsigned char* cfg = rows + (size_t)k * cfg_bytes;
+    const uint4* src = base + (w - k * stride_words);
+    // (section, row, byte in the row) of the word; the traversal records start at offset 0
+    uint32_t row = 0, in_row = 0, at = 0;
+    int slot = -1;
+    if (o < off.matk) {
+      if (o < off.nf) { row = o / kTravBytes; in_row = o - row * kTravBytes; at = 0; }
+      else if (o < off.ni) { row = (o - off.nf) / kNfBytes; in_row = o - off.nf - row * kNfBytes; at = kTravBytes; }
+      else { row = (o - off.ni) / kNiBytes; in_row = o - off.ni - row * kNiBytes; at = kTravBytes + kNfBytes; }
+      if ((int)row < n_nodes) slot = node_slot[row];
+      if (slot >= 0) src = (const uint4*)(cfg + (size_t)slot * kVarNodeBytes + at + in_row);
+    } else if (o >= off.mon && o < off.aux) {
+      row = (o - off.mon) / kMonBytes;
+      if ((int)row < n_mons) slot = mon_slot[row];
+      if (slot >= 0) src = (const uint4*)(cfg + mon_rows_at + (size_t)slot * kMonBytes + (o - off.mon - row * kMonBytes));
+    }
+    out[w] = *src;
+  }
+}
+
 size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 }  // namespace
@@ -1068,9 +1106,10 @@ extern "C" const char* optb_last_error(const optb_ctx* ctx) { return ctx ? ctx->
 // object's own `.bbox`): a stale box is still TESTED like the reference does, but never used for dismissal. A group is
 // cullable when its box contains the boxes of all its children, all of them cullable. Capped leaves count every
 // geometric hit, closest or not (optical_component.py:359-362): never cullable, nor is any group above them.
-static void cull_bits(const optb_scene_desc* d, std::vector<unsigned char>& cull) {
-  const int n = d->n_nodes;
-  cull.assign(n, 0);
+// One node's bit: `nf` is node i's node_f row; a group reads its children's rows and bits through row_of(j) / cull_of(j)
+// (node_i, which fixes the tree, comes from `d`).
+template <class RowOf, class CullOf>
+static bool cull_node(const optb_scene_desc* d, int i, const double* nf, RowOf row_of, CullOf cull_of) {
   auto contains = [](const double* outer, const double* inner) {
     for (int ax = 0; ax < 3; ax++) {
       const double tol = 1e-9 * std::max(1.0, std::max(fabs(inner[2 * ax]), fabs(inner[2 * ax + 1])));
@@ -1078,43 +1117,48 @@ static void cull_bits(const optb_scene_desc* d, std::vector<unsigned char>& cull
     }
     return true;
   };
-  for (int i = n - 1; i >= 0; i--) {  // children before parents (pre-order table, reverse scan)
-    const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
-    const double* nf = d->node_f + (size_t)i * OPTB_NF_STRIDE;
-    if (!ni[OPTB_NI_AABB]) continue;
-    const int g = ni[OPTB_NI_GEOM];
-    if (g == OPTB_G_GROUP || g == OPTB_G_GRID) {
-      bool ok = true;
-      for (int j = i + 1; j < ni[OPTB_NI_SKIP] && ok; j = d->node_i[(size_t)j * OPTB_NI_STRIDE + OPTB_NI_SKIP])
-        ok = cull[j] && contains(nf + OPTB_NF_AABB, d->node_f + (size_t)j * OPTB_NF_STRIDE + OPTB_NF_AABB);
-      cull[i] = ok && ni[OPTB_NI_SKIP] > i + 1;
-      continue;
-    }
-    if (ni[OPTB_NI_CAPSLOT] >= 0) continue;
-    const double* p = nf + OPTB_NF_P;
-    double e[6];  // geometric extent of the hittable points in the local frame
-    switch (g) {
-      case OPTB_G_CIRCLE: e[0] = e[1] = 0; e[2] = e[4] = -p[0]; e[3] = e[5] = p[0]; break;
-      case OPTB_G_RECT: e[0] = e[1] = 0; e[2] = -p[0]; e[3] = p[0]; e[4] = -p[1]; e[5] = p[1]; break;
-      case OPTB_G_SPHERE: for (int k = 0; k < 6; k++) e[k] = p[2 + k]; break;
-      case OPTB_G_ASPHERE: e[0] = p[6]; e[1] = p[7]; e[2] = e[4] = -p[0]; e[3] = e[5] = p[0]; break;
-      case OPTB_G_CYL: e[0] = e[2] = -p[0]; e[1] = e[3] = p[0]; e[4] = -p[1] / 2; e[5] = p[1] / 2; break;
-      default: continue;  // polygons, composite apertures: boxes are tested, not used for dismissal
-    }
-    if (!(e[0] <= e[1] && e[2] <= e[3] && e[4] <= e[5])) continue;
-    const double* T = nf + OPTB_NF_T;
-    const double* c = nf + OPTB_NF_ORIGIN;
-    double lab[6] = {INFINITY, -INFINITY, INFINITY, -INFINITY, INFINITY, -INFINITY};
-    for (int corner = 0; corner < 8; corner++) {
-      const double x = e[corner & 1], y = e[2 + ((corner >> 1) & 1)], z = e[4 + ((corner >> 2) & 1)];
-      for (int ax = 0; ax < 3; ax++) {
-        const double v = T[3 * ax] * x + T[3 * ax + 1] * y + T[3 * ax + 2] * z + c[ax];
-        lab[2 * ax] = std::min(lab[2 * ax], v); lab[2 * ax + 1] = std::max(lab[2 * ax + 1], v);
-      }
-    }
-    // (a curved leaf finds roots up to 1e-9 outside its bracket; the tolerance of `contains` covers that)
-    cull[i] = contains(nf + OPTB_NF_AABB, lab);
+  const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
+  if (!ni[OPTB_NI_AABB]) return false;
+  const int g = ni[OPTB_NI_GEOM];
+  if (g == OPTB_G_GROUP || g == OPTB_G_GRID) {
+    bool ok = true;
+    for (int j = i + 1; j < ni[OPTB_NI_SKIP] && ok; j = d->node_i[(size_t)j * OPTB_NI_STRIDE + OPTB_NI_SKIP])
+      ok = cull_of(j) && contains(nf + OPTB_NF_AABB, row_of(j) + OPTB_NF_AABB);
+    return ok && ni[OPTB_NI_SKIP] > i + 1;
   }
+  if (ni[OPTB_NI_CAPSLOT] >= 0) return false;
+  const double* p = nf + OPTB_NF_P;
+  double e[6];  // geometric extent of the hittable points in the local frame
+  switch (g) {
+    case OPTB_G_CIRCLE: e[0] = e[1] = 0; e[2] = e[4] = -p[0]; e[3] = e[5] = p[0]; break;
+    case OPTB_G_RECT: e[0] = e[1] = 0; e[2] = -p[0]; e[3] = p[0]; e[4] = -p[1]; e[5] = p[1]; break;
+    case OPTB_G_SPHERE: for (int k = 0; k < 6; k++) e[k] = p[2 + k]; break;
+    case OPTB_G_ASPHERE: e[0] = p[6]; e[1] = p[7]; e[2] = e[4] = -p[0]; e[3] = e[5] = p[0]; break;
+    case OPTB_G_CYL: e[0] = e[2] = -p[0]; e[1] = e[3] = p[0]; e[4] = -p[1] / 2; e[5] = p[1] / 2; break;
+    default: return false;  // polygons, composite apertures: boxes are tested, not used for dismissal
+  }
+  if (!(e[0] <= e[1] && e[2] <= e[3] && e[4] <= e[5])) return false;
+  const double* T = nf + OPTB_NF_T;
+  const double* c = nf + OPTB_NF_ORIGIN;
+  double lab[6] = {INFINITY, -INFINITY, INFINITY, -INFINITY, INFINITY, -INFINITY};
+  for (int corner = 0; corner < 8; corner++) {
+    const double x = e[corner & 1], y = e[2 + ((corner >> 1) & 1)], z = e[4 + ((corner >> 2) & 1)];
+    for (int ax = 0; ax < 3; ax++) {
+      const double v = T[3 * ax] * x + T[3 * ax + 1] * y + T[3 * ax + 2] * z + c[ax];
+      lab[2 * ax] = std::min(lab[2 * ax], v); lab[2 * ax + 1] = std::max(lab[2 * ax + 1], v);
+    }
+  }
+  // (a curved leaf finds roots up to 1e-9 outside its bracket; the tolerance of `contains` covers that)
+  return contains(nf + OPTB_NF_AABB, lab);
+}
+
+static void cull_bits(const optb_scene_desc* d, std::vector<unsigned char>& cull) {
+  const int n = d->n_nodes;
+  cull.assign(n, 0);
+  auto row_of = [d](int j) { return d->node_f + (size_t)j * OPTB_NF_STRIDE; };
+  auto cull_of = [&cull](int j) { return cull[j] != 0; };
+  for (int i = n - 1; i >= 0; i--)  // children before parents (pre-order table, reverse scan)
+    cull[i] = cull_node(d, i, row_of(i), row_of, cull_of);
 }
 
 // Device-side extras of an asphere row: k1 of the sign / Newton functor (AsphF) in the FOCAL slot, which a refractive
@@ -1126,74 +1170,78 @@ static void asphere_constants(double* nf, const int32_t* ni) {
   else nf[OPTB_NF_FOCAL] = (c[1] + 1.0) / ((c[1] - 1.0) * c[0] * c[0]);
 }
 
-// The kernels index the tables without bounds checks: reject anything that could walk out of them.
+// The kernels index the tables without bounds checks: reject anything that could walk out of them. Node i with the
+// rows `ni` / `nf` (d's own, or a sweep configuration's replacement of them) in the tables of `d`.
+static int validate_node(optb_ctx* ctx, const optb_scene_desc* d, int i, const int32_t* ni, const double* nf) {
+  const int g = ni[OPTB_NI_GEOM];
+  if (ni[OPTB_NI_SKIP] <= i || ni[OPTB_NI_SKIP] > d->n_nodes) return fail(ctx, -5, "scene: node skip pointer out of range");
+  if (g < OPTB_G_GROUP || g > OPTB_G_GRID) return fail(ctx, -5, "scene: unknown geometry kind");
+  if (g == OPTB_G_GRID) {  // lattice descriptor: inside the aux pool, every listed child a leaf of this subtree
+    const long long off = ni[OPTB_NI_AUX];
+    if (off < 0 || off + OPTB_GRID_CELLS > d->n_aux) return fail(ctx, -5, "scene: lattice descriptor out of range");
+    const double* gd = d->aux + off;
+    const double cells = gd[OPTB_GRID_NOUTER] * gd[OPTB_GRID_NINNER] + gd[OPTB_GRID_NEXT];
+    if (!(gd[OPTB_GRID_NOUTER] >= 1 && gd[OPTB_GRID_NINNER] >= 1 && gd[OPTB_GRID_NEXT] >= 0 && cells <= 1e8) ||
+        off + OPTB_GRID_CELLS + (long long)cells > d->n_aux)
+      return fail(ctx, -5, "scene: lattice descriptor out of range");
+    for (long long k = 0; k < (long long)cells; k++) {
+      const double c = gd[OPTB_GRID_CELLS + k];
+      if (!(c > i && c < ni[OPTB_NI_SKIP]) || d->node_i[(size_t)c * OPTB_NI_STRIDE + OPTB_NI_GEOM] == OPTB_G_GROUP ||
+          d->node_i[(size_t)c * OPTB_NI_STRIDE + OPTB_NI_GEOM] == OPTB_G_GRID)
+        return fail(ctx, -5, "scene: lattice child is not a leaf of the group's subtree");
+    }
+  }
+  if (g == OPTB_G_GROUP || g == OPTB_G_GRID) return 0;
+  if (ni[OPTB_NI_SKIP] != i + 1) return fail(ctx, -5, "scene: a leaf must skip to the next node");
+  if (ni[OPTB_NI_INTER] < OPTB_I_MIRROR || ni[OPTB_NI_INTER] > OPTB_I_PASS) return fail(ctx, -5, "scene: unknown interaction kind");
+  if (ni[OPTB_NI_MAT1] < 0 || ni[OPTB_NI_MAT1] >= d->n_materials || ni[OPTB_NI_MAT2] < 0 || ni[OPTB_NI_MAT2] >= d->n_materials)
+    return fail(ctx, -5, "scene: material index out of range");
+  if (ni[OPTB_NI_CAPSLOT] >= d->n_capslots) return fail(ctx, -5, "scene: cap slot out of range");
+  if (ni[OPTB_NI_LEAF] < 0 || ni[OPTB_NI_LEAF] >= d->n_leaves) return fail(ctx, -5, "scene: leaf index out of range");
+  auto poly_ok = [&](long long off) {
+    if (off < 0 || off + OPTB_POLY_HEADER > d->n_aux) return false;
+    const double nv = d->aux[off];
+    return nv >= 3 && nv <= 1e6 && off + OPTB_POLY_HEADER + 2 * (long long)nv <= d->n_aux;
+  };
+  const double* p = nf + OPTB_NF_P;
+  if ((g == OPTB_G_POLY2D || g == OPTB_G_POLY3D) && !poly_ok(ni[OPTB_NI_AUX])) return fail(ctx, -5, "scene: polygon record out of range");
+  if (g == OPTB_G_ASPHERE && ni[OPTB_NI_AUX] != OPTB_ASPH_PARAMETRIC && ni[OPTB_NI_AUX] != OPTB_ASPH_EXACT_SPH)
+    return fail(ctx, -5, "scene: unknown asphere form");
+  if (g == OPTB_G_CSG && (int)p[0] == 2) {  // nested composite: a well-formed postfix program in the aux pool
+    const long long off = ni[OPTB_NI_AUX];
+    if (off < 0 || off + 1 > d->n_aux) return fail(ctx, -5, "scene: CSG program out of range");
+    const double nt = d->aux[off];
+    if (!(nt >= 3 && nt <= 4096) || off + 1 + 3 * (long long)nt > d->n_aux) return fail(ctx, -5, "scene: CSG program out of range");
+    int depth = 0;
+    for (int k = 0; k < (int)nt; k++) {
+      const int code = (int)d->aux[off + 1 + 3 * k];
+      if (code == OPTB_G_CIRCLE || code == OPTB_G_RECT || code == OPTB_G_POLY2D) {
+        if (code == OPTB_G_POLY2D && !poly_ok((long long)d->aux[off + 2 + 3 * k])) return fail(ctx, -5, "scene: CSG polygon out of range");
+        if (++depth > OPTB_CSG_MAX_DEPTH) return fail(ctx, -5, "scene: CSG program nests too deep");
+      } else if (code == OPTB_CSG_SUBTRACT || code == OPTB_CSG_UNION) {
+        if (depth < 2) return fail(ctx, -5, "scene: malformed CSG program");
+        depth--;
+      } else {
+        return fail(ctx, -5, "scene: bad CSG token");
+      }
+    }
+    if (depth != 1) return fail(ctx, -5, "scene: malformed CSG program");
+  } else if (g == OPTB_G_CSG) {
+    if ((int)p[0] != 0 && (int)p[0] != 1) return fail(ctx, -5, "scene: bad CSG op");
+    for (int q = 0; q < 2; q++) {
+      const int k = (int)p[1 + 3 * q];
+      if (k != OPTB_G_CIRCLE && k != OPTB_G_RECT && k != OPTB_G_POLY2D) return fail(ctx, -5, "scene: bad CSG operand");
+      if (k == OPTB_G_POLY2D && !poly_ok((long long)p[2 + 3 * q])) return fail(ctx, -5, "scene: CSG polygon out of range");
+    }
+  }
+  return 0;
+}
+
 static int validate_desc(optb_ctx* ctx, const optb_scene_desc* d) {
   if (d->abi_version != OPTB_ABI_VERSION) return fail(ctx, -4, "scene ABI version mismatch");
   if (d->n_nodes < 0 || d->n_materials < 1) return fail(ctx, -5, "bad scene counts");
-  for (int i = 0; i < d->n_nodes; i++) {
-    const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
-    const int g = ni[OPTB_NI_GEOM];
-    if (ni[OPTB_NI_SKIP] <= i || ni[OPTB_NI_SKIP] > d->n_nodes) return fail(ctx, -5, "scene: node skip pointer out of range");
-    if (g < OPTB_G_GROUP || g > OPTB_G_GRID) return fail(ctx, -5, "scene: unknown geometry kind");
-    if (g == OPTB_G_GRID) {  // lattice descriptor: inside the aux pool, every listed child a leaf of this subtree
-      const long long off = ni[OPTB_NI_AUX];
-      if (off < 0 || off + OPTB_GRID_CELLS > d->n_aux) return fail(ctx, -5, "scene: lattice descriptor out of range");
-      const double* gd = d->aux + off;
-      const double cells = gd[OPTB_GRID_NOUTER] * gd[OPTB_GRID_NINNER] + gd[OPTB_GRID_NEXT];
-      if (!(gd[OPTB_GRID_NOUTER] >= 1 && gd[OPTB_GRID_NINNER] >= 1 && gd[OPTB_GRID_NEXT] >= 0 && cells <= 1e8) ||
-          off + OPTB_GRID_CELLS + (long long)cells > d->n_aux)
-        return fail(ctx, -5, "scene: lattice descriptor out of range");
-      for (long long k = 0; k < (long long)cells; k++) {
-        const double c = gd[OPTB_GRID_CELLS + k];
-        if (!(c > i && c < ni[OPTB_NI_SKIP]) || d->node_i[(size_t)c * OPTB_NI_STRIDE + OPTB_NI_GEOM] == OPTB_G_GROUP ||
-            d->node_i[(size_t)c * OPTB_NI_STRIDE + OPTB_NI_GEOM] == OPTB_G_GRID)
-          return fail(ctx, -5, "scene: lattice child is not a leaf of the group's subtree");
-      }
-    }
-    if (g == OPTB_G_GROUP || g == OPTB_G_GRID) continue;
-    if (ni[OPTB_NI_SKIP] != i + 1) return fail(ctx, -5, "scene: a leaf must skip to the next node");
-    if (ni[OPTB_NI_INTER] < OPTB_I_MIRROR || ni[OPTB_NI_INTER] > OPTB_I_PASS) return fail(ctx, -5, "scene: unknown interaction kind");
-    if (ni[OPTB_NI_MAT1] < 0 || ni[OPTB_NI_MAT1] >= d->n_materials || ni[OPTB_NI_MAT2] < 0 || ni[OPTB_NI_MAT2] >= d->n_materials)
-      return fail(ctx, -5, "scene: material index out of range");
-    if (ni[OPTB_NI_CAPSLOT] >= d->n_capslots) return fail(ctx, -5, "scene: cap slot out of range");
-    if (ni[OPTB_NI_LEAF] < 0 || ni[OPTB_NI_LEAF] >= d->n_leaves) return fail(ctx, -5, "scene: leaf index out of range");
-    auto poly_ok = [&](long long off) {
-      if (off < 0 || off + OPTB_POLY_HEADER > d->n_aux) return false;
-      const double nv = d->aux[off];
-      return nv >= 3 && nv <= 1e6 && off + OPTB_POLY_HEADER + 2 * (long long)nv <= d->n_aux;
-    };
-    const double* p = d->node_f + (size_t)i * OPTB_NF_STRIDE + OPTB_NF_P;
-    if ((g == OPTB_G_POLY2D || g == OPTB_G_POLY3D) && !poly_ok(ni[OPTB_NI_AUX])) return fail(ctx, -5, "scene: polygon record out of range");
-    if (g == OPTB_G_ASPHERE && ni[OPTB_NI_AUX] != OPTB_ASPH_PARAMETRIC && ni[OPTB_NI_AUX] != OPTB_ASPH_EXACT_SPH)
-      return fail(ctx, -5, "scene: unknown asphere form");
-    if (g == OPTB_G_CSG && (int)p[0] == 2) {  // nested composite: a well-formed postfix program in the aux pool
-      const long long off = ni[OPTB_NI_AUX];
-      if (off < 0 || off + 1 > d->n_aux) return fail(ctx, -5, "scene: CSG program out of range");
-      const double nt = d->aux[off];
-      if (!(nt >= 3 && nt <= 4096) || off + 1 + 3 * (long long)nt > d->n_aux) return fail(ctx, -5, "scene: CSG program out of range");
-      int depth = 0;
-      for (int k = 0; k < (int)nt; k++) {
-        const int code = (int)d->aux[off + 1 + 3 * k];
-        if (code == OPTB_G_CIRCLE || code == OPTB_G_RECT || code == OPTB_G_POLY2D) {
-          if (code == OPTB_G_POLY2D && !poly_ok((long long)d->aux[off + 2 + 3 * k])) return fail(ctx, -5, "scene: CSG polygon out of range");
-          if (++depth > OPTB_CSG_MAX_DEPTH) return fail(ctx, -5, "scene: CSG program nests too deep");
-        } else if (code == OPTB_CSG_SUBTRACT || code == OPTB_CSG_UNION) {
-          if (depth < 2) return fail(ctx, -5, "scene: malformed CSG program");
-          depth--;
-        } else {
-          return fail(ctx, -5, "scene: bad CSG token");
-        }
-      }
-      if (depth != 1) return fail(ctx, -5, "scene: malformed CSG program");
-    } else if (g == OPTB_G_CSG) {
-      if ((int)p[0] != 0 && (int)p[0] != 1) return fail(ctx, -5, "scene: bad CSG op");
-      for (int q = 0; q < 2; q++) {
-        const int k = (int)p[1 + 3 * q];
-        if (k != OPTB_G_CIRCLE && k != OPTB_G_RECT && k != OPTB_G_POLY2D) return fail(ctx, -5, "scene: bad CSG operand");
-        if (k == OPTB_G_POLY2D && !poly_ok((long long)p[2 + 3 * q])) return fail(ctx, -5, "scene: CSG polygon out of range");
-      }
-    }
-  }
+  for (int i = 0; i < d->n_nodes; i++)
+    if (int rc = validate_node(ctx, d, i, d->node_i + (size_t)i * OPTB_NI_STRIDE, d->node_f + (size_t)i * OPTB_NF_STRIDE)) return rc;
   return 0;
 }
 
@@ -1214,42 +1262,63 @@ static size_t blob_layout(const optb_scene_desc* d, SceneOff& off) {
   return o;
 }
 
+// Parent of every node, from the skip pointers (pre-order: the innermost open group that still covers i).
+static std::vector<int32_t> node_parents(const optb_scene_desc* d) {
+  std::vector<int32_t> parent(d->n_nodes, -1), open;
+  for (int i = 0; i < d->n_nodes; i++) {
+    const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
+    while (!open.empty() && d->node_i[(size_t)open.back() * OPTB_NI_STRIDE + OPTB_NI_SKIP] <= i) open.pop_back();
+    parent[i] = open.empty() ? -1 : open.back();
+    if (ni[OPTB_NI_GEOM] == OPTB_G_GROUP || ni[OPTB_NI_GEOM] == OPTB_G_GRID) open.push_back(i);
+  }
+  return parent;
+}
+
+// Box word of a traversal record: bit 0 = test the box (component_group.py:98-107), bit 1 = the box may dismiss by
+// distance (cull_bits).
+static int32_t box_word(const int32_t* ni, bool cull) { return (ni[OPTB_NI_AABB] ? 1 : 0) | (cull ? 2 : 0); }
+
+// Blob record of one monitor: the ABI record + the histogram constants derived from it (kMonBlobStride).
+static void mon_record(double* mf, const double* rec) {
+  memcpy(mf, rec, OPTB_MON_STRIDE * 8);
+  const double w = mf[OPTB_MON_HW] - (-mf[OPTB_MON_HW]), h = mf[OPTB_MON_HH] - (-mf[OPTB_MON_HH]);  // hi - lo as hist_bin forms it
+  mf[OPTB_MON_STRIDE] = OPTB_HIST_BINS / w; mf[OPTB_MON_STRIDE + 1] = w / OPTB_HIST_BINS;
+  mf[OPTB_MON_STRIDE + 2] = OPTB_HIST_BINS / h; mf[OPTB_MON_STRIDE + 3] = h / OPTB_HIST_BINS;
+}
+
 // Host image of one scene blob (zeroed `host`, blob_layout bytes); `cull` receives the cullable bit of every node.
 static void fill_blob(const optb_scene_desc* d, const SceneOff& off, unsigned char* host, std::vector<unsigned char>& cull) {
   const size_t b_nf = (size_t)d->n_nodes * OPTB_NF_STRIDE * 8, b_ni = (size_t)d->n_nodes * OPTB_NI_STRIDE * 4;
   if (d->n_nodes) {
     memcpy(host + off.nf, d->node_f, b_nf);
     memcpy(host + off.ni, d->node_i, b_ni);
-    // parent of every node, from the skip pointers (pre-order: the innermost open group that still covers i)
-    std::vector<int32_t> parent(d->n_nodes, -1), open;
-    for (int i = 0; i < d->n_nodes; i++) {
-      const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
-      while (!open.empty() && d->node_i[(size_t)open.back() * OPTB_NI_STRIDE + OPTB_NI_SKIP] <= i) open.pop_back();
-      parent[i] = open.empty() ? -1 : open.back();
-      if (ni[OPTB_NI_GEOM] == OPTB_G_GROUP || ni[OPTB_NI_GEOM] == OPTB_G_GRID) open.push_back(i);
-    }
+    const std::vector<int32_t> parent = node_parents(d);
     cull_bits(d, cull);
     for (int i = 0; i < d->n_nodes; i++) {  // compact traversal records
-      unsigned char* tv = host + off.trav + (size_t)i * 64;
+      unsigned char* tv = host + off.trav + (size_t)i * kTravBytes;
       const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
       memcpy(tv, d->node_f + (size_t)i * OPTB_NF_STRIDE + OPTB_NF_AABB, 48);
-      // box word: bit 0 = test the box (component_group.py:98-107), bit 1 = the box may dismiss by distance (cull_bits)
-      const int32_t pack[4] = {ni[OPTB_NI_GEOM], ni[OPTB_NI_SKIP], (ni[OPTB_NI_AABB] ? 1 : 0) | (cull[i] ? 2 : 0), parent[i]};
+      const int32_t pack[4] = {ni[OPTB_NI_GEOM], ni[OPTB_NI_SKIP], box_word(ni, cull[i]), parent[i]};
       memcpy(tv + 48, pack, 16);
     }
   }
   memcpy(host + off.matk, d->mat_kind, (size_t)d->n_materials * 4);
   memcpy(host + off.matf, d->mat_f, (size_t)d->n_materials * OPTB_MF_STRIDE * 8);
-  for (int m = 0; m < d->n_monitors; m++) {  // ABI record + the histogram constants derived from it (kMonBlobStride)
-    double* mf = (double*)(host + off.mon) + (size_t)m * kMonBlobStride;
-    memcpy(mf, d->mon_f + (size_t)m * OPTB_MON_STRIDE, OPTB_MON_STRIDE * 8);
-    const double w = mf[OPTB_MON_HW] - (-mf[OPTB_MON_HW]), h = mf[OPTB_MON_HH] - (-mf[OPTB_MON_HH]);  // hi - lo as hist_bin forms it
-    mf[OPTB_MON_STRIDE] = OPTB_HIST_BINS / w; mf[OPTB_MON_STRIDE + 1] = w / OPTB_HIST_BINS;
-    mf[OPTB_MON_STRIDE + 2] = OPTB_HIST_BINS / h; mf[OPTB_MON_STRIDE + 3] = h / OPTB_HIST_BINS;
-  }
+  for (int m = 0; m < d->n_monitors; m++)
+    mon_record((double*)(host + off.mon) + (size_t)m * kMonBlobStride, d->mon_f + (size_t)m * OPTB_MON_STRIDE);
   for (int i = 0; i < d->n_nodes; i++) asphere_constants((double*)(host + off.nf) + (size_t)i * OPTB_NF_STRIDE,
                                                          d->node_i + (size_t)i * OPTB_NI_STRIDE);
   if (d->n_aux) memcpy(host + off.aux, d->aux, (size_t)d->n_aux * 8);
+}
+
+// Most rays one interaction of a node can emit.
+static int node_children(const int32_t* ni, const double* nf) {
+  switch (ni[OPTB_NI_INTER]) {
+    case OPTB_I_MIRROR: return (nf[OPTB_NF_REFL] > 0) + (nf[OPTB_NF_TRANS] > 0);
+    case OPTB_I_REFRACT: return nf[OPTB_NF_REFL] > 0 ? 2 : 1;
+    case OPTB_I_THINLENS: case OPTB_I_PASS: return 1;
+    default: return 0;
+  }
 }
 
 // Scene-wide properties that pick the kernel variant. max_children: most children one interaction can emit (decides
@@ -1259,30 +1328,54 @@ static SceneProps scene_props(const optb_scene_desc* d) {
   SceneProps p{0, 0, 0, 0, 0};
   for (int i = 0; i < d->n_nodes; i++) {
     const int32_t* ni = d->node_i + (size_t)i * OPTB_NI_STRIDE;
-    const double* nf = d->node_f + (size_t)i * OPTB_NF_STRIDE;
     if (ni[OPTB_NI_AABB]) p.has_boxes = 1;
     if (ni[OPTB_NI_GEOM] == OPTB_G_ASPHERE) p.has_asph = 1;
     if (ni[OPTB_NI_GEOM] == OPTB_G_GRID) p.has_grid = 1;
     if (ni[OPTB_NI_INTER] == OPTB_I_PASS) p.has_pass = 1;
-    int k = 0;
-    switch (ni[OPTB_NI_INTER]) {
-      case OPTB_I_MIRROR: k = (nf[OPTB_NF_REFL] > 0) + (nf[OPTB_NF_TRANS] > 0); break;
-      case OPTB_I_REFRACT: k = nf[OPTB_NF_REFL] > 0 ? 2 : 1; break;
-      case OPTB_I_THINLENS: case OPTB_I_PASS: k = 1; break;
-      default: k = 0;
-    }
-    p.max_children = std::max(p.max_children, k);
+    p.max_children = std::max(p.max_children, node_children(ni, d->node_f + (size_t)i * OPTB_NF_STRIDE));
   }
   return p;
 }
 
-// One scene (n_cfg = 0) or a sweep of n_cfg configurations of one topology (descs checked by the caller): the
-// configuration blobs lie back to back at a stride of one blob.
-static int scene_upload(optb_ctx* ctx, const optb_scene_desc* ds, int n_cfg, optb_scene** out) {
+// First node_i column other than OPTB_NI_ORTHO in which two rows differ, or -1. The configurations of a sweep may differ
+// in that column only: a leaf index, skip pointer, material and cap slot mean the same in every configuration.
+static int ni_row_differs(const int32_t* a, const int32_t* b) {
+  for (int c = 0; c < OPTB_NI_STRIDE; c++)
+    if (c != OPTB_NI_ORTHO && a[c] != b[c]) return c;
+  return -1;
+}
+
+// Device buffer of at least `bytes`: the smallest retired blob that is large enough, else a new allocation.
+static cudaError_t blob_acquire(optb_ctx* ctx, size_t bytes, unsigned char** p, size_t* cap) {
+  int pick = -1;
+  for (int k = 0; k < 8; k++)
+    if (ctx->pool[k].p && ctx->pool[k].cap >= bytes && (pick < 0 || ctx->pool[k].cap < ctx->pool[pick].cap)) pick = k;
+  if (pick >= 0) {
+    *p = ctx->pool[pick].p; *cap = ctx->pool[pick].cap;
+    ctx->pool[pick].p = nullptr; ctx->pool[pick].cap = 0;
+    return cudaSuccess;
+  }
+  *cap = (bytes + 65535) & ~(size_t)65535;
+  return cudaMalloc((void**)p, *cap);
+}
+
+// Retire a device buffer that no kernel reads any more: into a free pool slot when it is small enough, else freed.
+static void blob_release(optb_ctx* ctx, unsigned char* p, size_t cap) {
+  int slot = -1;
+  if (ctx && cap <= ((size_t)64 << 20))
+    for (int k = 0; k < 8 && slot < 0; k++) if (!ctx->pool[k].p) slot = k;
+  if (slot >= 0) {
+    ctx->pool[slot].p = p; ctx->pool[slot].cap = cap;
+  } else {
+    cudaFree(p);
+  }
+}
+
+// Handle of one scene (n_cfg = 0) or of a sweep of n_cfg configurations with the sizes of `d`: layout, shared-memory
+// plan and a device blob of n_cfg configuration blobs back to back (contents and kernel-selection properties are the
+// caller's to fill).
+static int scene_alloc(optb_ctx* ctx, const optb_scene_desc* d, int n_cfg, optb_scene** out) {
   const int K = std::max(n_cfg, 1);
-  for (int k = 0; k < K; k++)
-    if (int rc = validate_desc(ctx, &ds[k])) return rc;
-  const optb_scene_desc* d = &ds[0];
   cudaSetDevice(ctx->device);
   optb_scene* s = new (std::nothrow) optb_scene();
   if (!s) return -3;
@@ -1294,8 +1387,31 @@ static int scene_upload(optb_ctx* ctx, const optb_scene_desc* ds, int n_cfg, opt
   const size_t o = stride * K;
   if (o > 0xfff00000ull) { delete s; return fail(ctx, -6, "scene too large"); }
   s->blob_bytes = (uint32_t)o; s->cfg_stride = (uint32_t)stride;
-  std::vector<unsigned char> host(o, 0);
+  size_t hist_bytes = (size_t)K * d->n_monitors * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 4;
+  size_t budget = ctx->smem_optin > 2048 ? ctx->smem_optin - 2048 : 0;
+  s->in_smem = !n_cfg && (o <= budget);  // sweep kernels read the tables from global memory (L1/L2)
+  size_t used = s->in_smem ? o : 0;
+  s->hist_smem = (hist_bytes > 0 && used + hist_bytes <= std::min<size_t>(budget, used + 65536));
+  s->smem_bytes = (uint32_t)(used + (s->hist_smem ? hist_bytes : 0));
   if (d->n_nodes) s->cull = new std::vector<unsigned char>();
+  cudaError_t e = blob_acquire(ctx, o, &s->d_blob, &s->blob_cap);
+  if (e != cudaSuccess) { delete s->cull; delete s; return fail(ctx, -10, "cudaMalloc(scene)", e); }
+  e = cudaEventCreateWithFlags(&s->last_use, cudaEventDisableTiming);
+  if (e != cudaSuccess) { optb_scene_destroy(ctx, s); return fail(ctx, -10, "cudaEventCreate(scene)", e); }
+  *out = s;
+  return 0;
+}
+
+// One scene (n_cfg = 0) or a sweep of n_cfg configurations of one topology (descs checked by the caller): the
+// configuration blobs lie back to back at a stride of one blob.
+static int scene_upload(optb_ctx* ctx, const optb_scene_desc* ds, int n_cfg, optb_scene** out) {
+  const int K = std::max(n_cfg, 1);
+  for (int k = 0; k < K; k++)
+    if (int rc = validate_desc(ctx, &ds[k])) return rc;
+  optb_scene* s = nullptr;
+  if (int rc = scene_alloc(ctx, &ds[0], n_cfg, &s)) return rc;
+  const size_t stride = s->cfg_stride;
+  std::vector<unsigned char> host(s->blob_bytes, 0);
   for (int k = 0; k < K; k++) {
     std::vector<unsigned char> cull_k;  // (cull bits are per configuration; the scene keeps the first one's)
     fill_blob(&ds[k], s->off, host.data() + stride * k, k == 0 && s->cull ? *s->cull : cull_k);
@@ -1303,27 +1419,8 @@ static int scene_upload(optb_ctx* ctx, const optb_scene_desc* ds, int n_cfg, opt
     s->max_children = std::max(s->max_children, p.max_children);
     s->has_boxes |= p.has_boxes; s->has_asph |= p.has_asph; s->has_grid |= p.has_grid; s->has_pass |= p.has_pass;
   }
-  size_t hist_bytes = (size_t)K * d->n_monitors * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 4;
-  size_t budget = ctx->smem_optin > 2048 ? ctx->smem_optin - 2048 : 0;
-  s->in_smem = !n_cfg && (o <= budget);  // sweep kernels read the tables from global memory (L1/L2)
-  size_t used = s->in_smem ? o : 0;
-  s->hist_smem = (hist_bytes > 0 && used + hist_bytes <= std::min<size_t>(budget, used + 65536));
-  s->smem_bytes = (uint32_t)(used + (s->hist_smem ? hist_bytes : 0));
-  cudaError_t e = cudaSuccess;
-  int pick = -1;  // smallest retired blob that is large enough
-  for (int k = 0; k < 8; k++)
-    if (ctx->pool[k].p && ctx->pool[k].cap >= o && (pick < 0 || ctx->pool[k].cap < ctx->pool[pick].cap)) pick = k;
-  if (pick >= 0) {
-    s->d_blob = ctx->pool[pick].p; s->blob_cap = ctx->pool[pick].cap;
-    ctx->pool[pick].p = nullptr; ctx->pool[pick].cap = 0;
-  } else {
-    s->blob_cap = (o + 65535) & ~(size_t)65535;
-    e = cudaMalloc((void**)&s->d_blob, s->blob_cap);
-    if (e != cudaSuccess) { delete s->cull; delete s; return fail(ctx, -10, "cudaMalloc(scene)", e); }
-  }
-  e = cudaMemcpy(s->d_blob, host.data(), o, cudaMemcpyHostToDevice);
-  if (e == cudaSuccess) e = cudaEventCreateWithFlags(&s->last_use, cudaEventDisableTiming);
-  if (e != cudaSuccess) { cudaFree(s->d_blob); delete s->cull; delete s; return fail(ctx, -10, "cudaMemcpy(scene)", e); }
+  cudaError_t e = cudaMemcpy(s->d_blob, host.data(), s->blob_bytes, cudaMemcpyHostToDevice);
+  if (e != cudaSuccess) { optb_scene_destroy(ctx, s); return fail(ctx, -10, "cudaMemcpy(scene)", e); }
   *out = s;
   return 0;
 }
@@ -1345,19 +1442,130 @@ extern "C" int optb_scene_upload_sweep(optb_ctx* ctx, const optb_scene_desc* des
       snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in its table sizes", k);
       return fail(ctx, -5, msg);
     }
-    // a leaf index, skip pointer, material slot and cap slot must mean the same in every configuration
-    for (int i = 0; i < d0->n_nodes; i++)
-      for (int c = 0; c < OPTB_NI_STRIDE; c++)
-        if (c != OPTB_NI_ORTHO && d->node_i[(size_t)i * OPTB_NI_STRIDE + c] != d0->node_i[(size_t)i * OPTB_NI_STRIDE + c]) {
-          snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in node_i row %d column %d", k, i, c);
-          return fail(ctx, -5, msg);
-        }
+    for (int i = 0; i < d0->n_nodes; i++) {
+      const int c = ni_row_differs(d->node_i + (size_t)i * OPTB_NI_STRIDE, d0->node_i + (size_t)i * OPTB_NI_STRIDE);
+      if (c >= 0) {
+        snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in node_i row %d column %d", k, i, c);
+        return fail(ctx, -5, msg);
+      }
+    }
     if (memcmp(d->mat_kind, d0->mat_kind, (size_t)d0->n_materials * 4)) {
       snprintf(msg, sizeof msg, "optb_scene_upload_sweep: configuration %d differs from configuration 0 in its material kinds", k);
       return fail(ctx, -5, msg);
     }
   }
   return scene_upload(ctx, descs, n_configs, out);
+}
+
+extern "C" int optb_scene_upload_sweep_rows(optb_ctx* ctx, const optb_scene_desc* base, int32_t n_configs,
+                                            const int32_t* nodes, int32_t n_var_nodes, const double* node_f,
+                                            const int32_t* node_i, const int32_t* monitors, int32_t n_var_monitors,
+                                            const double* mon_f, optb_scene** out) {
+  if (!ctx || !base || !out || n_var_nodes < 0 || n_var_monitors < 0 || (n_var_nodes && (!nodes || !node_f || !node_i)) ||
+      (n_var_monitors && (!monitors || !mon_f)))
+    return -1;
+  const optb_scene_desc* d = base;
+  char msg[768];
+  if (n_configs < 1) return fail(ctx, -5, "optb_scene_upload_sweep_rows: n_configs must be >= 1");
+  if (int rc = validate_desc(ctx, d)) return rc;
+  const int K = n_configs, N = d->n_nodes, M = d->n_monitors;
+  std::vector<int32_t> var_of(N, -1), mon_slot(std::max(M, 1), -1);
+  for (int v = 0; v < n_var_nodes; v++) {
+    const int i = nodes[v];
+    if (i < 0 || i >= N || var_of[i] >= 0) {
+      snprintf(msg, sizeof msg, "optb_scene_upload_sweep_rows: varied node %d (entry %d) is out of range or repeated", i, v);
+      return fail(ctx, -5, msg);
+    }
+    var_of[i] = v;
+  }
+  for (int w = 0; w < n_var_monitors; w++) {
+    const int m = monitors[w];
+    if (m < 0 || m >= M || mon_slot[m] >= 0) {
+      snprintf(msg, sizeof msg, "optb_scene_upload_sweep_rows: varied monitor %d (entry %d) is out of range or repeated", m, w);
+      return fail(ctx, -5, msg);
+    }
+    mon_slot[m] = w;
+  }
+  auto row_i = [&](int k, int v) { return node_i + ((size_t)k * n_var_nodes + v) * OPTB_NI_STRIDE; };
+  auto row_f = [&](int k, int v) { return node_f + ((size_t)k * n_var_nodes + v) * OPTB_NF_STRIDE; };
+  for (int k = 0; k < K; k++)
+    for (int v = 0; v < n_var_nodes; v++) {
+      const int i = nodes[v];
+      const int c = ni_row_differs(row_i(k, v), d->node_i + (size_t)i * OPTB_NI_STRIDE);
+      if (c >= 0) {
+        snprintf(msg, sizeof msg, "optb_scene_upload_sweep_rows: configuration %d differs from the base in node_i row %d column %d", k, i, c);
+        return fail(ctx, -5, msg);
+      }
+      if (validate_node(ctx, d, i, row_i(k, v), row_f(k, v))) {
+        snprintf(msg, sizeof msg, "optb_scene_upload_sweep_rows: configuration %d, node %d: %s", k, i, ctx->err);
+        return fail(ctx, -5, msg);
+      }
+    }
+  optb_scene* s = nullptr;
+  if (int rc = scene_alloc(ctx, d, K, &s)) return rc;
+  // Rows sent per configuration: the varied nodes and all their ancestors (slots in pre-order), whose cull bits follow
+  // their children's boxes and bits; every other node keeps the base's rows and bit. Then the varied monitors.
+  const std::vector<int32_t> parent = node_parents(d);
+  std::vector<int32_t> node_slot(std::max(N, 1), -1), U;
+  for (int v = 0; v < n_var_nodes; v++)
+    for (int i = nodes[v]; i >= 0 && node_slot[i] < 0; i = parent[i]) node_slot[i] = 0;
+  for (int i = 0; i < N; i++)
+    if (node_slot[i] >= 0) { node_slot[i] = (int32_t)U.size(); U.push_back(i); }
+  const size_t stride = s->cfg_stride, n_u = U.size();
+  const size_t maps_at = stride, rows_at = maps_at + align_up((node_slot.size() + mon_slot.size()) * 4, 16);
+  const size_t mon_rows_at = n_u * kVarNodeBytes, cfg_bytes = mon_rows_at + (size_t)n_var_monitors * kMonBytes;
+  // staging: base blob, slot maps, configuration rows
+  std::vector<unsigned char> host(rows_at + K * cfg_bytes, 0);
+  std::vector<unsigned char> cull_tmp;
+  std::vector<unsigned char>& cull = s->cull ? *s->cull : cull_tmp;
+  fill_blob(d, s->off, host.data(), cull);
+  memcpy(host.data() + maps_at, node_slot.data(), node_slot.size() * 4);
+  memcpy(host.data() + maps_at + node_slot.size() * 4, mon_slot.data(), mon_slot.size() * 4);
+  const SceneProps p = scene_props(d);  // kinds, boxes and interactions live in node_i: the same in every configuration
+  s->has_boxes = p.has_boxes; s->has_asph = p.has_asph; s->has_grid = p.has_grid; s->has_pass = p.has_pass;
+  for (int i = 0; i < N; i++)
+    if (var_of[i] < 0) s->max_children = std::max(s->max_children, node_children(d->node_i + (size_t)i * OPTB_NI_STRIDE, d->node_f + (size_t)i * OPTB_NF_STRIDE));
+  std::vector<unsigned char> cull_k(n_u);
+  for (int k = 0; k < K; k++) {
+    unsigned char* cfg = host.data() + rows_at + k * cfg_bytes;
+    auto nf_of = [&](int j) { return var_of[j] >= 0 ? row_f(k, var_of[j]) : d->node_f + (size_t)j * OPTB_NF_STRIDE; };
+    auto ni_of = [&](int j) { return var_of[j] >= 0 ? row_i(k, var_of[j]) : d->node_i + (size_t)j * OPTB_NI_STRIDE; };
+    auto cull_of = [&](int j) { return (node_slot[j] >= 0 ? cull_k[node_slot[j]] : cull[j]) != 0; };
+    for (size_t u = n_u; u-- > 0;) {  // children before parents
+      const int i = U[u];
+      cull_k[u] = cull_node(d, i, nf_of(i), nf_of, cull_of);
+      unsigned char* r = cfg + u * kVarNodeBytes;
+      memcpy(r, host.data() + s->off.trav + (size_t)i * kTravBytes, kTravBytes);  // kind, skip, parent: the base's
+      memcpy(r, nf_of(i) + OPTB_NF_AABB, 48);
+      const int32_t word = box_word(ni_of(i), cull_k[u]);
+      memcpy(r + 56, &word, 4);
+      memcpy(r + kTravBytes, nf_of(i), kNfBytes);
+      asphere_constants((double*)(r + kTravBytes), ni_of(i));
+      memcpy(r + kTravBytes + kNfBytes, ni_of(i), kNiBytes);
+    }
+    for (int v = 0; v < n_var_nodes; v++) s->max_children = std::max(s->max_children, node_children(row_i(k, v), row_f(k, v)));
+    for (int w = 0; w < n_var_monitors; w++)
+      mon_record((double*)(cfg + mon_rows_at + (size_t)w * kMonBytes), mon_f + ((size_t)k * n_var_monitors + w) * OPTB_MON_STRIDE);
+  }
+  // one copy of the staging, one kernel writing every configuration blob (legacy default stream: after the copy)
+  unsigned char* stage = nullptr;
+  size_t stage_cap = 0;
+  cudaError_t e = blob_acquire(ctx, host.size(), &stage, &stage_cap);
+  if (e == cudaSuccess) e = cudaMemcpy(stage, host.data(), host.size(), cudaMemcpyHostToDevice);
+  if (e == cudaSuccess) {
+    const uint32_t total = s->blob_bytes / 16;
+    const int grid = (int)std::min<long long>((total + 255) / 256, (long long)ctx->sm_count * 8);
+    sweep_build_kernel<<<std::max(grid, 1), 256>>>((uint4*)s->d_blob, (const uint4*)stage, stage + rows_at,
+                                                   (const int32_t*)(stage + maps_at), (const int32_t*)(stage + maps_at) + node_slot.size(),
+                                                   s->off, N, M, (uint32_t)(stride / 16), total, (uint32_t)cfg_bytes,
+                                                   (uint32_t)mon_rows_at);
+    e = cudaGetLastError();
+  }
+  if (e == cudaSuccess) e = cudaStreamSynchronize(0);
+  if (stage) blob_release(ctx, stage, stage_cap);
+  if (e != cudaSuccess) { optb_scene_destroy(ctx, s); return fail(ctx, -10, "optb_scene_upload_sweep_rows: building the configurations", e); }
+  *out = s;
+  return 0;
 }
 
 extern "C" int optb_scene_update_nodes(optb_ctx* ctx, optb_scene* s, const optb_scene_desc* d, const int32_t* nodes,
@@ -1388,7 +1596,7 @@ extern "C" int optb_scene_update_nodes(optb_ctx* ctx, optb_scene* s, const optb_
     cull_bits(d, now);
     for (int i = 0; i < d->n_nodes; i++) {
       if (now[i] == (*s->cull)[i]) continue;
-      const int32_t word = (d->node_i[(size_t)i * OPTB_NI_STRIDE + OPTB_NI_AABB] ? 1 : 0) | (now[i] ? 2 : 0);
+      const int32_t word = box_word(d->node_i + (size_t)i * OPTB_NI_STRIDE, now[i]);
       CK(cudaMemcpyAsync(s->d_blob + s->off.trav + (size_t)i * 64 + 56, &word, 4, cudaMemcpyHostToDevice, st), "update box word");
     }
     s->cull->swap(now);
@@ -1403,15 +1611,8 @@ extern "C" int optb_scene_destroy(optb_ctx* ctx, optb_scene* s) {
   if (!s) return 0;
   if (ctx) cudaSetDevice(ctx->device);
   if (s->d_blob) {
-    int slot = -1;
-    if (ctx && s->blob_cap <= ((size_t)64 << 20))
-      for (int k = 0; k < 8 && slot < 0; k++) if (!ctx->pool[k].p) slot = k;
     if (s->used) cudaEventSynchronize(s->last_use);  // no kernel may still be reading the blob
-    if (slot >= 0) {
-      ctx->pool[slot].p = s->d_blob; ctx->pool[slot].cap = s->blob_cap;
-    } else {
-      cudaFree(s->d_blob);
-    }
+    blob_release(ctx, s->d_blob, s->blob_cap);
   }
   if (s->last_use) cudaEventDestroy(s->last_use);
   delete s->cull;

@@ -166,19 +166,18 @@ class FlatScene:
         self.monitors = list(monitors)
         self.mon_f = np.zeros((max(len(self.monitors), 1), A.MON_STRIDE), dtype=np.float64)
         for k, m in enumerate(self.monitors):
-            T = np.asarray(m.transform_matrix, dtype=np.float64)
-            self.mon_f[k, A.MON_ORIGIN:A.MON_ORIGIN + 3] = np.asarray(m.origin, dtype=np.float64)
-            self.mon_f[k, A.MON_TINV:A.MON_TINV + 9] = np.linalg.inv(T).reshape(-1)
-            self.mon_f[k, A.MON_ORTHO] = float(_orthonormal(np.linalg.inv(T)))
-            self.mon_f[k, A.MON_HW] = m.width / 2
-            self.mon_f[k, A.MON_HH] = m.height / 2
-            self.mon_f[k, A.MON_TY:A.MON_TY + 3] = T @ np.array([0.0, 1.0, 0.0])
-            self.mon_f[k, A.MON_TZ:A.MON_TZ + 3] = T @ np.array([0.0, 0.0, 1.0])
+            monitor_record(m, self.mon_f[k])
         self.n_nodes = self.node_i.shape[0]
         self.n_leaves = len(self.leaves)
         self.n_materials = int(self.mat_kind.shape[0])  # >= 1 (a dummy row when nothing refracts)
         self.n_monitors = len(self.monitors)
         self.n_capslots = len(self.capslots)
+
+    @property
+    def cap_min(self) -> float:
+        """Smallest max_interact_count of a capped leaf (+inf without caps)."""
+        caps = self.node_f[self.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX]
+        return float(caps.min()) if caps.size else float("inf")
 
     @functools.cached_property
     def has_pass(self) -> bool:
@@ -651,6 +650,19 @@ class FlatScene:
         d.aux = self.aux.ctypes.data
         d._keepalive = self  # arrays must outlive the struct
         return d
+
+
+def monitor_record(m, row):
+    """Write monitor m's OPTB_MON_* record (include/optb.h) into `row` (float64 [A.MON_STRIDE]) and return it."""
+    T = np.asarray(m.transform_matrix, dtype=np.float64)
+    row[A.MON_ORIGIN:A.MON_ORIGIN + 3] = np.asarray(m.origin, dtype=np.float64)
+    row[A.MON_TINV:A.MON_TINV + 9] = np.linalg.inv(T).reshape(-1)
+    row[A.MON_ORTHO] = float(_orthonormal(np.linalg.inv(T)))
+    row[A.MON_HW] = m.width / 2
+    row[A.MON_HH] = m.height / 2
+    row[A.MON_TY:A.MON_TY + 3] = T @ np.array([0.0, 1.0, 0.0])
+    row[A.MON_TZ:A.MON_TZ + 3] = T @ np.array([0.0, 0.0, 1.0])
+    return row
 
 
 def material_value(m, wavelength_m: float = 0.0) -> float:

@@ -6,6 +6,11 @@ steps of `calibrate_symmetric_4f`, tolerance and Monte Carlo studies. One call p
 nearly idle (a few hundred rays occupy a few SMs, and every call pays an upload and a host synchronisation). A sweep
 uploads the K configurations as one sweep scene (include/optb.h `optb_scene_upload_sweep`) and traces K x N roots in
 one call: root k * N + r is ray r of the bundle in configuration k.
+
+`trace_sweep(tables)` flattens K whole tables. A study that moves one or two components of a large scene keeps a
+`SweepScene` instead: the table is flattened once, each configuration re-reads only the varied components and monitors
+(`FlatScene.refresh`), and the device builds the K configuration blobs from the base and those rows
+(`optb_scene_upload_sweep_rows`).
 """
 from __future__ import annotations
 
@@ -56,13 +61,16 @@ def _rays(rays):
     return len(arrs["ox"]), arrs["wavelength"], unit, arrs
 
 
-def _device_sweep(flats, rays, limit, record_hits=True, record_hist=False, engine=None, unit=None, arrs=None):
-    """The CUDA sweep: one sweep scene, one optb_trace over K x N roots, hit rows sorted into key order on the device."""
+def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, engine=None, unit=None, arrs=None):
+    """The CUDA sweep: one sweep scene, one optb_trace over K x N roots, hit rows sorted into key order on the device.
+    `configs`: the FlatScenes of the K configurations, or a SweepRows."""
     from .backend import Engine
     from .bundle import DeviceTrace, run_to_fit
 
     engine = engine or Engine.get()
-    K, M = len(flats), flats[0].n_monitors
+    rows = configs if isinstance(configs, SweepRows) else None
+    flat0, K = (rows.flat, rows.n_configs) if rows is not None else (configs[0], len(configs))
+    M = flat0.n_monitors
     if limit > (1 << 24) or M > 256:
         raise ValueError("trace_sweep sorts rows by a packed key: max_trace_num <= 2^24 and at most 256 monitors")
     if arrs is None:
@@ -73,8 +81,8 @@ def _device_sweep(flats, rays, limit, record_hits=True, record_hist=False, engin
         del rays_t["family"]   # every root is its own family (rays.family must be NULL on a sweep scene)
     n_roots = K * n
     cap = n_roots * max(M, 1) * 2 if record_hits else 0
-    dt, cnt = run_to_fit(lambda c: DeviceTrace(engine, flats[0], n, c, max_trace_num=limit, record_hist=record_hist,
-                                               configs=flats, **({} if unit is None else {"unit": unit})),
+    dt, cnt = run_to_fit(lambda c: DeviceTrace(engine, flat0, n, c, max_trace_num=limit, record_hist=record_hist,
+                                               configs=configs, **({} if unit is None else {"unit": unit})),
                          rays_t, n_roots, limit, cap)
     nh = int(cnt[A.C_HITS]) if record_hits else 0
     engine._sort_rows_on_device(dt.res, 0, nh, limit, M)
@@ -85,15 +93,18 @@ def _device_sweep(flats, rays, limit, record_hits=True, record_hist=False, engin
 
 
 class SweepResult:
-    """Result of `trace_sweep`. `hits`: the monitor-row columns of all configurations (CUDA tensors in (root, monitor,
-    pop) key order, so configuration-major; `hit_root` is the global root k * N + r); `hist_y` [K, M, 30],
-    `hist_yz` [K, M, 30, 30]; `counters`: OPTB_C_* totals over all configurations (numpy)."""
+    """Result of `trace_sweep` or `SweepScene.trace`. `hits`: the monitor-row columns of all configurations (CUDA
+    tensors in (root, monitor, pop) key order, so configuration-major; `hit_root` is the global root k * N + r);
+    `hist_y` [K, M, 30], `hist_yz` [K, M, 30, 30]; `counters`: OPTB_C_* totals over all configurations (numpy).
+    `monitors[k][m]`: monitor m as configuration k placed it (default: tables[k].monitors[m]), the frame `stats`,
+    `row_values` and `monitor` evaluate its rows in."""
 
-    def __init__(self, tables, n, out, engine=None):
+    def __init__(self, tables, n, out, engine=None, monitors=None):
         import torch
 
         self.tables, self.n, self.n_configs, self.engine = list(tables), int(n), len(tables), engine
-        K, M = self.n_configs, len(self.tables[0].monitors)
+        self.monitors = [list(t.monitors) for t in self.tables] if monitors is None else monitors
+        K, M = self.n_configs, len(self.monitors[0])
         self.counters = out["counters"]
         self.hist_y = out["hist_y"].reshape(K, -1, A.HIST_BINS)[:, :M]
         self.hist_yz = out["hist_yz"].reshape(K, -1, A.HIST_BINS, A.HIST_BINS)[:, :M]
@@ -113,14 +124,12 @@ class SweepResult:
             raise ValueError("SweepResult.stats / row_values: this sweep was traced with record_hits=False, so it kept no "
                              "monitor rows to summarise")
         if self._grouped is None:
-            M = len(self.tables[0].monitors)
-            monitors = [[t.monitors[m] for m in range(M)] for t in self.tables]
-            self._grouped = grouped_stats(self.hits, monitors, self.n, self.engine)
+            self._grouped = grouped_stats(self.hits, self.monitors, self.n, self.engine)
         return self._grouped
 
     def stats(self) -> dict:
         """Summaries of every configuration k and monitor m from one device call over all monitor rows
-        (`optb_monitor_stats_grouped`; each in the frame of tables[k].monitors[m]) and one copy back: the keys of
+        (`optb_monitor_stats_grouped`; each in the frame of monitors[k][m]) and one copy back: the keys of
         `DeviceMonitor.stats()` as numpy arrays [K, M] (hist_y [K, M, 30]), plus `std_tY` and `std_histy`. The same
         sweep gives the same bits on every call, so a ranking of configurations does not change between calls."""
         return self._grouped_stats()[0]
@@ -150,7 +159,7 @@ class SweepResult:
         """`DeviceMonitor` of monitor m in configuration k: every accessor of the reference's Monitor, on the device."""
         from .analytics import DeviceMonitor
 
-        return DeviceMonitor(self.tables[k].monitors[m], self.rows(k), m, engine=self.engine)
+        return DeviceMonitor(self.monitors[k][m], self.rows(k), m, engine=self.engine)
 
 
 def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hist=False, engine=None, tracer=None):
@@ -182,3 +191,162 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
     out = tracer(flats, rays, trace_cap(perfomance_limit), record_hits=record_hits, record_hist=record_hist,
                  engine=engine, unit=unit, arrs=arrs)
     return SweepResult(tables, n, out, engine)
+
+
+def _children(ni, nf):
+    """Most rays one interaction of each row can emit (FlatScene._physics's count, from the rows)."""
+    inter, refl, trans = ni[..., A.NI_INTER], nf[..., A.NF_REFL] > 0, nf[..., A.NF_TRANS] > 0
+    return np.select([inter == A.I_MIRROR, inter == A.I_REFRACT, (inter == A.I_THINLENS) | (inter == A.I_PASS)],
+                     [refl.astype(np.int64) + trans, 1 + refl.astype(np.int64), 1], 0)
+
+
+class SweepRows:
+    """K configurations of one scene as its base FlatScene plus the rows that differ (include/optb.h
+    `optb_scene_upload_sweep_rows`): configuration k is `flat` with node rows `nodes[v]` replaced by node_i[k, v] /
+    node_f[k, v] and monitor records `monitors[w]` by mon_f[k, w]. It stands for all K configurations wherever a sweep
+    needs a property of them (Scene, DeviceTrace, backend.runs_wavefront), without K FlatScenes on the host."""
+
+    def __init__(self, flat, n_configs, nodes, node_i, node_f, monitors, mon_f):
+        self.flat, self.n_configs = flat, int(n_configs)
+        self.nodes = np.ascontiguousarray(nodes, dtype=np.int32)
+        self.monitors = np.ascontiguousarray(monitors, dtype=np.int32)
+        self.node_i = np.ascontiguousarray(node_i, dtype=np.int32).reshape(self.n_configs, self.nodes.size, A.NI_STRIDE)
+        self.node_f = np.ascontiguousarray(node_f, dtype=np.float64).reshape(self.n_configs, self.nodes.size, A.NF_STRIDE)
+        self.mon_f = np.ascontiguousarray(mon_f, dtype=np.float64).reshape(self.n_configs, self.monitors.size, A.MON_STRIDE)
+        self.n_monitors, self.n_capslots, self.has_pass = flat.n_monitors, flat.n_capslots, flat.has_pass
+        fixed = np.ones(flat.n_nodes, dtype=bool)
+        fixed[self.nodes] = False
+        self.max_children = int(max(_children(flat.node_i[fixed], flat.node_f[fixed]).max(initial=0),
+                                     _children(self.node_i, self.node_f).max(initial=0)))
+        capped, capped_v = flat.node_i[fixed, A.NI_CAPSLOT] >= 0, self.node_i[..., A.NI_CAPSLOT] >= 0
+        self.cap_min = float(min(flat.node_f[fixed][capped, A.NF_CAPMAX].min(initial=np.inf),
+                                 self.node_f[capped_v][:, A.NF_CAPMAX].min(initial=np.inf)))
+
+    def materialise(self, k):
+        """Configuration k as a FlatScene of its own (tables only, like FlatScene.from_arrays)."""
+        d = self.flat.to_arrays()
+        d["node_i"], d["node_f"], d["mon_f"] = d["node_i"].copy(), d["node_f"].copy(), d["mon_f"].copy()
+        d["node_i"][self.nodes], d["node_f"][self.nodes], d["mon_f"][self.monitors] = self.node_i[k], self.node_f[k], self.mon_f[k]
+        d["counts"][4] = int(_children(d["node_i"], d["node_f"]).max(initial=0))
+        return type(self.flat).from_arrays(d)
+
+
+class _MonitorPose:
+    """A monitor's frame and size as one configuration left them: what SweepResult's statistics and monitor(k, m) read,
+    copied because the pose methods move the live object in place."""
+
+    def __init__(self, m):
+        self.origin = np.array(m.origin, dtype=np.float64)
+        self.transform_matrix = np.array(m.transform_matrix, dtype=np.float64)
+        self.tangent_Y, self.tangent_Z, self.normal = (np.array(getattr(m, a), dtype=np.float64)
+                                                       for a in ("tangent_Y", "tangent_Z", "normal"))
+        self.width, self.height = m.width, m.height
+
+
+class SweepScene:
+    """A sweep over configurations of one table that differ only in the components and monitors listed in `vary`
+    (tolerance and Monte Carlo studies, optimizer steps): the table is flattened once per distinct wavelength set and
+    kept, so repeated sweeps do not re-flatten a large scene.
+
+        sw = SweepScene(table, vary=[lens2, mon1])
+        res = sw.trace(rays, configure, n_configs)      # a SweepResult
+
+    `vary` holds objects of the table: components (leaves or groups, at any depth) and monitors of `table.monitors`.
+    What can vary is what `FlatScene.refresh` can rewrite in place: poses, apertures, reflectivity, transmission, focal
+    lengths, interact caps, monitor placement and size. A change of topology, of a material, of a polygon or
+    composite-aperture record or of the cap slots raises ValueError; so does a varied component inside a lattice group
+    (its lattice descriptor would have to be recomputed) and an object that is not in the table. Such sweeps go through
+    `trace_sweep(tables)`, which flattens every configuration."""
+
+    def __init__(self, table, vary):
+        self.table, self.vary = table, list(vary)
+        self._bases = {}   # wavelength set -> (FlatScene, varied components, node rows V, varied monitor indices, node_i[V])
+
+    def _what(self, j):
+        return f"vary[{j}] ({type(self.vary[j]).__name__})"
+
+    def _base(self, wls):
+        from .flatten import FlatScene
+
+        key = None if wls is None else tuple(wls)
+        if key in self._bases:
+            return self._bases[key]
+        flat = FlatScene(self.table.components, self.table.monitors, wavelengths_m=wls)
+        mon_index = {id(m): i for i, m in enumerate(flat.monitors)}
+        parents = flat._parents()
+        comps, rows, mons = [], set(), []
+        for j, obj in enumerate(self.vary):
+            first = flat._node_of.get(id(obj))
+            if first is None and id(obj) not in mon_index:
+                raise ValueError(f"SweepScene: {self._what(j)} is not a component or monitor of the table")
+            if id(obj) in mon_index:
+                mons.append(mon_index[id(obj)])
+            if first is None:
+                continue
+            up, p = [], parents.get(first, -1)
+            while p >= 0:
+                up.append(p)
+                p = parents.get(p, -1)
+            if any(flat.node_i[p, A.NI_GEOM] == A.G_GRID for p in up):
+                raise ValueError(f"SweepScene: {self._what(j)} lies in a lattice group, whose lattice descriptor a move "
+                                 "would change: trace such configurations with trace_sweep(tables)")
+            if flat.refresh(obj) is None:
+                raise ValueError(f"SweepScene: {self._what(j)} cannot be rewritten in place (it holds a lattice, a box "
+                                 "hierarchy, a polygon or composite-aperture record): trace such configurations with "
+                                 "trace_sweep(tables)")
+            comps.append((j, obj))
+            rows.update(range(first, int(flat.node_i[first, A.NI_SKIP])), up)
+        V = np.array(sorted(rows), dtype=np.int32)
+        base = self._bases[key] = (flat, comps, V, np.array(mons, dtype=np.int32), flat.node_i[V].copy())
+        return base
+
+    def trace(self, rays, configure, n_configs, perfomance_limit=None, record_hits=True, record_hist=False, engine=None,
+              tracer=None):
+        """Trace `rays` (a RayBundle or a list of Ray) through `n_configs` configurations in one device call; returns a
+        SweepResult whose `rows(k)`, `monitor(k, m)`, `stats()` and `row_values()` see configuration k's monitor
+        placement.
+
+        `configure(k)` puts the objects of `vary` into configuration k, with absolute values (the same configuration
+        whatever ran before it); it runs for k = 0 .. n_configs - 1 in order, and after the call the table stands in
+        configuration n_configs - 1. Limits, interact caps and record flags follow `trace_sweep`. `tracer(rows, rays,
+        max_trace_num, ...)` defaults to the CUDA sweep, where `rows` is the SweepRows of the configurations; the CPU
+        tests pass a stand-in."""
+        from .flatten import batch_wavelengths_m, monitor_record, trace_cap
+
+        K = int(n_configs)
+        if K < 1:
+            raise ValueError("SweepScene.trace: n_configs must be >= 1")
+        n, wl, unit, arrs = _rays(rays)
+        wl_unit = unit if unit is not None else getattr(self.table, "unit", 1e-2)
+        flat, comps, V, mons, ni0 = self._base(None if wl is None else batch_wavelengths_m(wl, wl_unit))
+        node_i = np.empty((K, V.size, A.NI_STRIDE), dtype=np.int32)
+        node_f = np.empty((K, V.size, A.NF_STRIDE), dtype=np.float64)
+        mon_f = np.zeros((K, mons.size, A.MON_STRIDE), dtype=np.float64)
+        cols = [c for c in range(A.NI_STRIDE) if c != A.NI_ORTHO]
+        owner = {}
+        for j, obj in comps:
+            first = flat._node_of[id(obj)]
+            owner.update({i: j for i in range(first, int(flat.node_i[first, A.NI_SKIP]))})
+        frames, varied_mons = [], set(mons.tolist())
+        for k in range(K):
+            configure(k)
+            for j, obj in comps:
+                if flat.refresh(obj) is None:
+                    raise ValueError(f"SweepScene: configuration {k} changes {self._what(j)} in a way the scene cannot "
+                                     "take in place (topology, a material, a polygon or composite-aperture record or its "
+                                     "cap slots): trace such configurations with trace_sweep(tables)")
+            node_i[k], node_f[k] = flat.node_i[V], flat.node_f[V]
+            bad = np.argwhere(node_i[k][:, cols] != ni0[:, cols])
+            if bad.size:
+                i, c = int(V[bad[0][0]]), cols[int(bad[0][1])]
+                raise ValueError(f"SweepScene: configuration {k} changes the {_NI_NAMES.get(c, f'node_i column {c}')} of "
+                                 f"{self._what(owner[i]) if i in owner else f'node {i}'}: trace such configurations with "
+                                 "trace_sweep(tables)")
+            for w, m in enumerate(mons.tolist()):
+                monitor_record(flat.monitors[m], mon_f[k, w])
+            live = list(flat.monitors)
+            frames.append([_MonitorPose(live[m]) if m in varied_mons else live[m] for m in range(len(live))])
+        rows = SweepRows(flat, K, V, node_i, node_f, mons, mon_f)
+        out = (tracer or _device_sweep)(rows, rays, trace_cap(perfomance_limit), record_hits=record_hits,
+                                        record_hist=record_hist, engine=engine, unit=unit, arrs=arrs)
+        return SweepResult([self.table] * K, n, out, engine, monitors=frames)

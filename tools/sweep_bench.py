@@ -9,9 +9,13 @@ Arms, alternated rep by rep (medians with min / max):
   c_e2e   one trace_sweep, including the K flattens
   c_dev   one sweep on FlatScenes built beforehand (sweep upload + trace + row sort)
   c_trace the trace of an uploaded sweep scene alone (CUDA events)
-Scenes: the 4f telescope over a 16 x 16 (F1, F2) grid (lens 2 and monitor 1 move) with N = 7, 1e3, 1e5; a splitting
-glass slab between two partially transmitting mirrors (tilt, index and reflectivity of the slab vary; roots
-reach the 300-pop cap), K = 64; ripa with one MMA group moved, K = 8, N = 1e4.
+  d       one SweepScene.trace: configure + FlatScene.refresh x K on a table flattened once, the varied rows uploaded
+          and the K configuration blobs built on the device (optb_scene_upload_sweep_rows), trace, row sort
+  d_build the blob-building kernel alone (torch.profiler kernel time, in a pass of its own after the timed reps), with
+          its write bandwidth: K x blob bytes over kernel time
+Scenes: the 4f telescope over a 16 x 16 (F1, F2) grid (lens 2 and monitor 1 move; arm b moves lens 2 only) with N = 7,
+1e3, 1e5; a splitting glass slab between two partially transmitting mirrors (tilt, index and reflectivity of the slab
+vary; roots reach the 300-pop cap), K = 64; ripa with one mirror of its first group moved, K = 8 and 64, N = 1e4.
 The _dev arms and b get a fixed live-ray budget and row capacity per root so that no attempt is repeated; the
 _e2e arms use the public entry points as they are (which grow it on overflow). Writes JSON lines to --out and stdout."""
 import argparse
@@ -30,7 +34,7 @@ from optable_b200 import _abi as A
 from optable_b200.backend import Engine
 from optable_b200.bundle import DeviceTrace, RayBundle, trace_bundle
 from optable_b200.flatten import FlatScene, batch_wavelengths_m
-from optable_b200.sweep import trace_sweep
+from optable_b200.sweep import SweepScene, trace_sweep
 from optable_b200.workloads import WORKLOADS, Scene, ripa, telescope_4f_grid
 
 
@@ -53,9 +57,32 @@ def checked(dt):
     return cnt
 
 
-def run_case(engine, name, tables, bundle, limit, reps, moved=None, out=None, live_per_root=None, rows_per_root=4):
+def blob_bytes(f):
+    """Bytes of one configuration blob (liboptb's blob_layout): 16-byte aligned sections."""
+    al = lambda b: (b + 15) // 16 * 16
+    return (al(max(f.n_nodes, 1) * 64) + al(f.n_nodes * A.NF_STRIDE * 8) + al(f.n_nodes * A.NI_STRIDE * 4)
+            + al(f.n_materials * 4) + al(f.n_materials * A.MF_STRIDE * 8) + al(max(f.n_monitors, 1) * (A.MON_STRIDE + 4) * 8)
+            + al(max(f.aux.size, 1) * 8))
+
+
+def build_kernel_ms(engine, rows, reps):
+    """Device time of the blob-building kernel per optb_scene_upload_sweep_rows call (torch.profiler)."""
+    from torch.profiler import ProfilerActivity, profile
+
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for _ in range(reps):
+            engine.upload_sweep(rows).close()
+        torch.cuda.synchronize()
+    ev = [e for e in prof.events() if "sweep_build_kernel" in e.name and e.device_type.name == "CUDA"]
+    if len(ev) != reps:
+        raise RuntimeError(f"expected {reps} sweep_build_kernel launches in the profile, found {len(ev)}")
+    return [e.device_time_total / 1e3 for e in ev]
+
+
+def run_case(engine, name, tables, bundle, limit, reps, moved=None, out=None, live_per_root=None, rows_per_root=4,
+             sweep=None):
     """moved: (builder of the base table, function(table, k) that applies configuration k's pose change, component
-    getter) for the b arm, or None."""
+    getter) for the b arm, or None. sweep: (table, varied objects, configure(k)) for the d arms, or None."""
     K, n = len(tables), bundle.n
     lim = None if limit is None else {"max_trace_num": limit}
     wls = batch_wavelengths_m(bundle.columns["wavelength"], 1e-2)
@@ -113,6 +140,9 @@ def run_case(engine, name, tables, bundle, limit, reps, moved=None, out=None, li
         return e0.elapsed_time(e1)
 
     cnt = checked(sdt)
+    if sweep is not None:
+        sw = SweepScene(sweep[0], sweep[1])
+        arms["d"] = lambda: sw.trace(bundle, sweep[2], K, lim, engine=engine)
     for f in arms.values():   # warm-up of every arm
         f()
     c_trace()
@@ -126,6 +156,28 @@ def run_case(engine, name, tables, bundle, limit, reps, moved=None, out=None, li
     rec = {"case": name, "K": K, "N": n, "roots": K * n, "leaves": flats[0].n_leaves,
            "interactions": int(cnt[A.C_INTERACTIONS]), "dropped": int(cnt[A.C_DROPPED]),
            "flatten_K_tables_ms": float(np.median(flat_ms)), **{k: stats(v) for k, v in times.items()}}
+    rec["c_trace_per_config_ms"] = rec["c_trace"]["median_ms"] / K
+    if sweep is not None:
+        captured = []
+
+        def grab(rows, *a, **kw):   # the SweepRows of one trace call, without tracing
+            captured.append(rows)
+            raise StopIteration
+
+        try:
+            sw.trace(bundle, sweep[2], K, lim, engine=engine, tracer=grab)
+        except StopIteration:
+            pass
+        rows = captured[0]
+        build = build_kernel_ms(engine, rows, reps)
+        nbytes = K * blob_bytes(rows.flat)
+        rec["d_build"] = stats(build)
+        rec["d_build_bytes_written"] = nbytes
+        rec["d_build_write_TBps"] = nbytes / (rec["d_build"]["median_ms"] * 1e-3) / 1e12
+        rec["d_varied_node_rows"], rec["d_varied_monitors"] = int(rows.nodes.size), int(rows.monitors.size)
+        rec["speedup_d_over_c_e2e"] = rec["c_e2e"]["median_ms"] / rec["d"]["median_ms"]
+        if "b" in rec:
+            rec["speedup_d_over_b"] = rec["b"]["median_ms"] / rec["d"]["median_ms"]
     rec["speedup_dev_a_over_c"] = rec["a_dev"]["median_ms"] / rec["c_dev"]["median_ms"]
     rec["speedup_e2e_a_over_c"] = rec["a_e2e"]["median_ms"] / rec["c_e2e"]["median_ms"]
     if "b" in rec:
@@ -150,6 +202,8 @@ def main():
     ap.add_argument("--out", default=None)
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--only", default=None, help="comma-separated case prefixes (4f, slab, ripa)")
+    ap.add_argument("--n4f", default="7,1000,100000", help="bundle sizes of the 4f cases")
+    ap.add_argument("--kripa", default="8,64", help="configuration counts of the ripa cases")
     args = ap.parse_args()
     q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                        capture_output=True, text=True).stdout.strip()
@@ -169,33 +223,42 @@ def main():
             f1, f2 = F[k // 16], F[k % 16]
             t.components[1].TX(43.17 + f1 + f2 - t.components[1].origin[0])
 
-        for n in (7, 1000, 100_000):
+        dbase = telescope_4f_grid(ob, F[0], F[0])
+
+        def configure(k):   # lens 2 and monitor 1 to configuration k's places
+            f1, f2 = F[k // 16], F[k % 16]
+            pose(dbase, k)
+            dbase.monitors[1].TX(43.17 + f1 + 2 * f2 - dbase.monitors[1].origin[0])
+
+        for n in [int(v) for v in args.n4f.split(",")]:
             reps = args.reps if n < 100_000 else max(3, args.reps // 2)
             run_case(engine, f"4f_grid_16x16_N{n}", tables, RayBundle.collimated_disc(n, radius=2.5), None, reps,
-                     (base, pose, lambda t: t.components[1]), args.out)
+                     (base, pose, lambda t: t.components[1]), args.out,
+                     sweep=(dbase, [dbase.components[1], dbase.monitors[1]], configure))
     if want("slab"):
         rng = np.random.default_rng(7)
         tables = [slab(1.45 + 0.1 * rng.uniform(), 0.1 + 0.2 * rng.uniform(), 0.1 * rng.uniform(-1, 1)) for _ in range(64)]
         bundle = RayBundle.collimated_disc(1000, x0=-3, radius=0.6, direction=(1.0, 0.01, 0.0))
         run_case(engine, "slab_cavity_split_K64_N1000", tables, bundle, 300, args.reps, None, args.out, live_per_root=600,
                  rows_per_root=160)
-    if want("ripa"):
+    for K in ([int(v) for v in args.kripa.split(",")] if want("ripa") else []):
         tables = []
-        for k in range(8):
+        for k in range(K):
             sc = ripa(ob, n_rays=0)
             sc.components[0].components[1].TX(1e-4 * k)
             tables.append(sc)
-        base = ripa(ob, n_rays=0)
-        dx = {"k": 0}
+        base, dbase = ripa(ob, n_rays=0), ripa(ob, n_rays=0)
+        dx = {id(base): 0, id(dbase): 0}
 
         def pose(t, k):
-            t.components[0].components[1].TX(1e-4 * (k - dx["k"]))
-            dx["k"] = k
+            t.components[0].components[1].TX(1e-4 * (k - dx[id(t)]))
+            dx[id(t)] = k
 
         w = WORKLOADS["c5_ripa_64"]
-        run_case(engine, "ripa_K8_N10000", tables, w.bundle(10_000, 0), w.max_trace_num, max(3, args.reps // 2),
+        run_case(engine, f"ripa_K{K}_N10000", tables, w.bundle(10_000, 0), w.max_trace_num, max(3, args.reps // 2),
                  (base, pose, lambda t: t.components[0].components[1]), args.out, live_per_root=64,
-                 rows_per_root=int(w.rows_per_ray * 2))
+                 rows_per_root=int(w.rows_per_ray * 2),
+                 sweep=(dbase, [dbase.components[0].components[1]], lambda k: pose(dbase, k)))
 
 
 if __name__ == "__main__":
