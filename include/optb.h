@@ -412,6 +412,32 @@ int optb_trace(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays,
 int optb_trace_host(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays,
                     const optb_params* params, optb_result* out);
 
+/* The launch plan of a trace, without tracing: which trace kernel variant optb_trace / optb_trace_host would run for
+ * (scene, rays, params) and with how much shared memory. Runs the same parameter checks as a trace that do not read
+ * the result buffers (the plan reads only rays->n and whether rays->family is set) and sets the kernel's shared-memory
+ * attribute as a trace does; enqueues nothing. out[5]:
+ *   out[0]  variant bits (OPTB_PLAN_*)
+ *   out[1]  scene blob bytes (all configurations of a sweep scene)
+ *   out[2]  dynamic shared memory the trace kernel launches with (blob and / or histograms)
+ *   out[3]  the selected kernel's static shared memory
+ *   out[4]  the device's opt-in shared memory per block (cudaDevAttrMaxSharedMemoryPerBlockOptin)
+ * A scene's tables are staged in shared memory when its blob fits the opt-in limit less the largest static shared
+ * memory of the shared-memory trace kernels, so that any later trace of the scene (diagnostics modes and family column
+ * included) can launch. Added without a change of OPTB_ABI_VERSION: no struct changed.                          */
+#define OPTB_PLAN_SMEM      (1u << 0)   /* tables staged in shared memory (else read from global memory) */
+#define OPTB_PLAN_SERIAL    (1u << 1)   /* family-serial path (binding interact caps) */
+#define OPTB_PLAN_BOX_SHIFT 2           /* 2 bits: 0 no boxes, 1 box walk, 2 box walk + lattice windows */
+#define OPTB_PLAN_BOX_MASK  (3u << OPTB_PLAN_BOX_SHIFT)
+#define OPTB_PLAN_ASPH      (1u << 4)   /* asphere root search compiled in */
+#define OPTB_PLAN_SPLIT     (1u << 5)   /* wavefront (splitting) form */
+#define OPTB_PLAN_FLAG      (1u << 6)   /* params.flag_ambiguity */
+#define OPTB_PLAN_BRENT     (1u << 7)   /* params.reference_roots */
+#define OPTB_PLAN_PASSK     (1u << 8)   /* pass-through leaves (OPTB_I_PASS) */
+#define OPTB_PLAN_SWEEP     (1u << 9)   /* sweep scene */
+#define OPTB_PLAN_HIST_SMEM (1u << 10)  /* histograms accumulated in shared memory (else global atomics); 0 without record_hist */
+int optb_trace_plan(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* params,
+                    int64_t out[5]);
+
 /* Put the first n_seg segment rows of `res` into (root, pop) order and its first n_hit monitor rows into
  * (root, monitor, pop) order, in place: what a caller of optb_trace does once it has read the counters (rows are
  * appended in device order). DEVICE pointers; NULL columns are skipped; the key columns (seg_root + seg_pop;

@@ -29,6 +29,9 @@ RF_ALIVE, RF_HASQ = 1, 2
  C_BOX_TESTS, C_FLAGGED, C_RESERVED) = range(12)
 C_COUNT = 12
 ST_SEG_OVERFLOW, ST_HIT_OVERFLOW, ST_WORK_OVERFLOW, ST_CAP_ORDER, ST_LUT_MISS = 1, 2, 4, 8, 16
+# optb_trace_plan: variant bits of out[0]
+PLAN_SMEM, PLAN_SERIAL, PLAN_BOX_SHIFT, PLAN_BOX_MASK = 1, 2, 2, 12
+PLAN_ASPH, PLAN_SPLIT, PLAN_FLAG, PLAN_BRENT, PLAN_PASSK, PLAN_SWEEP, PLAN_HIST_SMEM = 16, 32, 64, 128, 256, 512, 1024
 AMB_TIE, AMB_APERTURE, AMB_GRAZING, AMB_TIR, AMB_EPS, AMB_SCAN, AMB_SLAB = 1, 2, 4, 8, 16, 32, 64
 
 _vp = C.c_void_p
@@ -85,7 +88,7 @@ EXPORTED_SYMBOLS = (
     "optb_abi_version", "optb_ctx_create", "optb_ctx_destroy", "optb_last_error",
     "optb_scene_upload", "optb_scene_upload_sweep", "optb_scene_upload_sweep_rows", "optb_scene_destroy",
     "optb_scene_update_nodes", "optb_workspace_bytes", "optb_trace",
-    "optb_trace_host", "optb_measure_fp64_peak",
+    "optb_trace_host", "optb_trace_plan", "optb_measure_fp64_peak",
     "optb_sort_workspace_bytes", "optb_sort_rows", "optb_monitor_stats",
     "optb_monitor_stats_grouped_workspace_bytes", "optb_monitor_stats_grouped",
     "optb_comm_unique_id", "optb_comm_init", "optb_monitor_merge", "optb_comm_destroy",

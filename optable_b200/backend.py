@@ -45,6 +45,8 @@ def lib():
         L.optb_trace.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(A.Rays), C.POINTER(A.Params), C.POINTER(A.Result),
                                  C.c_void_p, C.c_int64, C.c_void_p]
         L.optb_trace_host.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(A.Rays), C.POINTER(A.Params), C.POINTER(A.Result)]
+        if hasattr(L, "optb_trace_plan"):   # (a library built before the entry point still traces)
+            L.optb_trace_plan.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(A.Rays), C.POINTER(A.Params), C.POINTER(C.c_int64)]
         L.optb_measure_fp64_peak.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
         L.optb_sort_workspace_bytes.restype = C.c_int64
         L.optb_sort_workspace_bytes.argtypes = [C.c_int64]
@@ -306,17 +308,13 @@ class Engine:
         """optb_trace_host: host buffers in, host buffers out (copies inside the call)."""
         self._check(lib().optb_trace_host(self._ctx, scene._h, C.byref(rays_struct), C.byref(params), C.byref(result)))
 
-    # -- convenience: exact-size traced result on the host, in reference order -------------------------
-    def trace_arrays(self, scene: Scene, arrs, max_trace_num=2000, unit=1e-2, record_segments=True, record_hits=True,
-                     record_hist=False, n_families=None, cap_counts=None, chain_len=0, max_live=None, flag_ambiguity=False,
-                     reference_roots=False):
-        """Trace a packed ray batch and return numpy result arrays trimmed and sorted to reference order
-        (segments by (root, pop); monitor rows by (root, monitor, pop))."""
-        torch = self.torch
+    def _arrays_params(self, scene: Scene, arrs, max_trace_num=2000, unit=1e-2, record_segments=True, record_hits=True,
+                       record_hist=False, n_families=None, cap_counts=None, chain_len=0, flag_ambiguity=False,
+                       reference_roots=False):
+        """optb_params of trace_arrays for a packed batch, and the initial interact-count table (None without caps)."""
         n = len(arrs["ox"])
         if n_families is None:
             n_families = int(arrs["family"].max()) + 1 if n else 1
-        rays_t = self.rays_to_device(arrs)
         flat = scene.flat
         caps0, slack = None, 0
         if flat.n_capslots:
@@ -325,14 +323,42 @@ class Engine:
             fam_size = np.bincount(arrs["family"], minlength=n_families).max() if n else 0
             capmax = flat.node_f[flat.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX].min()
             slack = int(caps0.max() + int(max_trace_num) * int(fam_size) <= capmax)
+        prm = self.make_params(max_trace_num, unit, record_segments, record_hits, record_hist, chain_len, n_families, slack,
+                               flag_ambiguity, reference_roots)
+        return prm, caps0
+
+    def trace_plan(self, scene: Scene, arrs, **params):
+        """The launch plan (optb_trace_plan) of `trace_arrays(scene, arrs, **params)`: a dict of the variant bits
+        (`bits`, OPTB_PLAN_*), `blob` bytes, `dynamic` and `static` shared memory of the kernel, and the device's
+        `optin` limit. Nothing is traced."""
+        prm, _ = self._arrays_params(scene, arrs, **params)
+        rs = A.Rays()
+        rs.n = len(arrs["ox"])
+        family = np.ascontiguousarray(arrs["family"], dtype=np.int32)
+        rs.family = family.ctypes.data        # (trace_arrays always passes the family column; the plan only tests it is set)
+        out = (C.c_int64 * 5)()
+        self._check(lib().optb_trace_plan(self._ctx, scene._h, C.byref(rs), C.byref(prm), out))
+        return dict(zip(("bits", "blob", "dynamic", "static", "optin"), (int(v) for v in out)))
+
+    # -- convenience: exact-size traced result on the host, in reference order -------------------------
+    def trace_arrays(self, scene: Scene, arrs, max_trace_num=2000, unit=1e-2, record_segments=True, record_hits=True,
+                     record_hist=False, n_families=None, cap_counts=None, chain_len=0, max_live=None, flag_ambiguity=False,
+                     reference_roots=False):
+        """Trace a packed ray batch and return numpy result arrays trimmed and sorted to reference order
+        (segments by (root, pop); monitor rows by (root, monitor, pop))."""
+        torch = self.torch
+        n = len(arrs["ox"])
+        prm, caps0 = self._arrays_params(scene, arrs, max_trace_num, unit, record_segments, record_hits, record_hist,
+                                         n_families, cap_counts, chain_len, flag_ambiguity, reference_roots)
+        n_families = prm.n_families
+        rays_t = self.rays_to_device(arrs)
+        flat = scene.flat
         # Row counts are only known after the trace. First try with capacities guessed from the batch; the
         # counters keep counting past the capacity, so an overflowing attempt is repeated once with exact sizes
         # (interact counts restart from caps0: every attempt gets a fresh table).
         pops_max = n * int(max_trace_num)
         nseg = min(pops_max, 8 * n + 1024) if record_segments else 0
         nhit = min(pops_max * flat.n_monitors, 8 * n + 1024) if record_hits else 0
-        prm = self.make_params(max_trace_num, unit, record_segments, record_hits, record_hist, chain_len, n_families, slack,
-                               flag_ambiguity, reference_roots)
         root_flags = torch.zeros(max(n, 1), dtype=torch.int32, device=f"cuda:{self.device}") if flag_ambiguity else None
         np_dt = {torch.float64: np.float64, torch.int64: np.int64, torch.int32: np.int32}
         # The live ray set of a splitting scene is not known in advance either: a root pops at most max_trace_num rays

@@ -1010,6 +1010,7 @@ struct optb_ctx {
   int device;
   int sm_count;
   size_t smem_optin;
+  size_t smem_static;  // largest static shared memory of the shared-memory trace kernels (smem_static_max)
   char err[512];
   // arena for optb_trace_host
   void* arena; size_t arena_bytes;
@@ -1042,6 +1043,9 @@ struct optb_scene {
 static int hist_mons(const optb_scene* s) { return s->n_mons * std::max(s->n_cfg, 1); }
 
 static int fail(optb_ctx* ctx, int code, const char* what, cudaError_t e = cudaSuccess) {
+  // A refused runtime call may also leave its error as the runtime's last error: clear it, so that a later
+  // cudaGetLastError check (the end of trace_impl) cannot report it a second time.
+  if (e != cudaSuccess) cudaGetLastError();
   if (ctx) {
     if (e != cudaSuccess) snprintf(ctx->err, sizeof ctx->err, "%s: %s", what, cudaGetErrorString(e));
     else snprintf(ctx->err, sizeof ctx->err, "%s", what);
@@ -1056,6 +1060,7 @@ extern "C" int64_t optb_sort_workspace_bytes(int64_t n_rows);
 static int sort_rows_dev(optb_ctx* ctx, const optb_result* res, const optb_result* dst, int64_t n_seg, int64_t n_hit,
                          const unsigned long long* d_counters, void* workspace, int64_t workspace_bytes, cudaStream_t st,
                          int end_bit);
+static cudaError_t smem_static_max(size_t* out);
 
 extern "C" int optb_ctx_create(int device, optb_ctx** out) {
   if (!out) return -1;
@@ -1071,7 +1076,8 @@ extern "C" int optb_ctx_create(int device, optb_ctx** out) {
       cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, device) != cudaSuccess ||
       cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device) != cudaSuccess ||
       cudaMallocHost((void**)&ctx->h_counters, sizeof(unsigned long long) * OPTB_C_COUNT) != cudaSuccess ||
-      cudaMallocHost((void**)&ctx->h_hdr, sizeof(Header)) != cudaSuccess) {
+      cudaMallocHost((void**)&ctx->h_hdr, sizeof(Header)) != cudaSuccess ||
+      smem_static_max(&ctx->smem_static) != cudaSuccess) {
     cudaGetLastError();
     optb_ctx_destroy(ctx);
     return -10;
@@ -1388,7 +1394,10 @@ static int scene_alloc(optb_ctx* ctx, const optb_scene_desc* d, int n_cfg, optb_
   if (o > 0xfff00000ull) { delete s; return fail(ctx, -6, "scene too large"); }
   s->blob_bytes = (uint32_t)o; s->cfg_stride = (uint32_t)stride;
   size_t hist_bytes = (size_t)K * d->n_monitors * OPTB_HIST_BINS * (OPTB_HIST_BINS + 1) * 4;
-  size_t budget = ctx->smem_optin > 2048 ? ctx->smem_optin - 2048 : 0;
+  // dynamic + static shared memory of a block may not exceed the opt-in limit. The budget takes the largest static
+  // size of the shared-memory kernels, not the one the scene's first trace selects: a later trace of the same scene
+  // with flag_ambiguity, reference_roots or a family column runs a general kind, which has the largest.
+  size_t budget = ctx->smem_optin > ctx->smem_static ? ctx->smem_optin - ctx->smem_static : 0;
   s->in_smem = !n_cfg && (o <= budget);  // sweep kernels read the tables from global memory (L1/L2)
   size_t used = s->in_smem ? o : 0;
   s->hist_smem = (hist_bytes > 0 && used + hist_bytes <= std::min<size_t>(budget, used + 65536));
@@ -1681,31 +1690,40 @@ SerialLayout serial_layout(long long n_rays, long long n_fam, long long ring_ent
 }
 
 using Kern = void (*)(const TraceArgs);
+// One trace_kernel instantiation and its template arguments as OPTB_PLAN_* bits (what optb_trace_plan reports)
+struct KernPick { Kern kern; uint32_t bits; };
+template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = false, bool BRENT = false, bool PASSK = false,
+          bool SWEEP = false>
+KernPick pick() {
+  return {trace_kernel<SMEM, SERIAL, BOXES, ASPH, SPLIT, FLAG, BRENT, PASSK, SWEEP>,
+          (SMEM ? OPTB_PLAN_SMEM : 0u) | (SERIAL ? OPTB_PLAN_SERIAL : 0u) | ((uint32_t)BOXES << OPTB_PLAN_BOX_SHIFT) |
+              (ASPH ? OPTB_PLAN_ASPH : 0u) | (SPLIT ? OPTB_PLAN_SPLIT : 0u) | (FLAG ? OPTB_PLAN_FLAG : 0u) |
+              (BRENT ? OPTB_PLAN_BRENT : 0u) | (PASSK ? OPTB_PLAN_PASSK : 0u) | (SWEEP ? OPTB_PLAN_SWEEP : 0u)};
+}
 // The parallel-path kinds, indexed by [box mode][aspheres][split]; SWEEP: each lane on its root's configuration
 template <bool SMEM, bool SWEEP = false>
-Kern parallel_kernel(int boxmode, bool asph, bool split) {
-#define OPTB_K(B, A, P) trace_kernel<SMEM, false, B, A, P, false, false, false, SWEEP>
+KernPick parallel_kernel(int boxmode, bool asph, bool split) {
+#define OPTB_K(B, A, P) pick<SMEM, false, B, A, P, false, false, false, SWEEP>()
 #define OPTB_KROW(B) {{OPTB_K(B, false, false), OPTB_K(B, false, true)}, {OPTB_K(B, true, false), OPTB_K(B, true, true)}}
-  static const Kern k[3][2][2] = {OPTB_KROW(0), OPTB_KROW(1), OPTB_KROW(2)};
+  static const KernPick k[3][2][2] = {OPTB_KROW(0), OPTB_KROW(1), OPTB_KROW(2)};
 #undef OPTB_KROW
 #undef OPTB_K
   return k[boxmode][asph ? 1 : 0][split ? 1 : 0];
 }
 // The general kind (box walk, aspheres, split) with one of the options only it carries
 template <bool SERIAL, bool FLAG, bool BRENT, bool PASSK>
-Kern general_kernel(bool smem) {
-  return smem ? trace_kernel<true, SERIAL, 1, true, true, FLAG, BRENT, PASSK>
-              : trace_kernel<false, SERIAL, 1, true, true, FLAG, BRENT, PASSK>;
+KernPick general_kernel(bool smem) {
+  return smem ? pick<true, SERIAL, 1, true, true, FLAG, BRENT, PASSK>() : pick<false, SERIAL, 1, true, true, FLAG, BRENT, PASSK>();
 }
 // The trace_kernel instantiation that runs a trace. Sweep scenes read their tables from global memory. The
 // family-serial path, the two diagnostics modes (params.reference_roots: brentq_dev roots; params.flag_ambiguity: the
 // A.9 pass at every pop) and pass-through leaves (OPTB_I_PASS) only exist in the general kind.
-Kern select_kernel(const optb_scene* scene, const optb_params* prm, bool serial, bool split) {
+KernPick select_kernel(const optb_scene* scene, const optb_params* prm, bool serial, bool split) {
   // box mode: 0 none, 1 pre-order walk with culling, 2 walk + lattice windows (scenes with OPTB_G_GRID groups)
   const int boxmode = !scene->has_boxes ? 0 : (scene->has_grid ? 2 : 1);
   const bool smem = scene->in_smem, asph = scene->has_asph;
   if (scene->n_cfg)
-    return scene->has_pass ? trace_kernel<false, false, 1, true, true, false, false, true, true>
+    return scene->has_pass ? pick<false, false, 1, true, true, false, false, true, true>()
                            : parallel_kernel<false, true>(boxmode, asph, split);
   if (prm->reference_roots)
     return serial ? general_kernel<true, false, true, false>(smem) : general_kernel<false, false, true, false>(smem);
@@ -1714,7 +1732,73 @@ Kern select_kernel(const optb_scene* scene, const optb_params* prm, bool serial,
   if (scene->has_pass) return general_kernel<false, false, false, true>(smem);
   return smem ? parallel_kernel<true>(boxmode, asph, split) : parallel_kernel<false>(boxmode, asph, split);
 }
+
+// What a trace launches: the kernel, its OPTB_PLAN_* bits, the dynamic shared memory of every launch and the
+// resident CTAs per SM at that size. trace_impl and optb_trace_plan both take it from launch_plan.
+struct LaunchPlan { KernPick k; uint32_t smem; int occ; };
 }  // namespace
+
+// Largest static shared memory over the trace kernels that stage the blob in shared memory (every kind a scene that
+// scene_alloc puts in shared memory can be traced with): the part of the opt-in window that is not the blob's.
+static cudaError_t smem_static_max(size_t* out) {
+  std::vector<Kern> ks;
+  for (int b = 0; b < 3; b++)
+    for (int a = 0; a < 2; a++)
+      for (int p = 0; p < 2; p++) ks.push_back(parallel_kernel<true>(b, a, p).kern);
+  ks.push_back(general_kernel<false, false, true, false>(true).kern);
+  ks.push_back(general_kernel<true, false, true, false>(true).kern);
+  ks.push_back(general_kernel<false, true, false, false>(true).kern);
+  ks.push_back(general_kernel<true, false, false, false>(true).kern);
+  ks.push_back(general_kernel<false, false, false, true>(true).kern);
+  size_t m = 0;
+  for (Kern k : ks) {
+    cudaFuncAttributes fa;
+    cudaError_t e = cudaFuncGetAttributes(&fa, (const void*)k);
+    if (e != cudaSuccess) return e;
+    m = std::max(m, fa.sharedSizeBytes);
+  }
+  *out = m;
+  return cudaSuccess;
+}
+
+// The kernel of a trace with these options and its launch configuration. Sets the kernel's dynamic shared-memory
+// attribute (a host call; nothing is enqueued): a plan CUDA refuses fails here, in the query as in the trace.
+static int launch_plan(optb_ctx* ctx, const optb_scene* scene, const optb_params* prm, bool serial, bool split,
+                       bool hist_smem, LaunchPlan* lp) {
+  lp->k = select_kernel(scene, prm, serial, split);
+  if (hist_smem) lp->k.bits |= OPTB_PLAN_HIST_SMEM;
+  lp->smem = scene->in_smem ? scene->smem_bytes : (hist_smem ? scene->smem_bytes : 0);
+  const Kern kern = lp->k.kern;
+  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<uint32_t>(lp->smem, 1024)), "smem attr");
+  lp->occ = 1;
+  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&lp->occ, kern, kBlock, lp->smem), "occupancy");
+  if (lp->occ < 1) lp->occ = 1;
+  return 0;
+}
+
+// The checks of a trace's arguments that do not read the result buffers (optb_trace_plan runs them too).
+static int check_trace_args(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm) {
+  if (rays->n >= 0xffffffffll) return fail(ctx, -7, "at most 2^32-1 rays per call");
+  // a sweep scene traces every ray through every configuration: root k * rays.n + r = ray r in configuration k
+  const long long n_roots = scene->n_cfg ? rays->n * scene->n_cfg : rays->n;
+  if (scene->n_cfg) {
+    if (n_roots >= 0xffffffffll) return fail(ctx, -7, "sweep: n_configs * rays.n must stay below 2^32");
+    if (needs_serial(scene, rays, prm))
+      return fail(ctx, -7, "sweep: the scene has interact caps; set params.caps_slack (sweeps have no family-serial path)");
+    if (prm->flag_ambiguity || prm->reference_roots)
+      return fail(ctx, -7, "sweep: flag_ambiguity and reference_roots are not available on sweep scenes");
+    if (rays->family) return fail(ctx, -7, "sweep: rays.family must be NULL (every root is its own family)");
+  }
+  // cap_counts is [n_capslots][n_families]; without a family column every initial ray is its own family (column
+  // index = ray index), so the table must have a column per ray
+  if (scene->n_caps > 0 && prm->n_families < 1) return fail(ctx, -7, "scene has interact caps: cap_counts/n_families required");
+  if (scene->n_caps > 0 && !rays->family && (long long)prm->n_families < n_roots)
+    return fail(ctx, -7, "scene has interact caps and rays.family is NULL: n_families must be >= rays.n (times n_configs for a sweep)");
+  if (needs_serial(scene, rays, prm) && prm->flag_ambiguity)
+    return fail(ctx, -7, "flag_ambiguity is not available on the family-serial path (binding interact caps)");
+  if (prm->reference_roots && prm->flag_ambiguity) return fail(ctx, -7, "reference_roots and flag_ambiguity are separate diagnostics modes");
+  return 0;
+}
 
 extern "C" int64_t optb_workspace_bytes(const optb_scene* scene, int64_t n_rays, int64_t max_live) {
   if (!scene || n_rays < 0) return -1;
@@ -1737,34 +1821,35 @@ extern "C" int optb_trace(optb_ctx* ctx, const optb_scene* scene, const optb_ray
   return trace_impl(ctx, scene, rays, prm, out, workspace, workspace_bytes, (cudaStream_t)stream_v, 0u, true);
 }
 
+extern "C" int optb_trace_plan(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
+                               int64_t out[5]) {
+  if (!ctx || !scene || !rays || !prm || !out) return -1;
+  cudaSetDevice(ctx->device);
+  if (int rc = check_trace_args(ctx, scene, rays, prm)) return rc;
+  const bool serial = needs_serial(scene, rays, prm), split = !serial && needs_wavefront(scene, prm);
+  LaunchPlan lp;
+  if (int rc = launch_plan(ctx, scene, prm, serial, split, prm->record_hist && scene->n_mons > 0 && scene->hist_smem, &lp))
+    return rc;
+  cudaFuncAttributes fa;
+  CK(cudaFuncGetAttributes(&fa, (const void*)lp.k.kern), "kernel attributes");
+  out[0] = lp.k.bits; out[1] = scene->blob_bytes; out[2] = lp.smem; out[3] = (int64_t)fa.sharedSizeBytes;
+  out[4] = (int64_t)ctx->smem_optin;
+  return 0;
+}
+
 static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* rays, const optb_params* prm,
                       optb_result* out, void* workspace, int64_t workspace_bytes, cudaStream_t st, uint32_t root_base,
                       bool zero_hist) {
   cudaSetDevice(ctx->device);
   if (!out->counters) return fail(ctx, -7, "result.counters is required");
-  if (rays->n >= 0xffffffffll) return fail(ctx, -7, "at most 2^32-1 rays per call");
-  // a sweep scene traces every ray through every configuration: root k * rays.n + r = ray r in configuration k
+  if (int rc = check_trace_args(ctx, scene, rays, prm)) return rc;
   const long long n_roots = scene->n_cfg ? rays->n * scene->n_cfg : rays->n;
-  if (scene->n_cfg) {
-    if (n_roots >= 0xffffffffll) return fail(ctx, -7, "sweep: n_configs * rays.n must stay below 2^32");
-    if (needs_serial(scene, rays, prm))
-      return fail(ctx, -7, "sweep: the scene has interact caps; set params.caps_slack (sweeps have no family-serial path)");
-    if (prm->flag_ambiguity || prm->reference_roots)
-      return fail(ctx, -7, "sweep: flag_ambiguity and reference_roots are not available on sweep scenes");
-    if (rays->family) return fail(ctx, -7, "sweep: rays.family must be NULL (every root is its own family)");
-  }
   if (prm->record_hits && out->hit_capacity > 0 && !out->hit_monitor && !out->hit_key) return fail(ctx, -7, "record_hits needs hit_monitor or hit_key");
   if (prm->record_hits && out->hit_key && (prm->max_trace_num > (1ll << 24) || scene->n_mons > 256))
     return fail(ctx, -7, "hit_key packs pop into 24 bits and the monitor into 8: max_trace_num <= 2^24 and <= 256 monitors");
   if (prm->flag_ambiguity && !out->root_flags) return fail(ctx, -7, "flag_ambiguity needs result.root_flags [rays.n]");
-  if (scene->n_caps > 0 && (!out->cap_counts || prm->n_families < 1)) return fail(ctx, -7, "scene has interact caps: cap_counts/n_families required");
-  // cap_counts is [n_capslots][n_families]; without a family column every initial ray is its own family (column
-  // index = ray index), so the table must have a column per ray
-  if (scene->n_caps > 0 && !rays->family && (long long)prm->n_families < n_roots)
-    return fail(ctx, -7, "scene has interact caps and rays.family is NULL: n_families must be >= rays.n (times n_configs for a sweep)");
+  if (scene->n_caps > 0 && !out->cap_counts) return fail(ctx, -7, "scene has interact caps: cap_counts/n_families required");
   const bool serial = needs_serial(scene, rays, prm);
-  if (serial && prm->flag_ambiguity) return fail(ctx, -7, "flag_ambiguity is not available on the family-serial path (binding interact caps)");
-  if (prm->reference_roots && prm->flag_ambiguity) return fail(ctx, -7, "reference_roots and flag_ambiguity are separate diagnostics modes");
   if (prm->record_hist && scene->n_mons && (!out->hist_y || (zero_hist && !out->hist_yz)))
     return fail(ctx, -7, "record_hist needs hist_y and hist_yz");
   const bool split = !serial && needs_wavefront(scene, prm);
@@ -1838,13 +1923,11 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
     a.gen_first = (uint32_t*)(ws + L.gen_first);
     a.gen_last = (uint32_t*)(ws + L.gen_last);
   }
-  uint32_t smem = scene->in_smem ? scene->smem_bytes : (a.hist_smem ? scene->smem_bytes : 0);
-  const Kern kern = select_kernel(scene, prm, serial, split);
-  CK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)std::max<uint32_t>(smem, 1024)), "smem attr");
-  int occ = 1;
-  CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kBlock, smem), "occupancy");
-  if (occ < 1) occ = 1;
-  const int full_grid = ctx->sm_count * occ;
+  LaunchPlan lp;
+  if (int rc = launch_plan(ctx, scene, prm, serial, split, a.hist_smem, &lp)) return rc;
+  const Kern kern = lp.k.kern;
+  const uint32_t smem = lp.smem;
+  const int full_grid = ctx->sm_count * lp.occ;
 
   unsigned long long gens = 0, launches = 0;
   long long n_in = n_roots;

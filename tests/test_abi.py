@@ -23,6 +23,13 @@ def test_header_and_python_mirror_agree():
     for name, val in (("OPTB_NI_STRIDE", A.NI_STRIDE), ("OPTB_NF_STRIDE", A.NF_STRIDE), ("OPTB_MON_STRIDE", A.MON_STRIDE),
                       ("OPTB_NF_CAPMAX", A.NF_CAPMAX), ("OPTB_POLY_HEADER", A.POLY_HEADER), ("OPTB_C_COUNT", A.C_COUNT)):
         assert re.search(rf"{name}\s*=\s*{val}\b", src), name
+    # optb_trace_plan's variant bits
+    plan = {m[0]: int(m[1]) for m in re.findall(r"#define OPTB_(PLAN_\w+)\s+\(1u << (\d+)\)", src)}
+    assert len(plan) == 9
+    for name, shift in plan.items():
+        assert getattr(A, name) == 1 << shift, name
+    assert re.search(rf"#define OPTB_PLAN_BOX_SHIFT\s+{A.PLAN_BOX_SHIFT}\b", src)
+    assert re.search(r"#define OPTB_PLAN_BOX_MASK\s+\(3u << OPTB_PLAN_BOX_SHIFT\)", src) and A.PLAN_BOX_MASK == 3 << A.PLAN_BOX_SHIFT
 
 
 def test_library_exports_all_symbols():
