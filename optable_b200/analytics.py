@@ -56,6 +56,17 @@ def grouped_stats(out: dict, monitors, rays_per_config=0, engine=None):
     root // rays_per_config (0: one configuration). Returns (stats_arrays dict of [K, M] arrays, per-row values
     [5, n]: y, z, tY, tZ, waist distance as a CUDA tensor aligned with the rows). Raises ValueError when a row belongs
     to no group (its monitor or configuration is out of range): the counts would not add up to the rows."""
+    s, per_row = grouped_slots(out, monitors, rays_per_config, engine)
+    return stats_arrays(s, monitor_widths(monitors)), per_row
+
+
+def monitor_widths(monitors):
+    """[K][M] widths of monitors[k][m], the second argument of `stats_arrays`."""
+    return [[float(m.width) for m in row] for row in monitors]
+
+
+def grouped_slots(out: dict, monitors, rays_per_config=0, engine=None):
+    """The raw stats slots [K, M, OPTB_MS_STRIDE] (numpy) and per-row values of `grouped_stats`."""
     from .backend import Engine
 
     K, M = len(monitors), len(monitors[0])
@@ -68,8 +79,7 @@ def grouped_stats(out: dict, monitors, rays_per_config=0, engine=None):
     if counted != n:
         raise ValueError(f"{n - counted} of {n} monitor rows belong to no (configuration, monitor) group of this "
                          f"{K} x {M} result: their monitor or configuration index is out of range")
-    widths = [[float(monitors[k][m].width) for m in range(M)] for k in range(K)]
-    return stats_arrays(s, widths), per_row
+    return s, per_row
 
 
 def monitor_stats(monitors, out: dict, engine=None) -> dict:

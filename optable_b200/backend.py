@@ -335,7 +335,8 @@ class Engine:
         rs = A.Rays()
         rs.n = len(arrs["ox"])
         family = np.ascontiguousarray(arrs["family"], dtype=np.int32)
-        rs.family = family.ctypes.data        # (trace_arrays always passes the family column; the plan only tests it is set)
+        if not scene.sweep:                   # (a sweep's roots are their own families: no family column)
+            rs.family = family.ctypes.data    # (trace_arrays always passes the family column; the plan only tests it is set)
         out = (C.c_int64 * 5)()
         self._check(lib().optb_trace_plan(self._ctx, scene._h, C.byref(rs), C.byref(prm), out))
         return dict(zip(("bits", "blob", "dynamic", "static", "optin"), (int(v) for v in out)))

@@ -144,3 +144,154 @@ def trace_sharded(table, bundle, perfomance_limit=None, group=None, gather=False
             rows = gather_rows(rows, n_rows, 0, group)
     out.update(rows)
     return out
+
+
+def _collective_device(group=None):
+    """Where tensors of a collective live: the current CUDA device under NCCL, the host under gloo."""
+    import torch.distributed as dist
+
+    return "cuda" if dist.get_backend(group) == "nccl" else "cpu"
+
+
+def _gather_configs(t, counts, group=None):
+    """All-gather of per-rank slices [K_r, ...] of a per-configuration array (uneven K_r = `counts`, rank order):
+    padded to the largest slice, returns the concatenation [sum K_r, ...] on every rank, on t's device. Not a sum:
+    each slice lands at its own configurations."""
+    import torch
+    import torch.distributed as dist
+
+    padded = torch.zeros((max(counts),) + tuple(t.shape[1:]), dtype=t.dtype, device=_collective_device(group))
+    padded[:t.shape[0]] = t
+    parts = [torch.empty_like(padded) for _ in counts]
+    dist.all_gather(parts, padded, group=group)
+    return torch.cat([p[:c] for p, c in zip(parts, counts)]).to(t.device)
+
+
+def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label, tracer, group=None, gather=False,
+                        record_hits=True, record_hist=False, engine=None, unit=None, arrs=None):
+    """Multi-GPU form of a sweep (`trace_sweep` / `SweepScene.trace` with `group=`): the K configurations are sharded
+    over the ranks of `group`, rank r owning the contiguous configurations [k0, k1) = shard_bounds(K, r, world) (equal
+    counts, no balancing by cost; K < world leaves ranks without configurations, which still take part in every
+    collective). Every group (k, m) of the monitor statistics is reduced on its own rows in a fixed order, so a
+    configuration that stays on one rank gets the bits of the one-GPU sweep: rows, histograms and statistics.
+
+    `prepare(k0, k1)` runs this rank's host side and returns (configs, shares): the FlatScenes or SweepRows of its
+    configurations (None when k0 == k1) and a list with one picklable item per configuration that every rank receives
+    (SweepScene: the frames of the varied monitors). `monitors`: the [K][M] monitor frames, or a function of the
+    gathered shares (configuration order) that returns them. A rank without configurations does not call `prepare`.
+
+    Before any trace, one exchange checks on every rank (so that no rank waits in a collective while another raised):
+    what `prepare` raised on any rank, the topology of the ranks' configurations (`sweep.topology_key`; ValueError
+    naming the first differing global configuration), interact caps, and the largest `max_children`. A rank whose
+    own configurations do not split while others do runs the wavefront kernels with chain_len = limit + 1, which
+    selects the variant the one-GPU sweep runs and never cuts a chain (a root pops at most `limit` times). The global
+    K * N < 2^32 bound is checked up front, since row keys are global.
+
+    After the trace: statistics of the rank's own rows (`optb_monitor_stats_grouped`, configurations numbered from
+    k0), all-gather of their slots and of the [K_r, M, ...] histograms, `merge_counters`, roots rebased to k * N + r
+    and, with `gather`, `gather_rows`. Returns (out, monitors): the result dict SweepResult reads (`shard`, `world`,
+    `holds`, `counters_local`, `chain_len`, `stats_slots`) and the [K][M] frames."""
+    import builtins
+
+    import torch
+    import torch.distributed as dist
+
+    from . import _abi as A
+    from .analytics import grouped_slots
+    from .sweep import SweepRows, topology_key, topology_mismatch
+
+    K, n = int(n_configs), int(n_rays)
+    who, what = label.split(": ")
+    if K * n >= 1 << 32:
+        raise ValueError(f"{who}: n_configs * rays ({K} x {n}) must stay below 2^32: row keys count roots over all "
+                         "configurations")
+    rank, world = dist.get_rank(group), dist.get_world_size(group)
+    bounds = [shard_bounds(K, r, world) for r in range(world)]
+    counts = [hi - lo for lo, hi in bounds]
+    k0, k1 = bounds[rank]
+    mismatch = lambda k, why: f"{label} {k} does not have the topology of {what} 0 ({why})"
+
+    # ---- this rank's host side, and one exchange of what every rank must know before any trace
+    mine = {"error": None, "key": None, "max_children": 0, "shares": []}
+    configs, err = None, None
+    try:
+        if k1 > k0:
+            configs, mine["shares"] = prepare(k0, k1)
+        if configs is not None:
+            rows = configs if isinstance(configs, SweepRows) else None
+            flats = [rows] if rows is not None else configs
+            flat0 = rows.flat if rows is not None else configs[0]
+            mine["key"] = topology_key(flat0)     # (sent even when a later configuration of this rank differs)
+            bad = topology_mismatch(configs) if rows is None else None
+            if bad is not None:
+                raise ValueError(mismatch(k0 + bad[0], bad[1]))
+            if flat0.n_capslots and min(f.cap_min for f in flats) < limit:
+                raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped component")
+            mine["max_children"] = max(f.max_children for f in flats)
+    except Exception as e:   # raised on every rank below
+        err, mine["error"] = e, (k0, type(e).__name__, str(e))
+    states = [None] * world
+    dist.all_gather_object(states, mine, group=group)
+    # (first configuration, exception name, message, rank that raised it or None): the earliest one is raised everywhere
+    found = [s["error"] + (r,) for r, s in enumerate(states) if s["error"] is not None]
+    ref = next((s["key"] for s in states if s["key"] is not None), None)
+    found += [(bounds[r][0], "ValueError", mismatch(bounds[r][0], f"its sizes, node kinds or material kinds differ; "
+                                                    f"rank {r} traces it"), None)
+              for r, s in enumerate(states) if s["key"] not in (None, ref)]
+    if found:
+        k, name, msg, r = min(found, key=lambda f: (f[0], f[3] is not None))
+        if r == rank:
+            raise err
+        cls = getattr(builtins, name, None)
+        cls = cls if isinstance(cls, type) and issubclass(cls, Exception) else RuntimeError
+        raise cls(msg if r is None else f"{msg} (raised on rank {r} of the sharded sweep)")
+    if callable(monitors):
+        monitors = monitors([x for s in states for x in s["shares"]])
+    M = len(monitors[0])
+    Mh = max(M, 1)       # the device keeps one histogram row per monitor, at least one per configuration
+    wide = max(s["max_children"] for s in states)
+    chain_len = int(limit) + 1 if configs is not None and wide > 1 >= mine["max_children"] else 0
+
+    # ---- this rank's trace
+    dev = _collective_device(group)
+    cols = A.HIT_I32 + A.HIT_U32 + A.HIT_F64
+    if configs is not None:
+        res = tracer(configs, rays, limit, record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
+                     arrs=arrs, chain_len=chain_len)
+        counters = np.asarray(res["counters"])
+    else:
+        dt = {k: torch.int32 for k in A.HIT_I32 + A.HIT_U32}
+        res = {k: torch.empty(0, dtype=dt.get(k, torch.float64), device=dev) for k in cols} if record_hits else {}
+        res["hist_y"] = torch.zeros((0, Mh, A.HIST_BINS), dtype=torch.int64, device=dev)
+        res["hist_yz"] = torch.zeros((0, Mh, A.HIST_BINS, A.HIST_BINS), dtype=torch.int64, device=dev)
+        counters = np.zeros(A.C_COUNT, dtype=np.int64)
+    rows = {k: res[k] for k in cols + ("hit_key",) if k in res}
+    n_rows = int(rows["hit_px"].numel()) if record_hits else 0
+
+    # ---- statistics of the own rows, before their roots are made global
+    out = {"shard": (k0, k1), "world": world, "holds": (0, K) if gather and record_hits else (k0, k1),
+           "counters_local": counters.copy(), "chain_len": chain_len, "stats_slots": None}
+    if record_hits:
+        slots = (torch.from_numpy(grouped_slots(rows, monitors[k0:k1], n, engine)[0]) if configs is not None
+                 else torch.zeros((0, M, A.MS_STRIDE), dtype=torch.float64))
+        out["stats_slots"] = _gather_configs(slots, counts, group).numpy()
+    if k0 and "hit_root" in rows:
+        r = (rows["hit_root"].long() & 0xFFFFFFFF) + k0 * n
+        rows["hit_root"] = (r - ((r >> 31) << 32)).to(rows["hit_root"].dtype)   # uint32 bit pattern in int32
+    if k0 and "hit_key" in rows:
+        rows["hit_key"] = rows["hit_key"] + ((k0 * n) << 32)
+
+    # ---- what every rank receives
+    hy = res["hist_y"].reshape(k1 - k0, Mh, A.HIST_BINS)
+    hyz = res["hist_yz"].reshape(k1 - k0, Mh, A.HIST_BINS, A.HIST_BINS)
+    if record_hist:
+        out["hist_y"], out["hist_yz"] = _gather_configs(hy, counts, group), _gather_configs(hyz, counts, group)
+    else:
+        out["hist_y"] = torch.zeros((K,) + tuple(hy.shape[1:]), dtype=hy.dtype, device=hy.device)
+        out["hist_yz"] = torch.zeros((K,) + tuple(hyz.shape[1:]), dtype=hyz.dtype, device=hyz.device)
+    out["counters"] = merge_counters(counters, group)
+    if gather and record_hits:
+        where = rows["hit_px"].device
+        rows = {k: v.to(where) for k, v in gather_rows({k: v.to(dev) for k, v in rows.items()}, n_rows, 0, group).items()}
+    out.update(rows)
+    return out, monitors

@@ -25,9 +25,10 @@ _NI_NAMES = {A.NI_GEOM: "geometry kind", A.NI_INTER: "interaction kind", A.NI_SK
              A.NI_LEAF: "leaf index"}
 
 
-def check_topology(flats):
-    """Raise ValueError naming the first FlatScene that does not have the topology of flats[0]: the same table sizes,
-    node_i rows identical except OPTB_NI_ORTHO, identical material kinds (what optb_scene_upload_sweep requires)."""
+def topology_mismatch(flats):
+    """(k, what) of the first FlatScene of `flats` that does not have the topology of flats[0], or None: the same
+    table sizes, node_i rows identical except OPTB_NI_ORTHO, identical material kinds (what optb_scene_upload_sweep
+    requires)."""
     f0 = flats[0]
     for k, f in enumerate(flats[1:], 1):
         what = None
@@ -47,7 +48,29 @@ def check_topology(flats):
             m = int(np.argmax(f.mat_kind != f0.mat_kind))
             what = f"material {m}: kind {f.mat_kind[m]} != {f0.mat_kind[m]}"
         if what is not None:
-            raise ValueError(f"trace_sweep: table {k} does not have the topology of table 0 ({what})")
+            return k, what
+    return None
+
+
+def check_topology(flats):
+    """Raise ValueError naming the first FlatScene that does not have the topology of flats[0] (`topology_mismatch`)."""
+    bad = topology_mismatch(flats)
+    if bad is not None:
+        raise ValueError(f"trace_sweep: table {bad[0]} does not have the topology of table 0 ({bad[1]})")
+
+
+def topology_key(flat) -> bytes:
+    """Digest of what `topology_mismatch` compares: equal digests, equal topology. Ranks of a sharded sweep compare
+    these instead of their tables."""
+    import hashlib
+
+    h = hashlib.sha256()
+    h.update(np.array([flat.n_nodes, flat.n_leaves, flat.n_materials, flat.n_monitors, flat.n_capslots, flat.aux.size],
+                      dtype=np.int64).tobytes())
+    cols = [c for c in range(A.NI_STRIDE) if c != A.NI_ORTHO]
+    h.update(np.ascontiguousarray(flat.node_i[:, cols], dtype=np.int32).tobytes())
+    h.update(np.ascontiguousarray(flat.mat_kind, dtype=np.int32).tobytes())
+    return h.digest()
 
 
 def _rays(rays):
@@ -61,9 +84,11 @@ def _rays(rays):
     return len(arrs["ox"]), arrs["wavelength"], unit, arrs
 
 
-def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, engine=None, unit=None, arrs=None):
+def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, engine=None, unit=None, arrs=None,
+                  chain_len=0):
     """The CUDA sweep: one sweep scene, one optb_trace over K x N roots, hit rows sorted into key order on the device.
-    `configs`: the FlatScenes of the K configurations, or a SweepRows."""
+    `configs`: the FlatScenes of the K configurations, or a SweepRows. `chain_len` > 0 runs the wavefront kernels
+    (a shard of a sharded sweep whose own configurations do not split, when others do)."""
     from .backend import Engine
     from .bundle import DeviceTrace, run_to_fit
 
@@ -82,7 +107,7 @@ def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, eng
     n_roots = K * n
     cap = n_roots * max(M, 1) * 2 if record_hits else 0
     dt, cnt = run_to_fit(lambda c: DeviceTrace(engine, flat0, n, c, max_trace_num=limit, record_hist=record_hist,
-                                               configs=configs, **({} if unit is None else {"unit": unit})),
+                                               chain_len=chain_len, configs=configs, **({} if unit is None else {"unit": unit})),
                          rays_t, n_roots, limit, cap)
     nh = int(cnt[A.C_HITS]) if record_hits else 0
     engine._sort_rows_on_device(dt.res, 0, nh, limit, M)
@@ -97,7 +122,13 @@ class SweepResult:
     tensors in (root, monitor, pop) key order, so configuration-major; `hit_root` is the global root k * N + r);
     `hist_y` [K, M, 30], `hist_yz` [K, M, 30, 30]; `counters`: OPTB_C_* totals over all configurations (numpy).
     `monitors[k][m]`: monitor m as configuration k placed it (default: tables[k].monitors[m]), the frame `stats`,
-    `row_values` and `monitor` evaluate its rows in."""
+    `row_values` and `monitor` evaluate its rows in.
+
+    Of a sharded call (`group=`): `shard` = (k0, k1), the configurations this rank traced, and `counters_local` its own
+    counters; `counters`, the histograms, `monitors` and `stats()` cover all K configurations on every rank. `hits`
+    holds this rank's rows with global roots, or every rank's rows with `gather=True`; `rows(k)` and `monitor(k, m)`
+    of a configuration whose rows this rank does not hold raise IndexError. `chain_len` > 0 when this rank ran the
+    wavefront kernels with that chain length to match the kernel variant of the one-GPU sweep (0 otherwise)."""
 
     def __init__(self, tables, n, out, engine=None, monitors=None):
         import torch
@@ -109,6 +140,9 @@ class SweepResult:
         self.hist_y = out["hist_y"].reshape(K, -1, A.HIST_BINS)[:, :M]
         self.hist_yz = out["hist_yz"].reshape(K, -1, A.HIST_BINS, A.HIST_BINS)[:, :M]
         self.hits = {k: v for k, v in out.items() if k.startswith("hit_")}
+        self.shard, self.counters_local, self.chain_len = out.get("shard"), out.get("counters_local"), out.get("chain_len", 0)
+        self._world = out.get("world", 1)
+        self._holds = out.get("holds", (0, K))      # the configurations whose rows `hits` holds
         root = self.hits.get("hit_root")
         if root is not None:   # rows are sorted by root: configuration k owns the roots [k N, (k + 1) N)
             starts = torch.arange(K + 1, dtype=torch.int64, device=root.device) * self.n
@@ -116,6 +150,13 @@ class SweepResult:
         else:
             self._bounds = [0] * (K + 1)
         self._grouped = None
+        # a sharded call summarises every configuration on the rank that holds its rows and gathers the slots, so
+        # stats() is never a collective (a script in which one rank asks must not hang)
+        self._stats = None
+        if out.get("stats_slots") is not None:
+            from .analytics import monitor_widths, stats_arrays
+
+            self._stats = stats_arrays(out["stats_slots"], monitor_widths(self.monitors))
 
     def _grouped_stats(self):
         from .analytics import grouped_stats
@@ -131,12 +172,13 @@ class SweepResult:
         """Summaries of every configuration k and monitor m from one device call over all monitor rows
         (`optb_monitor_stats_grouped`; each in the frame of monitors[k][m]) and one copy back: the keys of
         `DeviceMonitor.stats()` as numpy arrays [K, M] (hist_y [K, M, 30]), plus `std_tY` and `std_histy`. The same
-        sweep gives the same bits on every call, so a ranking of configurations does not change between calls."""
-        return self._grouped_stats()[0]
+        sweep gives the same bits on every call, so a ranking of configurations does not change between calls; a
+        sharded sweep gives the bits of the one-GPU sweep."""
+        return self._stats if self._stats is not None else self._grouped_stats()[0]
 
     def row_values(self) -> dict:
         """Per-row y, z, tY, tZ and waist_distance, each row evaluated in its own configuration's monitor frame: CUDA
-        tensors aligned with `hits`, from the same device call as `stats()`."""
+        tensors aligned with `hits` (after a sharded call: the rows this rank holds)."""
         v = self._grouped_stats()[1]
         return dict(zip(("y", "z", "tY", "tZ", "waist_distance"), v))
 
@@ -145,6 +187,13 @@ class SweepResult:
         bundle index r, plus its `hist_y` [M, 30] / `hist_yz` [M, 30, 30]: the shape of a `trace_bundle` result."""
         if not 0 <= k < self.n_configs:
             raise IndexError(f"configuration {k} of {self.n_configs}")
+        if not self._holds[0] <= k < self._holds[1]:
+            from .dist import shard_bounds
+
+            owner = next(r for r in range(self._world) if k < shard_bounds(self.n_configs, r, self._world)[1])
+            raise IndexError(f"configuration {k}: its rows are on rank {owner} of this sharded sweep (this rank holds "
+                             f"configurations [{self._holds[0]}, {self._holds[1]})); trace with gather=True to hold "
+                             "every configuration's rows on every rank")
         lo, hi = self._bounds[k], self._bounds[k + 1]
         out = {c: v[lo:hi] for c, v in self.hits.items()}
         if "hit_root" in out:
@@ -162,7 +211,18 @@ class SweepResult:
         return DeviceMonitor(self.monitors[k][m], self.rows(k), m, engine=self.engine)
 
 
-def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hist=False, engine=None, tracer=None):
+def _sharded(group):
+    """Whether `group=` asks for a sharded sweep: True (the default process group) or a ProcessGroup, under an
+    initialised torch.distributed; None / False, or no process group, is the one-GPU call."""
+    if group is None or group is False:
+        return False
+    import torch.distributed as dist
+
+    return dist.is_available() and dist.is_initialized()
+
+
+def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hist=False, engine=None, tracer=None,
+                group=None, gather=False):
     """Trace one bundle through every table of `tables` (K configurations of one scene, e.g. one builder function over
     a parameter grid) in one device call; returns a SweepResult.
 
@@ -174,9 +234,15 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
     Interact caps follow `trace_bundle`: every capped component needs max_interact_count >= max_trace_num in every
     configuration, else NotImplementedError.
 
+    `group=True` (the default process group) or a ProcessGroup shards the configurations over its ranks, one GPU
+    each (`optable_b200.dist.trace_sweep_sharded`): rank r flattens and traces only the contiguous configurations
+    `shard_bounds(K, r, world)`, and every rank gets the histograms, counters, monitor frames and `stats()` of all K;
+    `gather=True` also gives every rank every row. Each configuration's rows, histograms and statistics are the bits
+    of the one-GPU call.
+
     Like `trace_bundle`, a sweep is a tensor entry point: it does not fill `table.rays`, `Monitor._data_raw` or the
     components' `_interact_count`. `tracer(flats, rays, max_trace_num, record_hits=, record_hist=, engine=, unit=,
-    arrs=)` defaults to the CUDA sweep; the CPU tests pass a stand-in."""
+    arrs=)` (plus `chain_len=` when sharded) defaults to the CUDA sweep; the CPU tests pass a stand-in."""
     from .flatten import FlatScene, batch_wavelengths_m, trace_cap
 
     tables = list(tables)
@@ -185,9 +251,18 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
     n, wl, unit, arrs = _rays(rays)
     wl_unit = unit if unit is not None else getattr(tables[0], "unit", 1e-2)
     wls = None if wl is None else batch_wavelengths_m(wl, wl_unit)
-    flats = [FlatScene(t.components, t.monitors, wavelengths_m=wls) for t in tables]
-    check_topology(flats)
+    flatten = lambda ts: [FlatScene(t.components, t.monitors, wavelengths_m=wls) for t in ts]
     tracer = tracer or _device_sweep
+    if _sharded(group):
+        from .dist import trace_sweep_sharded
+
+        out, _ = trace_sweep_sharded(len(tables), n, rays, trace_cap(perfomance_limit),
+                                     lambda k0, k1: (flatten(tables[k0:k1]), None), [list(t.monitors) for t in tables],
+                                     "trace_sweep: table", tracer, group=None if group is True else group, gather=gather,
+                                     record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit, arrs=arrs)
+        return SweepResult(tables, n, out, engine)
+    flats = flatten(tables)
+    check_topology(flats)
     out = tracer(flats, rays, trace_cap(perfomance_limit), record_hits=record_hits, record_hist=record_hist,
                  engine=engine, unit=unit, arrs=arrs)
     return SweepResult(tables, n, out, engine)
@@ -301,7 +376,7 @@ class SweepScene:
         return base
 
     def trace(self, rays, configure, n_configs, perfomance_limit=None, record_hits=True, record_hist=False, engine=None,
-              tracer=None):
+              tracer=None, group=None, gather=False):
         """Trace `rays` (a RayBundle or a list of Ray) through `n_configs` configurations in one device call; returns a
         SweepResult whose `rows(k)`, `monitor(k, m)`, `stats()` and `row_values()` see configuration k's monitor
         placement.
@@ -310,15 +385,50 @@ class SweepScene:
         whatever ran before it); it runs for k = 0 .. n_configs - 1 in order, and after the call the table stands in
         configuration n_configs - 1. Limits, interact caps and record flags follow `trace_sweep`. `tracer(rows, rays,
         max_trace_num, ...)` defaults to the CUDA sweep, where `rows` is the SweepRows of the configurations; the CPU
-        tests pass a stand-in."""
-        from .flatten import batch_wavelengths_m, monitor_record, trace_cap
+        tests pass a stand-in.
+
+        `group=` / `gather=` shard the configurations as in `trace_sweep`: rank r calls `configure(k)` only for its own
+        configurations `shard_bounds(K, r, world)`, in order (and `configure(n_configs - 1)` once more at the end when
+        another rank owns that one), and the frames of the varied monitors are exchanged so that `monitors[k][m]`
+        holds every configuration's placement on every rank."""
+        from .flatten import batch_wavelengths_m, trace_cap
 
         K = int(n_configs)
         if K < 1:
             raise ValueError("SweepScene.trace: n_configs must be >= 1")
         n, wl, unit, arrs = _rays(rays)
         wl_unit = unit if unit is not None else getattr(self.table, "unit", 1e-2)
-        flat, comps, V, mons, ni0 = self._base(None if wl is None else batch_wavelengths_m(wl, wl_unit))
+        wls = None if wl is None else batch_wavelengths_m(wl, wl_unit)
+        tracer = tracer or _device_sweep
+        if _sharded(group):
+            from .dist import trace_sweep_sharded
+
+            def prepare(k0, k1):
+                rows, frames = self._configurations(wls, configure, k0, k1)
+                return rows, [{m: f for m, f in enumerate(fr) if isinstance(f, _MonitorPose)} for fr in frames]
+
+            live = list(self.table.monitors)
+            out, frames = trace_sweep_sharded(K, n, rays, trace_cap(perfomance_limit), prepare,
+                                              lambda poses: [[p.get(m, mon) for m, mon in enumerate(live)] for p in poses],
+                                              "SweepScene.trace: configuration", tracer,
+                                              group=None if group is True else group, gather=gather,
+                                              record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
+                                              arrs=arrs)
+            if not out["shard"][0] <= K - 1 < out["shard"][1]:
+                configure(K - 1)     # the documented end state: the table stands in the last configuration
+            return SweepResult([self.table] * K, n, out, engine, monitors=frames)
+        rows, frames = self._configurations(wls, configure, 0, K)
+        out = tracer(rows, rays, trace_cap(perfomance_limit), record_hits=record_hits, record_hist=record_hist,
+                     engine=engine, unit=unit, arrs=arrs)
+        return SweepResult([self.table] * K, n, out, engine, monitors=frames)
+
+    def _configurations(self, wls, configure, k0, k1):
+        """configure(k) for k = k0 .. k1 - 1 in order: the SweepRows of those configurations and their monitor frames
+        (a _MonitorPose snapshot for a varied monitor, the live monitor otherwise)."""
+        from .flatten import monitor_record
+
+        flat, comps, V, mons, ni0 = self._base(wls)
+        K = k1 - k0
         node_i = np.empty((K, V.size, A.NI_STRIDE), dtype=np.int32)
         node_f = np.empty((K, V.size, A.NF_STRIDE), dtype=np.float64)
         mon_f = np.zeros((K, mons.size, A.MON_STRIDE), dtype=np.float64)
@@ -328,25 +438,22 @@ class SweepScene:
             first = flat._node_of[id(obj)]
             owner.update({i: j for i in range(first, int(flat.node_i[first, A.NI_SKIP]))})
         frames, varied_mons = [], set(mons.tolist())
-        for k in range(K):
+        for c, k in enumerate(range(k0, k1)):
             configure(k)
             for j, obj in comps:
                 if flat.refresh(obj) is None:
                     raise ValueError(f"SweepScene: configuration {k} changes {self._what(j)} in a way the scene cannot "
                                      "take in place (topology, a material, a polygon or composite-aperture record or its "
                                      "cap slots): trace such configurations with trace_sweep(tables)")
-            node_i[k], node_f[k] = flat.node_i[V], flat.node_f[V]
-            bad = np.argwhere(node_i[k][:, cols] != ni0[:, cols])
+            node_i[c], node_f[c] = flat.node_i[V], flat.node_f[V]
+            bad = np.argwhere(node_i[c][:, cols] != ni0[:, cols])
             if bad.size:
-                i, c = int(V[bad[0][0]]), cols[int(bad[0][1])]
-                raise ValueError(f"SweepScene: configuration {k} changes the {_NI_NAMES.get(c, f'node_i column {c}')} of "
-                                 f"{self._what(owner[i]) if i in owner else f'node {i}'}: trace such configurations with "
-                                 "trace_sweep(tables)")
+                i, col = int(V[bad[0][0]]), cols[int(bad[0][1])]
+                raise ValueError(f"SweepScene: configuration {k} changes the {_NI_NAMES.get(col, f'node_i column {col}')} "
+                                 f"of {self._what(owner[i]) if i in owner else f'node {i}'}: trace such configurations "
+                                 "with trace_sweep(tables)")
             for w, m in enumerate(mons.tolist()):
-                monitor_record(flat.monitors[m], mon_f[k, w])
+                monitor_record(flat.monitors[m], mon_f[c, w])
             live = list(flat.monitors)
             frames.append([_MonitorPose(live[m]) if m in varied_mons else live[m] for m in range(len(live))])
-        rows = SweepRows(flat, K, V, node_i, node_f, mons, mon_f)
-        out = (tracer or _device_sweep)(rows, rays, trace_cap(perfomance_limit), record_hits=record_hits,
-                                        record_hist=record_hist, engine=engine, unit=unit, arrs=arrs)
-        return SweepResult([self.table] * K, n, out, engine, monitors=frames)
+        return SweepRows(flat, K, V, node_i, node_f, mons, mon_f), frames
