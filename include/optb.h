@@ -510,6 +510,38 @@ int optb_monitor_stats_grouped(optb_ctx* ctx, const optb_result* rows, int64_t f
                                const optb_monitor_frame* frames, double* stats, double* y, double* z, double* ty,
                                double* tz, double* waist, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- ABCD matrices of every configuration of a sweep (OpticalTable.calculate_abcd_matrix, optical_table.py:239-297) --
+ * For K configurations whose monitor mon0 and everything in front of it are the same, the three bundles of the finite
+ * differences are the same in every configuration, so two sweep traces over one sweep scene give every configuration's
+ * matrices:
+ *   sweep A: 2N rays, the nominal rays r (roots k * 2N + r) and the same rays shifted by disp along mon0's tangent_Y
+ *            (roots k * 2N + N + r);
+ *   sweep B: N rays, the shifted rays turned by rot about mon0's tangent_Z through their pivots (roots k * N + r).
+ * optb_sweep_abcd_pivots reads sweep A's rows of mon0: pivots[r][3] = configuration 0's nominal mon0 hit point of ray r
+ * (monitor-local, the reference's pivot; NaN when that ray has no single row), and first_bad = the smallest k * N + r
+ * whose nominal ray has not exactly one mon0 row or whose hit point differs in any bit from configuration 0's, else -1.
+ * A caller builds sweep B only when first_bad is -1.
+ * optb_sweep_abcd reads both sweeps' rows of mon1 and writes, for configuration k and ray r,
+ *   abcd[k][r][4] = A, B, C, D = (y1 - y0) / disp, (y2 - y0) / rot, (t1 - t0) / disp, (t2 - t0) / rot
+ * with y = local point . tangent_Y and t = lab direction . tangent_Y in frames[k] (DEVICE optb_monitor_frame[K], the
+ * per-row values optb_monitor_stats_grouped writes, bit for bit) for the nominal (0), shifted (1) and turned (2) ray,
+ * and counts[k][r][3] = that ray's mon1 rows in each of the three traces. A matrix is NaN unless all three counts are 1.
+ *   - rows: DEVICE columns (root: hit_root or hit_key; monitor: hit_monitor or hit_key; hit_px/py/pz; for
+ *     optb_sweep_abcd also hit_dx/dy/dz), in any order: a slot per (trace, k, r) counts its rows and is read only when
+ *     it holds exactly one, so equal rows give equal bits in any order and on every call.
+ *   - pivots, first_bad, abcd, counts: DEVICE memory; workspace: optb_sweep_abcd_workspace_bytes(N, K) bytes of device
+ *     memory (-1: N < 1, K < 1 or 2 K N >= 2^32), enough for either call.
+ * Fails with -7 when a column is missing, the monitor index is outside [0, 256), 2 K N >= 2^32, a row count is >= 2^31 - 1
+ * or the workspace is too small. Enqueued on `stream`, without a host synchronisation. Added without a change of
+ * OPTB_ABI_VERSION: no struct changed.                                                                               */
+int64_t optb_sweep_abcd_workspace_bytes(int64_t n_rays, int32_t n_configs);
+int optb_sweep_abcd_pivots(optb_ctx* ctx, const optb_result* rows, int64_t n, int64_t n_rays, int32_t n_configs,
+                           int32_t mon0, double* pivots, int64_t* first_bad, void* workspace, int64_t workspace_bytes,
+                           void* stream);
+int optb_sweep_abcd(optb_ctx* ctx, const optb_result* rows_a, int64_t n_a, const optb_result* rows_b, int64_t n_b,
+                    int64_t n_rays, int32_t n_configs, int32_t mon1, const optb_monitor_frame* frames, double disp,
+                    double rot, double* abcd, int32_t* counts, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* ---- multi-GPU monitor merge (SURVEY 8e) -----------------------------------------------------------------------
  * The path shards without a data-path collective: every rank (one process per GPU, one ctx each) traces its own block
  * of the initial rays against its own copy of the scene. The only exchange is the merge of the monitors at the end,

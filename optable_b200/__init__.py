@@ -17,6 +17,6 @@ from .assemblies import (ComponentGroup, GlassSlab, CircleGlassSlab, MLA, MMA, M
 from .monitors import Monitor
 from .solvers import solve_ray_bboxes_intersections, solve_ray_ray_intersection, solve_normal_to_normal_rotation
 from .table import OpticalTable, install, trace_table
-from .sweep import SweepResult, SweepScene, trace_sweep
+from .sweep import SweepABCD, SweepResult, SweepScene, sweep_abcd_matrix, trace_sweep
 
 __all__ = [n for n in dir() if not n.startswith("_")]

@@ -91,6 +91,7 @@ EXPORTED_SYMBOLS = (
     "optb_trace_host", "optb_trace_plan", "optb_measure_fp64_peak",
     "optb_sort_workspace_bytes", "optb_sort_rows", "optb_monitor_stats",
     "optb_monitor_stats_grouped_workspace_bytes", "optb_monitor_stats_grouped",
+    "optb_sweep_abcd_workspace_bytes", "optb_sweep_abcd_pivots", "optb_sweep_abcd",
     "optb_comm_unique_id", "optb_comm_init", "optb_monitor_merge", "optb_comm_destroy",
 )
 

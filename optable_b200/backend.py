@@ -55,6 +55,13 @@ def lib():
         L.optb_monitor_stats_grouped_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
         L.optb_monitor_stats_grouped.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_int64, C.c_int32,
                                                  C.c_int32, C.c_void_p, C.c_void_p] + [C.c_void_p] * 6 + [C.c_int64, C.c_void_p]
+        L.optb_sweep_abcd_workspace_bytes.restype = C.c_int64
+        L.optb_sweep_abcd_workspace_bytes.argtypes = [C.c_int64, C.c_int32]
+        L.optb_sweep_abcd_pivots.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_int32, C.c_int32,
+                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+        L.optb_sweep_abcd.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.POINTER(A.Result), C.c_int64, C.c_int64,
+                                      C.c_int32, C.c_int32, C.c_void_p, C.c_double, C.c_double, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_int64, C.c_void_p]
         if L.optb_abi_version() != A.ABI_VERSION:
             raise BackendError("liboptb.so ABI version does not match optable_b200._abi")
         _lib = L
@@ -443,10 +450,7 @@ class Engine:
         torch = self.torch
         dev = f"cuda:{self.device}"
         n, G = int(cols["hit_px"].numel()), int(n_configs) * int(n_monitors)
-        res = A.Result()
-        for k in A.HIT_I32 + A.HIT_U32 + A.HIT_F64 + ("hit_key",):
-            if cols.get(k) is not None:
-                setattr(res, k, cols[k].data_ptr())
+        res = self._hit_result(cols)
         frames_dev = torch.frombuffer(bytearray(frames), dtype=torch.uint8).to(dev)
         stats = torch.empty((G, A.MS_STRIDE), dtype=torch.float64, device=dev)
         per_row = torch.empty((5, max(n, 1)), dtype=torch.float64, device=dev)
@@ -461,6 +465,53 @@ class Engine:
                                                  ptr(0), ptr(1), ptr(2, has_d), ptr(3, has_d), ptr(4, has_d and has_q),
                                                  C.c_void_p(ws.data_ptr()), int(ws.numel()), C.c_void_p(st)))
         return stats, per_row[:, :n]
+
+    @staticmethod
+    def _hit_result(cols):
+        """optb_result whose hit columns point at the CUDA tensors of `cols` (absent columns stay NULL)."""
+        res = A.Result()
+        for k in A.HIT_I32 + A.HIT_U32 + A.HIT_F64 + ("hit_key",):
+            if cols.get(k) is not None:
+                setattr(res, k, cols[k].data_ptr())
+        return res
+
+    def sweep_abcd_pivots(self, cols, n_rays, n_configs, mon0):
+        """optb_sweep_abcd_pivots over the rows `cols` of sweep A (2 n_rays rays per configuration) on the current
+        stream. Returns the device tensors pivots [n_rays, 3] and first_bad [1] (int64; -1: every configuration shares
+        configuration 0's mon0 hit points)."""
+        torch = self.torch
+        dev = f"cuda:{self.device}"
+        res = self._hit_result(cols)
+        pivots = torch.empty((int(n_rays), 3), dtype=torch.float64, device=dev)
+        first_bad = torch.empty(1, dtype=torch.int64, device=dev)
+        L = lib()
+        ws = self._ws(max(int(L.optb_sweep_abcd_workspace_bytes(int(n_rays), int(n_configs))), 1))
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(L.optb_sweep_abcd_pivots(self._ctx, C.byref(res), int(cols["hit_px"].numel()), int(n_rays),
+                                             int(n_configs), int(mon0), C.c_void_p(pivots.data_ptr()),
+                                             C.c_void_p(first_bad.data_ptr()), C.c_void_p(ws.data_ptr()), int(ws.numel()),
+                                             C.c_void_p(st)))
+        return pivots, first_bad
+
+    def sweep_abcd(self, cols_a, cols_b, n_rays, n_configs, mon1, frames, disp, rot):
+        """optb_sweep_abcd over the rows of sweep A (`cols_a`, 2 n_rays rays per configuration) and sweep B (`cols_b`,
+        n_rays) on the current stream; `frames`: a ctypes array of n_configs MonitorFrame (mon1 in each
+        configuration). Returns the device tensors abcd [n_configs, n_rays, 4] and counts [n_configs, n_rays, 3]."""
+        torch = self.torch
+        dev = f"cuda:{self.device}"
+        ra, rb = self._hit_result(cols_a), self._hit_result(cols_b)
+        frames_dev = torch.frombuffer(bytearray(frames), dtype=torch.uint8).to(dev)
+        abcd = torch.empty((int(n_configs), int(n_rays), 4), dtype=torch.float64, device=dev)
+        counts = torch.empty((int(n_configs), int(n_rays), 3), dtype=torch.int32, device=dev)
+        L = lib()
+        ws = self._ws(max(int(L.optb_sweep_abcd_workspace_bytes(int(n_rays), int(n_configs))), 1))
+        st = torch.cuda.current_stream(self.device).cuda_stream
+        self._check(L.optb_sweep_abcd(self._ctx, C.byref(ra), int(cols_a["hit_px"].numel()), C.byref(rb),
+                                      int(cols_b["hit_px"].numel()), int(n_rays), int(n_configs), int(mon1),
+                                      C.c_void_p(frames_dev.data_ptr()), float(disp), float(rot),
+                                      C.c_void_p(abcd.data_ptr()), C.c_void_p(counts.data_ptr()),
+                                      C.c_void_p(ws.data_ptr()), int(ws.numel()), C.c_void_p(st)))
+        return abcd, counts
 
     @staticmethod
     def _raise_status(counters):

@@ -2847,6 +2847,170 @@ extern "C" int optb_monitor_stats_grouped(optb_ctx* ctx, const optb_result* rows
   return 0;
 }
 
+// ---- ABCD matrices of a sweep: the rows of (trace, configuration, ray) joined through a slot table -------------------
+// Slot s = (trace * K + k) * N + r counts the rows of ray r of configuration k at the monitor in one trace and keeps the
+// index of the first row it saw. A slot is read only when its count is 1, so the row it holds is the only one, whatever
+// order the atomics ran in: the results depend on the rows, not on their order.
+namespace {
+struct AbcdRows {
+  const double *px, *py, *pz, *dx, *dy, *dz, *qre, *t;  // what eval_row reads (qre = NULL: no waist distance)
+  const uint32_t* root; const int32_t* mon; const unsigned long long* key;
+};
+struct AbcdLayout { size_t count, row, total; };
+AbcdLayout abcd_layout(long long slots) {
+  AbcdLayout L{};
+  L.count = 0;
+  L.row = align_up((size_t)slots * 4, 256);
+  L.total = L.row + align_up((size_t)slots * 4, 256);
+  return L;
+}
+AbcdRows abcd_rows(const optb_result* r) {
+  AbcdRows a;
+  a.px = r->hit_px; a.py = r->hit_py; a.pz = r->hit_pz; a.dx = r->hit_dx; a.dy = r->hit_dy; a.dz = r->hit_dz;
+  a.qre = nullptr; a.t = r->hit_t;
+  a.root = r->hit_root; a.mon = r->hit_monitor; a.key = (const unsigned long long*)r->hit_key;
+  return a;
+}
+// the checks both entry points share; returns 0 or the fail() code
+int abcd_check(optb_ctx* ctx, const char* fn, const optb_result* r, bool slopes, int monitor, long long n,
+               long long n_rays, int n_configs) {
+  char msg[160];
+  const char* why = nullptr;
+  if (!r->hit_root && !r->hit_key) why = "the configuration and ray of a row need hit_root or hit_key";
+  else if (!r->hit_monitor && !r->hit_key) why = "the monitor of a row needs hit_monitor or hit_key";
+  else if (!r->hit_px || !r->hit_py || !r->hit_pz) why = "hit_px/py/pz are required";
+  else if (slopes && !(r->hit_dx && r->hit_dy && r->hit_dz)) why = "hit_dx/dy/dz are required";
+  else if (monitor < 0 || monitor > 255) why = "monitor index outside [0, 256)";
+  else if (2 * (long long)n_configs * n_rays >= (1ll << 32)) why = "2 * n_configs * n_rays must stay below 2^32";
+  else if (n >= 0x7fffffffll) why = "at most 2^31-1 rows";
+  if (!why) return 0;
+  snprintf(msg, sizeof msg, "%s: %s", fn, why);
+  return fail(ctx, -7, msg);
+}
+// slot of every row of `monitor` in a trace of `per_config` roots per configuration, `first_trace` the slot trace of
+// root offset 0 (sweep A: nominal 0, shifted 1 with per_config = 2N; sweep B: 2 with per_config = N); `n_traces` limits
+// the traces kept (the pivots keep only the nominal rows)
+__global__ void abcd_scatter_kernel(const AbcdRows a, long long n, int monitor, long long n_rays, int n_configs,
+                                    long long per_config, int first_trace, int n_traces, uint32_t* count, uint32_t* row) {
+  for (long long j = blockIdx.x * (long long)blockDim.x + threadIdx.x; j < n; j += (long long)gridDim.x * blockDim.x) {
+    const int m = a.mon ? a.mon[j] : (int)((a.key[j] >> 24) & 0xffu);
+    if (m != monitor) continue;
+    const long long root = a.root ? (long long)a.root[j] : (long long)(a.key[j] >> 32);
+    const long long k = root / per_config, rr = root - k * per_config;
+    const int tr = first_trace + (int)(rr / n_rays);
+    if (k >= n_configs || tr >= n_traces) continue;
+    const long long s = ((long long)tr * n_configs + k) * n_rays + rr % n_rays;
+    if (atomicAdd(&count[s], 1u) == 0u) row[s] = (uint32_t)j;
+  }
+}
+OPTB_DEV unsigned long long f64_bits(double v) { return (unsigned long long)__double_as_longlong(v); }
+__global__ void abcd_pivots_kernel(const AbcdRows a, long long n_rays, int n_configs, const uint32_t* count,
+                                   const uint32_t* row, double* pivots, unsigned long long* first_bad) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;   // k * N + r
+  if (i >= (long long)n_configs * n_rays) return;
+  const long long r = i % n_rays;
+  const bool one = count[i] == 1u, ref = count[r] == 1u;
+  bool bad = !one;
+  if (i < n_rays) {
+    double P[3] = {NAN, NAN, NAN};
+    if (one) {
+      const uint32_t j = row[i];
+      P[0] = a.px[j]; P[1] = a.py[j]; P[2] = a.pz[j];
+    }
+    pivots[3 * r + 0] = P[0]; pivots[3 * r + 1] = P[1]; pivots[3 * r + 2] = P[2];
+  } else if (one && ref) {
+    const uint32_t j = row[i], j0 = row[r];
+    bad = f64_bits(a.px[j]) != f64_bits(a.px[j0]) || f64_bits(a.py[j]) != f64_bits(a.py[j0]) ||
+          f64_bits(a.pz[j]) != f64_bits(a.pz[j0]);
+  }
+  if (bad) atomicMin(first_bad, (unsigned long long)i);   // -1 (all ones) loses to every index
+}
+__global__ void abcd_matrix_kernel(const AbcdRows a, const AbcdRows b, long long n_rays, int n_configs,
+                                   const optb_monitor_frame* frames, double disp, double rot, const uint32_t* count,
+                                   const uint32_t* row, double* abcd, int32_t* counts) {
+  const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;   // k * N + r
+  const long long KN = (long long)n_configs * n_rays;
+  if (i >= KN) return;
+  const uint32_t c0 = count[i], c1 = count[KN + i], c2 = count[2 * KN + i];
+  counts[3 * i + 0] = (int32_t)c0; counts[3 * i + 1] = (int32_t)c1; counts[3 * i + 2] = (int32_t)c2;
+  double* M = abcd + 4 * i;
+  if (c0 != 1u || c1 != 1u || c2 != 1u) {
+    M[0] = NAN; M[1] = NAN; M[2] = NAN; M[3] = NAN;
+    return;
+  }
+  const optb_monitor_frame f = frames[i / n_rays];
+  double y0, y1, y2, t0, t1, t2, z, tz, wd;
+  eval_row(a, (long long)row[i], f, y0, z, t0, tz, wd);
+  eval_row(a, (long long)row[KN + i], f, y1, z, t1, tz, wd);
+  eval_row(b, (long long)row[2 * KN + i], f, y2, z, t2, tz, wd);
+  M[0] = __ddiv_rn(__dsub_rn(y1, y0), disp); M[1] = __ddiv_rn(__dsub_rn(y2, y0), rot);
+  M[2] = __ddiv_rn(__dsub_rn(t1, t0), disp); M[3] = __ddiv_rn(__dsub_rn(t2, t0), rot);
+}
+}  // namespace
+
+extern "C" int64_t optb_sweep_abcd_workspace_bytes(int64_t n_rays, int32_t n_configs) {
+  if (n_rays < 1 || n_configs < 1 || 2 * (long long)n_configs * n_rays >= (1ll << 32)) return -1;
+  return (int64_t)abcd_layout(3ll * n_configs * n_rays).total;
+}
+
+extern "C" int optb_sweep_abcd_pivots(optb_ctx* ctx, const optb_result* rows, int64_t n, int64_t n_rays,
+                                      int32_t n_configs, int32_t mon0, double* pivots, int64_t* first_bad,
+                                      void* workspace, int64_t workspace_bytes, void* stream_v) {
+  if (!ctx || !rows || !pivots || !first_bad || n < 0 || n_rays < 1 || n_configs < 1) return -1;
+  if (int rc = abcd_check(ctx, "optb_sweep_abcd_pivots", rows, false, mon0, n, n_rays, n_configs)) return rc;
+  const long long KN = (long long)n_configs * n_rays;
+  const AbcdLayout L = abcd_layout(KN);
+  if (!workspace || workspace_bytes < (int64_t)L.total)
+    return fail(ctx, -7, "optb_sweep_abcd_pivots: workspace too small (optb_sweep_abcd_workspace_bytes)");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream_v;
+  unsigned char* ws = (unsigned char*)workspace;
+  uint32_t *count = (uint32_t*)(ws + L.count), *row = (uint32_t*)(ws + L.row);
+  const AbcdRows a = abcd_rows(rows);
+  CK(cudaMemsetAsync(count, 0, (size_t)KN * 4, st), "optb_sweep_abcd_pivots: clearing the slots");
+  CK(cudaMemsetAsync(first_bad, 0xff, sizeof(int64_t), st), "optb_sweep_abcd_pivots: clearing first_bad");
+  if (n > 0) {
+    const int grid = (int)std::min<long long>((n + 255) / 256, (long long)ctx->sm_count * 16);
+    abcd_scatter_kernel<<<grid, 256, 0, st>>>(a, n, mon0, n_rays, n_configs, 2 * n_rays, 0, 1, count, row);
+  }
+  abcd_pivots_kernel<<<(unsigned)((KN + 255) / 256), 256, 0, st>>>(a, n_rays, n_configs, count, row, pivots,
+                                                                    (unsigned long long*)first_bad);
+  CK(cudaGetLastError(), "optb_sweep_abcd_pivots");
+  return 0;
+}
+
+extern "C" int optb_sweep_abcd(optb_ctx* ctx, const optb_result* rows_a, int64_t n_a, const optb_result* rows_b,
+                               int64_t n_b, int64_t n_rays, int32_t n_configs, int32_t mon1,
+                               const optb_monitor_frame* frames, double disp, double rot, double* abcd, int32_t* counts,
+                               void* workspace, int64_t workspace_bytes, void* stream_v) {
+  if (!ctx || !rows_a || !rows_b || !frames || !abcd || !counts || n_a < 0 || n_b < 0 || n_rays < 1 || n_configs < 1)
+    return -1;
+  if (int rc = abcd_check(ctx, "optb_sweep_abcd", rows_a, true, mon1, n_a, n_rays, n_configs)) return rc;
+  if (int rc = abcd_check(ctx, "optb_sweep_abcd", rows_b, true, mon1, n_b, n_rays, n_configs)) return rc;
+  const long long KN = (long long)n_configs * n_rays;
+  const AbcdLayout L = abcd_layout(3 * KN);
+  if (!workspace || workspace_bytes < (int64_t)L.total)
+    return fail(ctx, -7, "optb_sweep_abcd: workspace too small (optb_sweep_abcd_workspace_bytes)");
+  cudaSetDevice(ctx->device);
+  cudaStream_t st = (cudaStream_t)stream_v;
+  unsigned char* ws = (unsigned char*)workspace;
+  uint32_t *count = (uint32_t*)(ws + L.count), *row = (uint32_t*)(ws + L.row);
+  const AbcdRows a = abcd_rows(rows_a), b = abcd_rows(rows_b);
+  CK(cudaMemsetAsync(count, 0, (size_t)(3 * KN) * 4, st), "optb_sweep_abcd: clearing the slots");
+  if (n_a > 0) {
+    const int grid = (int)std::min<long long>((n_a + 255) / 256, (long long)ctx->sm_count * 16);
+    abcd_scatter_kernel<<<grid, 256, 0, st>>>(a, n_a, mon1, n_rays, n_configs, 2 * n_rays, 0, 2, count, row);
+  }
+  if (n_b > 0) {
+    const int grid = (int)std::min<long long>((n_b + 255) / 256, (long long)ctx->sm_count * 16);
+    abcd_scatter_kernel<<<grid, 256, 0, st>>>(b, n_b, mon1, n_rays, n_configs, n_rays, 2, 3, count, row);
+  }
+  abcd_matrix_kernel<<<(unsigned)((KN + 255) / 256), 256, 0, st>>>(a, b, n_rays, n_configs, frames, disp, rot, count,
+                                                                    row, abcd, counts);
+  CK(cudaGetLastError(), "optb_sweep_abcd");
+  return 0;
+}
+
 // ---- multi-GPU monitor merge over NCCL (loaded at run time: no link-time dependency) ------------------------------
 namespace {
 // the few NCCL entry points used, with the ABI of nccl.h (ncclResult_t = int, ncclUniqueId = 128 bytes by value)

@@ -422,6 +422,33 @@ class SweepScene:
                      engine=engine, unit=unit, arrs=arrs)
         return SweepResult([self.table] * K, n, out, engine, monitors=frames)
 
+    def abcd_matrix(self, m0, m1, rays, configure, n_configs, disp=1e-5, rot=1e-5, perfomance_limit=None, engine=None,
+                    group=None):
+        """`OpticalTable.calculate_abcd_matrix(mon0, mon1, rays)` of every configuration from two sweep traces; returns
+        a SweepABCD (see `sweep_abcd_matrix`, whose preconditions and refusals hold here too).
+
+        `m0`, `m1`: monitor indices or monitors of the table. `configure(k)` runs once for every k = 0 .. n_configs - 1,
+        in order, as for `trace`; both bundles are traced through the configurations this builds. A configuration that
+        moves mon0 raises ValueError before anything is traced."""
+        from .flatten import batch_wavelengths_m, pack_rays, trace_cap
+
+        what = "SweepScene.abcd_matrix"
+        work, ids = _abcd_work(rays, group)
+        K = int(n_configs)
+        if K < 1:
+            raise ValueError(f"{what}: n_configs must be >= 1")
+        live = list(self.table.monitors)
+        m0, m1 = _monitor_index(live, m0, what), _monitor_index(live, m1, what)
+        arrs, _, unit = pack_rays(work)     # (both bundles have these wavelengths)
+        wls = batch_wavelengths_m(arrs["wavelength"], unit)
+        if self._base(wls)[0].n_capslots:
+            raise NotImplementedError(f"{what}: interact-capped components are not supported (the table method's three "
+                                      "traces carry their interact counts over from one to the next)")
+        rows, frames = self._configurations(wls, configure, 0, K)
+        _check_mon0(frames, m0, what)
+        return _abcd(rows, K, [self.table] * K, frames, m0, m1, work, ids, disp, rot, trace_cap(perfomance_limit),
+                     engine, what)
+
     def _configurations(self, wls, configure, k0, k1):
         """configure(k) for k = k0 .. k1 - 1 in order: the SweepRows of those configurations and their monitor frames
         (a _MonitorPose snapshot for a varied monitor, the live monitor otherwise)."""
@@ -457,3 +484,132 @@ class SweepScene:
             live = list(flat.monitors)
             frames.append([_MonitorPose(live[m]) if m in varied_mons else live[m] for m in range(len(live))])
         return SweepRows(flat, K, V, node_i, node_f, mons, mon_f), frames
+
+
+class SweepABCD:
+    """ABCD matrices of every configuration of a sweep (`sweep_abcd_matrix`, `SweepScene.abcd_matrix`).
+
+    `M` [K, N, 2, 2]: M[k, r] is what `OpticalTable.calculate_abcd_matrix(mon0, mon1, rays)` returns for ray r on
+    configuration k, rays in order of their ids `ids`; NaN where it is not defined. `row_counts` [K, N, 3]: the mon1 rows
+    of ray r in the nominal, the shifted and the turned trace. `defined` [K, N]: exactly one row in each trace. `valid`
+    [K]: every ray defined, the configurations for which the table method returns instead of raising. `traces`: the
+    SweepResults of the two sweeps (the nominal and shifted bundle, 2N rays; the turned bundle, N rays), so that
+    `traces[0].stats()` summarises the nominal trace at hand."""
+
+    def __init__(self, M, row_counts, ids, traces):
+        self.M, self.row_counts, self.ids, self.traces = M, row_counts, list(ids), tuple(traces)
+        self.defined = (row_counts == 1).all(-1)
+        self.valid = self.defined.all(-1)
+
+
+def _abcd_work(rays, group):
+    """calculate_abcd_matrix's `work` (copies of the rays, sorted by id) and the sorted ids, with its refusals."""
+    if group is not None and group is not False:
+        raise NotImplementedError("ABCD matrices of a sharded sweep (group=) are not supported: trace on one GPU")
+    rays = list(rays)
+    if not rays:
+        raise ValueError("No rays to trace in ABCD calculation.")
+    ids = [r._id for r in rays]
+    if len(set(ids)) != len(rays):
+        raise ValueError("Redundant ray ids in ABCD calculation.")
+    order = np.argsort(ids)
+    return [rays[i].copy() for i in order], [ids[i] for i in order]
+
+
+def _abcd_bundle_a(work, mon0, disp):
+    """The nominal rays and the same rays shifted by disp along mon0's tangent_Y: the one batch of
+    `OpticalTable._abcd_first_two_traces`."""
+    shift = mon0.tangent_Y * disp
+    return work + [r.copy()._Translate(shift) for r in work]
+
+
+def _abcd_bundle_b(work, mon0, pivots, disp, rot):
+    """The shifted rays turned by rot about mon0's tangent_Z through their pivots (the third trace of
+    calculate_abcd_matrix: the shift is not undone first)."""
+    shift, axis = mon0.tangent_Y * disp, mon0.tangent_Z
+    return [r.copy()._Translate(shift)._RotAround(axis, pivots[k], rot) for k, r in enumerate(work)]
+
+
+def _monitor_index(monitors, m, what):
+    if isinstance(m, (int, np.integer)):
+        if not 0 <= int(m) < len(monitors):
+            raise IndexError(f"{what}: monitor {int(m)} of {len(monitors)}")
+        return int(m)
+    for i, mon in enumerate(monitors):
+        if mon is m:
+            return i
+    raise ValueError(f"{what}: {type(m).__name__} is not a monitor of the table")
+
+
+def _check_mon0(monitors, m0, what):
+    """Every configuration must place mon0 (origin, tangents, size) exactly as configuration 0 does: then the three
+    bundles are the same in every configuration."""
+    ref = monitors[0][m0]
+    for k in range(1, len(monitors)):
+        mon = monitors[k][m0]
+        for a in ("origin", "tangent_Y", "tangent_Z", "width", "height"):
+            if not np.array_equal(np.asarray(getattr(mon, a), np.float64), np.asarray(getattr(ref, a), np.float64)):
+                raise ValueError(f"{what}: configuration {k} changes the {a} of mon0 (monitor {m0}): its ABCD bundles "
+                                 "would differ from configuration 0's, and sweeps that need a bundle per configuration "
+                                 "are not supported")
+
+
+def _abcd(configs, K, tables, monitors, m0, m1, work, ids, disp, rot, limit, engine, what):
+    """The device part of sweep_abcd_matrix / SweepScene.abcd_matrix: sweep A, the pivots, sweep B, the matrices."""
+    from .analytics import _frame
+    from .backend import Engine
+    from .flatten import pack_rays
+
+    engine = engine or Engine.get()
+    N, mon0 = len(work), monitors[0][m0]
+    arrs, _, unit = pack_rays(_abcd_bundle_a(work, mon0, disp))
+    res_a = SweepResult(tables, 2 * N, _device_sweep(configs, None, limit, engine=engine, unit=unit, arrs=arrs), engine,
+                        monitors=monitors)
+    pivots, first_bad = engine.sweep_abcd_pivots(res_a.hits, N, K, m0)
+    bad = int(first_bad.item())
+    if bad >= 0:
+        k, r = divmod(bad, N)
+        if k == 0:
+            raise ValueError(f"Rays at mon0 do not match the input rays. ({what}: ray id {ids[r]} has not exactly one "
+                             "row at mon0 in configuration 0)")
+        raise ValueError(f"{what}: in configuration {k}, ray id {ids[r]} does not cross mon0 exactly once at the point "
+                         "it crosses it in configuration 0: its ABCD bundles would differ from configuration 0's, and "
+                         "sweeps that need a bundle per configuration are not supported")
+    arrs, _, unit = pack_rays(_abcd_bundle_b(work, mon0, pivots.cpu().numpy(), disp, rot))
+    res_b = SweepResult(tables, N, _device_sweep(configs, None, limit, engine=engine, unit=unit, arrs=arrs), engine,
+                        monitors=monitors)
+    frames = (A.MonitorFrame * K)(*[_frame(monitors[k][m1]) for k in range(K)])
+    abcd, counts = engine.sweep_abcd(res_a.hits, res_b.hits, N, K, m1, frames, disp, rot)
+    return SweepABCD(abcd.cpu().numpy().reshape(K, N, 2, 2), counts.cpu().numpy(), ids, (res_a, res_b))
+
+
+def sweep_abcd_matrix(tables, m0, m1, rays, disp=1e-5, rot=1e-5, perfomance_limit=None, engine=None, group=None):
+    """`OpticalTable.calculate_abcd_matrix(mon0, mon1, rays)` of every table of `tables` (K configurations of one
+    scene, as for `trace_sweep`) from two sweep traces; returns a SweepABCD.
+
+    `m0`, `m1`: monitor indices, or monitors of tables[0]. The three bundles of the finite differences depend on the
+    scene only through mon0 and what lies in front of it, so every configuration must place mon0 exactly as
+    configuration 0 does and give every ray exactly one nominal mon0 hit point, bit-identical to configuration 0's
+    (then the bundles are the same for all K): otherwise ValueError, naming the configuration (and ray). Like the table
+    method: repeated ray ids raise ValueError; the pivots are configuration 0's mon0 hit points in monitor-local
+    coordinates. Interact-capped components raise NotImplementedError (the table method's three traces share their
+    counts), as does `group=`."""
+    from .flatten import FlatScene, batch_wavelengths_m, pack_rays, trace_cap
+
+    what = "sweep_abcd_matrix"
+    work, ids = _abcd_work(rays, group)
+    tables = list(tables)
+    if not tables:
+        raise ValueError(f"{what}: no tables")
+    monitors = [list(t.monitors) for t in tables]
+    m0, m1 = _monitor_index(monitors[0], m0, what), _monitor_index(monitors[0], m1, what)
+    _check_mon0(monitors, m0, what)
+    arrs, _, unit = pack_rays(work)     # (both bundles have these wavelengths)
+    wls = batch_wavelengths_m(arrs["wavelength"], unit)
+    flats = [FlatScene(t.components, t.monitors, wavelengths_m=wls) for t in tables]
+    check_topology(flats)
+    if flats[0].n_capslots:
+        raise NotImplementedError(f"{what}: interact-capped components are not supported (the table method's three "
+                                  "traces carry their interact counts over from one to the next)")
+    return _abcd(flats, len(tables), tables, monitors, m0, m1, work, ids, disp, rot, trace_cap(perfomance_limit), engine,
+                 what)
