@@ -448,16 +448,16 @@ int optb_sort_rows(optb_ctx* ctx, const optb_result* res, int64_t n_seg, int64_t
                    void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ---- monitor analytics on the device (SURVEY 8f item 2; monitor.py:78-253) ----------------------------------------
- * One fused pass over monitor rows that are still in HBM: for the rows [first, first + n) of `rows` that belong to
- * `monitor` (-1: every row of the range) it evaluates what the reference's Monitor accessors derive per row --
+ * Monitor rows that are still in HBM, reduced per group of rows (optb_monitor_stats_grouped below). For every row it
+ * evaluates, in its group's frame, what the reference's Monitor accessors derive per row --
  *   y = P_local . tangent_Y, z = P_local . tangent_Z   (get_yList / get_zList :78-100; LOCAL point, LAB tangent: the
  *                                                        reference's own convention, kept)
  *   tY = d . tangent_Y, tZ = d . tangent_Z             (get_tYList / tZList :137-157)
  *   waist distance = +-Re(q + t), minus when d . normal > 0   (get_waist_distance :202-216)
- * -- writes them to the optional per-row columns (NaN for rows of other monitors) and accumulates, in the same pass,
- * the row count, sum of intensities (sum_intensity / avg_intensity :236-242), first and second moments and extrema of
- * y and z, the sum of the waist distances and the 30-bin np.histogram of y over +-width/2 (_get_hist_y :195-200,
- * from which std_histy :244-249 follows). No row leaves the device.                                              */
+ * -- writes them to the optional per-row columns and accumulates, per group, the row count, sum of intensities
+ * (sum_intensity / avg_intensity :236-242), first and second moments and extrema of y and z, the sum of the waist
+ * distances and the 30-bin np.histogram of y over +-width/2 (_get_hist_y :195-200, from which std_histy :244-249
+ * follows) in the OPTB_MS_* slots. No row leaves the device.                                                     */
 typedef struct optb_monitor_frame {
   double tangent_y[3], tangent_z[3], normal[3]; /* Monitor.tangent_Y / tangent_Z / normal (lab frame) */
   double half_width, half_height;
@@ -466,7 +466,7 @@ enum {
   OPTB_MS_COUNT = 0, OPTB_MS_SUM_I = 1, OPTB_MS_SUM_Y = 2, OPTB_MS_SUM_YY = 3, OPTB_MS_SUM_Z = 4, OPTB_MS_SUM_ZZ = 5,
   OPTB_MS_SUM_WD = 6, OPTB_MS_MIN_Y = 7, OPTB_MS_MAX_Y = 8, OPTB_MS_MIN_Z = 9, OPTB_MS_MAX_Z = 10,
   OPTB_MS_SUM_TY = 11, OPTB_MS_SUM_TYTY = 12,
-  /* sums of (y - mean_y)^2, (z - mean_z)^2, (tY - mean_tY)^2 over the selected rows, taken in a second pass about the
+  /* sums of (y - mean_y)^2, (z - mean_z)^2, (tY - mean_tY)^2 over a group's rows, taken in a second pass about the
    * means of the first (std_y = sqrt(M2_Y / count) keeps full precision where SUM_YY / count - mean_y^2 cancels, e.g.
    * a small spot far off the monitor's axis). M2_TY is 0 without hit_dx..dz. Added in slots that were unused before,
    * without a change of OPTB_ABI_VERSION: no struct changed.                                                      */
@@ -474,25 +474,19 @@ enum {
   OPTB_MS_HIST = 16, /* 30 counts */
   OPTB_MS_STRIDE = 48
 };
-/* rows: DEVICE pointers (hit_px/py/pz, hit_intensity, hit_t required; hit_dx..dz for tY/tZ/waist sign, hit_q_re for the
- * waist distance; hit_monitor or hit_key when monitor >= 0). stats: device double[OPTB_MS_STRIDE], overwritten.
- * y, z, ty, tz, waist: device double[n] or NULL.                                                                  */
-int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_t first, int64_t n, int monitor,
-                       const optb_monitor_frame* frame, double* stats, double* y, double* z, double* ty, double* tz,
-                       double* waist, void* stream);
-
-/* The same summaries for every (configuration, monitor) group of the rows [first, first + n) in one call: what a scan,
- * an optimizer or a tolerance study ranks after one sweep (optb_scene_upload_sweep), or all monitors of one trace.
+/* The summaries of every (configuration, monitor) group of the rows [first, first + n) in one call: what a scan, an
+ * optimizer or a tolerance study ranks after one sweep (optb_scene_upload_sweep), or all monitors of one trace.
+ *   - rows: DEVICE pointers (hit_px/py/pz, hit_intensity, hit_t required; hit_dx..dz for tY/tZ/waist sign, hit_q_re for
+ *     the waist distance).
  *   - group of a row: g = k * n_monitors + m, k = root / rays_per_config (the K x N root numbering of a sweep scene;
  *     rays_per_config = 0: one configuration, k = 0), root from hit_root or else hit_key >> 32, m from hit_monitor or
  *     else (hit_key >> 24) & 0xff. A row with k >= n_configs or m outside [0, n_monitors) belongs to no group: its
  *     per-row outputs are NaN and it is counted nowhere (the counts then add up to less than n).
  *   - frames: DEVICE optb_monitor_frame[n_configs * n_monitors], group g evaluated in frames[g].
- *   - stats: DEVICE double[n_configs * n_monitors][OPTB_MS_STRIDE], overwritten; every group's slots mean what the
- *     OPTB_MS_* slots of optb_monitor_stats mean (M2_* about that group's own means; the histogram bins like
- *     np.histogram); a group without rows reads like optb_monitor_stats over no rows (zeros, min +inf, max -inf).
- *   - y, z, ty, tz, waist: DEVICE double[n] or NULL, row first + i at [i], evaluated in its group's frame; bit-identical
- *     to what optb_monitor_stats writes for that row and frame.
+ *   - stats: DEVICE double[n_configs * n_monitors][OPTB_MS_STRIDE], overwritten; group g's OPTB_MS_* slots over its
+ *     own rows (M2_* about that group's own means; the histogram bins like np.histogram); a group without rows reads
+ *     zeros, min +inf, max -inf.
+ *   - y, z, ty, tz, waist: DEVICE double[n] or NULL, row first + i at [i], evaluated in its group's frame.
  *   - rows may come in any order (sorted by optb_sort_rows, or in device append order).
  *   - deterministic: the same rows in the same order give bit-identical stats on every call, on any stream, whatever
  *     the device's SM count (rows are sorted by group, each group is reduced in tiles of a fixed size in a fixed order,

@@ -89,7 +89,7 @@ EXPORTED_SYMBOLS = (
     "optb_scene_upload", "optb_scene_upload_sweep", "optb_scene_upload_sweep_rows", "optb_scene_destroy",
     "optb_scene_update_nodes", "optb_workspace_bytes", "optb_trace",
     "optb_trace_host", "optb_trace_plan", "optb_measure_fp64_peak",
-    "optb_sort_workspace_bytes", "optb_sort_rows", "optb_monitor_stats",
+    "optb_sort_workspace_bytes", "optb_sort_rows",
     "optb_monitor_stats_grouped_workspace_bytes", "optb_monitor_stats_grouped",
     "optb_sweep_abcd_workspace_bytes", "optb_sweep_abcd_pivots", "optb_sweep_abcd",
     "optb_comm_unique_id", "optb_comm_init", "optb_monitor_merge", "optb_comm_destroy",

@@ -4,14 +4,14 @@ the row columns a bundle trace leaves in HBM, without copying rows to the host o
 `trace_bundle` returns one set of row columns for all monitors; `DeviceMonitor(table.monitors[m], out, m)` selects
 monitor m's rows. The per-row quantities (y, z, slopes, waist distances) and every summary that needs no ordering
 (row count, intensity sum / mean, moments and extrema of the spot, the 30-bin histogram behind `std_histy`) come from
-ONE fused pass of the library's own kernel over the rows (`optb_monitor_stats`, include/optb.h). Only the accessors the
-reference defines through a sort (`sort="YZ"` / `"ID"` views, `get_delta_pos`) order those columns with torch.sort
-(PyTorch as the array library). Row order "YZ" = lexicographic (y, z) of the monitor-local point like
-`Monitor.sortYZIndex`; "ID" = by initial ray (a bundle ray's id is its index); None = device append order.
+the library's grouped statistics kernels (`optb_monitor_stats_grouped`, include/optb.h), which reduce every group of
+rows in a fixed order: the same rows give the same bits on every call. `grouped_stats` and `monitor_stats` give the
+summaries of every (configuration, monitor) of a result in one call; a `DeviceMonitor` is one group of such a call.
+Only the accessors the reference defines through a sort (`sort="YZ"` / `"ID"` views, `get_delta_pos`) order those
+columns with torch.sort (PyTorch as the array library). Row order "YZ" = lexicographic (y, z) of the monitor-local
+point like `Monitor.sortYZIndex`; "ID" = by initial ray (a bundle ray's id is its index); None = device append order.
 """
 from __future__ import annotations
-
-import ctypes as C
 
 import numpy as np
 
@@ -28,9 +28,10 @@ def _frame(monitor) -> A.MonitorFrame:
 
 
 def stats_arrays(s, widths) -> dict:
-    """`DeviceMonitor.stats()` of many monitors at once: stats slots s [..., OPTB_MS_STRIDE] (numpy) -> the same keys as
-    arrays shaped s.shape[:-1] (hist_y: [..., 30]), plus `std_tY` (from OPTB_MS_M2_TY) and `std_histy` (the formula of
-    `DeviceMonitor.std_histy`; NaN for a monitor without rows in its histogram) for monitors of widths `widths`."""
+    """`DeviceMonitor.stats()` of many monitors at once: stats slots s [..., OPTB_MS_STRIDE] (numpy) -> its keys as
+    arrays shaped s.shape[:-1] (hist_y: [..., 30]), among them `std_tY` (from OPTB_MS_M2_TY) and `std_histy` (the
+    reference's Monitor.std_histy: the spread of the left bin edges weighted by the counts; NaN for a monitor without
+    rows in its histogram) for monitors of widths `widths`."""
     s = np.asarray(s, np.float64)
     n = np.maximum(s[..., A.MS_COUNT], 1.0)
     hist = s[..., A.MS_HIST:A.MS_HIST + A.HIST_BINS].astype(np.int64)
@@ -84,7 +85,7 @@ def grouped_slots(out: dict, monitors, rays_per_config=0, engine=None):
 
 def monitor_stats(monitors, out: dict, engine=None) -> dict:
     """`DeviceMonitor(monitors[m], out, m).stats()` of every monitor of a `trace_bundle` result in one device call:
-    the same keys as arrays shaped [M] (hist_y [M, 30]), plus `std_tY` and `std_histy` (see `stats_arrays`)."""
+    the same keys as arrays shaped [M] (hist_y [M, 30])."""
     s, _ = grouped_stats(out, [list(monitors)], 0, engine)
     return {k: v[0] for k, v in s.items()}
 
@@ -93,37 +94,24 @@ class DeviceMonitor:
     def __init__(self, monitor, out: dict, index: int, engine=None):
         import torch
 
-        from .backend import Engine, lib
+        from .backend import Engine
 
         self.monitor, self.torch = monitor, torch
-        any_col = out["hit_px"]
-        dev = any_col.device
-        self.engine = engine or Engine.get(dev.index or 0)
-        n = int(any_col.numel())
-        # ---- the fused pass: per-row y / z / tY / tZ / waist distance + all order-free summaries, straight from HBM
-        res = A.Result()
-        for k in A.HIT_I32 + A.HIT_U32 + A.HIT_F64 + ("hit_key",):
-            if out.get(k) is not None:
-                setattr(res, k, out[k].data_ptr())
-        fr = _frame(monitor)
-        f64 = torch.float64
-        has_d, has_q = out.get("hit_dx") is not None, out.get("hit_q_re") is not None
-        cols = torch.empty((5, max(n, 1)), dtype=f64, device=dev)
-        self._stats_dev = torch.empty(A.MS_STRIDE, dtype=f64, device=dev)
-        L = lib()
-        L.optb_monitor_stats.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_int, C.POINTER(A.MonitorFrame),
-                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
-        ptr = lambda r, ok=True: C.c_void_p(cols[r].data_ptr()) if ok else None
-        st = torch.cuda.current_stream(dev).cuda_stream
-        self.engine._check(L.optb_monitor_stats(self.engine._ctx, C.byref(res), 0, n, int(index), C.byref(fr),
-                                                C.c_void_p(self._stats_dev.data_ptr()), ptr(0), ptr(1), ptr(2, has_d),
-                                                ptr(3, has_d), ptr(4, has_d and has_q), C.c_void_p(st)))
-        sel = torch.nonzero(~torch.isnan(cols[0, :n])).squeeze(1)   # rows of this monitor (the kernel marks the others NaN)
+        self.engine = engine or Engine.get(out["hit_px"].device.index or 0)
+        # one grouped call with monitors 0..index, each in this monitor's frame: rows of higher monitors fall in no
+        # group, and group `index` holds this monitor's rows (the Engine is called directly because grouped_slots
+        # refuses rows outside every group)
+        frames = (A.MonitorFrame * (index + 1))(*[_frame(monitor)] * (index + 1))
+        stats, cols = self.engine.monitor_stats_grouped(out, frames, 1, index + 1)
+        self._slots = stats[index]
+        mon = out["hit_monitor"] if out.get("hit_monitor") is not None else (out["hit_key"] >> 24) & 0xFF
+        sel = torch.nonzero(mon == index).squeeze(1)
         col = lambda k: out[k][sel] if out.get(k) is not None else None
-        self._y, self._z = cols[0, :n][sel], cols[1, :n][sel]
-        self._ty = cols[2, :n][sel] if has_d else None
-        self._tz = cols[3, :n][sel] if has_d else None
-        self._wd = cols[4, :n][sel] if has_d and has_q else None
+        has_d, has_q = out.get("hit_dx") is not None, out.get("hit_q_re") is not None
+        self._y, self._z = cols[0][sel], cols[1][sel]
+        self._ty = cols[2][sel] if has_d else None
+        self._tz = cols[3][sel] if has_d else None
+        self._wd = cols[4][sel] if has_d and has_q else None
         if out.get("hit_key") is not None and out.get("hit_root") is None:
             key = out["hit_key"][sel]
             self.root, self.pop = (key >> 32) & 0xFFFFFFFF, key & 0xFFFFFF
@@ -140,19 +128,11 @@ class DeviceMonitor:
         self._stats = None
 
     def stats(self) -> dict:
-        """Order-free summaries of this monitor's rows from the fused kernel (one small device-to-host read)."""
+        """Order-free summaries of this monitor's rows, the keys of `stats_arrays` (one small device-to-host read):
+        `count` an int, `hist_y` an int64 array, every other key a float."""
         if self._stats is None:
-            s = self._stats_dev.cpu().numpy()
-            n = max(s[A.MS_COUNT], 1.0)
-            my, mz = s[A.MS_SUM_Y] / n, s[A.MS_SUM_Z] / n
-            self._stats = {
-                "count": int(s[A.MS_COUNT]), "sum_intensity": float(s[A.MS_SUM_I]), "avg_intensity": float(s[A.MS_SUM_I] / n),
-                "mean_y": float(my), "mean_z": float(mz),
-                "std_y": float(np.sqrt(s[A.MS_M2_Y] / n)), "std_z": float(np.sqrt(s[A.MS_M2_Z] / n)),
-                "min_y": float(s[A.MS_MIN_Y]), "max_y": float(s[A.MS_MAX_Y]), "min_z": float(s[A.MS_MIN_Z]), "max_z": float(s[A.MS_MAX_Z]),
-                "mean_waist_distance": float(s[A.MS_SUM_WD] / n), "mean_tY": float(s[A.MS_SUM_TY] / n),
-                "hist_y": s[A.MS_HIST:A.MS_HIST + A.HIST_BINS].astype(np.int64),
-            }
+            s = stats_arrays(self._slots.cpu().numpy(), float(self.monitor.width))
+            self._stats = {k: v if k == "hist_y" else int(v) if k == "count" else float(v) for k, v in s.items()}
         return self._stats
 
     @property
@@ -221,17 +201,13 @@ class DeviceMonitor:
 
     def _get_hist_y(self):
         """(counts, bin edges) of the 30-bin histogram of yList over +-width/2 (monitor.py:195-200), accumulated by
-        the fused kernel with np.histogram's binning."""
+        the statistics kernels with np.histogram's binning."""
         w = float(self.monitor.width)
         return self.stats()["hist_y"], np.linspace(-w / 2, w / 2, 31)
 
     @property
     def std_histy(self):
-        counts, edges = self._get_hist_y()
-        c = counts.astype(np.float64)
-        left = edges[:-1]
-        mean = (c * left).sum() / c.sum()
-        return float(np.sqrt((c * left ** 2).sum() / c.sum() - mean ** 2))
+        return self.stats()["std_histy"]
 
     def export_rays_npz(self, filename: str):
         """Same arrays as Monitor.export_rays_npz (monitor.py:255-269); this is the one place rows leave the device."""

@@ -2403,40 +2403,12 @@ extern "C" int optb_sort_rows(optb_ctx* ctx, const optb_result* res, int64_t n_s
   return sort_rows_dev(ctx, res, nullptr, n_seg, n_hit, nullptr, workspace, workspace_bytes, (cudaStream_t)stream_v, 64);
 }
 
-// ---- monitor analytics: one fused pass over the rows in HBM ---------------------------------------------------------
+// ---- monitor analytics on the rows in HBM ---------------------------------------------------------------------------
 namespace {
-struct StatsArgs {
-  const double *px, *py, *pz, *I, *t, *dx, *dy, *dz, *qre;
-  const int32_t* mon; const unsigned long long* key;
-  long long first, n; int monitor;
-  optb_monitor_frame f;
-  double *stats, *y, *z, *ty, *tz, *wd;
-};
-OPTB_DEV void atomic_min_f64(double* addr, double v) {
-  unsigned long long* a = (unsigned long long*)addr;
-  unsigned long long old = *a;
-  while (v < __longlong_as_double((long long)old)) {
-    const unsigned long long seen = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
-    if (seen == old) break;
-    old = seen;
-  }
-}
-OPTB_DEV void atomic_max_f64(double* addr, double v) {
-  unsigned long long* a = (unsigned long long*)addr;
-  unsigned long long old = *a;
-  while (v > __longlong_as_double((long long)old)) {
-    const unsigned long long seen = atomicCAS(a, old, (unsigned long long)__double_as_longlong(v));
-    if (seen == old) break;
-    old = seen;
-  }
-}
-__global__ void stats_init_kernel(double* s) {
-  const int k = threadIdx.x;
-  if (k < OPTB_MS_STRIDE) s[k] = (k == OPTB_MS_MIN_Y || k == OPTB_MS_MIN_Z) ? INFINITY : (k == OPTB_MS_MAX_Y || k == OPTB_MS_MAX_Z) ? -INFINITY : 0.0;
-}
 // What the Monitor accessors derive for row j in frame f: y, z (local point . lab tangent), tY, tZ and the signed waist
 // distance (NaN without hit_dx..dz, resp. hit_q_re); returns the row's bin of the 30-bin histogram of y (-1 outside).
-// One definition for the single-monitor and the grouped kernels, so that their per-row columns agree bit for bit.
+// One definition for the grouped statistics kernels and abcd_matrix_kernel, so that the per-row values they use agree
+// bit for bit.
 template <class Cols>
 OPTB_DEV int eval_row(const Cols& a, long long j, const optb_monitor_frame& f, double& y, double& z, double& ty,
                       double& tz, double& wd) {
@@ -2455,128 +2427,7 @@ OPTB_DEV int eval_row(const Cols& a, long long j, const optb_monitor_frame& f, d
   }
   return hist_bin(y, -f.half_width, f.half_width);
 }
-__global__ void __launch_bounds__(256) monitor_stats_kernel(const StatsArgs a) {
-  __shared__ unsigned int s_hist[OPTB_HIST_BINS];
-  __shared__ double s_red[8][8];
-  if (threadIdx.x < OPTB_HIST_BINS) s_hist[threadIdx.x] = 0u;
-  __syncthreads();
-  double cnt = 0, sI = 0, sy = 0, syy = 0, sz = 0, szz = 0, swd = 0, sty = 0, styty = 0;
-  double ymin = INFINITY, ymax = -INFINITY, zmin = INFINITY, zmax = -INFINITY;
-  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < a.n; k += (long long)gridDim.x * blockDim.x) {
-    const long long j = a.first + k;
-    bool mine = true;
-    if (a.monitor >= 0) mine = a.mon ? (a.mon[j] == a.monitor) : (int)((a.key[j] >> 24) & 0xffu) == a.monitor;
-    double y = NAN, z = NAN, ty = NAN, tz = NAN, wd = NAN;
-    if (mine) {
-      const int b = eval_row(a, j, a.f, y, z, ty, tz, wd);
-      cnt += 1.0; sI += a.I[j]; sy += y; syy = fma(y, y, syy); sz += z; szz = fma(z, z, szz);
-      ymin = fmin(ymin, y); ymax = fmax(ymax, y); zmin = fmin(zmin, z); zmax = fmax(zmax, z);
-      if (b >= 0) atomicAdd(&s_hist[b], 1u);
-      if (a.dx) {
-        sty += ty; styty = fma(ty, ty, styty);
-        if (a.qre) swd += wd;
-      }
-    }
-    if (a.y) a.y[k] = y;
-    if (a.z) a.z[k] = z;
-    if (a.ty) a.ty[k] = ty;
-    if (a.tz) a.tz[k] = tz;
-    if (a.wd) a.wd[k] = wd;
-  }
-  // block reduction: warp shuffles, then one atomic per block and quantity
-  double v[9] = {cnt, sI, sy, syy, sz, szz, swd, sty, styty};
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < 9; q++) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    ymin = fmin(ymin, __shfl_xor_sync(0xffffffffu, ymin, o)); ymax = fmax(ymax, __shfl_xor_sync(0xffffffffu, ymax, o));
-    zmin = fmin(zmin, __shfl_xor_sync(0xffffffffu, zmin, o)); zmax = fmax(zmax, __shfl_xor_sync(0xffffffffu, zmax, o));
-  }
-  const int slot[9] = {OPTB_MS_COUNT, OPTB_MS_SUM_I, OPTB_MS_SUM_Y, OPTB_MS_SUM_YY, OPTB_MS_SUM_Z, OPTB_MS_SUM_ZZ,
-                       OPTB_MS_SUM_WD, OPTB_MS_SUM_TY, OPTB_MS_SUM_TYTY};
-  if (lane == 0) {
-    for (int q = 0; q < 8; q++) s_red[q][wid] = q < 8 ? v[q] : 0.0;
-  }
-  __syncthreads();
-  if (threadIdx.x < 8) {
-    double tot = 0;
-    for (int w = 0; w < 8; w++) tot += s_red[threadIdx.x][w];
-    if (tot != 0.0) atomicAdd(&a.stats[slot[threadIdx.x]], tot);
-  }
-  if (lane == 0) {
-    if (v[8] != 0.0) atomicAdd(&a.stats[OPTB_MS_SUM_TYTY], v[8]);
-    if (ymin <= ymax) { atomic_min_f64(&a.stats[OPTB_MS_MIN_Y], ymin); atomic_max_f64(&a.stats[OPTB_MS_MAX_Y], ymax); }
-    if (zmin <= zmax) { atomic_min_f64(&a.stats[OPTB_MS_MIN_Z], zmin); atomic_max_f64(&a.stats[OPTB_MS_MAX_Z], zmax); }
-  }
-  __syncthreads();
-  if (threadIdx.x < OPTB_HIST_BINS && s_hist[threadIdx.x]) atomicAdd(&a.stats[OPTB_MS_HIST + threadIdx.x], (double)s_hist[threadIdx.x]);
-}
-// Second pass: sums of squares about the means the first pass left in `stats`. sum_yy / n - mean^2 cancels for a spot
-// far off axis (|mean| / std = 1e4 already loses 8 digits); centred sums keep the spread to rounding.
-__global__ void __launch_bounds__(256) monitor_m2_kernel(const StatsArgs a) {
-  __shared__ double s_red[3][8];
-  const double n = a.stats[OPTB_MS_COUNT];
-  if (n == 0.0) return;
-  const double my = a.stats[OPTB_MS_SUM_Y] / n, mz = a.stats[OPTB_MS_SUM_Z] / n, mty = a.stats[OPTB_MS_SUM_TY] / n;
-  double v[3] = {0.0, 0.0, 0.0};
-  for (long long k = blockIdx.x * (long long)blockDim.x + threadIdx.x; k < a.n; k += (long long)gridDim.x * blockDim.x) {
-    const long long j = a.first + k;
-    if (a.monitor >= 0 && (a.mon ? a.mon[j] != a.monitor : (int)((a.key[j] >> 24) & 0xffu) != a.monitor)) continue;
-    double y, z, ty, tz, wd;
-    eval_row(a, j, a.f, y, z, ty, tz, wd);
-    y -= my; z -= mz;
-    v[0] = fma(y, y, v[0]); v[1] = fma(z, z, v[1]);
-    if (a.dx) {
-      ty -= mty;
-      v[2] = fma(ty, ty, v[2]);
-    }
-  }
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-  for (int q = 0; q < 3; q++) {
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
-    if (lane == 0) s_red[q][wid] = v[q];
-  }
-  __syncthreads();
-  if (threadIdx.x < 3) {
-    double tot = 0;
-    for (int w = 0; w < 8; w++) tot += s_red[threadIdx.x][w];
-    if (tot != 0.0) atomicAdd(&a.stats[OPTB_MS_M2_Y + threadIdx.x], tot);
-  }
-}
 }  // namespace
-
-extern "C" int optb_monitor_stats(optb_ctx* ctx, const optb_result* rows, int64_t first, int64_t n, int monitor,
-                                  const optb_monitor_frame* frame, double* stats, double* y, double* z, double* ty,
-                                  double* tz, double* waist, void* stream_v) {
-  if (!ctx || !rows || !frame || !stats || first < 0 || n < 0) return -1;
-  if (!rows->hit_px || !rows->hit_py || !rows->hit_pz || !rows->hit_intensity || !rows->hit_t)
-    return fail(ctx, -7, "optb_monitor_stats: hit_px/py/pz, hit_intensity and hit_t are required");
-  if (monitor >= 0 && !rows->hit_monitor && !rows->hit_key) return fail(ctx, -7, "optb_monitor_stats: selecting a monitor needs hit_monitor or hit_key");
-  if ((ty || tz || waist) && !(rows->hit_dx && rows->hit_dy && rows->hit_dz)) return fail(ctx, -7, "optb_monitor_stats: slopes / waist distances need hit_dx, hit_dy, hit_dz");
-  if (waist && !rows->hit_q_re) return fail(ctx, -7, "optb_monitor_stats: waist distances need hit_q_re");
-  cudaSetDevice(ctx->device);
-  cudaStream_t st = (cudaStream_t)stream_v;
-  StatsArgs a;
-  a.px = rows->hit_px; a.py = rows->hit_py; a.pz = rows->hit_pz; a.I = rows->hit_intensity; a.t = rows->hit_t;
-  a.dx = rows->hit_dx && rows->hit_dy && rows->hit_dz ? rows->hit_dx : nullptr; a.dy = rows->hit_dy; a.dz = rows->hit_dz;
-  a.qre = rows->hit_q_re; a.mon = rows->hit_monitor; a.key = (const unsigned long long*)rows->hit_key;
-  a.first = first; a.n = n; a.monitor = monitor; a.f = *frame;
-  a.stats = stats; a.y = y; a.z = z; a.ty = ty; a.tz = tz; a.wd = waist;
-  stats_init_kernel<<<1, 64, 0, st>>>(stats);
-  if (n > 0) {
-    const int grid = (int)std::min<long long>((n + 255) / 256, (long long)ctx->sm_count * 8);
-    monitor_stats_kernel<<<grid, 256, 0, st>>>(a);
-    monitor_m2_kernel<<<grid, 256, 0, st>>>(a);
-  }
-  CK(cudaGetLastError(), "monitor_stats_kernel");
-  return 0;
-}
 
 // ---- grouped monitor analytics: every (configuration, monitor) of a result in one call, deterministically ---------
 // Rows are sorted by group (stable radix sort of (group, row index)), each group's run is cut into tiles of kGroupTile
@@ -2667,7 +2518,7 @@ OPTB_DEV bool find_tile(const GroupArgs& a, long long tile, int& g, uint32_t& ro
   row1 = min(row0 + (uint32_t)kGroupTile, a.start[g + 1]);
   return true;
 }
-// first pass over one tile: the sums, extrema and histogram of optb_monitor_stats, and the per-row outputs
+// first pass over one tile: the sums, extrema and histogram of the OPTB_MS_* slots, and the per-row outputs
 __global__ void __launch_bounds__(kGroupThreads) group_stats_kernel(const GroupArgs a) {
   __shared__ unsigned int s_hist[OPTB_HIST_BINS];
   __shared__ double s_red[OPTB_MS_M2_Y][kGroupThreads / 32];
@@ -2726,7 +2577,7 @@ __global__ void __launch_bounds__(kGroupThreads) group_stats_kernel(const GroupA
     a.part[(r < 3 ? OPTB_MS_M2_Y + r : OPTB_MS_HIST + OPTB_HIST_BINS + r - 3) * a.part_stride + tile] = 0.0;
   }
 }
-// second pass over one tile: sums of squares about the group's means (what monitor_m2_kernel does for one monitor)
+// second pass over one tile: sums of squares about the group's means
 __global__ void __launch_bounds__(kGroupThreads) group_m2_kernel(const GroupArgs a) {
   __shared__ double s_red[3][kGroupThreads / 32];
   int g; uint32_t row0, row1;
@@ -2763,7 +2614,7 @@ __global__ void __launch_bounds__(kGroupThreads) group_m2_kernel(const GroupArgs
   }
 }
 // one warp per group: slots [q0, q1) of stats[g] from the group's tile partials, in tile order (lane l takes tiles
-// l, l + 32, ...; then a fixed shuffle tree). A group without rows gets the values of optb_monitor_stats over no rows.
+// l, l + 32, ...; then a fixed shuffle tree). A group without rows gets zeros, min +inf and max -inf.
 __global__ void group_combine_kernel(const GroupArgs a, int q0, int q1) {
   const long long g = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
   if (g >= a.n_groups) return;

@@ -171,9 +171,9 @@ class SweepResult:
     def stats(self) -> dict:
         """Summaries of every configuration k and monitor m from one device call over all monitor rows
         (`optb_monitor_stats_grouped`; each in the frame of monitors[k][m]) and one copy back: the keys of
-        `DeviceMonitor.stats()` as numpy arrays [K, M] (hist_y [K, M, 30]), plus `std_tY` and `std_histy`. The same
-        sweep gives the same bits on every call, so a ranking of configurations does not change between calls; a
-        sharded sweep gives the bits of the one-GPU sweep."""
+        `DeviceMonitor.stats()` as numpy arrays [K, M] (hist_y [K, M, 30]). The same sweep gives the same bits on
+        every call, so a ranking of configurations does not change between calls; a sharded sweep gives the bits of
+        the one-GPU sweep."""
         return self._stats if self._stats is not None else self._grouped_stats()[0]
 
     def row_values(self) -> dict:

@@ -250,7 +250,7 @@ def test_device_monitor_analytics_match_host_monitor(tmp_path):
         assert float(dm.sum_intensity) == pytest.approx(host.sum_intensity, rel=1e-12)
         assert float(dm.std_histy) == pytest.approx(host.std_histy, rel=1e-12)
         counts, _ = host._get_hist_y()
-        np.testing.assert_array_equal(dm._get_hist_y()[0], counts)           # the fused kernel's own binning
+        np.testing.assert_array_equal(dm._get_hist_y()[0], counts)           # the statistics kernels' own binning
         np.testing.assert_array_equal(out["hist_y"][m].cpu().numpy(), counts)  # = the histogram the trace accumulated
         y, z = dm.get_yList(sort=None).cpu().numpy(), dm.get_zList(sort=None).cpu().numpy()
         hw, hh = float(mon.width) / 2, float(mon.height) / 2
@@ -323,7 +323,7 @@ def test_component_interact_single_pop_on_device():
 
 @pytest.mark.parametrize("name", ["doublet", "telescope_4f", "callable_material", "ripa2_simplified"])
 def test_device_monitor_analytics_match_reference_monitor_methods(name):
-    """f2: optable_b200.analytics.DeviceMonitor (fused optb_monitor_stats pass over rows that stay in HBM) against
+    """f2: optable_b200.analytics.DeviceMonitor (optb_monitor_stats_grouped over rows that stay in HBM) against
     what the REFERENCE's own Monitor methods returned after the reference's own trace (monitor.py:78-253; fixture
     tests/golden/monitor_analytics.npz, made by oracle/make_golden.py analytics)."""
     import os

@@ -1,8 +1,8 @@
 """GPU: monitor histograms and monitor statistics against numpy, exactly, at the bin edges.
 
 The contract is np.histogram(y, bins=30, range=(-w/2, w/2)) (and np.histogram2d for the (y, z) histogram), both for the
-histograms a trace accumulates (record_hist) and for the fused analytics pass (optb_monitor_stats). Comparing one device
-histogram with another cannot see a binning error, so every comparison here is with numpy of the rows themselves."""
+histograms a trace accumulates (record_hist) and for the monitor statistics (optb_monitor_stats_grouped). Comparing one
+device histogram with another cannot see a binning error, so every comparison here is with numpy of the rows themselves."""
 import ctypes as C
 import math
 
@@ -22,7 +22,7 @@ def engine():
     return Engine.get(0)
 
 
-# ---- optb_monitor_stats on row columns built directly -------------------------------------------------------------
+# ---- optb_monitor_stats_grouped on row columns built directly ----------------------------------------------------
 def _rows(y, z, seed=1, monitor=None, d=None):
     """Row columns of a monitor whose local hit points are (0, y, z), as CUDA tensors."""
     import torch
@@ -41,8 +41,9 @@ def _rows(y, z, seed=1, monitor=None, d=None):
     return host, cols
 
 
-def _monitor_stats(engine, cols, first, n, monitor, hw, hh, frame=None):
-    """One optb_monitor_stats call; returns (stats, per-row [y, z, tY, tZ, waist]) on the host."""
+def _monitor_stats(engine, cols, first, n, n_monitors, hw, hh, frame=None):
+    """One optb_monitor_stats_grouped call over rows [first, first + n), one configuration, monitors 0..n_monitors-1
+    all in one frame; returns (stats [n_monitors, OPTB_MS_STRIDE], per-row [y, z, tY, tZ, waist]) on the host."""
     import torch
 
     from optable_b200 import _abi as A
@@ -55,15 +56,17 @@ def _monitor_stats(engine, cols, first, n, monitor, hw, hh, frame=None):
     ty, tz, nrm = frame if frame is not None else ((0.0, 1.0, 0.0), (0.0, 0.0, 1.0), (1.0, 0.0, 0.0))
     fr.tangent_y[:], fr.tangent_z[:], fr.normal[:] = list(ty), list(tz), list(nrm)
     fr.half_width, fr.half_height = float(hw), float(hh)
-    stats = torch.full((A.MS_STRIDE,), 7.0, dtype=torch.float64, device="cuda")
+    frames = torch.frombuffer(bytearray((A.MonitorFrame * n_monitors)(*[fr] * n_monitors)), dtype=torch.uint8).cuda()
+    stats = torch.full((n_monitors, A.MS_STRIDE), 7.0, dtype=torch.float64, device="cuda")
     per_row = torch.full((5, max(n, 1)), 7.0, dtype=torch.float64, device="cuda")
     L = lib()
-    L.optb_monitor_stats.argtypes = [C.c_void_p, C.POINTER(A.Result), C.c_int64, C.c_int64, C.c_int, C.POINTER(A.MonitorFrame)] + \
-        [C.c_void_p] * 7
+    ws = torch.empty(int(L.optb_monitor_stats_grouped_workspace_bytes(n, n_monitors)), dtype=torch.uint8, device="cuda")
     st = torch.cuda.current_stream().cuda_stream
     ptr = lambda r: C.c_void_p(per_row[r].data_ptr())
-    engine._check(L.optb_monitor_stats(engine._ctx, C.byref(res), int(first), int(n), int(monitor), C.byref(fr),
-                                       C.c_void_p(stats.data_ptr()), ptr(0), ptr(1), ptr(2), ptr(3), ptr(4), C.c_void_p(st)))
+    engine._check(L.optb_monitor_stats_grouped(engine._ctx, C.byref(res), int(first), int(n), 0, 1, int(n_monitors),
+                                               C.c_void_p(frames.data_ptr()), C.c_void_p(stats.data_ptr()), ptr(0), ptr(1),
+                                               ptr(2), ptr(3), ptr(4), C.c_void_p(ws.data_ptr()), int(ws.numel()),
+                                               C.c_void_p(st)))
     torch.cuda.synchronize()
     return stats.cpu().numpy(), per_row[:, :n].cpu().numpy()
 
@@ -75,11 +78,11 @@ def _hist(stats):
 
 
 @pytest.mark.parametrize("hw", H.HALF_WIDTHS)
-def test_monitor_stats_hist_is_np_histogram_at_the_edges(engine, hw):
+def test_grouped_stats_hist_is_np_histogram_at_the_edges(engine, hw):
     y = H.edge_values(hw)
-    _, cols = _rows(y, np.zeros_like(y))
-    stats, per_row = _monitor_stats(engine, cols, 0, len(y), -1, hw, 1.0)
-    got = _hist(stats)
+    _, cols = _rows(y, np.zeros_like(y), monitor=np.zeros(len(y)))
+    stats, per_row = _monitor_stats(engine, cols, 0, len(y), 1, hw, 1.0)
+    got = _hist(stats[0])
     assert np.array_equal(got, H.numpy_hist(y, hw)), H.explain_hist(y, got, hw)
     np.testing.assert_array_equal(per_row[0], y)   # identity frame: y passes through unchanged (NaN included)
 
@@ -104,10 +107,9 @@ def _check_sums(stats, ref):
 
 
 def _check_rows(per_row, ref, sel, exact):
-    """Per-row outputs: the monitor's rows equal numpy (exact for an identity frame), every other row is NaN."""
+    """Per-row outputs of the selected rows equal numpy (exact for an identity frame)."""
     for r, k in enumerate(("y", "z", "ty", "tz", "wd")):
         got = per_row[r]
-        assert np.isnan(got[~sel]).all(), f"{k}: rows of other monitors must be NaN"
         if exact or k == "wd":
             np.testing.assert_array_equal(got[sel], ref[k], err_msg=k)
         else:   # a dot product of three terms: within 1e-15 of the sum of the magnitudes of its terms
@@ -119,9 +121,11 @@ def _check_rows(per_row, ref, sel, exact):
 @pytest.mark.parametrize("n,first,select", [
     (0, 10, "all"), (1, 0, "all"), (1000 + 37, 0, "all"), (1000 + 37, 0, "monitor"), (1000 + 37, 0, "key"),
     (5000, 123, "monitor"), (5000, 123, "key"), (1_000_000, 0, "all"), (1_000_000, 17, "monitor")])
-def test_monitor_stats_against_numpy(engine, n, first, select):
-    """Counts, histogram, extrema exact; sums to 1e-13 of fsum; per-row columns exact, NaN on other monitors' rows.
-    1e6 rows exceed the grid cap (sm_count * 8 blocks of 256), so the grid-stride loop runs more than once."""
+def test_grouped_stats_against_numpy(engine, n, first, select):
+    """Every group = monitor against numpy of its rows: counts, histogram, extrema exact; sums to 1e-13 of fsum; per-row
+    columns exact. Rows have monitors 0..2; "all" has a group for each, "monitor" and "key" (the monitor read from
+    hit_key) only for 0 and 1, so monitor 2's rows belong to no group and their per-row columns must be NaN. 1e6 rows
+    make a group of many tiles, combined in tile order."""
     import torch
 
     hw, hh = 2.5, 1.5
@@ -133,34 +137,37 @@ def test_monitor_stats_against_numpy(engine, n, first, select):
     z = rng.uniform(-1.2 * hh, 1.2 * hh, total)
     mon = rng.integers(0, 3, total)
     h, cols = _rows(y, z, seed=n, monitor=mon)
-    monitor = -1 if select == "all" else 1
+    M = 3 if select == "all" else 2
     if select == "key":   # root << 32 | monitor << 24 | pop, and no hit_monitor column
         key = (np.arange(total, dtype=np.int64) << 32) | (mon.astype(np.int64) << 24) | 5
         cols["hit_key"] = torch.from_numpy(key).cuda()
         del cols["hit_monitor"]
-    stats, per_row = _monitor_stats(engine, cols, first, n, monitor, hw, hh)
+    stats, per_row = _monitor_stats(engine, cols, first, n, M, hw, hh)
     from optable_b200 import _abi as A
 
+    assert np.isnan(per_row[:, mon[first:] >= M]).all(), "rows of no group must be NaN"
     win = np.zeros(total, bool)
     win[first:] = True
-    sel_all = win & ((mon == monitor) if monitor >= 0 else True)
-    sel = sel_all[first:]
-    ref = _numpy_stats(h, sel_all)
-    assert stats[A.MS_COUNT] == sel.sum()
-    got = _hist(stats)
-    assert np.array_equal(got, H.numpy_hist(ref["y"], hw)), H.explain_hist(ref["y"], got, hw)
-    if sel.sum() == 0:
-        assert stats[A.MS_MIN_Y] == math.inf and stats[A.MS_MAX_Y] == -math.inf
-        assert stats[A.MS_MIN_Z] == math.inf and stats[A.MS_MAX_Z] == -math.inf
-        assert (stats[:A.MS_MIN_Y] == 0).all() and (stats[A.MS_SUM_TY:A.MS_HIST + H.BINS] == 0).all()
-        return
-    assert stats[A.MS_MIN_Y] == ref["y"].min() and stats[A.MS_MAX_Y] == ref["y"].max()
-    assert stats[A.MS_MIN_Z] == ref["z"].min() and stats[A.MS_MAX_Z] == ref["z"].max()
-    _check_sums(stats, ref)
-    _check_rows(per_row, ref, sel, exact=True)
+    for g in range(M):
+        s = stats[g]
+        sel_all = win & (mon == g)
+        sel = sel_all[first:]
+        ref = _numpy_stats(h, sel_all)
+        assert s[A.MS_COUNT] == sel.sum(), g
+        got = _hist(s)
+        assert np.array_equal(got, H.numpy_hist(ref["y"], hw)), H.explain_hist(ref["y"], got, hw)
+        if sel.sum() == 0:
+            assert s[A.MS_MIN_Y] == math.inf and s[A.MS_MAX_Y] == -math.inf
+            assert s[A.MS_MIN_Z] == math.inf and s[A.MS_MAX_Z] == -math.inf
+            assert (s[:A.MS_MIN_Y] == 0).all() and (s[A.MS_SUM_TY:A.MS_HIST + H.BINS] == 0).all()
+            continue
+        assert s[A.MS_MIN_Y] == ref["y"].min() and s[A.MS_MAX_Y] == ref["y"].max()
+        assert s[A.MS_MIN_Z] == ref["z"].min() and s[A.MS_MAX_Z] == ref["z"].max()
+        _check_sums(s, ref)
+        _check_rows(per_row, ref, sel, exact=True)
 
 
-def test_monitor_stats_rotated_frame(engine):
+def test_grouped_stats_rotated_frame(engine):
     """A rotated frame: per-row columns within 1e-15 of numpy, sums within 1e-13; the histogram is numpy's of the y
     the kernel writes."""
     import torch
@@ -177,7 +184,8 @@ def test_monitor_stats_rotated_frame(engine):
     h, cols = _rows(rng.uniform(-3.2, 3.2, n), rng.uniform(-2.2, 2.2, n), seed=6, monitor=np.zeros(n))
     h["hit_px"] = rng.uniform(-0.5, 0.5, n)
     cols["hit_px"].copy_(torch.from_numpy(h["hit_px"]))
-    stats, per_row = _monitor_stats(engine, cols, 0, n, 0, hw, hh, frame=frame)
+    stats, per_row = _monitor_stats(engine, cols, 0, n, 1, hw, hh, frame=frame)
+    stats = stats[0]
     sel = np.ones(n, bool)
     ref = _numpy_stats(h, sel, frame=frame)
     assert stats[A.MS_COUNT] == n

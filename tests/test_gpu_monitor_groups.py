@@ -1,8 +1,8 @@
 """GPU: grouped monitor statistics (optb_monitor_stats_grouped, SweepResult.stats, analytics.monitor_stats).
 
 Every (configuration, monitor) group is checked against numpy of its own rows (counts, histograms and extrema exactly,
-sums to 1e-13 of math.fsum), against a separate DeviceMonitor per group on traced scenes, and for bit-identical results
-between calls and streams."""
+sums to 1e-13 of math.fsum), bit for bit against a separate DeviceMonitor per group on traced scenes, and for
+bit-identical results between calls and streams."""
 import ctypes as C
 import math
 from types import SimpleNamespace
@@ -220,33 +220,40 @@ def test_off_axis_spots_are_centred_per_group(engine, ratio):
 def test_bit_identical_between_calls_and_streams(engine, kind):
     import torch
 
+    from optable_b200.analytics import DeviceMonitor
+
     K, M, N, y, z, root, m, grp, hws = _case(kind, seed=3)
     cols = _to_device(_rows(y, z, root, m, seed=4))
     monitors = [_monitor(IDENTITY, hws[g]) for g in range(K * M)]
-    a, ra = _grouped(engine, cols, monitors, K, M, N)
-    b, rb = _grouped(engine, cols, monitors, K, M, N)
+
+    def call():
+        """The grouped call's stats and row values, and the stats of a DeviceMonitor of the last monitor as one array."""
+        stats, rows = _grouped(engine, cols, monitors, K, M, N)
+        d = DeviceMonitor(monitors[M - 1], cols, M - 1, engine=engine).stats()
+        return stats, rows, np.hstack(list(d.values())).astype(np.float64)
+
+    a, ra, da = call()
+    b, rb, db = call()
     side = torch.cuda.Stream()
     side.wait_stream(torch.cuda.current_stream())
     with torch.cuda.stream(side):
-        c, rc = _grouped(engine, cols, monitors, K, M, N)
-    for other, rows in ((b, rb), (c, rc)):
+        c, rc, dc = call()
+    assert da[0] > 0   # the DeviceMonitor's count
+    for other, rows, dm in ((b, rb, db), (c, rc, dc)):
         assert np.array_equal(a.view(np.int64), other.view(np.int64))
         assert np.array_equal(ra.view(np.int64), rows.view(np.int64))
+        assert np.array_equal(da.view(np.int64), dm.view(np.int64))
 
 
 # ---- traced scenes: the grouped call against one DeviceMonitor per (configuration, monitor) ---------------------------
 def _compare(s, rv, k, m, dm, mon, lo=0, hi=None):
-    """stats()[q][k, m] against DeviceMonitor dm's stats; the row values of monitor m among rows [lo, hi) (`mon`: the
-    hit_monitor column) bit for bit against dm's columns."""
+    """stats()[q][k, m] against DeviceMonitor dm's stats, and the row values of monitor m among rows [lo, hi) (`mon`: the
+    hit_monitor column) against dm's columns, all bit for bit: both reduce the same rows in the same tiles and order."""
     d = dm.stats()
-    assert s["count"][k, m] == d["count"], (k, m)
-    np.testing.assert_array_equal(s["hist_y"][k, m], d["hist_y"])
-    for q in ("min_y", "max_y", "min_z", "max_z"):
-        assert s[q][k, m] == d[q], (k, m, q)
-    for q in ("sum_intensity", "avg_intensity", "mean_y", "mean_z", "std_y", "std_z", "mean_waist_distance", "mean_tY"):
-        assert s[q][k, m] == pytest.approx(d[q], rel=1e-12, abs=1e-15), (k, m, q)
-    if d["count"]:
-        assert s["std_histy"][k, m] == pytest.approx(dm.std_histy, rel=1e-12, abs=1e-15, nan_ok=True), (k, m)
+    assert set(d) == set(s)
+    for q, v in d.items():
+        assert np.array_equal(s[q][k, m], v, equal_nan=True), (k, m, q)
+    assert np.array_equal(dm.std_histy, d["std_histy"], equal_nan=True), (k, m)
     sel = (mon[lo:hi] == m).nonzero().squeeze(1)
     for key, acc in (("y", dm.get_yList), ("z", dm.get_zList), ("tY", dm.get_tYList), ("tZ", dm.get_tZList),
                      ("waist_distance", dm.get_waist_distance)):

@@ -1,22 +1,28 @@
-"""CPU: the [K, M] summaries of SweepResult.stats / analytics.monitor_stats are DeviceMonitor.stats() and
-DeviceMonitor.std_histy of each group's slots, evaluated by DeviceMonitor's own code on the same slots."""
-from types import SimpleNamespace
-
+"""CPU: the summaries `stats_arrays` derives from stats slots, which `SweepResult.stats`, `analytics.monitor_stats` and
+`DeviceMonitor.stats` return, against the same formulas written for one group's slots with scalars."""
 import numpy as np
 import pytest
 
 from optable_b200 import _abi as A
-from optable_b200.analytics import DeviceMonitor, stats_arrays
+from optable_b200.analytics import stats_arrays
 
 
-class _Slots(DeviceMonitor):
-    """A DeviceMonitor whose fused pass already ran: only its stats slots and its monitor's width."""
-
-    def __init__(self, slots, width):
-        import torch
-
-        self._stats, self._stats_dev = None, torch.from_numpy(slots)
-        self.monitor = SimpleNamespace(width=width)
+def _reference(s, width):
+    """The summaries of one group's slots s [OPTB_MS_STRIDE] and monitor width, one scalar at a time."""
+    n = max(s[A.MS_COUNT], 1.0)
+    counts = s[A.MS_HIST:A.MS_HIST + A.HIST_BINS].astype(np.int64)
+    c, left = counts.astype(np.float64), np.linspace(-width / 2, width / 2, 31)[:-1]
+    with np.errstate(invalid="ignore", divide="ignore"):
+        mean = (c * left).sum() / c.sum()
+        std_histy = float(np.sqrt((c * left ** 2).sum() / c.sum() - mean ** 2))
+    return {
+        "count": int(s[A.MS_COUNT]), "sum_intensity": float(s[A.MS_SUM_I]), "avg_intensity": float(s[A.MS_SUM_I] / n),
+        "mean_y": float(s[A.MS_SUM_Y] / n), "mean_z": float(s[A.MS_SUM_Z] / n),
+        "std_y": float(np.sqrt(s[A.MS_M2_Y] / n)), "std_z": float(np.sqrt(s[A.MS_M2_Z] / n)),
+        "min_y": float(s[A.MS_MIN_Y]), "max_y": float(s[A.MS_MAX_Y]), "min_z": float(s[A.MS_MIN_Z]), "max_z": float(s[A.MS_MAX_Z]),
+        "mean_waist_distance": float(s[A.MS_SUM_WD] / n), "mean_tY": float(s[A.MS_SUM_TY] / n), "hist_y": counts,
+        "std_tY": float(np.sqrt(s[A.MS_M2_TY] / n)), "std_histy": std_histy,
+    }
 
 
 def _slots(rng, K, M):
@@ -41,7 +47,7 @@ def _slots(rng, K, M):
 
 
 @pytest.mark.parametrize("K,M", [(1, 3), (7, 2), (16, 5)])
-def test_stats_arrays_are_device_monitor_stats(K, M):
+def test_stats_arrays_against_scalar_formulas(K, M):
     rng = np.random.default_rng(K * 10 + M)
     s = _slots(rng, K, M)
     widths = rng.choice([5.0, 2.54, 1.0, 0.2, 12.7], (K, M))
@@ -49,12 +55,11 @@ def test_stats_arrays_are_device_monitor_stats(K, M):
     assert got["count"].shape == (K, M) and got["hist_y"].shape == (K, M, A.HIST_BINS)
     for k in range(K):
         for m in range(M):
-            dm = _Slots(np.ascontiguousarray(s[k, m]), widths[k, m])
-            want = dm.stats()
+            want = _reference(s[k, m], widths[k, m])
+            one = stats_arrays(s[k, m], widths[k, m])   # one group's slots, as DeviceMonitor.stats reads them
+            assert set(got) == set(one) == set(want)
             for q, v in want.items():
-                assert np.array_equal(got[q][k, m], v), (k, m, q)
-            assert got["std_tY"][k, m] == np.sqrt(s[k, m, A.MS_M2_TY] / max(s[k, m, A.MS_COUNT], 1.0))
+                assert np.array_equal(got[q][k, m], v, equal_nan=q == "std_histy"), (k, m, q)
+                assert np.array_equal(one[q], v, equal_nan=q == "std_histy"), (k, m, q)
             if s[k, m, A.MS_HIST:A.MS_HIST + A.HIST_BINS].sum() == 0:
                 assert np.isnan(got["std_histy"][k, m])
-            else:
-                assert got["std_histy"][k, m] == dm.std_histy, (k, m)
