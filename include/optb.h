@@ -353,8 +353,11 @@ int optb_scene_destroy(optb_ctx* ctx, optb_scene* scene);
  *   - K * N roots: root k * N + r is ray r in configuration k (seg_root, hit_root and hit_key carry that number, so
  *     optb_sort_rows gives configuration-major order); K * N must stay below 2^32 (-7 otherwise);
  *   - hist_y / hist_yz are [K][n_monitors][...]; root_flags would be [K * N]; counters are totals over all configurations;
- *   - rays.family must be NULL (every root is its own family); a scene with interact caps needs params.caps_slack
- *     (sweeps have no family-serial path; -7 otherwise); flag_ambiguity and reference_roots are rejected (-7);
+ *   - rays.family must be NULL (every root is its own family), except on a scene with interact caps and
+ *     params.caps_slack = 0: there rays.family (dense, < n_families) runs the family-serial sweep, with
+ *     params.n_families = F families per configuration and cap_counts [n_capslots][n_configs * n_families], in and
+ *     out, column k * F + f = family f in configuration k. A capped scene without a family column needs
+ *     params.caps_slack when it can split (-7 otherwise); flag_ambiguity and reference_roots are rejected (-7);
  *   - optb_workspace_bytes(scene, N, max_live) sizes for K * N roots (max_live counts over all configurations);
  *   - optb_scene_update_nodes is rejected (-7): upload the configurations again.
  * Every desc must have the same n_nodes, n_leaves, n_materials, n_monitors, n_capslots and n_aux, identical node_i rows

@@ -102,6 +102,13 @@ def runs_wavefront(flats, params: A.Params) -> bool:
                 or any(f.max_children > 1 or f.n_capslots > 0 or f.has_pass for f in flats))
 
 
+def caps_can_bind(count_max, fam_size, cap_min, max_trace_num) -> bool:
+    """Whether an interact cap can bind in a trace: a family's count grows by at most one per pop of each of its initial
+    rays, so a cap binds only if the largest initial count plus max_trace_num pops of the largest family can exceed the
+    smallest cap. Traces where it can run family-serially (params.caps_slack = 0)."""
+    return not int(count_max) + int(max_trace_num) * int(fam_size) <= cap_min
+
+
 class Scene:
     """Device-resident scene tables (optb_scene handle). With `configs` it is a sweep scene, and every trace runs its
     bundle through all `n_configs` configurations: `configs` is a list of FlatScene of one topology
@@ -326,10 +333,9 @@ class Engine:
         caps0, slack = None, 0
         if flat.n_capslots:
             caps0 = np.zeros((flat.n_capslots, n_families), np.int32) if cap_counts is None else np.array(cap_counts, np.int32)
-            # can any cap bind at all? a family's count grows by at most one per pop of each of its initial rays
             fam_size = np.bincount(arrs["family"], minlength=n_families).max() if n else 0
             capmax = flat.node_f[flat.node_i[:, A.NI_CAPSLOT] >= 0, A.NF_CAPMAX].min()
-            slack = int(caps0.max() + int(max_trace_num) * int(fam_size) <= capmax)
+            slack = int(not caps_can_bind(caps0.max(), fam_size, capmax, max_trace_num))
         prm = self.make_params(max_trace_num, unit, record_segments, record_hits, record_hist, chain_len, n_families, slack,
                                flag_ambiguity, reference_roots)
         return prm, caps0
@@ -342,8 +348,10 @@ class Engine:
         rs = A.Rays()
         rs.n = len(arrs["ox"])
         family = np.ascontiguousarray(arrs["family"], dtype=np.int32)
-        if not scene.sweep:                   # (a sweep's roots are their own families: no family column)
-            rs.family = family.ctypes.data    # (trace_arrays always passes the family column; the plan only tests it is set)
+        # (trace_arrays always passes the family column; the plan only tests it is set). A sweep's roots are their own
+        # families unless its caps can bind: that sweep runs family-serially, with the family column.
+        if not scene.sweep or (scene.flat.n_capslots and not prm.caps_slack):
+            rs.family = family.ctypes.data
         out = (C.c_int64 * 5)()
         self._check(lib().optb_trace_plan(self._ctx, scene._h, C.byref(rs), C.byref(prm), out))
         return dict(zip(("bits", "blob", "dynamic", "static", "optin"), (int(v) for v in out)))

@@ -111,33 +111,44 @@ class DeviceTrace:
     """Reusable device-side state for repeated traces of same-shaped bundles through one scene: scene tables,
     result buffers and workspace are allocated once; `run` only enqueues kernels. With `configs` (the FlatScenes of a
     sweep, `flat` = configs[0], or a SweepRows, `flat` = its base) the scene is a sweep scene and one run traces the
-    bundle through every configuration."""
+    bundle through every configuration.
+
+    `cap_counts` (a sweep of Ray objects whose interact caps can bind: [n_capslots, n_configs * n_families], column
+    k * n_families + f = family f in configuration k) runs the family-serial sweep: every run starts from these counts,
+    and the rays must carry a `family` column (< n_families)."""
 
     def __init__(self, engine, flat, n_rays, hit_capacity, seg_capacity=0, hit_columns=HIT_COLUMNS_ALL,
-                 max_trace_num=2000, unit=1e-2, record_hist=False, chain_len=0, flag_ambiguity=False, configs=None):
+                 max_trace_num=2000, unit=1e-2, record_hist=False, chain_len=0, flag_ambiguity=False, configs=None,
+                 cap_counts=None, n_families=None):
         import torch
 
         self.engine, self.flat, self.torch = engine, flat, torch
         self.scene = engine.upload(flat) if configs is None else engine.upload_sweep(configs)
         n_roots = n_rays * self.scene.n_configs
-        self.res, self.t = engine.alloc_result(self.scene, seg_capacity, hit_capacity, n_roots,
+        serial = cap_counts is not None and flat.n_capslots > 0
+        self.res, self.t = engine.alloc_result(self.scene, seg_capacity, hit_capacity,
+                                               self.scene.n_configs * n_families if serial else n_roots,
                                                hit_columns=tuple(hit_columns) + (() if "hit_key" in hit_columns else ("hit_monitor",)))
+        self._caps0 = torch.from_numpy(np.ascontiguousarray(cap_counts, dtype=np.int32)).to(self.t["cap_counts"].device) if serial else None
         if flag_ambiguity:
             self.t["root_flags"] = torch.zeros(max(int(n_rays), 1), dtype=torch.int32, device=f"cuda:{engine.device}")
             self.res.root_flags = self.t["root_flags"].data_ptr()
         slack = 0
-        if flat.n_capslots:
+        if flat.n_capslots and not serial:
             # a bundle ray is its own `_id` family starting from zero counts: a cap can only bind if it is
-            # smaller than the pop budget. Binding caps need Ray objects (OpticalTable.ray_tracing).
+            # smaller than the pop budget. Binding caps need Ray objects (OpticalTable.ray_tracing, trace_sweep).
             if min(f.cap_min for f in self.scene.configs) < max_trace_num:
-                raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped component")
+                raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped "
+                                          "component (a sweep of Ray objects with ids lifts this)")
             slack = 1
         self.prm = engine.make_params(max_trace_num, unit, seg_capacity > 0, hit_capacity > 0, record_hist, chain_len,
-                                      n_roots, slack, flag_ambiguity)
+                                      n_families if serial else n_roots, slack, flag_ambiguity)
         self.hit_columns = tuple(k for k in HIT_COLUMNS_ALL + ("hit_key",) if k in self.t)
 
     def run(self, rays_t, max_live=None):
-        if self.flat.n_capslots:
+        if self._caps0 is not None:
+            self.t["cap_counts"].copy_(self._caps0)   # every attempt starts from the initial counts
+        elif self.flat.n_capslots:
             self.t["cap_counts"].zero_()  # a bundle is a fresh set of ray ids every time
         self.engine.trace_device(self.scene, rays_t, self.prm, self.res, max_live)
 

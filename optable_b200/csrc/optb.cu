@@ -122,7 +122,8 @@ OPTB_DEV unsigned long long warp_alloc(unsigned long long* ctr) {
   return base + __popc(m & ((1u << lane) - 1u));
 }
 
-template <bool SWEEP = false>
+// SERIAL (with SWEEP): the family-serial sweep numbers the families itself, so the family column is not read here
+template <bool SWEEP = false, bool SERIAL = false>
 OPTB_DEV void load_ray(const TraceArgs& a, long long i, Ray& r, bool& solo, uint32_t& gcount, uint32_t& pop_base) {
   if (a.gen0) {
     const optb_rays& s = a.in0;
@@ -139,7 +140,7 @@ OPTB_DEV void load_ray(const TraceArgs& a, long long i, Ray& r, bool& solo, uint
 #undef OPTB_COL
     r.flags = s.flags ? s.flags[in] : (OPTB_RF_ALIVE | OPTB_RF_HASQ);
     r.root = (uint32_t)i + a.root_base; r.pop = 0;
-    r.family = s.family ? s.family[i] : (int32_t)r.root;
+    if constexpr (!(SWEEP && SERIAL)) r.family = s.family ? s.family[i] : (int32_t)r.root;
     solo = true; gcount = 1; pop_base = 0;
   } else {
     // Children stay where the previous generation's kernel wrote them (slot 2*parent + k of the sparse buffer);
@@ -525,7 +526,8 @@ OPTB_DEV void closest_hit(const TraceArgs& a, const SceneView& sv, const Ray& ra
 // of the closed-form / Newton root.
 // PASSK = the scene has an OPTB_I_PASS leaf (a Monitor listed as a component): only the general variants carry that body.
 // SWEEP = a sweep scene (optb_scene_upload_sweep): every lane reads the tables of its root's configuration from global
-// memory (a warp may straddle configurations); the kernels of ordinary scenes do not carry it.
+// memory (a warp may straddle configurations); the kernels of ordinary scenes do not carry it. With SERIAL, work item
+// i is family i % F of configuration i / F (F = families per configuration), and all its roots read that configuration.
 template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = false, bool BRENT = false, bool PASSK = false,
           bool SWEEP = false>
 // Resident CTAs per SM: scenes staged in shared memory are bound by dependent fp64 chains and lose more to the
@@ -534,7 +536,7 @@ template <bool SMEM, bool SERIAL, int BOXES, bool ASPH, bool SPLIT, bool FLAG = 
 __global__ void __launch_bounds__(kBlock, (SMEM || ASPH || SERIAL) ? 4 : 5)
 trace_kernel(const __grid_constant__ TraceArgs a) {
   constexpr int MAXCH = (SPLIT || SERIAL) ? 2 : 1;
-  static_assert(!SWEEP || (!SMEM && !SERIAL && !FLAG && !BRENT), "sweeps run the parallel path from global memory");
+  static_assert(!SWEEP || (!SMEM && !FLAG && !BRENT), "sweeps run from global memory, without the diagnostics modes");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   __shared__ __align__(8) unsigned long long mbar;
   // The closest-hit search only needs a ray's geometry. Its radiometric state (intensity, wavelength, q, path
@@ -622,11 +624,12 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
         while (y > lo && a.fam_roots[y - 1] > v) { a.fam_roots[y] = a.fam_roots[y - 1]; y--; }
         a.fam_roots[y] = v;
       }
+      if constexpr (SWEEP) { if (lo < hi) sweep_view(a, a.fam_roots[lo], sv); }
       const long long ring = (long long)i * a.qcap;
       for (uint32_t x = lo; x < hi; x++) {
         Ray ray; bool solo; uint32_t gcount, pop_base0;
         const uint32_t root = a.fam_roots[x];
-        load_ray(a, root, ray, solo, gcount, pop_base0);
+        load_ray<SWEEP, true>(a, root, ray, solo, gcount, pop_base0);
         uint32_t head = 0, tail = 0, pops = 0;
         ring_put(a.w, ring, ray); tail = 1;
         while ((long long)pops < a.max_trace && head != tail) {
@@ -638,8 +641,8 @@ trace_kernel(const __grid_constant__ TraceArgs a) {
           const bool hit = node >= 0;
           const int32_t* ni = sv.ni + (hit ? node : 0) * OPTB_NI_STRIDE;
           const double* nf = sv.nf + (hit ? node : 0) * OPTB_NF_STRIDE;
-          emit_segment(a, sv, ray, hit ? t : ray.len, hit ? (ray.flags & ~OPTB_RF_ALIVE) : ray.flags,
-                       hit ? ni[OPTB_NI_LEAF] : -1, s_hist, c_hits);
+          emit_segment<SWEEP>(a, sv, ray, hit ? t : ray.len, hit ? (ray.flags & ~OPTB_RF_ALIVE) : ray.flags,
+                              hit ? ni[OPTB_NI_LEAF] : -1, s_hist, c_hits);
           if (!hit) continue;
           c_inter++;
           double ox, oy, oz, dx, dy, dz;
@@ -923,6 +926,21 @@ __global__ void fam_scatter_kernel(const int32_t* __restrict__ family, long long
                                    unsigned int* __restrict__ cursor, uint32_t* __restrict__ roots) {
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
     int f = family ? family[i] : (int32_t)i;
+    roots[off[f] + atomicAdd(&cursor[f], 1u)] = (uint32_t)i;
+  }
+}
+// The same for a sweep of n rays per configuration and n_fam families per configuration: root k * n + r belongs to
+// family k * n_fam + family[r]
+__global__ void fam_count_sweep_kernel(const int32_t* __restrict__ family, long long n_roots, uint32_t n, int n_fam,
+                                       unsigned int* __restrict__ counts) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_roots; i += (long long)gridDim.x * blockDim.x)
+    atomicAdd(&counts[(i / n) * n_fam + family[i % n]], 1u);
+}
+__global__ void fam_scatter_sweep_kernel(const int32_t* __restrict__ family, long long n_roots, uint32_t n, int n_fam,
+                                         const unsigned int* __restrict__ off, unsigned int* __restrict__ cursor,
+                                         uint32_t* __restrict__ roots) {
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n_roots; i += (long long)gridDim.x * blockDim.x) {
+    const long long f = (i / n) * n_fam + family[i % n];
     roots[off[f] + atomicAdd(&cursor[f], 1u)] = (uint32_t)i;
   }
 }
@@ -1722,6 +1740,7 @@ KernPick select_kernel(const optb_scene* scene, const optb_params* prm, bool ser
   // box mode: 0 none, 1 pre-order walk with culling, 2 walk + lattice windows (scenes with OPTB_G_GRID groups)
   const int boxmode = !scene->has_boxes ? 0 : (scene->has_grid ? 2 : 1);
   const bool smem = scene->in_smem, asph = scene->has_asph;
+  if (scene->n_cfg && serial) return pick<false, true, 1, true, true, false, false, false, true>();
   if (scene->n_cfg)
     return scene->has_pass ? pick<false, false, 1, true, true, false, false, true, true>()
                            : parallel_kernel<false, true>(boxmode, asph, split);
@@ -1739,7 +1758,8 @@ struct LaunchPlan { KernPick k; uint32_t smem; int occ; };
 }  // namespace
 
 // Largest static shared memory over the trace kernels that stage the blob in shared memory (every kind a scene that
-// scene_alloc puts in shared memory can be traced with): the part of the opt-in window that is not the blob's.
+// scene_alloc puts in shared memory can be traced with) and the family-serial sweep kind: the part of the opt-in window
+// that is not the blob's or the histograms'.
 static cudaError_t smem_static_max(size_t* out) {
   std::vector<Kern> ks;
   for (int b = 0; b < 3; b++)
@@ -1750,6 +1770,7 @@ static cudaError_t smem_static_max(size_t* out) {
   ks.push_back(general_kernel<false, true, false, false>(true).kern);
   ks.push_back(general_kernel<true, false, false, false>(true).kern);
   ks.push_back(general_kernel<false, false, false, true>(true).kern);
+  ks.push_back(pick<false, true, 1, true, true, false, false, false, true>().kern);
   size_t m = 0;
   for (Kern k : ks) {
     cudaFuncAttributes fa;
@@ -1783,11 +1804,16 @@ static int check_trace_args(optb_ctx* ctx, const optb_scene* scene, const optb_r
   const long long n_roots = scene->n_cfg ? rays->n * scene->n_cfg : rays->n;
   if (scene->n_cfg) {
     if (n_roots >= 0xffffffffll) return fail(ctx, -7, "sweep: n_configs * rays.n must stay below 2^32");
-    if (needs_serial(scene, rays, prm))
-      return fail(ctx, -7, "sweep: the scene has interact caps; set params.caps_slack (sweeps have no family-serial path)");
+    // the family-serial sweep: a family column on a scene whose caps may bind
+    const bool serial_sweep = rays->family && scene->n_caps > 0 && !prm->caps_slack;
+    if (needs_serial(scene, rays, prm) && !serial_sweep)
+      return fail(ctx, -7, "sweep: the scene has interact caps; set params.caps_slack, or give rays.family for the "
+                           "family-serial sweep");
     if (prm->flag_ambiguity || prm->reference_roots)
       return fail(ctx, -7, "sweep: flag_ambiguity and reference_roots are not available on sweep scenes");
-    if (rays->family) return fail(ctx, -7, "sweep: rays.family must be NULL (every root is its own family)");
+    if (rays->family && !serial_sweep) return fail(ctx, -7, "sweep: rays.family must be NULL (every root is its own family)");
+    if (serial_sweep && (long long)prm->n_families * scene->n_cfg >= 0x7fffffffll)
+      return fail(ctx, -7, "sweep: n_configs * n_families must stay below 2^31");
   }
   // cap_counts is [n_capslots][n_families]; without a family column every initial ray is its own family (column
   // index = ray index), so the table must have a column per ray
@@ -1858,19 +1884,20 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   SerialLayout SL{};
   long long n_fam = 0, qcap = 0;
   if (serial) {
-    n_fam = rays->family ? prm->n_families : rays->n;
+    // a sweep has n_families families in each configuration: global family k * n_families + f
+    n_fam = rays->family ? (long long)prm->n_families * std::max(scene->n_cfg, 1) : rays->n;
     if (n_fam < 1) return fail(ctx, -7, "n_families must be >= 1");
     const long long want = std::min<long long>(prm->max_trace_num + 2, 1ll << 20);
-    const size_t fixed = serial_layout(rays->n, n_fam, 1).total;
+    const size_t fixed = serial_layout(n_roots, n_fam, 1).total;
     if ((size_t)workspace_bytes <= fixed) return fail(ctx, -8, "workspace too small (see optb_workspace_bytes)");
     long long lo = 1, hi = std::max<long long>(want, 2) * n_fam;
     while (lo < hi) {
       long long mid = lo + (hi - lo + 1) / 2;
-      if ((int64_t)serial_layout(rays->n, n_fam, mid).total <= workspace_bytes) lo = mid; else hi = mid - 1;
+      if ((int64_t)serial_layout(n_roots, n_fam, mid).total <= workspace_bytes) lo = mid; else hi = mid - 1;
     }
     qcap = std::min<long long>(lo / n_fam, want);
     if (qcap < 4) return fail(ctx, -8, "workspace too small for the per-family FIFO (see optb_workspace_bytes)");
-    SL = serial_layout(rays->n, n_fam, qcap * n_fam);
+    SL = serial_layout(n_roots, n_fam, qcap * n_fam);
     L.hdr = SL.hdr;
   } else if (split) {
     // find the largest wavefront capacity the given workspace supports
@@ -1938,10 +1965,14 @@ static int trace_impl(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
     CK(cudaMemsetAsync(off, 0, (size_t)(n_fam + 2) * 4, st), "memset family offsets");
     CK(cudaMemsetAsync(cursor, 0, (size_t)(n_fam + 1) * 4, st), "memset family cursors");
     const int g = (int)std::min<long long>(full_grid * 4, (n_in + 255) / 256);
-    fam_count_kernel<<<g, 256, 0, st>>>(rays->family, n_in, off);
+    const uint32_t n_cfg_rays = (uint32_t)rays->n;
+    if (scene->n_cfg) fam_count_sweep_kernel<<<g, 256, 0, st>>>(rays->family, n_in, n_cfg_rays, prm->n_families, off);
+    else fam_count_kernel<<<g, 256, 0, st>>>(rays->family, n_in, off);
     scan_sums_kernel<<<1, 1024, 0, st>>>(off, (int)(n_fam + 1), hdr, a.counters, 0xffffffffu);  // exclusive, in place
-    fam_scatter_kernel<<<g, 256, 0, st>>>(rays->family, n_in, off, cursor, roots);
+    if (scene->n_cfg) fam_scatter_sweep_kernel<<<g, 256, 0, st>>>(rays->family, n_in, n_cfg_rays, prm->n_families, off, cursor, roots);
+    else fam_scatter_kernel<<<g, 256, 0, st>>>(rays->family, n_in, off, cursor, roots);
     a.fam_off = off; a.fam_roots = roots; a.qcap = (uint32_t)qcap;
+    if (scene->n_cfg) a.n_families = (int)n_fam;  // cap_counts [n_capslots][n_configs * n_families]
     a.w = make_raybuf(ws + SL.ring, qcap * n_fam);
     a.fam_shared = 0;
     a.n_in = n_fam;
@@ -2059,7 +2090,8 @@ static int trace_host(optb_ctx* ctx, const optb_scene* scene, const optb_rays* r
   const int64_t sortb = sorted ? optb_sort_workspace_bytes(std::max(cseg, chit)) : 0;
   const bool hist = prm->record_hist && scene->n_mons;
   const size_t hy = (size_t)hist_mons(scene) * OPTB_HIST_BINS * 8, hyz = hy * OPTB_HIST_BINS;
-  const size_t capb = (size_t)scene->n_caps * std::max(prm->n_families, 1) * 4;
+  // the family-serial sweep: [n_capslots][n_configs * n_families]
+  const size_t capb = (size_t)scene->n_caps * std::max(prm->n_families, 1) * (rays->family ? std::max(scene->n_cfg, 1) : 1) * 4;
   if (!ctx->s_h2d) {
     CK(cudaStreamCreateWithFlags(&ctx->s_h2d, cudaStreamNonBlocking), "stream");
     CK(cudaStreamCreateWithFlags(&ctx->s_run, cudaStreamNonBlocking), "stream");

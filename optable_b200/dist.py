@@ -168,23 +168,27 @@ def _gather_configs(t, counts, group=None):
 
 
 def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label, tracer, group=None, gather=False,
-                        record_hits=True, record_hist=False, engine=None, unit=None, arrs=None):
+                        record_hits=True, record_hist=False, engine=None, unit=None, arrs=None, fam_ids=None):
     """Multi-GPU form of a sweep (`trace_sweep` / `SweepScene.trace` with `group=`): the K configurations are sharded
     over the ranks of `group`, rank r owning the contiguous configurations [k0, k1) = shard_bounds(K, r, world) (equal
     counts, no balancing by cost; K < world leaves ranks without configurations, which still take part in every
     collective). Every group (k, m) of the monitor statistics is reduced on its own rows in a fixed order, so a
     configuration that stays on one rank gets the bits of the one-GPU sweep: rows, histograms and statistics.
 
-    `prepare(k0, k1)` runs this rank's host side and returns (configs, shares): the FlatScenes or SweepRows of its
-    configurations (None when k0 == k1) and a list with one picklable item per configuration that every rank receives
-    (SweepScene: the frames of the varied monitors). `monitors`: the [K][M] monitor frames, or a function of the
+    `prepare(k0, k1)` runs this rank's host side and returns (configs, shares, caps0): the FlatScenes or SweepRows of
+    its configurations (None when k0 == k1), a list with one picklable item per configuration that every rank receives
+    (SweepScene: the frames of the varied monitors, else None) and the starting interact counts of its configurations
+    (`sweep.initial_counts` of the families `fam_ids` of a list of Ray, or None). `monitors`: the [K][M] monitor frames, or a function of the
     gathered shares (configuration order) that returns them. A rank without configurations does not call `prepare`.
 
     Before any trace, one exchange checks on every rank (so that no rank waits in a collective while another raised):
     what `prepare` raised on any rank, the topology of the ranks' configurations (`sweep.topology_key`; ValueError
     naming the first differing global configuration), interact caps, and the largest `max_children`. A rank whose
     own configurations do not split while others do runs the wavefront kernels with chain_len = limit + 1, which
-    selects the variant the one-GPU sweep runs and never cuts a chain (a root pops at most `limit` times). The global
+    selects the variant the one-GPU sweep runs and never cuts a chain (a root pops at most `limit` times). For a list
+    of Ray on a capped scene, every rank also sends its largest starting count and its smallest cap, so that all ranks
+    decide as the one-GPU sweep does, over all K configurations, whether to trace family-serially (`sweep.caps_bind`;
+    chain_len is then 0); the [K, S, F] `interact_counts` are all-gathered. The global
     K * N < 2^32 bound is checked up front, since row keys are global.
 
     After the trace: statistics of the rank's own rows (`optb_monitor_stats_grouped`, configurations numbered from
@@ -198,7 +202,8 @@ def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label
 
     from . import _abi as A
     from .analytics import grouped_slots
-    from .sweep import SweepRows, topology_key, topology_mismatch
+    from .backend import caps_can_bind
+    from .sweep import SweepRows, largest_family, topology_key, topology_mismatch
 
     K, n = int(n_configs), int(n_rays)
     who, what = label.split(": ")
@@ -212,11 +217,12 @@ def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label
     mismatch = lambda k, why: f"{label} {k} does not have the topology of {what} 0 ({why})"
 
     # ---- this rank's host side, and one exchange of what every rank must know before any trace
-    mine = {"error": None, "key": None, "max_children": 0, "shares": []}
-    configs, err = None, None
+    mine = {"error": None, "key": None, "max_children": 0, "shares": [], "caps": (0, float("inf"), 0)}
+    configs, err, caps0 = None, None, None
     try:
         if k1 > k0:
-            configs, mine["shares"] = prepare(k0, k1)
+            configs, shares, caps0 = prepare(k0, k1)
+            mine["shares"] = shares or []
         if configs is not None:
             rows = configs if isinstance(configs, SweepRows) else None
             flats = [rows] if rows is not None else configs
@@ -225,9 +231,12 @@ def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label
             bad = topology_mismatch(configs) if rows is None else None
             if bad is not None:
                 raise ValueError(mismatch(k0 + bad[0], bad[1]))
-            if flat0.n_capslots and min(f.cap_min for f in flats) < limit:
-                raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped component")
+            cap_min = min(f.cap_min for f in flats)
+            if flat0.n_capslots and arrs is None and cap_min < limit:
+                raise NotImplementedError("bundle traces need max_interact_count >= max_trace_num on every capped "
+                                          "component (a sweep of Ray objects with ids lifts this)")
             mine["max_children"] = max(f.max_children for f in flats)
+            mine["caps"] = (int(caps0.max(initial=0)) if caps0 is not None else 0, cap_min, flat0.n_capslots)
     except Exception as e:   # raised on every rank below
         err, mine["error"] = e, (k0, type(e).__name__, str(e))
     states = [None] * world
@@ -250,14 +259,18 @@ def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label
     M = len(monitors[0])
     Mh = max(M, 1)       # the device keeps one histogram row per monitor, at least one per configuration
     wide = max(s["max_children"] for s in states)
-    chain_len = int(limit) + 1 if configs is not None and wide > 1 >= mine["max_children"] else 0
+    n_caps = max(s["caps"][2] for s in states)
+    counted = fam_ids is not None and n_caps > 0     # a list of Ray on a capped scene: interact_counts are returned
+    serial = counted and caps_can_bind(max(s["caps"][0] for s in states), largest_family(arrs),
+                                       min(s["caps"][1] for s in states), limit)
+    chain_len = int(limit) + 1 if configs is not None and wide > 1 >= mine["max_children"] and not serial else 0
 
     # ---- this rank's trace
     dev = _collective_device(group)
     cols = A.HIT_I32 + A.HIT_U32 + A.HIT_F64
     if configs is not None:
         res = tracer(configs, rays, limit, record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
-                     arrs=arrs, chain_len=chain_len)
+                     arrs=arrs, chain_len=chain_len, **({"caps0": caps0, "serial": serial} if counted else {}))
         counters = np.asarray(res["counters"])
     else:
         dt = {k: torch.int32 for k in A.HIT_I32 + A.HIT_U32}
@@ -290,6 +303,10 @@ def trace_sweep_sharded(n_configs, n_rays, rays, limit, prepare, monitors, label
         out["hist_y"] = torch.zeros((K,) + tuple(hy.shape[1:]), dtype=hy.dtype, device=hy.device)
         out["hist_yz"] = torch.zeros((K,) + tuple(hyz.shape[1:]), dtype=hyz.dtype, device=hyz.device)
     out["counters"] = merge_counters(counters, group)
+    if counted:
+        mine_counts = (torch.from_numpy(np.asarray(res["interact_counts"])) if configs is not None
+                       else torch.zeros((0, n_caps, len(fam_ids)), dtype=torch.int32))
+        out["interact_counts"] = _gather_configs(mine_counts, counts, group).numpy()
     if gather and record_hits:
         where = rows["hit_px"].device
         rows = {k: v.to(where) for k, v in gather_rows({k: v.to(dev) for k, v in rows.items()}, n_rows, 0, group).items()}

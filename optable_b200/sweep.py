@@ -74,21 +74,63 @@ def topology_key(flat) -> bytes:
 
 
 def _rays(rays):
-    """(n, wavelength column, unit, packed host arrays or None) of a RayBundle or a list of Ray."""
+    """(n, wavelength column, unit, packed host arrays or None, family ids or None) of a RayBundle or a list of Ray."""
     from .bundle import RayBundle
     from .flatten import pack_rays
 
     if isinstance(rays, RayBundle):
-        return rays.n, rays.columns.get("wavelength"), None, None
-    arrs, _, unit = pack_rays(list(rays))
-    return len(arrs["ox"]), arrs["wavelength"], unit, arrs
+        return rays.n, rays.columns.get("wavelength"), None, None, None
+    arrs, fam_ids, unit = pack_rays(list(rays))
+    return len(arrs["ox"]), arrs["wavelength"], unit, arrs, fam_ids
+
+
+def initial_counts(cap_components, fam_ids):
+    """The starting interact counts of a sweep of Ray objects, [n_capslots, K * F] int32: column k * F + f holds
+    `cap_components[k][s]._interact_count` of ray id fam_ids[f] (F = len(fam_ids)). None for a bundle (fam_ids None)
+    or a scene without caps."""
+    if fam_ids is None or not cap_components or not len(cap_components[0]):
+        return None
+    F = len(fam_ids)
+    out = np.zeros((len(cap_components[0]), len(cap_components) * F), np.int32)
+    for k, comps in enumerate(cap_components):
+        for s, c in enumerate(comps):
+            out[s, k * F:(k + 1) * F] = [c._interact_count.get(rid, 0) for rid in fam_ids]
+    return out
+
+
+def largest_family(arrs) -> int:
+    """Initial rays of the largest `_id` family of a packed batch (0 when empty)."""
+    return int(np.bincount(arrs["family"]).max()) if len(arrs["family"]) else 0
+
+
+def caps_bind(caps0, arrs, cap_min, limit) -> bool:
+    """Whether a sweep of the packed Ray batch `arrs` from the initial counts `caps0` needs the family-serial path:
+    the rule of `Engine._arrays_params` over all its configurations (`cap_min`: their smallest cap)."""
+    from .backend import caps_can_bind
+
+    return caps_can_bind(caps0.max(initial=0), largest_family(arrs), cap_min, limit)
+
+
+def _family_counts(table, caps0, family, K, n, serial):
+    """`SweepResult.interact_counts` [K, S, F] from the device's cap table: the family-serial table itself
+    ([S, K * F]), or, where no cap can bind (every root its own family, counted from zero: [S, >= K * n]), the initial
+    counts plus the counts of each family's roots."""
+    S, F = caps0.shape[0], caps0.shape[1] // K
+    if serial:
+        c = np.asarray(table[:, :K * F]).reshape(S, K, F)
+    else:
+        c = caps0.reshape(S, K, F).astype(np.int64)
+        np.add.at(c, (slice(None), slice(None), np.asarray(family)), np.asarray(table[:, :K * n]).reshape(S, K, n))
+    return np.ascontiguousarray(c.transpose(1, 0, 2), dtype=np.int32)
 
 
 def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, engine=None, unit=None, arrs=None,
-                  chain_len=0):
+                  chain_len=0, caps0=None, serial=False):
     """The CUDA sweep: one sweep scene, one optb_trace over K x N roots, hit rows sorted into key order on the device.
     `configs`: the FlatScenes of the K configurations, or a SweepRows. `chain_len` > 0 runs the wavefront kernels
-    (a shard of a sharded sweep whose own configurations do not split, when others do)."""
+    (a shard of a sharded sweep whose own configurations do not split, when others do). `caps0` (Ray objects on a
+    capped scene: `initial_counts`) adds `interact_counts` [K, S, F] to the result; with `serial` (`caps_bind`) the
+    sweep runs family-serially from these counts."""
     from .backend import Engine
     from .bundle import DeviceTrace, run_to_fit
 
@@ -103,16 +145,21 @@ def _device_sweep(configs, rays, limit, record_hits=True, record_hist=False, eng
     else:
         n = len(arrs["ox"])
         rays_t = engine.rays_to_device(arrs)
-        del rays_t["family"]   # every root is its own family (rays.family must be NULL on a sweep scene)
+        if not serial:
+            del rays_t["family"]   # every root is its own family (rays.family must be NULL on a parallel sweep)
     n_roots = K * n
     cap = n_roots * max(M, 1) * 2 if record_hits else 0
+    serial_kw = {"cap_counts": caps0, "n_families": caps0.shape[1] // K} if serial else {}
     dt, cnt = run_to_fit(lambda c: DeviceTrace(engine, flat0, n, c, max_trace_num=limit, record_hist=record_hist,
-                                               chain_len=chain_len, configs=configs, **({} if unit is None else {"unit": unit})),
+                                               chain_len=chain_len, configs=configs, **serial_kw,
+                                               **({} if unit is None else {"unit": unit})),
                          rays_t, n_roots, limit, cap)
     nh = int(cnt[A.C_HITS]) if record_hits else 0
     engine._sort_rows_on_device(dt.res, 0, nh, limit, M)
     out = {k: dt.t[k][:nh] for k in dt.hit_columns} if record_hits else {}
     out["hist_y"], out["hist_yz"], out["counters"] = dt.t["hist_y"], dt.t["hist_yz"], cnt
+    if caps0 is not None:
+        out["interact_counts"] = _family_counts(dt.t["cap_counts"].cpu().numpy(), caps0, arrs["family"], K, n, serial)
     dt.scene.close()
     return out
 
@@ -128,9 +175,15 @@ class SweepResult:
     counters; `counters`, the histograms, `monitors` and `stats()` cover all K configurations on every rank. `hits`
     holds this rank's rows with global roots, or every rank's rows with `gather=True`; `rows(k)` and `monitor(k, m)`
     of a configuration whose rows this rank does not hold raise IndexError. `chain_len` > 0 when this rank ran the
-    wavefront kernels with that chain length to match the kernel variant of the one-GPU sweep (0 otherwise)."""
+    wavefront kernels with that chain length to match the kernel variant of the one-GPU sweep (0 otherwise).
 
-    def __init__(self, tables, n, out, engine=None, monitors=None):
+    Of a sweep of Ray objects: `family_ids`, the ray id of each interact-cap family (`pack_rays` order);
+    `cap_components` [K][S], the capped components of each configuration (FlatScene cap-slot order); and
+    `interact_counts`, int32 [K, S, F]: interact_counts[k, s, f] is what cap_components[k][s]._interact_count[
+    family_ids[f]] would hold after tables[k].ray_tracing(rays). A sweep does not write these counts back. A RayBundle
+    sweep has none of the three (None)."""
+
+    def __init__(self, tables, n, out, engine=None, monitors=None, family_ids=None, cap_components=None):
         import torch
 
         self.tables, self.n, self.n_configs, self.engine = list(tables), int(n), len(tables), engine
@@ -142,6 +195,11 @@ class SweepResult:
         self.hits = {k: v for k, v in out.items() if k.startswith("hit_")}
         self.shard, self.counters_local, self.chain_len = out.get("shard"), out.get("counters_local"), out.get("chain_len", 0)
         self._world = out.get("world", 1)
+        self.family_ids = None if family_ids is None else list(family_ids)
+        self.interact_counts = out.get("interact_counts")
+        if self.interact_counts is None and family_ids is not None:    # a scene without caps
+            self.interact_counts = np.zeros((K, 0, len(family_ids)), np.int32)
+        self._cap_components = cap_components
         self._holds = out.get("holds", (0, K))      # the configurations whose rows `hits` holds
         root = self.hits.get("hit_root")
         if root is not None:   # rows are sorted by root: configuration k owns the roots [k N, (k + 1) N)
@@ -157,6 +215,12 @@ class SweepResult:
             from .analytics import monitor_widths, stats_arrays
 
             self._stats = stats_arrays(out["stats_slots"], monitor_widths(self.monitors))
+
+    @property
+    def cap_components(self):
+        if callable(self._cap_components):
+            self._cap_components = self._cap_components()
+        return self._cap_components
 
     def _grouped_stats(self):
         from .analytics import grouped_stats
@@ -230,9 +294,13 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
     flattened with the bundle's wavelength set; tables whose topology differs from tables[0] (node count, component
     kinds, material kinds, ...) raise ValueError naming the first such table and what differs. Poses, apertures,
     reflectivities, glass coefficients and monitor placement may differ.
-    `rays`: a RayBundle or a list of Ray (packed with pack_rays; every ray is its own interact-cap family).
-    Interact caps follow `trace_bundle`: every capped component needs max_interact_count >= max_trace_num in every
-    configuration, else NotImplementedError.
+    `rays`: a RayBundle or a list of Ray (packed with pack_rays).
+    Interact caps: a list of Ray is traced as `tables[k].ray_tracing(rays)` would trace it, with the rays' `_id`
+    families and the components' current `_interact_count` as starting counts. Where a cap can bind (the rule of
+    `Engine.trace_arrays`, over all configurations), every family runs serially in the reference's order (the
+    family-serial sweep kernel); the final counts are `SweepResult.interact_counts`. A RayBundle follows
+    `trace_bundle`: every ray is its own family counted from zero, and every capped component needs
+    max_interact_count >= max_trace_num in every configuration, else NotImplementedError.
 
     `group=True` (the default process group) or a ProcessGroup shards the configurations over its ranks, one GPU
     each (`optable_b200.dist.trace_sweep_sharded`): rank r flattens and traces only the contiguous configurations
@@ -242,13 +310,14 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
 
     Like `trace_bundle`, a sweep is a tensor entry point: it does not fill `table.rays`, `Monitor._data_raw` or the
     components' `_interact_count`. `tracer(flats, rays, max_trace_num, record_hits=, record_hist=, engine=, unit=,
-    arrs=)` (plus `chain_len=` when sharded) defaults to the CUDA sweep; the CPU tests pass a stand-in."""
+    arrs=)` (plus `chain_len=` when sharded, and `caps0=`, `serial=` for Ray objects on a capped scene) defaults to
+    the CUDA sweep; the CPU tests pass a stand-in."""
     from .flatten import FlatScene, batch_wavelengths_m, trace_cap
 
     tables = list(tables)
     if not tables:
         raise ValueError("trace_sweep: no tables")
-    n, wl, unit, arrs = _rays(rays)
+    n, wl, unit, arrs, fam_ids = _rays(rays)
     wl_unit = unit if unit is not None else getattr(tables[0], "unit", 1e-2)
     wls = None if wl is None else batch_wavelengths_m(wl, wl_unit)
     flatten = lambda ts: [FlatScene(t.components, t.monitors, wavelengths_m=wls) for t in ts]
@@ -256,16 +325,25 @@ def trace_sweep(tables, rays, perfomance_limit=None, record_hits=True, record_hi
     if _sharded(group):
         from .dist import trace_sweep_sharded
 
-        out, _ = trace_sweep_sharded(len(tables), n, rays, trace_cap(perfomance_limit),
-                                     lambda k0, k1: (flatten(tables[k0:k1]), None), [list(t.monitors) for t in tables],
-                                     "trace_sweep: table", tracer, group=None if group is True else group, gather=gather,
-                                     record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit, arrs=arrs)
-        return SweepResult(tables, n, out, engine)
+        def prepare(k0, k1):
+            flats = flatten(tables[k0:k1])
+            return flats, None, initial_counts([f.capslots for f in flats], fam_ids)
+
+        out, _ = trace_sweep_sharded(len(tables), n, rays, trace_cap(perfomance_limit), prepare,
+                                     [list(t.monitors) for t in tables], "trace_sweep: table", tracer,
+                                     group=None if group is True else group, gather=gather, record_hits=record_hits,
+                                     record_hist=record_hist, engine=engine, unit=unit, arrs=arrs, fam_ids=fam_ids)
+        comps = None if fam_ids is None else (lambda: [list(f.capslots) for f in flatten(tables)])
+        return SweepResult(tables, n, out, engine, family_ids=fam_ids, cap_components=comps)
     flats = flatten(tables)
     check_topology(flats)
-    out = tracer(flats, rays, trace_cap(perfomance_limit), record_hits=record_hits, record_hist=record_hist,
-                 engine=engine, unit=unit, arrs=arrs)
-    return SweepResult(tables, n, out, engine)
+    limit = trace_cap(perfomance_limit)
+    caps0 = initial_counts([f.capslots for f in flats], fam_ids)
+    kw = {} if caps0 is None else {"caps0": caps0, "serial": caps_bind(caps0, arrs, min(f.cap_min for f in flats), limit)}
+    out = tracer(flats, rays, limit, record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
+                 arrs=arrs, **kw)
+    return SweepResult(tables, n, out, engine, family_ids=fam_ids,
+                       cap_components=None if fam_ids is None else [list(f.capslots) for f in flats])
 
 
 def _children(ni, nf):
@@ -385,7 +463,8 @@ class SweepScene:
         whatever ran before it); it runs for k = 0 .. n_configs - 1 in order, and after the call the table stands in
         configuration n_configs - 1. Limits, interact caps and record flags follow `trace_sweep`. `tracer(rows, rays,
         max_trace_num, ...)` defaults to the CUDA sweep, where `rows` is the SweepRows of the configurations; the CPU
-        tests pass a stand-in.
+        tests pass a stand-in. The starting interact counts of a list of Ray are the table's, read after each
+        `configure(k)`.
 
         `group=` / `gather=` shard the configurations as in `trace_sweep`: rank r calls `configure(k)` only for its own
         configurations `shard_bounds(K, r, world)`, in order (and `configure(n_configs - 1)` once more at the end when
@@ -396,16 +475,17 @@ class SweepScene:
         K = int(n_configs)
         if K < 1:
             raise ValueError("SweepScene.trace: n_configs must be >= 1")
-        n, wl, unit, arrs = _rays(rays)
+        n, wl, unit, arrs, fam_ids = _rays(rays)
         wl_unit = unit if unit is not None else getattr(self.table, "unit", 1e-2)
         wls = None if wl is None else batch_wavelengths_m(wl, wl_unit)
         tracer = tracer or _device_sweep
+        comps = None if fam_ids is None else (lambda: [list(self._base(wls)[0].capslots)] * K)
         if _sharded(group):
             from .dist import trace_sweep_sharded
 
             def prepare(k0, k1):
-                rows, frames = self._configurations(wls, configure, k0, k1)
-                return rows, [{m: f for m, f in enumerate(fr) if isinstance(f, _MonitorPose)} for fr in frames]
+                rows, frames, caps0 = self._configurations(wls, configure, k0, k1, fam_ids)
+                return rows, [{m: f for m, f in enumerate(fr) if isinstance(f, _MonitorPose)} for fr in frames], caps0
 
             live = list(self.table.monitors)
             out, frames = trace_sweep_sharded(K, n, rays, trace_cap(perfomance_limit), prepare,
@@ -413,14 +493,16 @@ class SweepScene:
                                               "SweepScene.trace: configuration", tracer,
                                               group=None if group is True else group, gather=gather,
                                               record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
-                                              arrs=arrs)
+                                              arrs=arrs, fam_ids=fam_ids)
             if not out["shard"][0] <= K - 1 < out["shard"][1]:
                 configure(K - 1)     # the documented end state: the table stands in the last configuration
-            return SweepResult([self.table] * K, n, out, engine, monitors=frames)
-        rows, frames = self._configurations(wls, configure, 0, K)
-        out = tracer(rows, rays, trace_cap(perfomance_limit), record_hits=record_hits, record_hist=record_hist,
-                     engine=engine, unit=unit, arrs=arrs)
-        return SweepResult([self.table] * K, n, out, engine, monitors=frames)
+            return SweepResult([self.table] * K, n, out, engine, monitors=frames, family_ids=fam_ids, cap_components=comps)
+        rows, frames, caps0 = self._configurations(wls, configure, 0, K, fam_ids)
+        limit = trace_cap(perfomance_limit)
+        kw = {} if caps0 is None else {"caps0": caps0, "serial": caps_bind(caps0, arrs, rows.cap_min, limit)}
+        out = tracer(rows, rays, limit, record_hits=record_hits, record_hist=record_hist, engine=engine, unit=unit,
+                     arrs=arrs, **kw)
+        return SweepResult([self.table] * K, n, out, engine, monitors=frames, family_ids=fam_ids, cap_components=comps)
 
     def abcd_matrix(self, m0, m1, rays, configure, n_configs, disp=1e-5, rot=1e-5, perfomance_limit=None, engine=None,
                     group=None):
@@ -444,14 +526,15 @@ class SweepScene:
         if self._base(wls)[0].n_capslots:
             raise NotImplementedError(f"{what}: interact-capped components are not supported (the table method's three "
                                       "traces carry their interact counts over from one to the next)")
-        rows, frames = self._configurations(wls, configure, 0, K)
+        rows, frames, _ = self._configurations(wls, configure, 0, K)
         _check_mon0(frames, m0, what)
         return _abcd(rows, K, [self.table] * K, frames, m0, m1, work, ids, disp, rot, trace_cap(perfomance_limit),
                      engine, what)
 
-    def _configurations(self, wls, configure, k0, k1):
-        """configure(k) for k = k0 .. k1 - 1 in order: the SweepRows of those configurations and their monitor frames
-        (a _MonitorPose snapshot for a varied monitor, the live monitor otherwise)."""
+    def _configurations(self, wls, configure, k0, k1, fam_ids=None):
+        """configure(k) for k = k0 .. k1 - 1 in order: the SweepRows of those configurations, their monitor frames
+        (a _MonitorPose snapshot for a varied monitor, the live monitor otherwise) and the `initial_counts` of the
+        families `fam_ids`, read after each configure(k) (None without fam_ids or caps)."""
         from .flatten import monitor_record
 
         flat, comps, V, mons, ni0 = self._base(wls)
@@ -464,9 +547,10 @@ class SweepScene:
         for j, obj in comps:
             first = flat._node_of[id(obj)]
             owner.update({i: j for i in range(first, int(flat.node_i[first, A.NI_SKIP]))})
-        frames, varied_mons = [], set(mons.tolist())
+        frames, varied_mons, counts = [], set(mons.tolist()), []
         for c, k in enumerate(range(k0, k1)):
             configure(k)
+            counts.append(initial_counts([flat.capslots], fam_ids))
             for j, obj in comps:
                 if flat.refresh(obj) is None:
                     raise ValueError(f"SweepScene: configuration {k} changes {self._what(j)} in a way the scene cannot "
@@ -483,7 +567,8 @@ class SweepScene:
                 monitor_record(flat.monitors[m], mon_f[c, w])
             live = list(flat.monitors)
             frames.append([_MonitorPose(live[m]) if m in varied_mons else live[m] for m in range(len(live))])
-        return SweepRows(flat, K, V, node_i, node_f, mons, mon_f), frames
+        caps0 = np.concatenate(counts, axis=1) if counts and counts[0] is not None else None
+        return SweepRows(flat, K, V, node_i, node_f, mons, mon_f), frames, caps0
 
 
 class SweepABCD:
